@@ -11,8 +11,8 @@ working set (state + outputs) exceeds the 126 MB L2 ("inputs larger than L2").
 
 Prints ONE JSON line (rank 0):
   value       device-timed throughput, inputs resident in HBM: CUDA-graph replay of exactly K launches on one stream,
-              CUDA events on that stream; the K-step region is repeated until >= 50 ms were timed, median reported,
-              MAX over ranks.
+              CUDA events on that stream around those K steps (after W eager warm-up steps and untimed replays of the
+              graph right ahead of them, lead_in_regions(K)), MAX over ranks.
   e2e         the same metric through the host-buffer C-ABI call (ngw_step_host_begin/_end): pinned H2D of the actions,
               one launch, D2H of obs/reward/done/step_cost/result every step, >= 200 steps; observation rows in the
               compact NGW_OBS_U8 layout (uint8 lidar ranges + int32 inventory tail; `int32_rows` = the default layout);
@@ -23,6 +23,7 @@ Prints ONE JSON line (rank 0):
   cpu_baseline  the C port of the reference path (oracle/ngw_oracle.c) on all host threads, and — when the unmodified
               Python reference is installed under baseline/_ref — its single-process and process-pool throughput.
 `--impl reference` times the C port alone (rank 0 only), same config keys.
+`--dump-outputs DIR` writes what the last timed step of `value` returned (rank 0) as DIR/<name>.npy, see dump_outputs().
 """
 import argparse
 import json
@@ -50,6 +51,17 @@ E2E_MIN_STEPS = 400
 E2E_CHUNK = 50                # e2e loops are timed in chunks of this many steps, median chunk reported
 REFERENCE_FLOOR_S = 2.0
 C4_TOTAL_ENVS = 1048576
+DUMP_LIMIT_BYTES = 64 << 20       # --dump-outputs: above this a fixed, seeded sample of env rows is written
+QUEUE_SLEEP_CYCLES = 4000000      # ~2 ms of device spin ahead of a timed region, see time_regions
+LEAD_IN_STEPS = 2048              # untimed steps replayed right ahead of the exactly-K-step `value` region
+
+
+def lead_in_regions(K):
+    """Untimed replays of the K-step region ahead of the timed one (a function of K alone, so that the batches always
+    advance by the same number of steps): the timed steps run in the steady state that the 2nd .. nth region of a
+    longer run sees (on a B200 at its 1000 W limit, 1965 MHz, a 20-step C2 region measured 1-3 % slower right behind a
+    single untimed replay than in a long back-to-back run)."""
+    return max(1, -(-LEAD_IN_STEPS // K))
 
 
 def build_c2_chain(num_envs=1, device=None):
@@ -396,9 +408,11 @@ class Workload(object):
             r = torch.randint(0, 1 << 30, (self.envs,), generator=gen, device=dev, dtype=torch.int64)
             self.act_sets.append((r % per_env_n).to(torch.int32))
         self.reset_error_flags = sum(int((h.error_flags != 0).sum().item()) for h in self.batches)
+        self.last = None                                # batch of the latest step() call (in a capture: the last replayed)
 
     def step(self, i):
-        self.batches[i % self.n_batches].step(self.act_sets[i % self.n_sets], **self.kw)
+        self.last = i % self.n_batches
+        self.batches[self.last].step(self.act_sets[i % self.n_sets], **self.kw)
 
     def launches(self):
         return sum(h.launch_count() for h in self.batches)
@@ -412,10 +426,12 @@ class Workload(object):
         self.batches = []
 
 
-def time_regions(wl, K, dev, world, floor_ms=VALUE_FLOOR_MS, n_streams=1, max_regions=4000):
+def time_regions(wl, K, dev, world, floor_ms=VALUE_FLOOR_MS, n_streams=1, max_regions=4000, n_regions=None):
     """Exactly K steps per region as CUDA-graph replays on one launching stream, CUDA events on that stream around every
-    region; barrier + synchronize on both sides of the whole measurement.  Returns (region durations in ms, wall
-    bracket, launches per step, steps per graph)."""
+    region; barrier + synchronize on both sides of the whole measurement.  The region is repeated until floor_ms were
+    timed, or exactly n_regions times when that is given (then the batches advance by a number of steps that does not
+    depend on the speed of the build).  Returns (region durations in ms, wall bracket, launches per step, steps per
+    graph)."""
     import torch
     import torch.distributed as dist
     n_b = wl.n_batches
@@ -457,26 +473,36 @@ def time_regions(wl, K, dev, world, floor_ms=VALUE_FLOOR_MS, n_streams=1, max_re
         if graph_rem:
             graph_rem.replay()
 
-    with torch.cuda.stream(stream):
-        region()                                                         # graph warm-up (uploads the exec graphs)
-    torch.cuda.synchronize(dev)
-    # how many regions make the floor: probe one
-    p0, p1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-    with torch.cuda.stream(stream):
-        p0.record(stream)
-        region()
-        p1.record(stream)
-    torch.cuda.synchronize(dev)
-    n_regions = int(min(max_regions, max(3, np.ceil(floor_ms / max(p0.elapsed_time(p1), 1e-3)))))
+    fixed = n_regions is not None
+    if not fixed:
+        with torch.cuda.stream(stream):
+            region()                                                     # graph warm-up (uploads the exec graphs)
+        torch.cuda.synchronize(dev)
+        # how many regions make the floor: probe one
+        p0, p1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+        with torch.cuda.stream(stream):
+            p0.record(stream)
+            region()
+            p1.record(stream)
+        torch.cuda.synchronize(dev)
+        n_regions = int(min(max_regions, max(3, np.ceil(floor_ms / max(p0.elapsed_time(p1), 1e-3)))))
+        if world > 1:
+            t = torch.tensor([n_regions], device=dev)
+            dist.all_reduce(t, op=dist.ReduceOp.MAX)
+            n_regions = int(t.item())
     if world > 1:
-        t = torch.tensor([n_regions], device=dev)
-        dist.all_reduce(t, op=dist.ReduceOp.MAX)
-        n_regions = int(t.item())
         dist.barrier()
     torch.cuda.synchronize(dev)
     evs = [torch.cuda.Event(enable_timing=True) for _ in range(n_regions + 1)]
     t0 = time.perf_counter()
     with torch.cuda.stream(stream):
+        if fixed:
+            # the graph warm-up (uploads the exec graphs; lead_in_regions(K) replays) runs right ahead of the timed
+            # regions, and both wait behind a device spin while the host enqueues them: the first event does not time
+            # the host's graph launch
+            torch.cuda._sleep(QUEUE_SLEEP_CYCLES)
+            for _ in range(lead_in_regions(K)):
+                region()
         evs[0].record(stream)
         for r in range(n_regions):
             region()
@@ -486,6 +512,30 @@ def time_regions(wl, K, dev, world, floor_ms=VALUE_FLOOR_MS, n_streams=1, max_re
         dist.barrier()
     t1 = time.perf_counter()
     return [evs[r].elapsed_time(evs[r + 1]) for r in range(n_regions)], (t0, t1), launches_per_step, g_steps
+
+
+def dump_outputs(wl, out_dir):
+    """What the last timed step returned to its caller, for comparing two builds output by output: the observation rows,
+    reward, done, step_cost and result of the batch that step advanced, as float32 DIR/<name>.npy.  When they would
+    exceed DUMP_LIMIT_BYTES, the same fixed, seeded sample of env rows is kept of each (its indices: env_index.npy)."""
+    import torch
+    h = wl.batches[wl.last]
+    torch.cuda.synchronize(h.device)
+    outs = {'obs': h.obs[:, :h.obs_dim], 'reward': h.reward, 'done': h.done, 'step_cost': h.step_cost,
+            'result': h.result}
+    if not h.obs_dim:
+        del outs['obs']
+    row_bytes = 4 * sum(t[0].numel() for t in outs.values())
+    index = None
+    if h.n * row_bytes > DUMP_LIMIT_BYTES:
+        index = np.sort(np.random.RandomState(0).choice(h.n, DUMP_LIMIT_BYTES // row_bytes, replace=False))
+        rows = torch.from_numpy(index).to(h.device)
+        outs = {name: t[rows] for name, t in outs.items()}
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in outs.items():
+        np.save(os.path.join(out_dir, name + '.npy'), t.cpu().numpy().astype(np.float32))
+    if index is not None:
+        np.save(os.path.join(out_dir, 'env_index.npy'), index.astype(np.float64))
 
 
 def pcie_probe(dev, d2h_bytes, h2d_bytes, world, reps=60):
@@ -611,7 +661,9 @@ def run_ours(args, rank, world, local_rank):
     for i in range(W):                                                  # warm-up: eager launches
         wl.step(i)
     torch.cuda.synchronize(dev)
-    regions, (t_wall0, t_wall1), launches_per_step, g_steps = time_regions(wl, K, dev, world)
+    regions, (t_wall0, t_wall1), launches_per_step, g_steps = time_regions(wl, K, dev, world, n_regions=1)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(wl, args.dump_outputs)                             # before anything else steps these batches
     ms_region = float(np.median(regions))
     overlapped_per_graph = wl.overlapped_launches_per_graph
     ov_regions = time_regions(wl, K, dev, world, n_streams=min(3, n_batches))[0]
@@ -899,7 +951,11 @@ def main():
     ap.add_argument('--no-cpu-baseline', action='store_true')
     ap.add_argument('--no-workloads', action='store_true', help='skip the C3/C4/C5 measurements of the default line')
     ap.add_argument('--workload', default='C2', choices=['C2', 'C3', 'C4', 'C4-blocked', 'C5'])
+    ap.add_argument('--dump-outputs', metavar='DIR',
+                    help='write the outputs of the last timed step as DIR/<name>.npy (float32, at most 64 MB)')
     args = ap.parse_args()
+    if args.dump_outputs and args.impl == 'reference':
+        ap.error('--dump-outputs writes the outputs of the GPU path (--impl ours)')
     rank = int(os.environ.get('RANK', '0'))
     world = int(os.environ.get('WORLD_SIZE', '1'))
     local_rank = int(os.environ.get('LOCAL_RANK', '0'))

@@ -1,8 +1,8 @@
 #!/usr/bin/env python
-"""Golden-trace generator: runs the UNMODIFIED reference (/root/reference, via oracle/gymstub) and
+"""Golden-trace generator: runs the UNMODIFIED reference (via oracle/gymstub) and
 records reset states, actions and every step's outputs into tests/golden/traces.npz.
 
-Run where the reference is importable (/root/reference in the build container, or the baseline/_ref install):
+Run where the reference is installed under baseline/_ref (see __graft_entry__.install_reference):
 
     python oracle/gen_golden.py            # ~1-2 min, rewrites tests/golden/traces.npz
 

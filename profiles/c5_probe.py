@@ -1,6 +1,6 @@
 import os, sys, time
 import numpy as np, torch
-sys.path.insert(0, '/root/repo')
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import bench
 from gym_novel_gridworlds_b200.runtime import BatchHandle
 desc, compiled, envs, rule, kw = bench.build_workload('C5')

@@ -1,5 +1,5 @@
-import time, cProfile, pstats, sys
-sys.path.insert(0, '/root/repo')
+import os, time, cProfile, pstats, sys
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import torch
 from examples.random_action import build
 env = build(65536); env.reset()

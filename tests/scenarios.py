@@ -41,14 +41,11 @@ def build_chain(ns, desc, **make_kwargs):
 
 
 def reference_root():
-    """Where the unmodified reference package lives: /root/reference in the build container, else the copy that
-    __graft_entry__.build() installs under git-ignored baseline/_ref (it travels to the GPU box with the snapshot)."""
+    """Where the unmodified reference package lives: the copy that __graft_entry__.build() installs under git-ignored
+    baseline/_ref when the upstream sources are at hand; None when it is not installed."""
     import os
-    here = os.path.dirname(os.path.abspath(__file__))
-    for root in ('/root/reference', os.path.join(here, '..', 'baseline', '_ref')):
-        if os.path.isdir(os.path.join(root, 'gym_novel_gridworlds')):
-            return os.path.abspath(root)
-    return None
+    root = os.path.join(os.path.dirname(os.path.abspath(__file__)), '..', 'baseline', '_ref')
+    return os.path.abspath(root) if os.path.isdir(os.path.join(root, 'gym_novel_gridworlds')) else None
 
 
 def reference_namespace(ref_root=None):
@@ -59,7 +56,7 @@ def reference_namespace(ref_root=None):
     stub = os.path.abspath(os.path.join(here, '..', 'oracle', 'gymstub'))
     root = ref_root or reference_root()
     if root is None:
-        raise RuntimeError("the reference package is neither at /root/reference nor under baseline/_ref")
+        raise RuntimeError("the reference package is not installed under baseline/_ref")
     for p in (stub, root):
         if p not in sys.path:
             sys.path.insert(0, p)

@@ -1,9 +1,12 @@
 """bench.py without a GPU: the algorithmic-bytes formula reproduces SURVEY §8d, the workloads compile, and the
-`--impl reference` arm prints the contract's JSON line."""
+`--impl reference` arm prints the contract's JSON line.  With one: `--dump-outputs` writes the last timed step."""
 import json
 import os
 import subprocess
 import sys
+
+import numpy as np
+import pytest
 
 import bench
 
@@ -33,3 +36,35 @@ def test_reference_arm_prints_the_contract_line():
     assert line['cpu_baseline']['kind'] == 'port' and line['cpu_baseline']['cores'] >= 1
     assert line['e2e']['h2d_bytes_per_step'] == 0 and line['e2e']['d2h_bytes_per_step'] == 0
     assert line['metric'] == json.load(open(os.path.join(ROOT, 'BASELINE.json')))['metric']
+
+
+@pytest.mark.gpu
+def test_dump_outputs_hold_the_last_of_exactly_k_timed_steps(tmp_path):
+    """`--steps K --warmup W --dump-outputs DIR`: the headline batches take W eager steps, lead_in_regions(K) untimed and
+    one timed replay of the K-step graph, and DIR holds what the last of those steps returned — the same arrays an
+    in-process replay of that step sequence produces."""
+    import torch
+    K, W = 5, 3
+    out = subprocess.run([sys.executable, os.path.join(ROOT, 'bench.py'), '--steps', str(K), '--warmup', str(W),
+                          '--no-workloads', '--no-cpu-baseline', '--dump-outputs', str(tmp_path)],
+                         capture_output=True, text=True, timeout=900, cwd=ROOT)
+    assert out.returncode == 0, out.stderr
+    line = json.loads(out.stdout.strip().splitlines()[-1])
+    assert line['steps'] == K and line['timing']['regions'] == 1
+    got = {name: np.load(str(tmp_path / (name + '.npy'))) for name in ('obs', 'reward', 'done', 'step_cost', 'result')}
+    assert sorted(os.listdir(str(tmp_path))) == sorted(name + '.npy' for name in got)
+    assert got['obs'].shape == (bench.ENVS_PER_BATCH, 63)
+    assert all(a.dtype == np.float32 for a in got.values()) and sum(a.nbytes for a in got.values()) <= bench.DUMP_LIMIT_BYTES
+
+    wl = bench.Workload('C2', 0, 1, torch.device('cuda', 0))
+    for i in range(W):
+        wl.step(i)
+    for _ in range(bench.lead_in_regions(K) + 1):
+        for i in range(K):
+            wl.step(i)
+    h = wl.batches[(K - 1) % wl.n_batches]
+    want = {'obs': h.obs[:, :h.obs_dim], 'reward': h.reward, 'done': h.done, 'step_cost': h.step_cost,
+            'result': h.result}
+    for name, t in want.items():
+        assert np.array_equal(got[name], t.cpu().numpy().astype(np.float32)), name
+    wl.close()
