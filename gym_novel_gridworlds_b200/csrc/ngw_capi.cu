@@ -220,11 +220,9 @@ static int build_lidar_tables(const ngw_config& c, int map_size, LidarDev& ld, s
         if (lines)
             for (int k = K - 1; k >= 0; k--) ld.firstk[ld.disp[1][k] - 1] = (uint8_t)(k + 1);   // first sample reaching cell d
     }
-    if (getenv("NGW_NO_LINE_LIDAR")) lines = false;
-    if (getenv("NGW_NO_FAST_LIDAR")) { fast = false; lines = false; }
     if (!lines) { memset(ld.firstk, 0, sizeof(ld.firstk)); memset(ld.rot, 0, sizeof(ld.rot)); }
     ld.fast = fast ? 1 : 0;
-    ld.lines = lines ? (getenv("NGW_LINE_LIDAR_BIG") ? 2 : 1) : 0;   // 2: A/B knob, line gather also on grids above 32x32
+    ld.lines = lines ? 1 : 0;
     if (!fast && lin) {
         int n = 4 * B * K;
         lin->resize(n);
@@ -255,25 +253,7 @@ static int create_init(ngw_handle* h, const ngw_config* cfgs, int32_t n_cfgs, in
                        int32_t device, int64_t first_env_gid, uint64_t seed, const cudaDeviceProp& prop) {
     h->device = device; h->n = n_envs; h->np = (n_envs + 31) / 32 * 32; h->first_gid = first_env_gid; h->seed = seed;
     h->ms = map_size; h->cells = map_size * map_size; h->n_cfgs = n_cfgs;
-    h->use_tma = getenv("NGW_NO_TMA") == nullptr;
-    h->collect_stats = getenv("NGW_NO_STATS") == nullptr;
-    h->force_global_cfg = getenv("NGW_GLOBAL_CFG") != nullptr;
-    h->plain_store = getenv("NGW_PLAIN_STORE") != nullptr;
-    h->use_pdl = getenv("NGW_NO_PDL") == nullptr;
-    h->pdl_in_graph = getenv("NGW_NO_PDL_GRAPH") == nullptr;
-    h->early_state = getenv("NGW_NO_EARLY_STATE") == nullptr;
-    h->wshape = getenv("NGW_WSHAPE") ? atoi(getenv("NGW_WSHAPE")) : 1;
     h->concurrent = getenv("NGW_NO_CONCURRENT") == nullptr;
-    h->concurrent_waves = getenv("NGW_NO_CONCURRENT_WAVES") == nullptr;
-    h->rollout2 = getenv("NGW_NO_ROLLOUT2") == nullptr;
-    h->alias = getenv("NGW_NO_ALIAS") == nullptr;
-    h->row_pad = getenv("NGW_NO_ROW_PAD") == nullptr;
-    if (const char* rg = getenv("NGW_RESET_GRID")) { int v = atoi(rg); if (v >= 1 && v <= 4) h->reset_grid = v; }
-    h->pdl_early = getenv("NGW_NO_PDL_EARLY") == nullptr;   // trigger right after the wait: C2 7.70 -> 7.60 us/step
-    // streaming data (each tile is read once and its observations written once per step) should not linger in L2:
-    // measured on C2 9.15 -> 8.82 us/step, C3 29.3 -> 28.0, C5 278 -> 274 (hinting the inventory store as well: 9.0)
-    h->cache_hints = getenv("NGW_HINTS") ? atoi(getenv("NGW_HINTS")) : 3;
-    h->dbg_skip = getenv("NGW_SKIP") ? atoi(getenv("NGW_SKIP")) : 0;   // attribution runs only: results are wrong
     if (const char* km = getenv("NGW_DEBUG_KEY_MASK")) h->key_mask = (uint32_t)strtoul(km, nullptr, 0);   // test knob: key ties
     for (int i = 0; i < n_cfgs; i++) {
         const ngw_config& c = cfgs[i];
@@ -352,16 +332,7 @@ static int create_init(ngw_handle* h, const ngw_config* cfgs, int32_t n_cfgs, in
     int tiles_per_sm = (227 * 1024) / (one_tile + 1024);
     int warps = tiles_per_sm >= 6 ? 2 : 4;
     if (n_cfgs > 1 && warps == 2) warps = 1;      // mixed batches: a second warp repeats the per-lane config reads (C4 129 vs 139 us)
-    if (const char* w = getenv("NGW_WARPS")) {                      // tuning knob: warps per tile
-        int v = atoi(w);
-        if (v == 1 || v == 2 || v == 4) warps = v;
-    }
     h->warps = warps;
-    h->tiles_per_cta = 0;                                           // 0 = chosen per launch (see launch_step1_nc)
-    if (const char* t = getenv("NGW_CTILES")) {                     // tuning knob: tile groups per CTA, 1..15
-        int v = atoi(t);
-        if (v >= 1 && v <= 15) h->tiles_per_cta = v;
-    }
     // line-gather lidar with one geometry for the whole batch (the common case): the kernel skips the per-lane dispatch
     h->lidar_mode = 1;
     for (int i = 0; i < n_cfgs; i++) {
@@ -371,15 +342,14 @@ static int create_init(ngw_handle* h, const ngw_config* cfgs, int32_t n_cfgs, in
     if (n_cfgs > 1 && !h->lidar_uniform) h->lidar_mode = 0;
     if (map_size > 32) h->lidar_mode = 0;           // large grids: pointer-walking beams (lidar_observe decides per lane)
 #define NGW_SMEM_ATTR(K) CK(cudaFuncSetAttribute(K, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024))
-#define NGW_SMEM_ATTR4(K, T, O) NGW_SMEM_ATTR((K<T, 0, O>)); NGW_SMEM_ATTR((K<T, 1, O>)); NGW_SMEM_ATTR((K<T, 4, O>)); NGW_SMEM_ATTR((K<T, 16, O>))
-    NGW_SMEM_ATTR4(step1_kernel, true, true); NGW_SMEM_ATTR4(step1_kernel, true, false);
-    NGW_SMEM_ATTR4(step1_kernel, false, true);
+#define NGW_SMEM_ATTR4(K, O) NGW_SMEM_ATTR((K<0, O>)); NGW_SMEM_ATTR((K<1, O>)); NGW_SMEM_ATTR((K<4, O>)); NGW_SMEM_ATTR((K<16, O>))
+    NGW_SMEM_ATTR4(step1_kernel, true); NGW_SMEM_ATTR4(step1_kernel, false);
 #undef NGW_SMEM_ATTR4
     // the queued-reset kernel shares SMs with the next handle's step CTAs: both must want the same (maximal) shared-memory
     // carve-out, or the SM would have to drain before it can be reconfigured
     CK(cudaFuncSetAttribute(reset_list_kernel, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
-    NGW_SMEM_ATTR((step1_kernel<true, 0, true, true>)); NGW_SMEM_ATTR((step1_kernel<true, 1, true, true>));
-    NGW_SMEM_ATTR((step1_kernel<true, 4, true, true>)); NGW_SMEM_ATTR((step1_kernel<true, 16, true, true>));
+    NGW_SMEM_ATTR((step1_kernel<0, true, true>)); NGW_SMEM_ATTR((step1_kernel<1, true, true>));
+    NGW_SMEM_ATTR((step1_kernel<4, true, true>)); NGW_SMEM_ATTR((step1_kernel<16, true, true>));
     NGW_SMEM_ATTR((step1w_kernel<0, 8>)); NGW_SMEM_ATTR((step1w_kernel<1, 8>)); NGW_SMEM_ATTR((step1w_kernel<4, 8>)); NGW_SMEM_ATTR((step1w_kernel<16, 8>));
     NGW_SMEM_ATTR((step1w_kernel<0, 16>)); NGW_SMEM_ATTR((step1w_kernel<1, 16>)); NGW_SMEM_ATTR((step1w_kernel<4, 16>)); NGW_SMEM_ATTR((step1w_kernel<16, 16>));
     if (ngw_rollout_init()) return 1;
@@ -504,16 +474,13 @@ static StepParams step_params(ngw_handle* h, const int32_t* actions, void* obs, 
     p.dcfgs = h->d_cfgs; p.map = h->map; p.pose = h->pose; p.inv = h->inv; p.cfg_id = h->cfg_id; p.episode = h->episode;
     p.ep_len = h->ep_len; p.err = h->err; p.actions = actions;
     p.obs = h->obs_dim > 0 ? static_cast<unsigned char*>(obs) : nullptr; p.reward = reward;
-    p.done = done; p.cost = cost; p.result = result; p.stats = h->collect_stats ? h->stats : nullptr;
+    p.done = done; p.cost = cost; p.result = result; p.stats = h->stats;
     p.env_begin = begin; p.env_end = end; p.first_gid = h->first_gid; p.seed = h->seed;
     p.ms = h->ms; p.cells = h->cells; p.inv_stride = h->inv_stride; p.obs_dim = h->obs_dim;
     p.map_bytes = h->map_bytes; p.inv_bytes = h->inv_bytes; p.obs_bytes = h->obs_bytes;
     p.obs_row_bytes = h->obs_row_bytes; p.obs_u8 = h->obs_u8;
     p.auto_reset = auto_reset; p.max_episode_steps = max_episode_steps;
-    p.plain_store = h->plain_store ? 1 : 0;
     p.lidar_uniform = h->lidar_uniform ? 1 : 0;
-    p.cache_hints = h->cache_hints;
-    p.dbg_skip = h->dbg_skip;
     p.msg = h->msg; p.reset_list = h->reset_list; p.reset_count = h->reset_ctl;
     p.n_steps = 1;
     return p;
@@ -525,18 +492,12 @@ static bool is_multi(const StepParams& p) {
     return p.n_steps > 1 || p.random_policy || p.done_count != nullptr || p.actions_out != nullptr || p.policy_w != nullptr;
 }
 
-void pdl_attr(ngw_handle* h, cudaStream_t s, cudaLaunchConfig_t& lc, cudaLaunchAttribute* attr) {
+void pdl_attr(cudaLaunchConfig_t& lc, cudaLaunchAttribute* attr) {
     attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
     attr[0].val.programmaticStreamSerializationAllowed = 1;
     // PDL (trigger once a CTA's stores are issued, see the kernels): the next launch's prologue overlaps this launch's
     // store phase; C2 CUDA-graph replay 9.3 -> 8.6 us/step.  (An early trigger at kernel entry measured slower.)
-    bool pdl = h->use_pdl;
-    if (pdl && !h->pdl_in_graph) {                  // A/B knob only: the capture query costs a driver call per launch
-        cudaStreamCaptureStatus cap = cudaStreamCaptureStatusNone;
-        cudaStreamIsCapturing(s, &cap);
-        pdl = cap == cudaStreamCaptureStatusNone;
-    }
-    lc.attrs = attr; lc.numAttrs = pdl ? 1 : 0;
+    lc.attrs = attr; lc.numAttrs = 1;
 }
 
 // caller buffers of a one-step launch (for the independence proof of this launch and of the next one)
@@ -563,10 +524,10 @@ static cudaError_t launch_step1_nc(ngw_handle* h, StepParams p, cudaStream_t s) 
     p.off_luts = NGW_CTA_HDR;
     p.off_groups = p.off_luts + luts;
     // shared-memory row stride of the observation tile: rows of a multiple of 8 words get 16 bytes of padding
-    p.obs_srow = p.obs_row_bytes + (((p.obs_row_bytes >> 2) % 8 == 0 && p.obs_row_bytes > 0 && h->row_pad) ? 16 : 0);
+    p.obs_srow = p.obs_row_bytes + (((p.obs_row_bytes >> 2) % 8 == 0 && p.obs_row_bytes > 0) ? 16 : 0);
     p.group_bytes = (NGW_GROUP_HDR + p.map_bytes + p.inv_bytes + 32 * p.obs_srow + 127) & ~127;
     // alias plan (one tile per CTA, see step1_kernel<.., kAlias>): the observation tile shares the rows' shared memory
-    bool alias = h->alias && h->use_tma && h->tiles_per_cta <= 1;
+    bool alias = true;
     for (const DevConfig& dc : h->h_cfgs)
         if (dc.c.n_inv_obs > NGW_REGSINK_TAIL || (dc.c.n_beams > 0 && !dc.lidar.lines && !dc.lidar.fast)) alias = false;
     const int alias_bytes = (NGW_GROUP_HDR + ((p.map_bytes + p.inv_bytes) > 32 * p.obs_srow ? (p.map_bytes + p.inv_bytes) : 32 * p.obs_srow) + 127) & ~127;
@@ -578,18 +539,13 @@ static cudaError_t launch_step1_nc(ngw_handle* h, StepParams p, cudaStream_t s) 
     // packed into two CTAs per SM.  A launch of several waves runs one tile per CTA: small CTAs retire independently,
     // which staggers the load / compute / store phases of neighbouring tiles (C3 28.5 vs 31.7 us).
     const long long per_sm = (227 * 1024 - p.off_groups) / p.group_bytes;
-    int C = h->tiles_per_cta;
-    if (C <= 0) {
-        if (tiles <= per_sm * h->sm_count && per_sm >= 4) {
-            C = (int)((tiles + 2 * h->sm_count - 1) / (2 * h->sm_count));
-            const int c_cap = (int)((113 * 1024 - p.off_groups) / p.group_bytes);
-            if (C > c_cap) C = c_cap;
-            if (C > 512 / (32 * G)) C = 512 / (32 * G);
-        } else {
-            C = 1;
-        }
+    int C = 1;
+    if (tiles <= per_sm * h->sm_count && per_sm >= 4) {
+        C = (int)((tiles + 2 * h->sm_count - 1) / (2 * h->sm_count));
+        const int c_cap = (int)((113 * 1024 - p.off_groups) / p.group_bytes);
+        if (C > c_cap) C = c_cap;
+        if (C > 512 / (32 * G)) C = 512 / (32 * G);
     }
-    if (!h->use_tma) C = 1;                         // the plain-copy A/B kernel exists as one tile per CTA only
     if (C > 15) C = 15;
     if (C > 512 / (32 * G)) C = 512 / (32 * G);
     while (C > 1 && (size_t)p.off_groups + (size_t)C * p.group_bytes > 227 * 1024) C--;
@@ -605,11 +561,10 @@ static cudaError_t launch_step1_nc(ngw_handle* h, StepParams p, cudaStream_t s) 
     // only for one-wave launches: with several waves the loads of later waves never wait anyway, and issuing them ahead
     // of the tile's zero-fill measured 4 % slower (C4 122 vs 127 us)
     const StreamTail me = launch_tail(p);
-    const int mode = claim_stream(h, s, h->early_state && h->use_pdl, &me);
+    const int mode = claim_stream(h, s, true, &me);
     // independent of the predecessor (see claim_stream): no thread waits for it except the gate CTA (block 0)
-    p.concurrent = (mode == 2 && h->concurrent && h->concurrent_waves && p.actions != nullptr) ? 1 : 0;
+    p.concurrent = (mode == 2 && h->concurrent && p.actions != nullptr) ? 1 : 0;
     p.early_state = (p.concurrent || (mode >= 1 && C > 1)) ? 1 : 0;
-    p.pdl_early = h->pdl_early ? 1 : 0;
     const size_t smem = (size_t)p.off_groups + (size_t)C * p.group_bytes;
     args.p = p;
     for (int i = 0; i < NC && i < h->n_cfgs; i++) args.cfg[i] = h->h_cfgs[i];
@@ -619,17 +574,13 @@ static cudaError_t launch_step1_nc(ngw_handle* h, StepParams p, cudaStream_t s) 
     lc.dynamicSmemBytes = smem;
     lc.stream = s;
     cudaLaunchAttribute attr[1];
-    pdl_attr(h, s, lc, attr);
+    pdl_attr(lc, attr);
     cudaError_t e;
-    if (C == 1) {
-        if (alias) e = cudaLaunchKernelEx(&lc, (step1_kernel<true, NC, true, true>), args);
-        else if (h->use_tma) e = cudaLaunchKernelEx(&lc, step1_kernel<true, NC, true>, args);
-        else e = cudaLaunchKernelEx(&lc, step1_kernel<false, NC, true>, args);
-    } else {
-        e = cudaLaunchKernelEx(&lc, step1_kernel<true, NC, false>, args);
-    }
+    if (alias) e = cudaLaunchKernelEx(&lc, step1_kernel<NC, true, true>, args);
+    else if (C == 1) e = cudaLaunchKernelEx(&lc, step1_kernel<NC, true, false>, args);
+    else e = cudaLaunchKernelEx(&lc, step1_kernel<NC, false, false>, args);
     if (e == cudaSuccess) {
-        note_launched(s, p.actions != nullptr && lc.numAttrs == 1);
+        note_launched(s, p.actions != nullptr);
         h->concurrent_launches += p.concurrent;
         h->last_step_concurrent = p.concurrent != 0;
     }
@@ -641,7 +592,6 @@ static cudaError_t launch_step1_nc(ngw_handle* h, StepParams p, cudaStream_t s) 
 template <int NC>
 static cudaError_t launch_step1w_nc(ngw_handle* h, StepParams p, cudaStream_t s) {
     static thread_local StepArgs<NC> args;
-    if (h->wshape == 0 || !h->use_tma) return cudaErrorNotSupported;
     if (h->obs_dim > 0 && h->lidar_mode != 1) return cudaErrorNotSupported;     // needs the line-gather lidar (register sink)
     int max_tail = 0;
     for (const DevConfig& dc : h->h_cfgs) max_tail = dc.c.n_inv_obs > max_tail ? dc.c.n_inv_obs : max_tail;
@@ -649,7 +599,7 @@ static cudaError_t launch_step1w_nc(ngw_handle* h, StepParams p, cudaStream_t s)
     const int luts = (NGW_MAX_MAP_SIZE + NGW_MAX_ITEMS * (NC > 0 ? NC : 0) + 127) & ~127;
     p.off_luts = NGW_WCTA_HDR;
     p.off_groups = p.off_luts + luts;
-    p.obs_srow = p.obs_row_bytes + (((p.obs_row_bytes >> 2) % 8 == 0 && p.obs_row_bytes > 0 && h->row_pad) ? 16 : 0);
+    p.obs_srow = p.obs_row_bytes + (((p.obs_row_bytes >> 2) % 8 == 0 && p.obs_row_bytes > 0) ? 16 : 0);
     const int in_bytes = p.map_bytes + p.inv_bytes, obs_tile = p.obs ? 32 * p.obs_srow : 0;
     p.group_bytes = (NGW_WTILE_HDR + (in_bytes > obs_tile ? in_bytes : obs_tile) + 127) & ~127;
     const long long tiles = (p.env_end - p.env_begin + 31) / 32;
@@ -659,24 +609,21 @@ static cudaError_t launch_step1w_nc(ngw_handle* h, StepParams p, cudaStream_t s)
     if (c_cap < 1) return cudaErrorNotSupported;
     const StreamTail me = launch_tail(p);
     const bool one_wave = tiles <= (long long)c_cap * h->sm_count;
-    const int mode = claim_stream(h, s, h->early_state && h->use_pdl, &me);
+    const int mode = claim_stream(h, s, true, &me);
     p.early_state = mode >= 1 ? 1 : 0;
     // (one-wave launches overlap whole; with several waves the next launch fills the SMs as the last wave drains)
-    p.concurrent = (mode == 2 && h->concurrent && (one_wave || h->concurrent_waves) && p.actions != nullptr) ? 1 : 0;
-    p.pdl_early = h->pdl_early ? 1 : 0;
-    int C = h->tiles_per_cta;
-    if (C <= 0) {
-        // Tiles per CTA (r02_sweep16, 29..31).  One wave, waiting for the predecessor: one CTA per SM (C2 7.3 us; two
-        // 7-tile CTAs: 8.5).  One wave, overlapped: two CTAs per SM and launch, of which THREE fit an SM — one and a half
-        // launches resident: C2 5.68 us vs 5.89 with 14 tiles per CTA, and 5.89 again when a slimmer header lets four
-        // 7-tile CTAs in.  Several waves: 8 (C3 19.5 / 20.3 / 20.4 us with 8 / 4 / 6, C4 98.6 / 99.9 / 99.7; odd counts
-        // leave partial CTAs).
-        if (!one_wave) C = h->wshape == 3 ? c_cap : 8;
-        else if (p.concurrent || (g_first_in_capture && h->concurrent && h->use_pdl && p.actions != nullptr))
-            C = (int)((tiles + 2 * h->sm_count - 1) / (2 * h->sm_count));   // (a capture's first launch waits, but its successor overlaps it)
-        else C = (int)((tiles + h->sm_count - 1) / h->sm_count);
-        if (C < 1) C = 1;
-    }
+    p.concurrent = (mode == 2 && h->concurrent && p.actions != nullptr) ? 1 : 0;
+    // Tiles per CTA (r02_sweep16, 29..31).  One wave, waiting for the predecessor: one CTA per SM (C2 7.3 us; two
+    // 7-tile CTAs: 8.5).  One wave, overlapped: two CTAs per SM and launch, of which THREE fit an SM — one and a half
+    // launches resident: C2 5.68 us vs 5.89 with 14 tiles per CTA, and 5.89 again when a slimmer header lets four
+    // 7-tile CTAs in.  Several waves: 8 (C3 19.5 / 20.3 / 20.4 us with 8 / 4 / 6, C4 98.6 / 99.9 / 99.7; odd counts
+    // leave partial CTAs).
+    int C;
+    if (!one_wave) C = 8;
+    else if (p.concurrent || (g_first_in_capture && h->concurrent && p.actions != nullptr))
+        C = (int)((tiles + 2 * h->sm_count - 1) / (2 * h->sm_count));   // (a capture's first launch waits, but its successor overlaps it)
+    else C = (int)((tiles + h->sm_count - 1) / h->sm_count);
+    if (C < 1) C = 1;
     if (C > c_cap) C = c_cap;
     if (C > tiles) C = (int)tiles;
     p.tiles_per_cta = C;
@@ -690,21 +637,23 @@ static cudaError_t launch_step1w_nc(ngw_handle* h, StepParams p, cudaStream_t s)
     lc.gridDim = dim3((unsigned)((tiles + C - 1) / C)); lc.blockDim = dim3(32 * (C + 1)); lc.dynamicSmemBytes = smem;
     lc.stream = s;
     cudaLaunchAttribute attr[1];
-    pdl_attr(h, s, lc, attr);
+    pdl_attr(lc, attr);
     cudaError_t e;
     if (max_tail <= 8) e = cudaLaunchKernelEx(&lc, step1w_kernel<NC, 8>, args);
     else e = cudaLaunchKernelEx(&lc, step1w_kernel<NC, 16>, args);
     if (e == cudaSuccess) {
-        note_launched(s, p.actions != nullptr && lc.numAttrs == 1);
+        note_launched(s, p.actions != nullptr);
         h->concurrent_launches += p.concurrent;
         h->last_step_concurrent = p.concurrent != 0;
     }
     return e;
 }
 
+static const int kResetCtasPerSmOverlapped = 1;    // queued-reset grid behind an overlapped step, see launch_step
+
 static int launch_step(ngw_handle* h, const StepParams& p, cudaStream_t s) {
     if (p.env_end <= p.env_begin) return 0;
-    int nc = h->force_global_cfg ? 0 : h->n_cfgs;
+    const int nc = h->n_cfgs;
     cudaError_t e;
     if (is_multi(p)) {
         e = ngw_launch_rollout(h, p, s);                  // ngw_rollout.cu
@@ -728,7 +677,7 @@ static int launch_step(ngw_handle* h, const StepParams& p, cudaStream_t s) {
         // Grid: alone, four CTAs per SM regenerate the queue fastest (C5: ~2000 envs in 52 us).  When this step overlapped
         // its predecessor — rotating handles inside a capture — the NEXT handle's step will overlap this kernel: then ONE
         // CTA per SM (11 KB, 16 K registers) fits next to that step's full set of CTAs and the resets hide behind it.
-        const int rl_ctas = h->sm_count * (h->last_step_concurrent ? h->reset_grid : 4);
+        const int rl_ctas = h->sm_count * (h->last_step_concurrent ? kResetCtasPerSmOverlapped : 4);
         cudaLaunchConfig_t lc;
         memset(&lc, 0, sizeof(lc));
         lc.gridDim = dim3((unsigned)rl_ctas); lc.blockDim = dim3(32 * NGW_RESET_WARPS);

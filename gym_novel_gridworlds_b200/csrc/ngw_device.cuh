@@ -596,7 +596,6 @@ __device__ __forceinline__ void lidar_lines(const EnvRow& e, const ngw_config& c
 __device__ __forceinline__ int lidar_line_share(int g, int G) {
     if (G == 1) return 0xF;
     if (G == 2) return g == 0 ? 0x3 : 0xC;
-    if (G == 3) return g == 0 ? 0x3 : (g == 1 ? 0x4 : 0x8);
     return g < 4 ? (1 << g) : 0;
 }
 
@@ -670,15 +669,16 @@ __device__ __forceinline__ void lidar_observe(const EnvRow& e, const DevConfig& 
                                               bool with_tail) {
     const ngw_config& cfg = dc.c;
     const int B = cfg.n_beams, K = cfg.max_range, L = cfg.n_lidar_items;
-    if (dc.lidar.lines && luts.slot != nullptr && (e.ms <= 32 || !dc.lidar.fast || dc.lidar.lines == 2)) {
+    // (`lines` implies `fast`, so `!fast` never holds here; written out, it keeps observe_masked_kernel at 62 registers
+    // instead of 68 and rollout_kernel's spills where they were)
+    if (dc.lidar.lines && luts.slot != nullptr && (e.ms <= 32 || !dc.lidar.fast)) {
         const int sel = lidar_line_share(g, G);
         if (sel) lidar_lines<kSafe, Sink>(e, cfg, tables, luts, obs, sel);
     } else if (dc.lidar.fast) {
         if (G == 1) lidar_fast<8, Sink>(e, cfg, tables, obs, zero, 0);
         else if (G == 2) lidar_fast<4, Sink>(e, cfg, tables, obs, zero, g * 4);
-        else if (G == 3) { if (g < 2) lidar_fast<3, Sink>(e, cfg, tables, obs, zero, g * 3); else lidar_fast<2, Sink>(e, cfg, tables, obs, zero, 6); }
         else if (G == 4) lidar_fast<2, Sink>(e, cfg, tables, obs, zero, g * 2);
-        else lidar_fast<1, Sink>(e, cfg, tables, obs, zero, g);
+        else lidar_fast<1, Sink>(e, cfg, tables, obs, zero, g);         // G == 8: the reset kernel's observation pass
     } else {
         const int cells = e.ms * e.ms;
         const int pos = e.r * e.ms + e.c;

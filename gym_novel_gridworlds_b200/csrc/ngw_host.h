@@ -18,19 +18,11 @@ struct ngw_handle {
     long long n = 0, np = 0, first_gid = 0;
     unsigned long long seed = 0;
     int ms = 0, cells = 0, inv_stride = 0, obs_dim = 0, n_cfgs = 0;
-    int map_bytes = 0, inv_bytes = 0, obs_bytes = 0, warps = 2, tiles_per_cta = 0, lidar_mode = 0;
+    int map_bytes = 0, inv_bytes = 0, obs_bytes = 0, warps = 2, lidar_mode = 0;
     int obs_u8 = 0, obs_row_bytes = 0;             // observation row layout (ngw_set_obs_format)
-    int cache_hints = 3, dbg_skip = 0;
     uint32_t key_mask = 0xFFFFFFFFu;
-    bool use_tma = true, collect_stats = true, force_global_cfg = false, plain_store = false, use_pdl = true;
-    bool pdl_in_graph = true, early_state = true, pdl_early = true;
     bool lidar_uniform = false;
-    int wshape = 1;                                // 1: launches take the warp-per-tile kernel when it supports them, 0: never
     bool concurrent = true;                        // independent consecutive launches may overlap (NGW_NO_CONCURRENT)
-    bool concurrent_waves = true;                  // ... also launches of several waves (NGW_NO_CONCURRENT_WAVES)
-    bool rollout2 = true;                          // lane-pair rollout kernel (NGW_NO_ROLLOUT2)
-    bool row_pad = true;                           // shared-memory observation rows of 8k words get 16 bytes of padding (NGW_NO_ROW_PAD)
-    bool alias = true;                             // tile-group kernel, one tile per CTA: observation tile aliases the rows (NGW_NO_ALIAS)
     DevConfig* d_cfgs = nullptr;
     std::vector<int16_t*> d_luts;
     std::vector<DevConfig> h_cfgs;
@@ -41,7 +33,6 @@ struct ngw_handle {
     int32_t* reset_list = nullptr; int32_t* reset_ctl = nullptr;   // auto-reset queue; ctl[0] = count, ctl[1] = finished CTAs
     int sm_count = 148;
     long long launches = 0, concurrent_launches = 0;
-    int reset_grid = 1;                            // CTAs per SM of the queued-reset kernel when it overlaps the next step (NGW_RESET_GRID)
     bool last_step_concurrent = false;             // the latest one-step launch overlapped its predecessor
     // host-buffer path: its own stream, ordered against the caller's streams with events
     cudaStream_t hs = nullptr;
@@ -67,7 +58,7 @@ struct StreamTail {                       // the latest library launch on a stre
 int fail(const std::string& m);
 // see ngw_capi.cu
 int claim_stream(ngw_handle* h, cudaStream_t s, bool want_early, const StreamTail* mine = nullptr);
-void pdl_attr(ngw_handle* h, cudaStream_t s, cudaLaunchConfig_t& lc, cudaLaunchAttribute* attr);
+void pdl_attr(cudaLaunchConfig_t& lc, cudaLaunchAttribute* attr);
 // ngw_rollout.cu
 cudaError_t ngw_launch_rollout(ngw_handle* h, const StepParams& p, cudaStream_t s);
 int ngw_rollout_init();

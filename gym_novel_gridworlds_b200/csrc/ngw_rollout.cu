@@ -9,14 +9,13 @@
     } while (0)
 
 int ngw_rollout_init() {
-    // (rollout_kernel is the fallback behind rollout2_kernel: inline configs for one config, the global table otherwise;
-    // its plain-copy twin exists for the NGW_NO_TMA A/B only with the global table)
-    NGW_SMEM_ATTR((rollout_kernel<true, 0>)); NGW_SMEM_ATTR((rollout_kernel<true, 1>)); NGW_SMEM_ATTR((rollout_kernel<false, 0>));
+    // (rollout_kernel is the fallback behind rollout2_kernel: inline configs for one config, the global table otherwise)
+    NGW_SMEM_ATTR((rollout_kernel<0>)); NGW_SMEM_ATTR((rollout_kernel<1>));
     return 0;
 }
 
 // K-step rollout launches (ngw_rollout / ngw_rollout_policy): one tile per CTA, tile resident across the steps
-template <int NC, bool kTma = true>
+template <int NC>
 static cudaError_t launch_rollout_nc(ngw_handle* h, StepParams p, cudaStream_t s) {
     static thread_local StepArgs<NC> args;          // host staging of the argument block (copied by the launch); per thread,
                                                     // so distinct handles stay independent across host threads
@@ -40,8 +39,8 @@ static cudaError_t launch_rollout_nc(ngw_handle* h, StepParams p, cudaStream_t s
     lc.gridDim = dim3((unsigned)tiles); lc.blockDim = dim3(32 * warps); lc.dynamicSmemBytes = smem;
     lc.stream = s;
     cudaLaunchAttribute attr[1];
-    pdl_attr(h, s, lc, attr);
-    return cudaLaunchKernelEx(&lc, rollout_kernel<kTma, NC>, args);
+    pdl_attr(lc, attr);
+    return cudaLaunchKernelEx(&lc, rollout_kernel<NC>, args);
 }
 
 // K-step rollout launches in the lane-pair shape (rollout2_kernel); cudaErrorNotSupported -> rollout_kernel
@@ -66,7 +65,7 @@ static cudaError_t launch_rollout2_na(ngw_handle* h, StepParams p, cudaStream_t 
     lc.gridDim = dim3((unsigned)tiles); lc.blockDim = dim3(64); lc.dynamicSmemBytes = smem;
     lc.stream = s;
     cudaLaunchAttribute attr[1];
-    pdl_attr(h, s, lc, attr);
+    pdl_attr(lc, attr);
     static bool attr_set = false;       // per instantiation
     if (!attr_set) { cudaFuncSetAttribute(rollout2_kernel<NC, A4>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024); attr_set = true; }
     return cudaLaunchKernelEx(&lc, rollout2_kernel<NC, A4>, args);
@@ -74,7 +73,7 @@ static cudaError_t launch_rollout2_na(ngw_handle* h, StepParams p, cudaStream_t 
 
 template <int NC>
 static cudaError_t launch_rollout2_nc(ngw_handle* h, const StepParams& p, cudaStream_t s) {
-    if (h->wshape == 0 || !h->use_tma || h->ms > 32 || !h->rollout2) return cudaErrorNotSupported;
+    if (h->ms > 32) return cudaErrorNotSupported;
     if (h->obs_dim > 0 && h->lidar_mode != 1) return cudaErrorNotSupported;
     for (const DevConfig& dc : h->h_cfgs)
         if (dc.c.n_inv_obs > NGW_REGSINK_TAIL) return cudaErrorNotSupported;
@@ -88,10 +87,9 @@ static cudaError_t launch_rollout2_nc(ngw_handle* h, const StepParams& p, cudaSt
 }
 
 cudaError_t ngw_launch_rollout(ngw_handle* h, const StepParams& p, cudaStream_t s) {
-    const int nc = h->force_global_cfg ? 0 : h->n_cfgs;
+    const int nc = h->n_cfgs;
     cudaError_t e = nc == 1 ? launch_rollout2_nc<1>(h, p, s) : launch_rollout2_nc<0>(h, p, s);
     if (e != cudaErrorNotSupported) return e;
-    if (!h->use_tma) return launch_rollout_nc<0, false>(h, p, s);
     if (nc == 1) return launch_rollout_nc<1>(h, p, s);
     return launch_rollout_nc<0>(h, p, s);
 }

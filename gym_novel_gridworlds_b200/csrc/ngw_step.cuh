@@ -35,7 +35,9 @@ __device__ __forceinline__ void bulk_g2s(void* dst_smem, const void* src_gmem, u
                  "l"(src_gmem), "r"(bytes), "r"(smem_u32(bar))
                  : "memory");
 }
-// L2 cache-hinted variants (createpolicy + .L2::cache_hint)
+// L2 cache-hinted variants (createpolicy + .L2::cache_hint).  The kernels load the state tiles and store the observation
+// tile evict_first: streaming data (each tile is read once and its observations written once per step) should not linger
+// in L2 — measured on C2 9.15 -> 8.82 us/step, C3 29.3 -> 28.0, C5 278 -> 274 (hinting the inventory store as well: 9.0)
 __device__ __forceinline__ uint64_t policy_evict_first() {
     uint64_t pol;
     asm volatile("createpolicy.fractional.L2::evict_first.b64 %0, 1.0;" : "=l"(pol));
@@ -95,7 +97,7 @@ struct StepParams {
     uint8_t* done;
     float* cost;
     uint8_t* result;
-    double* stats;              // [NGW_STAT_SLOTS][NGW_STAT_COUNT] or nullptr
+    double* stats;              // [NGW_STAT_SLOTS][NGW_STAT_COUNT]
     long long env_begin, env_end;   // env range of this launch (env_begin multiple of 32)
     long long first_gid;
     unsigned long long seed;
@@ -111,16 +113,10 @@ struct StepParams {
     int tiles_per_cta, g_shift, n_tiles;                 // one-step kernel: tile groups per CTA, log2(warps per tile), tiles
     int lidar_mode;             // 1: every config takes the line-gather path with one shared geometry (the common case)
     int early_state;            // 1: this handle's state is complete already, state loads may precede griddepcontrol.wait
-    int pdl_early;              // 1: trigger the dependent launch right after the wait (A/B knob NGW_PDL_EARLY)
     int concurrent;             // step1w_kernel: 1 = this launch is independent of its predecessor (another handle's step, proven
                                 // adjacent in a stream capture, disjoint buffers): the tile warps do not wait for it, only the gate warp
     int auto_reset, max_episode_steps;
     int lidar_uniform;          // every config has the same beam tables (then config 0's are read, warp-uniformly)
-    int cache_hints;            // bit 0: state tiles are loaded L2::evict_first, bit 1: the observation tile is stored evict_first
-    int plain_store;            // 1 => write tiles back with ordinary coalesced stores instead of TMA bulk stores
-    int dbg_skip;               // attribution knob (NGW_SKIP, results are then WRONG): 1 step, 2 lidar, 4 outputs + statistics,
-                                // 8 observation store, 16 inventory store, 64 return after griddepcontrol.wait,
-                                // 128 return once the tile has landed
     // K-step rollout (n_steps > 1 or random policy): the tile stays in shared memory across the steps
     int n_steps;                // steps per launch (1 for ngw_step)
     int random_policy;          // 1 => actions drawn on the device (Philox), `actions` is only a non-null marker
@@ -218,7 +214,7 @@ __device__ __forceinline__ void tile_stats(double* stats, int slot, int lane, in
 #define NGW_CLASS1_OPS ((1u << NGW_OP_FORWARD) | (1u << NGW_OP_BREAK) | (1u << NGW_OP_PLACE_TREE_TAP) | \
                         (1u << NGW_OP_EXTRACT_RUBBER) | (1u << NGW_OP_EXTRACT_STRING) | (1u << NGW_OP_CHOP) | (1u << NGW_OP_JUMP))
 
-template <bool kTma, int NC>
+template <int NC>
 __global__ void __launch_bounds__(256) rollout_kernel(const __grid_constant__ StepArgs<NC> args) {
     extern __shared__ __align__(128) unsigned char smem[];
     const StepParams& p = args.p;
@@ -244,7 +240,7 @@ __global__ void __launch_bounds__(256) rollout_kernel(const __grid_constant__ St
     const int8_t* gmap = p.map + e0 * p.cells;
     int32_t* ginv = p.inv + e0 * p.inv_stride;
     if (threadIdx.x == 0) {
-        if (kTma) mbar_init(bar, 1);
+        mbar_init(bar, 1);
         *reinterpret_cast<uint64_t*>(szero) = 0ull;
     }
     if (NC > 0) {                                                    // config tables are kernel arguments (constant bank)
@@ -266,25 +262,11 @@ __global__ void __launch_bounds__(256) rollout_kernel(const __grid_constant__ St
     asm volatile("griddepcontrol.wait;" ::: "memory");               // previous kernel of the stream done + visible
 
     // ---- stage the tile: grid rows + inventory rows (state arrays are padded, a full tile is always readable)
-    if (kTma) {
-        if (threadIdx.x == 0) {
-            mbar_expect_tx(bar, (uint32_t)(p.map_bytes + p.inv_bytes));
-            if (p.cache_hints & 1) {
-                uint64_t pol = policy_evict_first();
-                bulk_g2s_hint(smap, gmap, (uint32_t)p.map_bytes, bar, pol);
-                bulk_g2s_hint(sinv, ginv, (uint32_t)p.inv_bytes, bar, pol);
-            } else {
-                bulk_g2s(smap, gmap, (uint32_t)p.map_bytes, bar);
-                bulk_g2s(sinv, ginv, (uint32_t)p.inv_bytes, bar);
-            }
-        }
-    } else {
-        const uint4* s4 = reinterpret_cast<const uint4*>(gmap);
-        uint4* d4 = reinterpret_cast<uint4*>(smap);
-        for (int i = threadIdx.x; i < (p.map_bytes >> 4); i += blockDim.x) d4[i] = s4[i];
-        s4 = reinterpret_cast<const uint4*>(ginv);
-        d4 = reinterpret_cast<uint4*>(sinv);
-        for (int i = threadIdx.x; i < (p.inv_bytes >> 4); i += blockDim.x) d4[i] = s4[i];
+    if (threadIdx.x == 0) {
+        mbar_expect_tx(bar, (uint32_t)(p.map_bytes + p.inv_bytes));
+        uint64_t pol = policy_evict_first();
+        bulk_g2s_hint(smap, gmap, (uint32_t)p.map_bytes, bar, pol);
+        bulk_g2s_hint(sinv, ginv, (uint32_t)p.inv_bytes, bar, pol);
     }
     if (closed_loop) {                                               // the policy's weights, once per CTA
         const int n_w = p.obs_dim * p.policy_actions;
@@ -317,8 +299,8 @@ __global__ void __launch_bounds__(256) rollout_kernel(const __grid_constant__ St
         if (valid && given_actions) action = p.actions[e];
     }
 
-    if (kTma) mbar_wait(bar, 0);
-    __syncthreads();                                                 // plain copies / policy weights visible to the step warp
+    mbar_wait(bar, 0);
+    __syncthreads();                                                 // policy weights visible to the step warp
 
     EnvRow env;
     env.m = smap + lane * p.cells;
@@ -400,8 +382,7 @@ __global__ void __launch_bounds__(256) rollout_kernel(const __grid_constant__ St
                     env.r = ps.x; env.c = ps.y; env.facing = ps.z; env.sel = ps.w;
                 }
             }
-            if (p.stats != nullptr)
-                tile_stats(p.stats, (int)blockIdx.x, lane, valid, o.done, success, did_reset, invalid, o.reward, o.cost);
+            tile_stats(p.stats, (int)blockIdx.x, lane, valid, o.done, success, did_reset, invalid, o.reward, o.cost);
             action = next_action;
         }
         if (closed_loop && !use_sink) {                               // the last policy observation must not leak into the final one
@@ -431,17 +412,14 @@ __global__ void __launch_bounds__(256) rollout_kernel(const __grid_constant__ St
 
     // ---- write back: inventory tile and observation tile.  Every thread orders its generic-proxy writes to the tiles
     //      before the async proxy reads them (fence before the barrier), then one thread issues.
-    if (kTma) fence_async_smem();
+    fence_async_smem();
     __syncthreads();
     asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
-    if (kTma && full_tile && !p.plain_store) {
+    if (full_tile) {
         if (threadIdx.x == 0) {
             bulk_s2g(ginv, sinv, (uint32_t)p.inv_bytes);
-            if (p.obs != nullptr) {
-                unsigned char* gobs = p.obs + e0 * p.obs_row_bytes;
-                if (p.cache_hints & 2) bulk_s2g_hint(gobs, sobs, (uint32_t)p.obs_bytes, policy_evict_first());
-                else bulk_s2g(gobs, sobs, (uint32_t)p.obs_bytes);
-            }
+            if (p.obs != nullptr)
+                bulk_s2g_hint(p.obs + e0 * p.obs_row_bytes, sobs, (uint32_t)p.obs_bytes, policy_evict_first());
             bulk_commit();
             bulk_wait_read<0>();                                     // shared memory must outlive the bulk stores' reads
         }
@@ -492,7 +470,7 @@ __device__ __forceinline__ void group_sync(int grp, int G) {
 // kAlias (one tile per CTA only): the observation tile ALIASES the grid / inventory rows, as in step1w_kernel — the lidar
 // hits and the inventory tail wait in registers (RegSink) until the rows have been consumed.  A 40x40 tile is then 52 KB
 // instead of 61 KB: four tiles per SM instead of three (C5).
-template <bool kTma, int NC, bool kOne, bool kAlias = false>
+template <int NC, bool kOne, bool kAlias = false>
 __global__ void __launch_bounds__(512) step1_kernel(const __grid_constant__ StepArgs<NC> args) {
     extern __shared__ __align__(128) unsigned char smem[];
     const StepParams& p = args.p;
@@ -530,7 +508,7 @@ __global__ void __launch_bounds__(512) step1_kernel(const __grid_constant__ Step
     // ---- prologue without global state: barriers, zero pad, lidar tables
     if (threadIdx.x < 8) scta[threadIdx.x] = 0;
     if (gt == 0) {
-        if (kTma) mbar_init(bar, 1);
+        mbar_init(bar, 1);
         *reinterpret_cast<uint64_t*>(szero) = 0ull;
     }
     if (NC > 0) {                                                     // config tables are kernel arguments (constant bank)
@@ -554,30 +532,16 @@ __global__ void __launch_bounds__(512) step1_kernel(const __grid_constant__ Step
     int32_t* ginv = p.inv + e0 * p.inv_stride;
     uint64_t pol_first = 0;
     auto issue_loads = [&]() {
-        if (kTma) {
-            if (gt == 0) {
-                mbar_expect_tx(bar, (uint32_t)(p.map_bytes + p.inv_bytes));
-                if (p.cache_hints) pol_first = policy_evict_first();
-                if (p.cache_hints & 1) {
-                    bulk_g2s_hint(smap, gmap, (uint32_t)p.map_bytes, bar, pol_first);
-                    bulk_g2s_hint(sinv, ginv, (uint32_t)p.inv_bytes, bar, pol_first);
-                } else {
-                    bulk_g2s(smap, gmap, (uint32_t)p.map_bytes, bar);
-                    bulk_g2s(sinv, ginv, (uint32_t)p.inv_bytes, bar);
-                }
-            }
-        } else {
-            const uint4* s4 = reinterpret_cast<const uint4*>(gmap);
-            uint4* d4 = reinterpret_cast<uint4*>(smap);
-            for (int i = gt; i < (p.map_bytes >> 4); i += 32 * G) d4[i] = s4[i];
-            s4 = reinterpret_cast<const uint4*>(ginv);
-            d4 = reinterpret_cast<uint4*>(sinv);
-            for (int i = gt; i < (p.inv_bytes >> 4); i += 32 * G) d4[i] = s4[i];
+        if (gt == 0) {
+            mbar_expect_tx(bar, (uint32_t)(p.map_bytes + p.inv_bytes));
+            pol_first = policy_evict_first();
+            bulk_g2s_hint(smap, gmap, (uint32_t)p.map_bytes, bar, pol_first);
+            bulk_g2s_hint(sinv, ginv, (uint32_t)p.inv_bytes, bar, pol_first);
         }
     };
     const int n_cls = G >= 2 ? 2 : 1;                                 // warps that take part in the step
     uchar4 ps = make_uchar4(0, 0, 0, 0);
-    const bool early = p.early_state && active && !(p.dbg_skip & 64);
+    const bool early = p.early_state && active;
     if (early) {
         issue_loads();
         if (g < n_cls) ps = __ldcg(&p.pose[e]);
@@ -595,9 +559,10 @@ __global__ void __launch_bounds__(512) step1_kernel(const __grid_constant__ Step
     }
     if (!p.concurrent) {
         asm volatile("griddepcontrol.wait;" ::: "memory");            // previous kernel of the stream done + visible
-        if (p.pdl_early) asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
+        // trigger right after the wait (rather than once the stores are issued): C2 7.70 -> 7.60 us/step
+        asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
     }
-    if (!active || (p.dbg_skip & 64)) { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); return; }
+    if (!active) { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); return; }
     if (!early) issue_loads();
 
     // ---- while the copies fly: per-lane scalars
@@ -610,9 +575,7 @@ __global__ void __launch_bounds__(512) step1_kernel(const __grid_constant__ Step
         if (stepping && valid) action = __ldcg(&p.actions[e]);
     }
 
-    if (kTma) mbar_wait(bar, 0);
-    else group_sync<kOne>(grp, G);
-    if (p.dbg_skip & 128) { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); return; }
+    mbar_wait(bar, 0);
 
     EnvRow env;
     env.m = smap + lane * p.cells;
@@ -642,7 +605,7 @@ __global__ void __launch_bounds__(512) step1_kernel(const __grid_constant__ Step
                     bits |= 1u << 20;
                     atomicOr(&p.err[e], NGW_ERR_INVALID_ACTION);
                 } else {
-                    if (!(p.dbg_skip & 1)) step_env(env, cfg, a, o);
+                    step_env(env, cfg, a, o);
                     if (o.goal) bits |= 1u << 18;
                     int finished = o.done;
                     if (p.max_episode_steps > 0) {
@@ -677,12 +640,11 @@ __global__ void __launch_bounds__(512) step1_kernel(const __grid_constant__ Step
     group_sync<kOne>(grp, G);                                               // step results (grid, inventory, hand-over) visible to the group
     ps = sout[lane].ps;
     env.r = ps.x; env.c = ps.y; env.facing = ps.z; env.sel = ps.w;
-    const bool tma_store = kTma && full_tile && !p.plain_store;
     if (kAlias && stepping) {                                         // the inventory tile leaves before its rows are overwritten
-        if (tma_store) {
+        if (full_tile) {
             fence_async_smem();
             group_sync<kOne>(grp, G);
-            if (gt == 0 && !(p.dbg_skip & 16)) { bulk_s2g(ginv, sinv, (uint32_t)p.inv_bytes); bulk_commit(); }
+            if (gt == 0) { bulk_s2g(ginv, sinv, (uint32_t)p.inv_bytes); bulk_commit(); }
         } else {
             const uint4* s4 = reinterpret_cast<const uint4*>(sinv);
             uint4* d4 = reinterpret_cast<uint4*>(ginv);
@@ -696,7 +658,7 @@ __global__ void __launch_bounds__(512) step1_kernel(const __grid_constant__ Step
             RegSink<NGW_REGSINK_TAIL> sink;
             sink.init(p.obs_u8);
             const bool look = valid && cfg.n_beams > 0;
-            if (look && !(p.dbg_skip & 2)) {
+            if (look) {
                 LidarLuts luts;
                 if (NC > 0) { luts.slot = sslot + cfg_i * NGW_MAX_ITEMS; luts.firstk = sfirstk; }
                 else { luts.slot = p.dcfgs[cfg_i].c.lidar_slot; luts.firstk = p.dcfgs[cfg_i].lidar.firstk; }
@@ -719,7 +681,7 @@ __global__ void __launch_bounds__(512) step1_kernel(const __grid_constant__ Step
             }
         }
     } else
-    if (p.obs != nullptr && valid && cfg.n_beams > 0 && !(p.dbg_skip & 2)) {
+    if (p.obs != nullptr && valid && cfg.n_beams > 0) {
         ObsRow orow;
         orow.p = sobs + lane * p.obs_srow;
         orow.u8 = p.obs_u8;
@@ -739,22 +701,18 @@ __global__ void __launch_bounds__(512) step1_kernel(const __grid_constant__ Step
 
     // ---- write back: inventory tile (only when stepping) and observation tile.  Every thread orders its generic-proxy
     //      writes to the tiles before the async proxy reads them (fence before the barrier), then one thread issues.
-    if (kTma) fence_async_smem();
+    fence_async_smem();
     group_sync<kOne>(grp, G);
     const bool padded_rows = p.obs_srow != p.obs_row_bytes;
-    if (kTma && full_tile && !p.plain_store) {
-        if (!kAlias && gt == 0 && stepping && !(p.dbg_skip & 16)) bulk_s2g(ginv, sinv, (uint32_t)p.inv_bytes);
-        if (p.obs != nullptr && !(p.dbg_skip & 8)) {
+    if (full_tile) {
+        if (!kAlias && gt == 0 && stepping) bulk_s2g(ginv, sinv, (uint32_t)p.inv_bytes);
+        if (p.obs != nullptr) {
             unsigned char* gobs = p.obs + e0 * p.obs_row_bytes;
             if (!padded_rows) {                                       // the tile is one contiguous span on both sides
-                if (gt == 0) {
-                    if (p.cache_hints & 2) bulk_s2g_hint(gobs, sobs, (uint32_t)p.obs_bytes, pol_first);
-                    else bulk_s2g(gobs, sobs, (uint32_t)p.obs_bytes);
-                }
+                if (gt == 0) bulk_s2g_hint(gobs, sobs, (uint32_t)p.obs_bytes, pol_first);
             } else if (g == 0) {                                      // padded rows in shared memory: lane l stores row l
-                if (p.cache_hints & 2) bulk_s2g_hint(gobs + lane * p.obs_row_bytes, sobs + lane * p.obs_srow,
-                                                     (uint32_t)p.obs_row_bytes, lane == 0 ? pol_first : policy_evict_first());
-                else bulk_s2g(gobs + lane * p.obs_row_bytes, sobs + lane * p.obs_srow, (uint32_t)p.obs_row_bytes);
+                bulk_s2g_hint(gobs + lane * p.obs_row_bytes, sobs + lane * p.obs_srow, (uint32_t)p.obs_row_bytes,
+                              lane == 0 ? pol_first : policy_evict_first());
             }
         }
         if (g == 0) bulk_commit();
@@ -775,7 +733,7 @@ __global__ void __launch_bounds__(512) step1_kernel(const __grid_constant__ Step
     }
 
     // ---- per-env outputs (full lines, one warp) and episode statistics, behind the tile stores
-    if (g == 0 && stepping && !(p.dbg_skip & 4)) {
+    if (g == 0 && stepping) {
         const uint4 raw = *reinterpret_cast<const uint4*>(&sout[lane]);
         const uint32_t bits = raw.y;
         const int reward = (int)(short)(bits & 0xFFFFu);
@@ -788,47 +746,45 @@ __global__ void __launch_bounds__(512) step1_kernel(const __grid_constant__ Step
             p.result[e] = (uint8_t)((bits >> 17) & 1u);
             if (p.msg != nullptr) p.msg[e] = (uint16_t)raw.w;
         }
-        if (p.stats != nullptr) {
-            // warp reductions, then shared-memory accumulators of the CTA; the last group to arrive flushes them with one
-            // set of global atomics per CTA
-            const uint32_t stepped = valid ? (bits >> 21) & 1u : 0u;
-            const uint32_t a_cnt = stepped | ((valid ? (bits >> 16) & 1u : 0u) << 10) | (((bits >> 18) & 1u) << 20);     // steps | episodes | successes
-            const uint32_t b_cnt = ((bits >> 19) & 1u) | (((bits >> 20) & 1u) << 10);                                       // resets | invalid
-            const uint32_t a_sum = __reduce_add_sync(0xFFFFFFFFu, valid ? a_cnt : 0u);
-            const uint32_t b_sum = __reduce_add_sync(0xFFFFFFFFu, valid ? b_cnt : 0u);
-            const int r_sum = __reduce_add_sync(0xFFFFFFFFu, valid ? reward : 0);
-            const float c_sum = warp_sum(valid ? cost : 0.0f);
-            if (lane == 0) {
-                int a_tot = (int)a_sum, b_tot = (int)b_sum, r_tot = r_sum;
-                float c_tot = c_sum;
-                bool flush = true;
-                if (!kOne) {                                          // several groups: fold in shared memory, the last one flushes
-                    atomicAdd(&scta[0], a_tot);
-                    atomicAdd(&scta[1], b_tot);
-                    atomicAdd(&scta[2], r_tot);
-                    atomicAdd(reinterpret_cast<float*>(&scta[3]), c_tot);
-                    __threadfence_block();
-                    const int n_groups = min(p.tiles_per_cta, p.n_tiles - ((int)blockIdx.x - p.concurrent) * p.tiles_per_cta);
-                    flush = atomicAdd(&scta[4], 1) == n_groups - 1;
-                    if (flush) {
-                        __threadfence_block();
-                        a_tot = *reinterpret_cast<volatile int*>(&scta[0]); b_tot = *reinterpret_cast<volatile int*>(&scta[1]);
-                        r_tot = *reinterpret_cast<volatile int*>(&scta[2]);
-                        c_tot = *reinterpret_cast<volatile float*>(&scta[3]);
-                    }
-                }
+        // warp reductions, then shared-memory accumulators of the CTA; the last group to arrive flushes them with one
+        // set of global atomics per CTA
+        const uint32_t stepped = valid ? (bits >> 21) & 1u : 0u;
+        const uint32_t a_cnt = stepped | ((valid ? (bits >> 16) & 1u : 0u) << 10) | (((bits >> 18) & 1u) << 20);     // steps | episodes | successes
+        const uint32_t b_cnt = ((bits >> 19) & 1u) | (((bits >> 20) & 1u) << 10);                                       // resets | invalid
+        const uint32_t a_sum = __reduce_add_sync(0xFFFFFFFFu, valid ? a_cnt : 0u);
+        const uint32_t b_sum = __reduce_add_sync(0xFFFFFFFFu, valid ? b_cnt : 0u);
+        const int r_sum = __reduce_add_sync(0xFFFFFFFFu, valid ? reward : 0);
+        const float c_sum = warp_sum(valid ? cost : 0.0f);
+        if (lane == 0) {
+            int a_tot = (int)a_sum, b_tot = (int)b_sum, r_tot = r_sum;
+            float c_tot = c_sum;
+            bool flush = true;
+            if (!kOne) {                                          // several groups: fold in shared memory, the last one flushes
+                atomicAdd(&scta[0], a_tot);
+                atomicAdd(&scta[1], b_tot);
+                atomicAdd(&scta[2], r_tot);
+                atomicAdd(reinterpret_cast<float*>(&scta[3]), c_tot);
+                __threadfence_block();
+                const int n_groups = min(p.tiles_per_cta, p.n_tiles - ((int)blockIdx.x - p.concurrent) * p.tiles_per_cta);
+                flush = atomicAdd(&scta[4], 1) == n_groups - 1;
                 if (flush) {
-                    const int n_step = a_tot & 1023, n_done = (a_tot >> 10) & 1023, n_succ = (a_tot >> 20) & 1023;
-                    const int n_reset = b_tot & 1023, n_inv = (b_tot >> 10) & 1023;
-                    double* sg = p.stats + (size_t)(blockIdx.x % NGW_STAT_SLOTS) * NGW_STAT_COUNT;
-                    atomicAdd(&sg[NGW_STAT_STEPS], (double)(n_step - n_inv));
-                    atomicAdd(&sg[NGW_STAT_REWARD_SUM], (double)r_tot);
-                    atomicAdd(&sg[NGW_STAT_COST_SUM], (double)c_tot);
-                    if (n_done) atomicAdd(&sg[NGW_STAT_EPISODES], (double)n_done);
-                    if (n_succ) atomicAdd(&sg[NGW_STAT_SUCCESSES], (double)n_succ);
-                    if (n_reset) atomicAdd(&sg[NGW_STAT_RESETS], (double)n_reset);
-                    if (n_inv) atomicAdd(&sg[NGW_STAT_INVALID], (double)n_inv);
+                    __threadfence_block();
+                    a_tot = *reinterpret_cast<volatile int*>(&scta[0]); b_tot = *reinterpret_cast<volatile int*>(&scta[1]);
+                    r_tot = *reinterpret_cast<volatile int*>(&scta[2]);
+                    c_tot = *reinterpret_cast<volatile float*>(&scta[3]);
                 }
+            }
+            if (flush) {
+                const int n_step = a_tot & 1023, n_done = (a_tot >> 10) & 1023, n_succ = (a_tot >> 20) & 1023;
+                const int n_reset = b_tot & 1023, n_inv = (b_tot >> 10) & 1023;
+                double* sg = p.stats + (size_t)(blockIdx.x % NGW_STAT_SLOTS) * NGW_STAT_COUNT;
+                atomicAdd(&sg[NGW_STAT_STEPS], (double)(n_step - n_inv));
+                atomicAdd(&sg[NGW_STAT_REWARD_SUM], (double)r_tot);
+                atomicAdd(&sg[NGW_STAT_COST_SUM], (double)c_tot);
+                if (n_done) atomicAdd(&sg[NGW_STAT_EPISODES], (double)n_done);
+                if (n_succ) atomicAdd(&sg[NGW_STAT_SUCCESSES], (double)n_succ);
+                if (n_reset) atomicAdd(&sg[NGW_STAT_RESETS], (double)n_reset);
+                if (n_inv) atomicAdd(&sg[NGW_STAT_INVALID], (double)n_inv);
             }
         }
     }
@@ -836,7 +792,7 @@ __global__ void __launch_bounds__(512) step1_kernel(const __grid_constant__ Step
     // Programmatic dependent launch: this group's work is issued; once every group of the CTA got here the next kernel of
     // the stream may start scheduling its CTAs (its prologue touches no global state: it overlaps this kernel's stores).
     asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
-    if (kTma && g == 0) bulk_wait_read<0>();                          // shared memory must outlive the bulk stores' reads
+    if (g == 0) bulk_wait_read<0>();                                  // shared memory must outlive the bulk stores' reads
 }
 
 // ------------------------------------------------------------------ the ONE-STEP kernel, WARP-PER-TILE shape (one-wave launches)
@@ -908,31 +864,23 @@ __global__ void __launch_bounds__(512, 2) step1w_kernel(const __grid_constant__ 
     // next launch start, so at most two consecutive launches are ever in flight and this grid cannot complete before its
     // predecessor has.  In concurrent mode the tile warps below never wait: the two launches step different batches.
     if (wid == p.tiles_per_cta) {
-        if (p.concurrent || p.pdl_early) {
-            asm volatile("griddepcontrol.wait;" ::: "memory");
-            asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
-        }
+        asm volatile("griddepcontrol.wait;" ::: "memory");
+        asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
         return;
     }
 
     const int8_t* gmap = p.map + e0 * p.cells;
     int32_t* ginv = p.inv + e0 * p.inv_stride;
-    uint64_t pol_first = 0;
-    if (p.cache_hints) pol_first = policy_evict_first();
+    const uint64_t pol_first = policy_evict_first();
     auto issue_loads = [&]() {
         if (lane == 0) {
             mbar_expect_tx(bar, in_bytes);
-            if (p.cache_hints & 1) {
-                bulk_g2s_hint(smap, gmap, (uint32_t)p.map_bytes, bar, pol_first);
-                bulk_g2s_hint(sinv, ginv, (uint32_t)p.inv_bytes, bar, pol_first);
-            } else {
-                bulk_g2s(smap, gmap, (uint32_t)p.map_bytes, bar);
-                bulk_g2s(sinv, ginv, (uint32_t)p.inv_bytes, bar);
-            }
+            bulk_g2s_hint(smap, gmap, (uint32_t)p.map_bytes, bar, pol_first);
+            bulk_g2s_hint(sinv, ginv, (uint32_t)p.inv_bytes, bar, pol_first);
         }
     };
     uchar4 ps = make_uchar4(0, 0, 0, 0);
-    const bool early = p.early_state && active && !(p.dbg_skip & 64);
+    const bool early = p.early_state && active;
     if (early) {                                                      // see step1_kernel: this handle's state is complete already
         issue_loads();
         ps = __ldcg(&p.pose[e]);   // L2 only: launches overlap, an SM's L1 is not a safe place for another grid's data
@@ -941,7 +889,7 @@ __global__ void __launch_bounds__(512, 2) step1w_kernel(const __grid_constant__ 
     zero_span(region_a + in_bytes + (uint32_t)lane * 16u, region_a + obs_tile);
     if (!p.concurrent) asm volatile("griddepcontrol.wait;" ::: "memory");   // previous kernel of the stream done + visible
     // (the gate warp has let the dependent launch start by now or will: it is co-resident — half an SM per launch)
-    if (!active || (p.dbg_skip & 64)) return;
+    if (!active) return;
     if (!early) {
         issue_loads();
         ps = __ldcg(&p.pose[e]);   // L2 only: launches overlap, an SM's L1 is not a safe place for another grid's data
@@ -954,7 +902,6 @@ __global__ void __launch_bounds__(512, 2) step1w_kernel(const __grid_constant__ 
     if (stepping && valid) action = __ldcg(&p.actions[e]);
 
     mbar_wait(bar, 0);
-    if (p.dbg_skip & 128) return;
 
     EnvRow env;
     env.m = smap + lane * p.cells;
@@ -981,7 +928,7 @@ __global__ void __launch_bounds__(512, 2) step1w_kernel(const __grid_constant__ 
                 counts |= 1u << 24;
                 atomicOr(&p.err[e], NGW_ERR_INVALID_ACTION);
             } else {
-                if (!(p.dbg_skip & 1)) step_env(env, cfg, a, o);
+                step_env(env, cfg, a, o);
                 int finished = o.done;
                 if (p.max_episode_steps > 0) {
                     int len = __ldcg(&p.ep_len[e]) + 1;
@@ -1003,10 +950,10 @@ __global__ void __launch_bounds__(512, 2) step1w_kernel(const __grid_constant__ 
             }
         }
         // ---- store 1: the inventory tile leaves as soon as the step is done
-        if (full_tile && !p.plain_store) {
+        if (full_tile) {
             fence_async_smem();
             __syncwarp();
-            if (lane == 0 && !(p.dbg_skip & 16)) { bulk_s2g(ginv, sinv, (uint32_t)p.inv_bytes); bulk_commit(); }
+            if (lane == 0) { bulk_s2g(ginv, sinv, (uint32_t)p.inv_bytes); bulk_commit(); }
         } else {
             __syncwarp();
             const uint4* s4 = reinterpret_cast<const uint4*>(sinv);
@@ -1020,7 +967,7 @@ __global__ void __launch_bounds__(512, 2) step1w_kernel(const __grid_constant__ 
         RegSink<NT> sink;
         sink.init(p.obs_u8);
         const bool look = valid && cfg.n_beams > 0;
-        if (look && !(p.dbg_skip & 2)) {
+        if (look) {
             LidarLuts luts;
             if (NC > 0) { luts.slot = sslot + cfg_i * NGW_MAX_ITEMS; luts.firstk = sfirstk; }
             else { luts.slot = p.dcfgs[cfg_i].c.lidar_slot; luts.firstk = p.dcfgs[cfg_i].lidar.firstk; }
@@ -1037,21 +984,14 @@ __global__ void __launch_bounds__(512, 2) step1w_kernel(const __grid_constant__ 
             sink.flush(region_a + (uint32_t)(lane * p.obs_srow), smem_u32(gbase + 16),
                        p.obs_u8 ? ((n_lidar + 3) & ~3) : 4 * n_lidar, cfg.n_inv_obs);
         }
-        if (full_tile && !p.plain_store) {
+        if (full_tile) {
             fence_async_smem();
             __syncwarp();
-            if (!(p.dbg_skip & 8)) {
-                unsigned char* gobs = p.obs + e0 * p.obs_row_bytes;
-                if (p.obs_srow == p.obs_row_bytes) {                  // the tile is one contiguous span on both sides
-                    if (lane == 0) {
-                        if (p.cache_hints & 2) bulk_s2g_hint(gobs, sobs, (uint32_t)p.obs_bytes, pol_first);
-                        else bulk_s2g(gobs, sobs, (uint32_t)p.obs_bytes);
-                    }
-                } else {                                              // padded rows in shared memory: lane l stores row l
-                    if (p.cache_hints & 2) bulk_s2g_hint(gobs + lane * p.obs_row_bytes, sobs + lane * p.obs_srow,
-                                                         (uint32_t)p.obs_row_bytes, pol_first);
-                    else bulk_s2g(gobs + lane * p.obs_row_bytes, sobs + lane * p.obs_srow, (uint32_t)p.obs_row_bytes);
-                }
+            unsigned char* gobs = p.obs + e0 * p.obs_row_bytes;
+            if (p.obs_srow == p.obs_row_bytes) {                      // the tile is one contiguous span on both sides
+                if (lane == 0) bulk_s2g_hint(gobs, sobs, (uint32_t)p.obs_bytes, pol_first);
+            } else {                                                  // padded rows in shared memory: lane l stores row l
+                bulk_s2g_hint(gobs + lane * p.obs_row_bytes, sobs + lane * p.obs_srow, (uint32_t)p.obs_row_bytes, pol_first);
             }
             bulk_commit();
         } else {
@@ -1066,7 +1006,7 @@ __global__ void __launch_bounds__(512, 2) step1w_kernel(const __grid_constant__ 
     }
 
     // ---- per-env outputs (lane = env: full lines) and episode statistics
-    if (stepping && !(p.dbg_skip & 4)) {
+    if (stepping) {
         if (valid) {
             p.pose[e] = ps;
             p.reward[e] = (float)o.reward;
@@ -1075,45 +1015,43 @@ __global__ void __launch_bounds__(512, 2) step1w_kernel(const __grid_constant__ 
             p.result[e] = (uint8_t)o.result;
             if (p.msg != nullptr) p.msg[e] = (uint16_t)o.msg;
         }
-        if (p.stats != nullptr) {
-            // warp reductions -> this warp's slot in shared memory; the last warp of the CTA to arrive folds the slots and
-            // issues one set of global atomics per CTA
-            const uint32_t c_all = __reduce_add_sync(0xFFFFFFFFu, counts);            // five counts <= 32: 6 bits apiece
-            const int r_sum = __reduce_add_sync(0xFFFFFFFFu, o.reward);
-            const float c_sum = warp_sum(o.cost);
-            int4* slots = reinterpret_cast<int4*>(smem + 64);
-            const int n_tiles_cta = min(p.tiles_per_cta, p.n_tiles - (int)blockIdx.x * p.tiles_per_cta);
-            int last = 0;
-            if (lane == 0) {
-                slots[wid] = make_int4((int)c_all, r_sum, __float_as_int(c_sum), 0);
-                __threadfence_block();
-                last = atomicAdd(&scta[0], 1) == n_tiles_cta - 1;
+        // warp reductions -> this warp's slot in shared memory; the last warp of the CTA to arrive folds the slots and
+        // issues one set of global atomics per CTA
+        const uint32_t c_all = __reduce_add_sync(0xFFFFFFFFu, counts);            // five counts <= 32: 6 bits apiece
+        const int r_sum = __reduce_add_sync(0xFFFFFFFFu, o.reward);
+        const float c_sum = warp_sum(o.cost);
+        int4* slots = reinterpret_cast<int4*>(smem + 64);
+        const int n_tiles_cta = min(p.tiles_per_cta, p.n_tiles - (int)blockIdx.x * p.tiles_per_cta);
+        int last = 0;
+        if (lane == 0) {
+            slots[wid] = make_int4((int)c_all, r_sum, __float_as_int(c_sum), 0);
+            __threadfence_block();
+            last = atomicAdd(&scta[0], 1) == n_tiles_cta - 1;
+        }
+        if (__shfl_sync(0xFFFFFFFFu, last, 0)) {
+            __threadfence_block();
+            int4 v = make_int4(0, 0, 0, 0);
+            if (lane < n_tiles_cta) {
+                const volatile int* sv = reinterpret_cast<const volatile int*>(&slots[lane]);
+                v.x = sv[0]; v.y = sv[1]; v.z = sv[2];
             }
-            if (__shfl_sync(0xFFFFFFFFu, last, 0)) {
-                __threadfence_block();
-                int4 v = make_int4(0, 0, 0, 0);
-                if (lane < n_tiles_cta) {
-                    const volatile int* sv = reinterpret_cast<const volatile int*>(&slots[lane]);
-                    v.x = sv[0]; v.y = sv[1]; v.z = sv[2];
-                }
-                // counts of up to 16 warps x 32 lanes need 10 bits: widen before the second reduction
-                const uint32_t lo = ((uint32_t)v.x & 63u) | ((((uint32_t)v.x >> 6) & 63u) << 10) | ((((uint32_t)v.x >> 12) & 63u) << 20);
-                const uint32_t hi = (((uint32_t)v.x >> 18) & 63u) | ((((uint32_t)v.x >> 24) & 63u) << 10);
-                const uint32_t a_tot = __reduce_add_sync(0xFFFFFFFFu, lo), b_tot = __reduce_add_sync(0xFFFFFFFFu, hi);
-                const int r_tot = __reduce_add_sync(0xFFFFFFFFu, v.y);
-                const float c_tot = warp_sum(__int_as_float(v.z));
-                if (lane == 0) {
-                    const int n_step = a_tot & 1023, n_done = (a_tot >> 10) & 1023, n_succ = (a_tot >> 20) & 1023;
-                    const int n_reset = b_tot & 1023, n_inv = (b_tot >> 10) & 1023;
-                    double* sg = p.stats + (size_t)(blockIdx.x % NGW_STAT_SLOTS) * NGW_STAT_COUNT;
-                    atomicAdd(&sg[NGW_STAT_STEPS], (double)(n_step - n_inv));
-                    atomicAdd(&sg[NGW_STAT_REWARD_SUM], (double)r_tot);
-                    atomicAdd(&sg[NGW_STAT_COST_SUM], (double)c_tot);
-                    if (n_done) atomicAdd(&sg[NGW_STAT_EPISODES], (double)n_done);
-                    if (n_succ) atomicAdd(&sg[NGW_STAT_SUCCESSES], (double)n_succ);
-                    if (n_reset) atomicAdd(&sg[NGW_STAT_RESETS], (double)n_reset);
-                    if (n_inv) atomicAdd(&sg[NGW_STAT_INVALID], (double)n_inv);
-                }
+            // counts of up to 16 warps x 32 lanes need 10 bits: widen before the second reduction
+            const uint32_t lo = ((uint32_t)v.x & 63u) | ((((uint32_t)v.x >> 6) & 63u) << 10) | ((((uint32_t)v.x >> 12) & 63u) << 20);
+            const uint32_t hi = (((uint32_t)v.x >> 18) & 63u) | ((((uint32_t)v.x >> 24) & 63u) << 10);
+            const uint32_t a_tot = __reduce_add_sync(0xFFFFFFFFu, lo), b_tot = __reduce_add_sync(0xFFFFFFFFu, hi);
+            const int r_tot = __reduce_add_sync(0xFFFFFFFFu, v.y);
+            const float c_tot = warp_sum(__int_as_float(v.z));
+            if (lane == 0) {
+                const int n_step = a_tot & 1023, n_done = (a_tot >> 10) & 1023, n_succ = (a_tot >> 20) & 1023;
+                const int n_reset = b_tot & 1023, n_inv = (b_tot >> 10) & 1023;
+                double* sg = p.stats + (size_t)(blockIdx.x % NGW_STAT_SLOTS) * NGW_STAT_COUNT;
+                atomicAdd(&sg[NGW_STAT_STEPS], (double)(n_step - n_inv));
+                atomicAdd(&sg[NGW_STAT_REWARD_SUM], (double)r_tot);
+                atomicAdd(&sg[NGW_STAT_COST_SUM], (double)c_tot);
+                if (n_done) atomicAdd(&sg[NGW_STAT_EPISODES], (double)n_done);
+                if (n_succ) atomicAdd(&sg[NGW_STAT_SUCCESSES], (double)n_succ);
+                if (n_reset) atomicAdd(&sg[NGW_STAT_RESETS], (double)n_reset);
+                if (n_inv) atomicAdd(&sg[NGW_STAT_INVALID], (double)n_inv);
             }
         }
     }
@@ -1377,30 +1315,27 @@ __global__ void __launch_bounds__(64, 14) rollout2_kernel(const __grid_constant_
         if (p.done_count != nullptr) p.done_count[e] = n_done;
         if (p.msg != nullptr) p.msg[e] = (uint16_t)o.msg;
     }
-    if (p.stats != nullptr) {
-        const int steps = (valid && low) ? p.n_steps - n_invalid : 0;
-        const int s_steps = __reduce_add_sync(0xFFFFFFFFu, steps), s_rew = __reduce_add_sync(0xFFFFFFFFu, reward_sum);
-        const int s_done = __reduce_add_sync(0xFFFFFFFFu, n_done), s_succ = __reduce_add_sync(0xFFFFFFFFu, n_succ);
-        const int s_reset = __reduce_add_sync(0xFFFFFFFFu, n_reset), s_inv = __reduce_add_sync(0xFFFFFFFFu, n_invalid);
-        const float s_cost = warp_sum(cost_sum);
-        if (lane == 0) {
-            double* sg = p.stats + (size_t)(blockIdx.x % NGW_STAT_SLOTS) * NGW_STAT_COUNT;
-            atomicAdd(&sg[NGW_STAT_STEPS], (double)s_steps);
-            atomicAdd(&sg[NGW_STAT_REWARD_SUM], (double)s_rew);
-            atomicAdd(&sg[NGW_STAT_COST_SUM], (double)s_cost);
-            if (s_done) atomicAdd(&sg[NGW_STAT_EPISODES], (double)s_done);
-            if (s_succ) atomicAdd(&sg[NGW_STAT_SUCCESSES], (double)s_succ);
-            if (s_reset) atomicAdd(&sg[NGW_STAT_RESETS], (double)s_reset);
-            if (s_inv) atomicAdd(&sg[NGW_STAT_INVALID], (double)s_inv);
-        }
+    const int steps = (valid && low) ? p.n_steps - n_invalid : 0;
+    const int s_steps = __reduce_add_sync(0xFFFFFFFFu, steps), s_rew = __reduce_add_sync(0xFFFFFFFFu, reward_sum);
+    const int s_done = __reduce_add_sync(0xFFFFFFFFu, n_done), s_succ = __reduce_add_sync(0xFFFFFFFFu, n_succ);
+    const int s_reset = __reduce_add_sync(0xFFFFFFFFu, n_reset), s_inv = __reduce_add_sync(0xFFFFFFFFu, n_invalid);
+    const float s_cost = warp_sum(cost_sum);
+    if (lane == 0) {
+        double* sg = p.stats + (size_t)(blockIdx.x % NGW_STAT_SLOTS) * NGW_STAT_COUNT;
+        atomicAdd(&sg[NGW_STAT_STEPS], (double)s_steps);
+        atomicAdd(&sg[NGW_STAT_REWARD_SUM], (double)s_rew);
+        atomicAdd(&sg[NGW_STAT_COST_SUM], (double)s_cost);
+        if (s_done) atomicAdd(&sg[NGW_STAT_EPISODES], (double)s_done);
+        if (s_succ) atomicAdd(&sg[NGW_STAT_SUCCESSES], (double)s_succ);
+        if (s_reset) atomicAdd(&sg[NGW_STAT_RESETS], (double)s_reset);
+        if (s_inv) atomicAdd(&sg[NGW_STAT_INVALID], (double)s_inv);
     }
 
     // ---- inventory tile out, final observation into the aliased region, observation tile out
     fence_async_smem();
     __syncthreads();                                                  // both warps are done stepping
     asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
-    const bool tma_store = full_tile && !p.plain_store;
-    if (tma_store) {
+    if (full_tile) {
         if (threadIdx.x == 0) { bulk_s2g(ginv, sinv, (uint32_t)p.inv_bytes); bulk_commit(); }
     } else {
         const uint4* s4 = reinterpret_cast<const uint4*>(sinv);
@@ -1437,13 +1372,11 @@ __global__ void __launch_bounds__(64, 14) rollout2_kernel(const __grid_constant_
                 for (int i = 0; i < NGW_REGSINK_TAIL; i++) if (i < n_tail) tl[i] = tail[i];
             }
         }
-        if (tma_store) {
+        if (full_tile) {
             fence_async_smem();
             __syncthreads();
             if (threadIdx.x == 0) {
-                unsigned char* gobs = p.obs + e0 * p.obs_row_bytes;
-                if (p.cache_hints & 2) bulk_s2g_hint(gobs, sobs, (uint32_t)p.obs_bytes, policy_evict_first());
-                else bulk_s2g(gobs, sobs, (uint32_t)p.obs_bytes);
+                bulk_s2g_hint(p.obs + e0 * p.obs_row_bytes, sobs, (uint32_t)p.obs_bytes, policy_evict_first());
                 bulk_commit();
             }
         } else {

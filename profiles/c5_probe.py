@@ -13,7 +13,7 @@ def run(kw, n=60):
     torch.cuda.synchronize(); e0=torch.cuda.Event(enable_timing=True); e1=torch.cuda.Event(enable_timing=True); e0.record()
     for i in range(n): hs[i%2].step(acts[i%4], **kw)
     e1.record(); torch.cuda.synchronize(); return e0.elapsed_time(e1)/n*1e3
-print('G', os.environ.get('NGW_WARPS'), 'no reset us/step', run({}), ' with staggered reset', end=' ')
+print('no reset us/step', run({}), ' with staggered reset', end=' ')
 for h in hs: h.ep_len.copy_(torch.randint(0,256,(envs,),device='cuda',dtype=torch.int32))
 print(run(dict(auto_reset=True, max_episode_steps=256)))
 # time of a full reset of the batch

@@ -1,5 +1,5 @@
-"""A/B sweep of the step kernel's tuning knobs (environment variables read by ngw_create) on the BASELINE workloads.
-    python profiles/sweep.py C2 "NGW_WARPS=1" "NGW_WARPS=2 NGW_TILES=2" ...     -> one JSON line per variant
+"""A/B sweep of environment settings read by ngw_create on the BASELINE workloads.
+    python profiles/sweep.py C2 "" "NGW_NO_CONCURRENT=1" ...     -> one JSON line per variant
 Timing = bench.py's: rotating batches (> L2), CUDA-graph replay on one stream, CUDA events, >= 40 ms per measurement."""
 import json
 import os
