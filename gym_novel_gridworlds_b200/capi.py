@@ -9,7 +9,7 @@ from . import opcodes as oc
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, 'csrc', 'libngw_b200.so')
 ABI_VERSION = 11
-OBS_I32, OBS_U8 = 0, 1
+OBS_I32, OBS_U8, OBS_HITS = 0, 1, 2
 
 
 class ActionEntryC(C.Structure):

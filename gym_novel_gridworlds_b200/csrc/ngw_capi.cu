@@ -237,13 +237,12 @@ int ngw_lidar_path(const ngw_config* cfg, int32_t map_size) {
     return build_lidar_tables(*cfg, map_size, ld, nullptr);
 }
 
-static int obs_row_bytes_of(const ngw_handle* h, int u8) {
+static int obs_row_bytes_of(const ngw_handle* h, int format) {
     int best = 0;
     for (const DevConfig& dc : h->h_cfgs) {
         const ngw_config& c = dc.c;
         if (c.n_beams <= 0) continue;
-        const int nl = c.n_lidar_items * c.n_beams;
-        const int b = u8 ? ((nl + 3) & ~3) + 4 * c.n_inv_obs : 4 * (nl + c.n_inv_obs);
+        const int b = obs_tail_offset(format, c.n_lidar_items, c.n_beams) + 4 * c.n_inv_obs;
         if (b > best) best = b;
     }
     return best;
@@ -322,8 +321,8 @@ static int create_init(ngw_handle* h, const ngw_config* cfgs, int32_t n_cfgs, in
     // bytes of one 32-env tile of each array
     h->map_bytes = 32 * h->cells;                       // multiple of 32
     h->inv_bytes = 128 * h->inv_stride;
-    h->obs_u8 = 0;
-    h->obs_row_bytes = obs_row_bytes_of(h, 0);
+    h->obs_format = NGW_OBS_I32;
+    h->obs_row_bytes = obs_row_bytes_of(h, NGW_OBS_I32);
     h->obs_bytes = 32 * h->obs_row_bytes;
     const int one_tile = NGW_SMEM_HDR + 512 + 1280 + h->map_bytes + h->inv_bytes + 128 * h->obs_dim;
     if (one_tile > 227 * 1024) return fail("ngw_create: map too large for shared memory");
@@ -363,19 +362,20 @@ int ngw_state(ngw_handle* h, ngw_state_view* o) {
     o->episode = h->episode; o->ep_len = h->ep_len; o->error_flags = h->err;
     o->inv_stride = h->inv_stride; o->obs_dim = h->obs_dim; o->n_envs = h->n; o->n_envs_padded = h->np;
     o->map_size = h->ms; o->n_configs = h->n_cfgs;
-    o->obs_format = h->obs_u8 ? NGW_OBS_U8 : NGW_OBS_I32; o->obs_row_bytes = h->obs_row_bytes;
+    o->obs_format = h->obs_format; o->obs_row_bytes = h->obs_row_bytes;
     return 0;
 }
 
 int ngw_set_obs_format(ngw_handle* h, int32_t format) {
     if (!h) return fail("null handle");
-    if (format != NGW_OBS_I32 && format != NGW_OBS_U8) return fail("ngw_set_obs_format: unknown format");
-    if (format == NGW_OBS_U8)
+    if (format != NGW_OBS_I32 && format != NGW_OBS_U8 && format != NGW_OBS_HITS)
+        return fail("ngw_set_obs_format: unknown format");
+    if (format != NGW_OBS_I32)                     // both narrow layouts store a range in one byte
         for (const DevConfig& dc : h->h_cfgs)
             if (dc.c.max_range > 255) return fail("ngw_set_obs_format: max_range does not fit a byte");
     if (h->host_dirty) { cudaStreamSynchronize(h->hs); h->host_dirty = false; }
-    h->obs_u8 = format == NGW_OBS_U8;
-    h->obs_row_bytes = obs_row_bytes_of(h, h->obs_u8);
+    h->obs_format = format;
+    h->obs_row_bytes = obs_row_bytes_of(h, format);
     h->obs_bytes = 32 * h->obs_row_bytes;
     return 0;
 }
@@ -431,7 +431,7 @@ static ResetParams reset_params(ngw_handle* h, const uint8_t* mask, int phase) {
     p.ep_len = h->ep_len; p.err = h->err; p.mask = mask; p.n_envs = h->n; p.first_gid = h->first_gid; p.seed = h->seed;
     p.ms = h->ms; p.cells = h->cells; p.inv_stride = h->inv_stride; p.phase = phase; p.zero_byte = h->zero_byte;
     p.reset_list = h->reset_list; p.reset_count = h->reset_ctl; p.done_ctas = h->reset_ctl + 1; p.obs = nullptr;
-    p.obs_dim = h->obs_dim; p.obs_row_bytes = h->obs_row_bytes; p.obs_u8 = h->obs_u8;
+    p.obs_dim = h->obs_dim; p.obs_row_bytes = h->obs_row_bytes; p.obs_format = h->obs_format;
     p.key_mask = h->key_mask;
     return p;
 }
@@ -478,7 +478,7 @@ static StepParams step_params(ngw_handle* h, const int32_t* actions, void* obs, 
     p.env_begin = begin; p.env_end = end; p.first_gid = h->first_gid; p.seed = h->seed;
     p.ms = h->ms; p.cells = h->cells; p.inv_stride = h->inv_stride; p.obs_dim = h->obs_dim;
     p.map_bytes = h->map_bytes; p.inv_bytes = h->inv_bytes; p.obs_bytes = h->obs_bytes;
-    p.obs_row_bytes = h->obs_row_bytes; p.obs_u8 = h->obs_u8;
+    p.obs_row_bytes = h->obs_row_bytes; p.obs_format = h->obs_format;
     p.auto_reset = auto_reset; p.max_episode_steps = max_episode_steps;
     p.lidar_uniform = h->lidar_uniform ? 1 : 0;
     p.msg = h->msg; p.reset_list = h->reset_list; p.reset_count = h->reset_ctl;
@@ -757,7 +757,8 @@ int ngw_rollout_policy(ngw_handle* h, const int32_t* weights, const int32_t* bia
     if (!weights || !bias || n_policy_actions < 1 || n_policy_actions > 16)
         return fail("ngw_rollout_policy: need weights, bias and 1..16 policy actions");
     if (h->obs_dim == 0 || !obs) return fail("ngw_rollout_policy: needs a LidarInFront observation (and an obs buffer)");
-    if (h->obs_u8) return fail("ngw_rollout_policy: the linear policy reads int32 observation rows (NGW_OBS_I32)");
+    if (h->obs_format != NGW_OBS_I32)
+        return fail("ngw_rollout_policy: the linear policy reads int32 observation rows (NGW_OBS_I32)");
     if (n_steps < 1) return fail("ngw_rollout_policy: n_steps must be >= 1");
     if (!reward_sum || !cost_sum || !last_done || !last_result) return fail("ngw_rollout_policy: null output pointer");
     if ((uintptr_t)obs & 15) return fail("ngw_rollout_policy: obs must be 16-byte aligned");

@@ -381,20 +381,30 @@ struct DevConfig {
     LidarDev lidar;
 };
 
-// One env's observation row: lidar part as int32 (the reference's vector) or as uint8 (NGW_OBS_U8: ranges are
-// <= max_range <= 90, so the narrowing is exact), followed by the int32 inventory tail at byte offset tail_off.
+// Byte offset of the int32 inventory tail in a row of layout `fmt` (NGW_OBS_*) for a config of L lidar items, B beams.
+__host__ __device__ __forceinline__ int obs_tail_offset(int fmt, int L, int B) {
+    return fmt == NGW_OBS_I32 ? 4 * L * B : fmt == NGW_OBS_U8 ? ((L * B + 3) & ~3) : ((2 * B + 3) & ~3);
+}
+
+// One env's observation row: lidar part as int32 (the reference's vector), as uint8 (NGW_OBS_U8: ranges are
+// <= max_range <= 90, so the narrowing is exact) or as one (item, range) byte pair per beam (NGW_OBS_HITS), followed by
+// the int32 inventory tail.  Sinks get a beam's hit as (beam, lidar slot): the hits row stores them apart, the vector
+// layouts at beam * L + slot.  Each beam owns its own entry, so warps / lanes sharing a row never touch the same bytes.
 struct ObsRow {
     unsigned char* p;
-    int u8;
-    __device__ __forceinline__ void put(int idx, int v) const {
-        if (u8) p[idx] = (unsigned char)v;
-        else reinterpret_cast<int32_t*>(p)[idx] = v;
+    int fmt;                            // NGW_OBS_I32 / NGW_OBS_U8 / NGW_OBS_HITS
+    __device__ __forceinline__ void put(int beam, int slot, int L, int v) const {
+        if (fmt == NGW_OBS_I32) reinterpret_cast<int32_t*>(p)[beam * L + slot] = v;
+        else if (fmt == NGW_OBS_U8) p[beam * L + slot] = (unsigned char)v;
+        else reinterpret_cast<uint16_t*>(p)[beam] = (uint16_t)((slot + 1) | (v << 8));
     }
-    __device__ __forceinline__ void put_beam(int, bool hit, int idx, int v) const { if (hit) put(idx, v); }
-    __device__ __forceinline__ int32_t* tail(int n_lidar) const {
-        return reinterpret_cast<int32_t*>(p + (u8 ? ((n_lidar + 3) & ~3) : 4 * n_lidar));
+    __device__ __forceinline__ void put_beam(int, bool hit, int beam, int slot, int L, int v) const {
+        if (hit) put(beam, slot, L, v);
     }
-    __device__ __forceinline__ void put_tail(int n_lidar, int i, int v) const { tail(n_lidar)[i] = v; }
+    __device__ __forceinline__ int32_t* tail(int L, int B) const {
+        return reinterpret_cast<int32_t*>(p + obs_tail_offset(fmt, L, B));
+    }
+    __device__ __forceinline__ void put_tail(int L, int B, int i, int v) const { tail(L, B)[i] = v; }
 };
 
 // Observation "sink" of the closed-loop rollout: instead of materialising the (sparse) observation row and scanning it,
@@ -409,13 +419,14 @@ struct PolicySink {
 #pragma unroll
         for (int a = 0; a < 16; a++) acc[a] = a < A ? bias[a] : 0;
     }
-    __device__ __forceinline__ void put(int idx, int v) {
+    __device__ __forceinline__ void add(int idx, int v) {               // obs[idx] = v
         const int32_t* row = w + idx * A;
 #pragma unroll
         for (int a = 0; a < 16; a++) if (a < A) acc[a] += v * row[a];
     }
-    __device__ __forceinline__ void put_beam(int, bool hit, int idx, int v) { if (hit) put(idx, v); }
-    __device__ __forceinline__ void put_tail(int n_lidar, int i, int v) { if (v != 0) put(n_lidar + i, v); }
+    __device__ __forceinline__ void put(int beam, int slot, int L, int v) { add(beam * L + slot, v); }
+    __device__ __forceinline__ void put_beam(int, bool hit, int beam, int slot, int L, int v) { if (hit) put(beam, slot, L, v); }
+    __device__ __forceinline__ void put_tail(int L, int B, int i, int v) { if (v != 0) add(L * B + i, v); }
     __device__ __forceinline__ int argmax(int n_valid) const {       // first maximum over the env's valid action ids
         int best = 0, best_v = acc[0];
 #pragma unroll
@@ -430,37 +441,42 @@ struct PolicySink {
 #define NGW_REGSINK_TAIL 16
 template <int NT>
 struct RegSink {
-    uint32_t hit[8];                    // per compass direction: (byte offset in the row << 8) | range, 0 = nothing seen
+    uint32_t hit[8];                    // per compass direction: (beam << 16) | (lidar slot << 8) | range, 0 = nothing seen
     int32_t tail[NT];
-    int sh;                             // log2 of the bytes per lidar entry (2: int32 rows, 0: NGW_OBS_U8 rows)
-    __device__ __forceinline__ void init(int u8) {
-        sh = u8 ? 0 : 2;
+    int sh;                             // log2 of the bytes per lidar entry (2: int32 rows, 0: NGW_OBS_U8, 1: NGW_OBS_HITS)
+    __device__ __forceinline__ void init(int fmt) {
+        sh = fmt == NGW_OBS_I32 ? 2 : fmt == NGW_OBS_U8 ? 0 : 1;
 #pragma unroll
         for (int a = 0; a < 8; a++) hit[a] = 0u;
 #pragma unroll
         for (int i = 0; i < NT; i++) tail[i] = 0;
     }
-    __device__ __forceinline__ void put_beam(int a, bool on, int idx, int v) {   // every position is written exactly once
-        const uint32_t packed = on ? (((uint32_t)idx << sh) << 8) | (uint32_t)v : 0u;
+    __device__ __forceinline__ void put_beam(int a, bool on, int beam, int slot, int L, int v) {   // every position is written exactly once
+        const uint32_t packed = on ? ((uint32_t)beam << 16) | ((uint32_t)slot << 8) | (uint32_t)v : 0u;   // (range >= 1)
 #pragma unroll
         for (int j = 0; j < 8; j++) if (j == a) hit[j] = packed;
     }
-    __device__ __forceinline__ void put_tail(int, int i, int v) {
+    __device__ __forceinline__ void put_tail(int, int, int i, int v) {
 #pragma unroll
         for (int j = 0; j < NT; j++) if (j == i) tail[j] = v;
     }
-    __device__ __forceinline__ void put(int, int) {}                 // (generic LUT walk: never taken with this sink)
+    __device__ __forceinline__ void put(int, int, int, int) {}       // (generic LUT walk: never taken with this sink)
     // row: the lane's (zeroed) observation row, dump: a scratch word, both as shared-memory addresses.  Branch-free: a
     // beam that saw nothing and a tail slot beyond n_tail store to the dump word instead.
-    __device__ __forceinline__ void flush(uint32_t row, uint32_t dump, int tail_off, int n_tail) const {
-        if (sh) {
+    // L: lidar items of the lane's config.
+    __device__ __forceinline__ void flush(uint32_t row, uint32_t dump, int L, int tail_off, int n_tail) const {
+        if (sh == 1) {                                                // (item, range) halfword at byte 2 * beam
 #pragma unroll
             for (int a = 0; a < 8; a++)
-                asm volatile("st.shared.b32 [%0], %1;" ::"r"(hit[a] ? row + (hit[a] >> 8) : dump), "r"(hit[a] & 0xFFu) : "memory");
+                asm volatile("st.shared.u16 [%0], %1;" ::"r"(hit[a] ? row + ((hit[a] >> 16) << 1) : dump),
+                             "r"(((hit[a] & 0xFFu) << 8) + ((hit[a] >> 8) & 0xFFu) + 1u) : "memory");
         } else {
 #pragma unroll
-            for (int a = 0; a < 8; a++)
-                asm volatile("st.shared.u8 [%0], %1;" ::"r"(hit[a] ? row + (hit[a] >> 8) : dump), "r"(hit[a]) : "memory");
+            for (int a = 0; a < 8; a++) {
+                const uint32_t off = ((hit[a] >> 16) * (uint32_t)L + ((hit[a] >> 8) & 0xFFu)) << sh;
+                if (sh == 2) asm volatile("st.shared.b32 [%0], %1;" ::"r"(hit[a] ? row + off : dump), "r"(hit[a] & 0xFFu) : "memory");
+                else asm volatile("st.shared.u8 [%0], %1;" ::"r"(hit[a] ? row + off : dump), "r"(hit[a]) : "memory");
+            }
         }
         const uint32_t t = row + (uint32_t)tail_off;
 #pragma unroll
@@ -557,7 +573,7 @@ __device__ __forceinline__ void line_beams(MaskT occ, int p, int stride, const i
         const int k = diagonal ? (int)luts.firstk[n - 1] : (n <= K ? n : 0);   // obsw:52-58: sample index of that cell, 0 = beyond max_beam_range
         const int id = here[side ? -n * stride : n * stride];
         const int slot = luts.slot[id];                               // -1: occludes but is not a lidar item (Q2)
-        obs.put_beam(a, slot >= 0 && n != 0 && k != 0, ((a - rot) & 7) * L + slot, k);
+        obs.put_beam(a, slot >= 0 && n != 0 && k != 0, (a - rot) & 7, slot, L, k);
     }
 }
 
@@ -640,7 +656,7 @@ __device__ __forceinline__ void lidar_fast(const EnvRow& e, const ngw_config& cf
 #pragma unroll
     for (int j = 0; j < NB; j++) {                                    // (sinks with positions: j-th beam of this warp's share)
         const int slot = hit[j] ? (int)cfg.lidar_slot[hit[j] & 0xFF] : -1;   // -1: occludes but is not a lidar item (Q2)
-        obs.put_beam(j, slot >= 0, (b0 + j) * L + slot, (int)(hit[j] >> 8));
+        obs.put_beam(j, slot >= 0, b0 + j, slot, L, (int)(hit[j] >> 8));
     }
 }
 
@@ -649,14 +665,14 @@ __device__ __forceinline__ void lidar_fast(const EnvRow& e, const ngw_config& cf
 // so without late-injected items the tail is an id range and the copy needs no table; NT bounds the unrolled copy.
 template <typename Sink, int NT = 16>
 __device__ __forceinline__ void obs_tail(const EnvRow& e, const ngw_config& cfg, Sink& obs, int tail_first) {
-    const int n_tail = cfg.n_inv_obs, n_lidar = cfg.n_lidar_items * cfg.n_beams;
+    const int n_tail = cfg.n_inv_obs, L = cfg.n_lidar_items, B = cfg.n_beams;
     if (tail_first >= 0 && n_tail <= NT) {
         const int32_t* src = e.inv + tail_first;
 #pragma unroll
-        for (int i = 0; i < NT; i++) if (i < n_tail) obs.put_tail(n_lidar, i, src[i]);
+        for (int i = 0; i < NT; i++) if (i < n_tail) obs.put_tail(L, B, i, src[i]);
         return;
     }
-    for (int i = 0; i < n_tail; i++) obs.put_tail(n_lidar, i, e.inv[cfg.inv_obs_item[i]]);
+    for (int i = 0; i < n_tail; i++) obs.put_tail(L, B, i, e.inv[cfg.inv_obs_item[i]]);
 }
 
 // `tables`: the beam tables to walk with — the env's own config, or (mixed batches whose configs all share one lidar
@@ -690,7 +706,7 @@ __device__ __forceinline__ void lidar_observe(const EnvRow& e, const DevConfig& 
                 int id = e.m[idx];
                 if (id != 0) {
                     int slot = cfg.lidar_slot[id];
-                    if (slot >= 0) obs.put(b * L + slot, k + 1);
+                    if (slot >= 0) obs.put(b, slot, L, k + 1);
                     break;
                 }
             }

@@ -19,7 +19,7 @@ struct ngw_handle {
     unsigned long long seed = 0;
     int ms = 0, cells = 0, inv_stride = 0, obs_dim = 0, n_cfgs = 0;
     int map_bytes = 0, inv_bytes = 0, obs_bytes = 0, warps = 2, lidar_mode = 0;
-    int obs_u8 = 0, obs_row_bytes = 0;             // observation row layout (ngw_set_obs_format)
+    int obs_format = NGW_OBS_I32, obs_row_bytes = 0;   // observation row layout (ngw_set_obs_format)
     uint32_t key_mask = 0xFFFFFFFFu;
     bool lidar_uniform = false;
     bool concurrent = true;                        // independent consecutive launches may overlap (NGW_NO_CONCURRENT)

@@ -25,7 +25,7 @@ struct ResetParams {
     int32_t* reset_count;
     int32_t* done_ctas;
     unsigned char* obs;         // observation rows of obs_row_bytes bytes (layout as in the step kernel)
-    int obs_dim, obs_row_bytes, obs_u8;
+    int obs_dim, obs_row_bytes, obs_format;
     uint32_t key_mask;          // 0xFFFFFFFF; test knob NGW_DEBUG_KEY_MASK forces ties between the subset-sampling keys
 };
 
@@ -126,7 +126,7 @@ __global__ void __launch_bounds__(32 * NGW_RESET_WARPS) reset_list_kernel(const 
         if (p.obs != nullptr) {                                       // observation of the new episode replaces the row
             ObsRow orow;
             orow.p = p.obs + e * p.obs_row_bytes;
-            orow.u8 = p.obs_u8;
+            orow.fmt = p.obs_format;
             uint32_t* row = reinterpret_cast<uint32_t*>(orow.p);
             for (int k = lane; k < (p.obs_row_bytes >> 2); k += 32) row[k] = 0;
             if (lane == 0) sc.hist[0] = 0;                                // a shared-memory byte that reads 0
@@ -178,7 +178,7 @@ __global__ void observe_masked_kernel(const ResetParams p) {
     env.r = ps.x; env.c = ps.y; env.facing = ps.z; env.sel = ps.w;
     ObsRow orow;
     orow.p = p.obs + e * p.obs_row_bytes;
-    orow.u8 = p.obs_u8;
+    orow.fmt = p.obs_format;
     uint32_t* row = reinterpret_cast<uint32_t*>(orow.p);
     for (int i = 0; i < (p.obs_row_bytes >> 2); i++) row[i] = 0;
     LidarLuts luts;

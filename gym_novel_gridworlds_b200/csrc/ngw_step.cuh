@@ -92,7 +92,7 @@ struct StepParams {
     int32_t* ep_len;
     uint32_t* err;
     const int32_t* actions;     // nullptr => observe only (no step, no outputs but obs)
-    unsigned char* obs;         // nullptr => no observation; rows of obs_row_bytes bytes (int32 or uint8 lidar part)
+    unsigned char* obs;         // nullptr => no observation; rows of obs_row_bytes bytes (layout obs_format)
     float* reward;
     uint8_t* done;
     float* cost;
@@ -103,7 +103,7 @@ struct StepParams {
     unsigned long long seed;
     int ms, cells, inv_stride, obs_dim;
     int map_bytes, inv_bytes, obs_bytes;                 // bytes of one 32-env tile of each array
-    int obs_row_bytes, obs_u8;                           // observation row layout (NGW_OBS_I32 / NGW_OBS_U8)
+    int obs_row_bytes, obs_format;                       // observation row layout (NGW_OBS_I32 / NGW_OBS_U8 / NGW_OBS_HITS)
     int obs_srow;               // one-step kernel: row stride of the observation tile in SHARED memory: obs_row_bytes, or
                                 // 16 bytes more when the row is a multiple of 8 words (64-word rows would put every
                                 // lane's row on the same bank: C4 / C5 measured 64-71 % of their shared wavefronts as conflicts)
@@ -290,7 +290,7 @@ __global__ void __launch_bounds__(256) rollout_kernel(const __grid_constant__ St
     }
     ObsRow orow;
     orow.p = sobs + lane * p.obs_row_bytes;
-    orow.u8 = p.obs_u8;
+    orow.fmt = p.obs_format;
     uchar4 ps = make_uchar4(0, 0, 0, 0);
     int action = 0;
     const bool given_actions = !(p.random_policy || closed_loop);     // else `actions` is only a non-null marker
@@ -341,7 +341,7 @@ __global__ void __launch_bounds__(256) rollout_kernel(const __grid_constant__ St
                     const int D = cfg.n_lidar_items * cfg.n_beams + cfg.n_inv_obs;
                     for (int j = 0; j < D; j++) {
                         const int v = row[j];
-                        if (v != 0) sink.put(j, v);                    // the observation is sparse (<= 8 hits + inventory)
+                        if (v != 0) sink.add(j, v);                    // the observation is sparse (<= 8 hits + inventory)
                     }
                     action = sink.argmax(n_valid);
                 }
@@ -656,7 +656,7 @@ __global__ void __launch_bounds__(512) step1_kernel(const __grid_constant__ Step
     if (kAlias) {
         if (p.obs != nullptr) {
             RegSink<NGW_REGSINK_TAIL> sink;
-            sink.init(p.obs_u8);
+            sink.init(p.obs_format);
             const bool look = valid && cfg.n_beams > 0;
             if (look) {
                 LidarLuts luts;
@@ -675,16 +675,15 @@ __global__ void __launch_bounds__(512) step1_kernel(const __grid_constant__ Step
             }
             group_sync<kOne>(grp, G);
             if (look) {
-                const int n_lidar = cfg.n_lidar_items * cfg.n_beams;
-                sink.flush(smem_u32(sobs) + (uint32_t)(lane * p.obs_srow), smem_u32(gbase + 16),
-                       p.obs_u8 ? ((n_lidar + 3) & ~3) : 4 * n_lidar, g == G - 1 ? cfg.n_inv_obs : 0);
+                sink.flush(smem_u32(sobs) + (uint32_t)(lane * p.obs_srow), smem_u32(gbase + 16), cfg.n_lidar_items,
+                           obs_tail_offset(p.obs_format, cfg.n_lidar_items, cfg.n_beams), g == G - 1 ? cfg.n_inv_obs : 0);
             }
         }
     } else
     if (p.obs != nullptr && valid && cfg.n_beams > 0) {
         ObsRow orow;
         orow.p = sobs + lane * p.obs_srow;
-        orow.u8 = p.obs_u8;
+        orow.fmt = p.obs_format;
         LidarLuts luts;
         if (NC > 0) { luts.slot = sslot + cfg_i * NGW_MAX_ITEMS; luts.firstk = sfirstk; }
         else { luts.slot = p.dcfgs[cfg_i].c.lidar_slot; luts.firstk = p.dcfgs[cfg_i].lidar.firstk; }
@@ -965,7 +964,7 @@ __global__ void __launch_bounds__(512, 2) step1w_kernel(const __grid_constant__ 
     // ---- LidarInFront of the new state, into registers
     if (p.obs != nullptr) {
         RegSink<NT> sink;
-        sink.init(p.obs_u8);
+        sink.init(p.obs_format);
         const bool look = valid && cfg.n_beams > 0;
         if (look) {
             LidarLuts luts;
@@ -980,9 +979,8 @@ __global__ void __launch_bounds__(512, 2) step1w_kernel(const __grid_constant__ 
         zero_span(region_a + (uint32_t)lane * 16u, region_a + (in_bytes < obs_tile ? in_bytes : obs_tile));
         __syncwarp();
         if (look) {
-            const int n_lidar = cfg.n_lidar_items * cfg.n_beams;
-            sink.flush(region_a + (uint32_t)(lane * p.obs_srow), smem_u32(gbase + 16),
-                       p.obs_u8 ? ((n_lidar + 3) & ~3) : 4 * n_lidar, cfg.n_inv_obs);
+            sink.flush(region_a + (uint32_t)(lane * p.obs_srow), smem_u32(gbase + 16), cfg.n_lidar_items,
+                       obs_tail_offset(p.obs_format, cfg.n_lidar_items, cfg.n_beams), cfg.n_inv_obs);
         }
         if (full_tile) {
             fence_async_smem();
@@ -1093,7 +1091,9 @@ __device__ __forceinline__ uint32_t pair_gather(const PairLine& ln, int ms_rt) {
     return occ & ln.mask;
 }
 
-// the two beams of one line -> (observation index << 8) | range, 0 = nothing reported
+// the two beams of one line -> (observation index << 8) | range (the policy's dot product), or with kSplit
+// (beam << 16) | (lidar slot << 8) | range (observation rows of any layout); 0 = nothing reported
+template <bool kSplit>
 __device__ __forceinline__ void pair_beams(uint32_t occ, const PairLine& ln, const int8_t* here, bool diagonal, int K, int L,
                                            int rot, const LidarLuts& luts, uint32_t& hit_pos, uint32_t& hit_neg) {
     const int p = ln.pos;
@@ -1109,13 +1109,14 @@ __device__ __forceinline__ void pair_beams(uint32_t occ, const PairLine& ln, con
         const int k = diagonal ? kd : (n <= K ? n : 0);
         const int id = here[side ? -n * ln.stride : n * ln.stride];
         const int slot = luts.slot[id];                               // -1: occludes but is not a lidar item (Q2)
-        const uint32_t h = (slot >= 0 && n != 0 && k != 0) ? ((uint32_t)(((a - rot) & 7) * L + slot) << 8) | (uint32_t)k : 0u;
+        const uint32_t at = kSplit ? ((uint32_t)((a - rot) & 7) << 8) | (uint32_t)slot : (uint32_t)(((a - rot) & 7) * L + slot);
+        const uint32_t h = (slot >= 0 && n != 0 && k != 0) ? (at << 8) | (uint32_t)k : 0u;
         if (side) hit_neg = h; else hit_pos = h;
     }
 }
 
-// the four hits of this lane's two lines (half 0: row, column; half 1: diagonal, anti-diagonal)
-template <int MS>
+// the four hits of this lane's two lines (half 0: row, column; half 1: diagonal, anti-diagonal), packed as pair_beams<kSplit>
+template <int MS, bool kSplit>
 __device__ __forceinline__ void pair_lidar(const EnvRow& e, const ngw_config& cfg, const LidarDev& t, const LidarLuts& luts,
                                            int half, uint32_t hit[4]) {
     const int ms = MS > 0 ? MS : e.ms;
@@ -1133,8 +1134,8 @@ __device__ __forceinline__ void pair_lidar(const EnvRow& e, const ngw_config& cf
     const int K = cfg.max_range, L = cfg.n_lidar_items;
     const int rot = (int)((*reinterpret_cast<const uint32_t*>(t.rot) >> (8 * e.facing)) & 7u);
     const int8_t* here = e.m + r * ms + c;
-    pair_beams(o1, l1, here, half != 0, K, L, rot, luts, hit[0], hit[1]);
-    pair_beams(o2, l2, here, half != 0, K, L, rot, luts, hit[2], hit[3]);
+    pair_beams<kSplit>(o1, l1, here, half != 0, K, L, rot, luts, hit[0], hit[1]);
+    pair_beams<kSplit>(o2, l2, here, half != 0, K, L, rot, luts, hit[2], hit[3]);
 }
 
 // score[a] += v * W[idx][a], a < 4 * A4; W rows are 16 * A4 bytes in shared memory
@@ -1238,8 +1239,8 @@ __global__ void __launch_bounds__(64, 14) rollout2_kernel(const __grid_constant_
             for (int a = 0; a < 16; a++) acc[a] = (a < 4 * A4 && low) ? spol[a] : 0;
             if (cfg.n_beams > 0) {
                 uint32_t hit[4];
-                if (p.ms == 10) pair_lidar<10>(env, cfg, geom, luts, half, hit);
-                else pair_lidar<0>(env, cfg, geom, luts, half, hit);
+                if (p.ms == 10) pair_lidar<10, false>(env, cfg, geom, luts, half, hit);
+                else pair_lidar<0, false>(env, cfg, geom, luts, half, hit);
 #pragma unroll
                 for (int j = 0; j < 4; j++)
                     if (hit[j]) policy_mac<A4>(acc, spol + 16, (int)(hit[j] >> 8), (int)(hit[j] & 0xFFu));
@@ -1348,8 +1349,8 @@ __global__ void __launch_bounds__(64, 14) rollout2_kernel(const __grid_constant_
         const bool look = valid && cfg.n_beams > 0;
         const int n_tail = cfg.n_inv_obs, tf = dc.lidar.tail_first;
         if (look) {
-            if (p.ms == 10) pair_lidar<10>(env, cfg, geom, luts, half, hit);
-            else pair_lidar<0>(env, cfg, geom, luts, half, hit);
+            if (p.ms == 10) pair_lidar<10, true>(env, cfg, geom, luts, half, hit);
+            else pair_lidar<0, true>(env, cfg, geom, luts, half, hit);
 #pragma unroll
             for (int i = 0; i < NGW_REGSINK_TAIL; i++)
                 tail[i] = i < n_tail ? env.inv[tf >= 0 ? tf + i : (int)cfg.inv_obs_item[i]] : 0;
@@ -1363,11 +1364,12 @@ __global__ void __launch_bounds__(64, 14) rollout2_kernel(const __grid_constant_
         if (look) {
             ObsRow orow;
             orow.p = sobs + el * p.obs_row_bytes;
-            orow.u8 = p.obs_u8;
+            orow.fmt = p.obs_format;
 #pragma unroll
-            for (int j = 0; j < 4; j++) if (hit[j]) orow.put((int)(hit[j] >> 8), (int)(hit[j] & 0xFFu));
+            for (int j = 0; j < 4; j++)
+                if (hit[j]) orow.put((int)(hit[j] >> 16), (int)((hit[j] >> 8) & 0xFFu), cfg.n_lidar_items, (int)(hit[j] & 0xFFu));
             if (low) {
-                int32_t* tl = orow.tail(n_lidar);
+                int32_t* tl = orow.tail(cfg.n_lidar_items, cfg.n_beams);
 #pragma unroll
                 for (int i = 0; i < NGW_REGSINK_TAIL; i++) if (i < n_tail) tl[i] = tail[i];
             }

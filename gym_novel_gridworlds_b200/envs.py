@@ -44,7 +44,8 @@ class NovelGridworldBatchEnv(Env):
         self.messages = bool(messages)
         # strict_actions: a batched step raises like the reference (wrappers.py:76, pogostick_v1_env.py:236) when any env
         # was given an id its chain rejects — one device-to-host read per step; off, the step is a no-op for that env,
-        # info['invalid'] marks it and the sticky error flag / NGW_STAT_INVALID count it.  obs_format: 'i32' | 'u8' rows.
+        # info['invalid'] marks it and the sticky error flag / NGW_STAT_INVALID count it.  obs_format: 'i32' | 'u8' | 'hits'
+        # rows (runtime.obs_to_vector turns the narrow ones back into the reference's vector).
         self.strict_actions = bool(strict_actions)
         self.obs_format = obs_format
 

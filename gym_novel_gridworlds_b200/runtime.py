@@ -30,6 +30,76 @@ def _ptr(t):
     return None if t is None else C.c_void_p(t.data_ptr())
 
 
+_OBS_FORMATS = {'i32': capi.OBS_I32, 'u8': capi.OBS_U8, 'hits': capi.OBS_HITS}
+
+
+def _tail_offset(c, obs_format):
+    """Byte offset of the int32 inventory tail in a narrow row of config `c` (include/ngw.h, NGW_OBS_U8 / NGW_OBS_HITS)."""
+    n = c.n_lidar_items * c.n_beams if obs_format == 'u8' else 2 * c.n_beams
+    return (n + 3) & ~3
+
+
+def _split_rows(rows, c, obs_format):
+    nl, ni = c.n_lidar_items * c.n_beams, c.n_inv_obs
+    if obs_format == 'i32':
+        return rows[:, :nl], rows[:, nl:nl + ni]
+    off = _tail_offset(c, obs_format)
+    tail = rows[:, off:off + 4 * ni]
+    tail = tail.view(torch.int32) if isinstance(tail, torch.Tensor) else tail.view(np.int32)
+    if obs_format == 'u8':
+        return rows[:, :nl], tail
+    return rows[:, :2 * c.n_beams].reshape(rows.shape[0], c.n_beams, 2), tail
+
+
+def _rows_to_vector(rows, c, obs_format, width):
+    """int32 [n, width] vector of config `c` from rows (torch) laid out for that config.  Only bounded index arithmetic:
+    rows of another config (mixed batches, discarded by the caller) decode to garbage but never index out of range."""
+    n, L, B = rows.shape[0], c.n_lidar_items, c.n_beams
+    lidar, tail = _split_rows(rows, c, obs_format)
+    out = torch.zeros((n, width), dtype=torch.int32, device=rows.device)
+    if obs_format == 'hits':
+        item = lidar[:, :, 0].to(torch.int64)
+        rng = torch.where((item > 0) & (item <= L), lidar[:, :, 1].to(torch.int32), 0)
+        vec = torch.zeros((n, B, L), dtype=torch.int32, device=rows.device)
+        vec.scatter_(2, (item - 1).clamp(0, L - 1).unsqueeze(2), rng.unsqueeze(2))
+        out[:, :L * B] = vec.view(n, L * B)
+    else:
+        out[:, :L * B] = lidar.to(torch.int32)
+    out[:, L * B:L * B + c.n_inv_obs] = tail
+    return out
+
+
+def obs_to_vector(rows, compiled, obs_format, cfg_ids=None):
+    """The reference's observation vector (observation_wrappers.py:70-80), int32 [n, obs_dim], from observation rows
+    of any layout ('i32', 'u8', 'hits'; include/ngw.h).  obs_dim is the widest config's; an env's entries beyond its own
+    config's L*B + I_obs are 0, as in an 'i32' row.  `compiled`: the batch's compiled chain(s); `cfg_ids` [n]: each
+    row's config index (None = config 0).  A CUDA tensor is decoded with torch ops only (no host synchronisation, so
+    the call can be captured in a CUDA graph) and gives a tensor; a numpy array gives a numpy array.  Needs no library."""
+    compiled = list(compiled) if isinstance(compiled, (list, tuple)) else [compiled]
+    if obs_format not in _OBS_FORMATS:
+        raise ValueError("unknown obs_format %r" % (obs_format,))
+    as_numpy = not isinstance(rows, torch.Tensor)
+    if as_numpy:
+        rows = np.ascontiguousarray(rows)
+        rows = torch.from_numpy(rows if rows.flags.writeable else rows.copy())
+        if cfg_ids is not None:
+            cfg_ids = torch.from_numpy(np.asarray(cfg_ids, dtype=np.int64))
+    width = max([cc.c.n_lidar_items * cc.c.n_beams + cc.c.n_inv_obs for cc in compiled if cc.c.n_beams > 0] or [0])
+    if obs_format == 'i32':
+        out = rows[:, :width].to(torch.int32).clone()
+    else:
+        out = torch.zeros((rows.shape[0], width), dtype=torch.int32, device=rows.device)
+        for k, cc in enumerate(compiled):
+            if cc.c.n_beams <= 0:
+                continue
+            vec = _rows_to_vector(rows, cc.c, obs_format, width)
+            if cfg_ids is None:
+                out = vec
+                break
+            out = torch.where((cfg_ids.to(rows.device) == k).unsqueeze(1), vec, out)
+    return out.numpy() if as_numpy else out
+
+
 class BatchHandle(object):
     def __init__(self, compiled, n_envs, device=None, seed=0, first_env_gid=0, cfg_id=None, obs_format='i32'):
         if not torch.cuda.is_available():
@@ -49,11 +119,12 @@ class BatchHandle(object):
         self._h = C.c_void_p()
         capi.check(self.lib, self.lib.ngw_create(C.byref(self._h), cfgs, len(self.compiled), self.n, self.map_size,
                                                  self.device.index, int(first_env_gid), int(seed) & (2 ** 64 - 1)))
-        if obs_format not in ('i32', 'u8'):
-            raise ValueError("obs_format must be 'i32' (the reference's vector as int32) or 'u8' (uint8 lidar ranges)")
+        if obs_format not in _OBS_FORMATS:
+            raise ValueError("obs_format must be 'i32' (the reference's vector as int32), 'u8' (uint8 lidar ranges) or "
+                             "'hits' (one (item, range) byte pair per beam)")
         self.obs_format = obs_format
-        if obs_format == 'u8':
-            capi.check(self.lib, self.lib.ngw_set_obs_format(self._h, capi.OBS_U8))
+        if obs_format != 'i32':
+            capi.check(self.lib, self.lib.ngw_set_obs_format(self._h, _OBS_FORMATS[obs_format]))
         sv = StateViewC()
         capi.check(self.lib, self.lib.ngw_state(self._h, C.byref(sv)))
         self.inv_stride, self.obs_dim, self.n_padded = sv.inv_stride, sv.obs_dim, sv.n_envs_padded
@@ -73,7 +144,7 @@ class BatchHandle(object):
         self.error_flags = view(sv.error_flags, (self.n_padded,), '<i4')[:self.n]
         with torch.cuda.device(self.device):
             d = max(self.obs_dim, 1)
-            if obs_format == 'u8':       # rows: uint8 lidar ranges | pad to 4 | int32 inventory tail (see split_obs)
+            if obs_format != 'i32':      # rows: uint8 lidar ranges or hits | pad to 4 | int32 inventory tail (see split_obs)
                 self.obs = torch.zeros((self.n, max(self.obs_row_bytes, 4)), dtype=torch.uint8, device=self.device)
             else:
                 self.obs = torch.zeros((self.n, d), dtype=torch.int32, device=self.device)
@@ -143,16 +214,19 @@ class BatchHandle(object):
         return m.view(count, self.map_size, self.map_size), p, v
 
     def split_obs(self, obs, cfg=0):
-        """(lidar ranges [n, L*B], inventory tail [n, I_obs]) views of an observation buffer of this handle's format
-        (torch tensor or numpy array) for config `cfg` — the two halves of observation_wrappers.py:70-80."""
-        c = self.compiled[cfg].c
-        nl, ni = c.n_lidar_items * c.n_beams, c.n_inv_obs
-        if self.obs_format == 'i32':
-            return obs[:, :nl], obs[:, nl:nl + ni]
-        off = (nl + 3) & ~3
-        tail = obs[:, off:off + 4 * ni]
-        tail = tail.view(torch.int32) if isinstance(tail, torch.Tensor) else tail.view(np.int32)
-        return obs[:, :nl], tail
+        """(lidar part, inventory tail int32 [n, I_obs]) views of an observation buffer of this handle's format (torch
+        tensor or numpy array) for config `cfg` — the two halves of observation_wrappers.py:70-80.  The lidar part is the
+        ranges [n, L*B] ('i32', 'u8') or the (item, range) pairs uint8 [n, B, 2] ('hits')."""
+        return _split_rows(obs, self.compiled[cfg].c, self.obs_format)
+
+    def obs_vector(self, rows=None):
+        """The reference's int32 vector [n, obs_dim] of observation rows of this handle (default: self.obs); see
+        obs_to_vector."""
+        rows = self.obs if rows is None else rows
+        cfg_ids = None
+        if len(self.compiled) > 1:
+            cfg_ids = self.cfg_id if isinstance(rows, torch.Tensor) else self.cfg_id.cpu().numpy()
+        return obs_to_vector(rows, self.compiled, self.obs_format, cfg_ids)
 
     def reset(self, mask=None, want_obs=True):
         mk = None
@@ -209,7 +283,7 @@ class BatchHandle(object):
     def capture_policy_rollout(self, policy, n_steps, auto_reset=False, max_episode_steps=0):
         """SURVEY §8f N1, general policy hook: ONE CUDA graph of n_steps x [actions = policy(obs); ngw_step(actions)].
         `policy` is any callable made of torch ops on the current stream mapping the handle's observation tensor
-        (int32 [n, obs_dim], or uint8 rows with obs_format='u8') to an int32 action tensor [n]; observations and actions
+        (int32 [n, obs_dim], or uint8 rows with obs_format 'u8' / 'hits') to an int32 action tensor [n]; observations and actions
         never leave the device and the host is out of the loop (tests/train.py:122-135 is the use case).  Returns
         (graph, record): `graph.replay()` advances every env by n_steps; `record` holds the tensors the graph fills
         (actions [n_steps, n], reward_sum, cost_sum, done_count, and the handle's obs/reward/done/... of the last step)."""
@@ -256,14 +330,14 @@ class BatchHandle(object):
             n = self.n
             # ONE pinned block mirroring the library's device staging (observation rows | pad to 16 | reward | step_cost |
             # done | result): ngw_step_host then brings a whole step back with a single device-to-host copy
-            row = max(self.obs_row_bytes, 4) if self.obs_format == 'u8' else 4 * d
+            row = max(self.obs_row_bytes, 4) if self.obs_format != 'i32' else 4 * d
             obs_bytes = n * row if self.obs_dim else 0
             off = (obs_bytes + 15) & ~15
             block = torch.zeros(off + 10 * n + 64, dtype=torch.uint8).pin_memory()
             small = block[off:off + 10 * n]
             if self.obs_dim == 0:
                 host_obs = torch.zeros((n, 1), dtype=torch.int32)
-            elif self.obs_format == 'u8':
+            elif self.obs_format != 'i32':
                 host_obs = block[:obs_bytes].view(n, row)
             else:
                 host_obs = block[:obs_bytes].view(torch.int32).view(n, d)
@@ -477,7 +551,7 @@ class ChainRuntime(object):
 
     def lidar_observation(self):
         obs = self.handle.observe()
-        if self.handle.obs_format != 'u8':
+        if self.handle.obs_format == 'i32':
             obs = obs[:, :self.compiled.obs_dim]
         return obs[0].cpu().numpy().astype(np.int64) if self.single else obs
 
@@ -557,7 +631,7 @@ class ChainRuntime(object):
             b.map, b.agent_location, b.agent_facing_id = h.map, h.pose[:, 0:2], h.pose[:, 2]
             b.inventory_items_quantity = {n: h.inventory[:, i] for i, n in enumerate(cc.item_names) if n in b.items}
         if cc.reset_returns == 'lidar':
-            o = obs if h.obs_format == 'u8' else obs[:, :cc.obs_dim]
+            o = obs if h.obs_format != 'i32' else obs[:, :cc.obs_dim]
             return o[0].cpu().numpy().astype(np.int64) if self.single else o
         return self.dict_observation()
 
@@ -592,7 +666,7 @@ class ChainRuntime(object):
                     'message': decode_message(h.msg[0].item(), cc)}
             o = (obs[0, :cc.obs_dim].cpu().numpy().astype(np.int64) if cc.obs_dim else self.dict_observation())
             return o, b.last_reward, b.last_done, info
-        lidar_cols = slice(None) if h.obs_format == 'u8' else slice(0, cc.obs_dim)     # u8 rows: see BatchHandle.split_obs
+        lidar_cols = slice(None) if h.obs_format != 'i32' else slice(0, cc.obs_dim)    # narrow rows: see BatchHandle.split_obs
         if isinstance(action, torch.Tensor) and action.is_cuda:
             obs, reward, done, cost, result = h.step(action, self.auto_reset, self.max_episode_steps)
             self._check_actions(action)

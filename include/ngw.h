@@ -200,13 +200,20 @@ enum ngw_msg {
 enum { NGW_STAT_STEPS = 0, NGW_STAT_EPISODES = 1, NGW_STAT_SUCCESSES = 2, NGW_STAT_REWARD_SUM = 3,
        NGW_STAT_COST_SUM = 4, NGW_STAT_RESETS = 5, NGW_STAT_INVALID = 6, NGW_STAT_RESERVED = 7, NGW_STAT_COUNT = 8 };
 
-/* Observation row layouts (ngw_set_obs_format).  Both carry the reference's vector (observation_wrappers.py:70-80):
+/* Observation row layouts (ngw_set_obs_format).  All three carry the reference's vector (observation_wrappers.py:70-80):
  * L*B lidar ranges (beam-major, L lidar items per beam) followed by the I_obs inventory quantities.
  *   NGW_OBS_I32 (default): int32 [L*B + I_obs]                         row = 4 * obs_dim bytes
  *   NGW_OBS_U8           : uint8 [L*B], zero padding to a multiple of 4, int32 [I_obs]
  *                          (a range is <= max_beam_range <= 90, so the byte is exact; inventory counts are unbounded
- *                          (quirk Q8) and stay int32).  C2: 56 + 28 = 84 bytes instead of 252. */
-enum { NGW_OBS_I32 = 0, NGW_OBS_U8 = 1 };
+ *                          (quirk Q8) and stay int32).  C2: 56 + 28 = 84 bytes instead of 252.
+ *   NGW_OBS_HITS         : uint8 [B][2], zero padding to a multiple of 4, int32 [I_obs]
+ *                          A beam stops at the first non-air cell, so it has at most one nonzero entry among its L.  Pair b
+ *                          (beam order of the vector's beam-major blocks) is (item, range): item = the reference's
+ *                          lidar_items_id value 1..L (lidar slot + 1), range = the 1-based sample index the vector holds;
+ *                          (0, 0) when the beam reports nothing.  vec[b*L + item - 1] = range wherever item != 0.
+ *                          C2: 16 + 28 = 44 bytes.
+ * Row bytes are the maximum over the batch's configs; each env's row is laid out with its own config's L, B and I_obs. */
+enum { NGW_OBS_I32 = 0, NGW_OBS_U8 = 1, NGW_OBS_HITS = 2 };
 
 /* raw device pointers of the struct-of-arrays state owned by a handle (get_observation's live references) */
 typedef struct {
@@ -223,7 +230,7 @@ typedef struct {
     int64_t n_envs_padded;
     int32_t map_size;
     int32_t n_configs;
-    int32_t obs_format;  /* NGW_OBS_I32 / NGW_OBS_U8 */
+    int32_t obs_format;  /* NGW_OBS_I32 / NGW_OBS_U8 / NGW_OBS_HITS */
     int32_t obs_row_bytes; /* bytes per env of the observation buffers handed to ngw_step / ngw_reset / ngw_observe */
 } ngw_state_view;
 
@@ -242,7 +249,8 @@ int ngw_state(ngw_handle* h, ngw_state_view* out);
 
 /* Choose the observation row layout for every following call (default NGW_OBS_I32).  The observation pointers of
  * ngw_step / ngw_step_host / ngw_reset / ngw_observe / ngw_rollout then address rows of ngw_state_view.obs_row_bytes
- * bytes.  NGW_OBS_U8 cuts the device-to-host traffic of the host-buffer path from 266 to 94 bytes per env-step on C2. */
+ * bytes.  NGW_OBS_U8 cuts the device-to-host traffic of the host-buffer path from 266 to 94 bytes per env-step on C2,
+ * NGW_OBS_HITS to 54.  ngw_rollout_policy needs NGW_OBS_I32. */
 int ngw_set_obs_format(ngw_handle* h, int32_t format);
 
 /* Which LidarInFront path the kernels take for this config on this map size (no GPU needed): 0 no lidar wrapper,
