@@ -248,6 +248,21 @@ static int obs_row_bytes_of(const ngw_handle* h, int format) {
     return best;
 }
 
+// Function attributes of every kernel, on the current device (the handle's: create_init runs after cudaSetDevice).
+static int set_kernel_attributes() {
+#define NGW_SMEM_ATTR(K) CK(cudaFuncSetAttribute(K, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024))
+#define NGW_SMEM_ATTR4(K, ...) NGW_SMEM_ATTR((K<0, __VA_ARGS__>)); NGW_SMEM_ATTR((K<1, __VA_ARGS__>)); \
+                               NGW_SMEM_ATTR((K<4, __VA_ARGS__>)); NGW_SMEM_ATTR((K<16, __VA_ARGS__>))
+    NGW_SMEM_ATTR4(step1_kernel, true, true); NGW_SMEM_ATTR4(step1_kernel, true, false); NGW_SMEM_ATTR4(step1_kernel, false, false);
+    NGW_SMEM_ATTR4(step1w_kernel, 8); NGW_SMEM_ATTR4(step1w_kernel, 16);
+#undef NGW_SMEM_ATTR4
+#undef NGW_SMEM_ATTR
+    // the queued-reset kernel shares SMs with the next handle's step CTAs: both must want the same (maximal) shared-memory
+    // carve-out, or the SM would have to drain before it can be reconfigured
+    CK(cudaFuncSetAttribute(reset_list_kernel, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
+    return ngw_rollout_set_attributes();              // ngw_rollout.cu
+}
+
 static int create_init(ngw_handle* h, const ngw_config* cfgs, int32_t n_cfgs, int64_t n_envs, int32_t map_size,
                        int32_t device, int64_t first_env_gid, uint64_t seed, const cudaDeviceProp& prop) {
     h->device = device; h->n = n_envs; h->np = (n_envs + 31) / 32 * 32; h->first_gid = first_env_gid; h->seed = seed;
@@ -340,20 +355,7 @@ static int create_init(ngw_handle* h, const ngw_config* cfgs, int32_t n_cfgs, in
     }
     if (n_cfgs > 1 && !h->lidar_uniform) h->lidar_mode = 0;
     if (map_size > 32) h->lidar_mode = 0;           // large grids: pointer-walking beams (lidar_observe decides per lane)
-#define NGW_SMEM_ATTR(K) CK(cudaFuncSetAttribute(K, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024))
-#define NGW_SMEM_ATTR4(K, O) NGW_SMEM_ATTR((K<0, O>)); NGW_SMEM_ATTR((K<1, O>)); NGW_SMEM_ATTR((K<4, O>)); NGW_SMEM_ATTR((K<16, O>))
-    NGW_SMEM_ATTR4(step1_kernel, true); NGW_SMEM_ATTR4(step1_kernel, false);
-#undef NGW_SMEM_ATTR4
-    // the queued-reset kernel shares SMs with the next handle's step CTAs: both must want the same (maximal) shared-memory
-    // carve-out, or the SM would have to drain before it can be reconfigured
-    CK(cudaFuncSetAttribute(reset_list_kernel, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
-    NGW_SMEM_ATTR((step1_kernel<0, true, true>)); NGW_SMEM_ATTR((step1_kernel<1, true, true>));
-    NGW_SMEM_ATTR((step1_kernel<4, true, true>)); NGW_SMEM_ATTR((step1_kernel<16, true, true>));
-    NGW_SMEM_ATTR((step1w_kernel<0, 8>)); NGW_SMEM_ATTR((step1w_kernel<1, 8>)); NGW_SMEM_ATTR((step1w_kernel<4, 8>)); NGW_SMEM_ATTR((step1w_kernel<16, 8>));
-    NGW_SMEM_ATTR((step1w_kernel<0, 16>)); NGW_SMEM_ATTR((step1w_kernel<1, 16>)); NGW_SMEM_ATTR((step1w_kernel<4, 16>)); NGW_SMEM_ATTR((step1w_kernel<16, 16>));
-    if (ngw_rollout_init()) return 1;
-#undef NGW_SMEM_ATTR
-    return 0;
+    return set_kernel_attributes();
 }
 
 int ngw_state(ngw_handle* h, ngw_state_view* o) {
@@ -492,12 +494,17 @@ static bool is_multi(const StepParams& p) {
     return p.n_steps > 1 || p.random_policy || p.done_count != nullptr || p.actions_out != nullptr || p.policy_w != nullptr;
 }
 
-void pdl_attr(cudaLaunchConfig_t& lc, cudaLaunchAttribute* attr) {
-    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[0].val.programmaticStreamSerializationAllowed = 1;
-    // PDL (trigger once a CTA's stores are issued, see the kernels): the next launch's prologue overlaps this launch's
-    // store phase; C2 CUDA-graph replay 9.3 -> 8.6 us/step.  (An early trigger at kernel entry measured slower.)
-    lc.attrs = attr; lc.numAttrs = 1;
+// shared-memory row stride of a one-step kernel's observation tile (StepParams::obs_srow): rows of a multiple of 8 words
+// get 16 bytes of padding
+static int obs_srow(int obs_row_bytes) {
+    return obs_row_bytes + (((obs_row_bytes >> 2) % 8 == 0 && obs_row_bytes > 0) ? 16 : 0);
+}
+
+// after a one-step launch: the stream's record for the next launch's independence proof, and the handle's counters
+static void note_step_launched(ngw_handle* h, cudaStream_t s, const StepParams& p) {
+    note_launched(s, p.actions != nullptr);
+    h->concurrent_launches += p.concurrent;
+    h->last_step_concurrent = p.concurrent != 0;
 }
 
 // caller buffers of a one-step launch (for the independence proof of this launch and of the next one)
@@ -518,13 +525,10 @@ static StreamTail launch_tail(const StepParams& p) {
 // one-step launches (ngw_step / ngw_step_host / ngw_observe): several tile groups per CTA
 template <int NC>
 static cudaError_t launch_step1_nc(ngw_handle* h, StepParams p, cudaStream_t s) {
-    static thread_local StepArgs<NC> args;
     // ---- shared-memory plan: CTA header | lidar tables | tiles_per_cta x (group header | grid | inventory | observation)
-    const int luts = (NGW_MAX_MAP_SIZE + NGW_MAX_ITEMS * (NC > 0 ? NC : 0) + 127) & ~127;
     p.off_luts = NGW_CTA_HDR;
-    p.off_groups = p.off_luts + luts;
-    // shared-memory row stride of the observation tile: rows of a multiple of 8 words get 16 bytes of padding
-    p.obs_srow = p.obs_row_bytes + (((p.obs_row_bytes >> 2) % 8 == 0 && p.obs_row_bytes > 0) ? 16 : 0);
+    p.off_groups = p.off_luts + lut_bytes<NC>();
+    p.obs_srow = obs_srow(p.obs_row_bytes);
     p.group_bytes = (NGW_GROUP_HDR + p.map_bytes + p.inv_bytes + 32 * p.obs_srow + 127) & ~127;
     // alias plan (one tile per CTA, see step1_kernel<.., kAlias>): the observation tile shares the rows' shared memory
     bool alias = true;
@@ -566,24 +570,12 @@ static cudaError_t launch_step1_nc(ngw_handle* h, StepParams p, cudaStream_t s) 
     p.concurrent = (mode == 2 && h->concurrent && p.actions != nullptr) ? 1 : 0;
     p.early_state = (p.concurrent || (mode >= 1 && C > 1)) ? 1 : 0;
     const size_t smem = (size_t)p.off_groups + (size_t)C * p.group_bytes;
-    args.p = p;
-    for (int i = 0; i < NC && i < h->n_cfgs; i++) args.cfg[i] = h->h_cfgs[i];
-    cudaLaunchConfig_t lc;
-    memset(&lc, 0, sizeof(lc));
-    lc.gridDim = dim3((unsigned)((tiles + C - 1) / C) + (p.concurrent ? 1u : 0u)); lc.blockDim = dim3(32 * G * C);
-    lc.dynamicSmemBytes = smem;
-    lc.stream = s;
-    cudaLaunchAttribute attr[1];
-    pdl_attr(lc, attr);
+    const dim3 grid((unsigned)((tiles + C - 1) / C) + (p.concurrent ? 1u : 0u)), block(32 * G * C);
     cudaError_t e;
-    if (alias) e = cudaLaunchKernelEx(&lc, step1_kernel<NC, true, true>, args);
-    else if (C == 1) e = cudaLaunchKernelEx(&lc, step1_kernel<NC, true, false>, args);
-    else e = cudaLaunchKernelEx(&lc, step1_kernel<NC, false, false>, args);
-    if (e == cudaSuccess) {
-        note_launched(s, p.actions != nullptr);
-        h->concurrent_launches += p.concurrent;
-        h->last_step_concurrent = p.concurrent != 0;
-    }
+    if (alias) e = launch_tiles<NC>(step1_kernel<NC, true, true>, h, p, grid, block, smem, s);
+    else if (C == 1) e = launch_tiles<NC>(step1_kernel<NC, true, false>, h, p, grid, block, smem, s);
+    else e = launch_tiles<NC>(step1_kernel<NC, false, false>, h, p, grid, block, smem, s);
+    if (e == cudaSuccess) note_step_launched(h, s, p);
     return e;
 }
 
@@ -591,15 +583,13 @@ static cudaError_t launch_step1_nc(ngw_handle* h, StepParams p, cudaStream_t s) 
 // qualify and the caller should take the tile-group kernel
 template <int NC>
 static cudaError_t launch_step1w_nc(ngw_handle* h, StepParams p, cudaStream_t s) {
-    static thread_local StepArgs<NC> args;
     if (h->obs_dim > 0 && h->lidar_mode != 1) return cudaErrorNotSupported;     // needs the line-gather lidar (register sink)
     int max_tail = 0;
     for (const DevConfig& dc : h->h_cfgs) max_tail = dc.c.n_inv_obs > max_tail ? dc.c.n_inv_obs : max_tail;
     if (max_tail > NGW_REGSINK_TAIL) return cudaErrorNotSupported;
-    const int luts = (NGW_MAX_MAP_SIZE + NGW_MAX_ITEMS * (NC > 0 ? NC : 0) + 127) & ~127;
     p.off_luts = NGW_WCTA_HDR;
-    p.off_groups = p.off_luts + luts;
-    p.obs_srow = p.obs_row_bytes + (((p.obs_row_bytes >> 2) % 8 == 0 && p.obs_row_bytes > 0) ? 16 : 0);
+    p.off_groups = p.off_luts + lut_bytes<NC>();
+    p.obs_srow = obs_srow(p.obs_row_bytes);
     const int in_bytes = p.map_bytes + p.inv_bytes, obs_tile = p.obs ? 32 * p.obs_srow : 0;
     p.group_bytes = (NGW_WTILE_HDR + (in_bytes > obs_tile ? in_bytes : obs_tile) + 127) & ~127;
     const long long tiles = (p.env_end - p.env_begin + 31) / 32;
@@ -630,23 +620,19 @@ static cudaError_t launch_step1w_nc(ngw_handle* h, StepParams p, cudaStream_t s)
     p.n_tiles = (int)tiles;
     p.lidar_mode = h->lidar_mode;
     const size_t smem = (size_t)p.off_groups + (size_t)C * p.group_bytes;
-    args.p = p;
-    for (int i = 0; i < NC && i < h->n_cfgs; i++) args.cfg[i] = h->h_cfgs[i];
-    cudaLaunchConfig_t lc;
-    memset(&lc, 0, sizeof(lc));
-    lc.gridDim = dim3((unsigned)((tiles + C - 1) / C)); lc.blockDim = dim3(32 * (C + 1)); lc.dynamicSmemBytes = smem;
-    lc.stream = s;
-    cudaLaunchAttribute attr[1];
-    pdl_attr(lc, attr);
+    const dim3 grid((unsigned)((tiles + C - 1) / C)), block(32 * (C + 1));
     cudaError_t e;
-    if (max_tail <= 8) e = cudaLaunchKernelEx(&lc, step1w_kernel<NC, 8>, args);
-    else e = cudaLaunchKernelEx(&lc, step1w_kernel<NC, 16>, args);
-    if (e == cudaSuccess) {
-        note_launched(s, p.actions != nullptr);
-        h->concurrent_launches += p.concurrent;
-        h->last_step_concurrent = p.concurrent != 0;
-    }
+    if (max_tail <= 8) e = launch_tiles<NC>(step1w_kernel<NC, 8>, h, p, grid, block, smem, s);
+    else e = launch_tiles<NC>(step1w_kernel<NC, 16>, h, p, grid, block, smem, s);
+    if (e == cudaSuccess) note_step_launched(h, s, p);
     return e;
+}
+
+// one-step launches: the warp-per-tile shape where it qualifies, else the tile-group kernel
+template <int NC>
+static cudaError_t launch_one_step(ngw_handle* h, const StepParams& p, cudaStream_t s) {
+    const cudaError_t e = launch_step1w_nc<NC>(h, p, s);
+    return e == cudaErrorNotSupported ? launch_step1_nc<NC>(h, p, s) : e;
 }
 
 static const int kResetCtasPerSmOverlapped = 1;    // queued-reset grid behind an overlapped step, see launch_step
@@ -655,20 +641,11 @@ static int launch_step(ngw_handle* h, const StepParams& p, cudaStream_t s) {
     if (p.env_end <= p.env_begin) return 0;
     const int nc = h->n_cfgs;
     cudaError_t e;
-    if (is_multi(p)) {
-        e = ngw_launch_rollout(h, p, s);                  // ngw_rollout.cu
-    } else {
-        if (nc == 0 || nc > 16) e = launch_step1w_nc<0>(h, p, s);
-        else if (nc == 1) e = launch_step1w_nc<1>(h, p, s);
-        else if (nc <= 4) e = launch_step1w_nc<4>(h, p, s);
-        else e = launch_step1w_nc<16>(h, p, s);
-        if (e == cudaErrorNotSupported) {
-            if (nc == 0 || nc > 16) e = launch_step1_nc<0>(h, p, s);
-            else if (nc == 1) e = launch_step1_nc<1>(h, p, s);
-            else if (nc <= 4) e = launch_step1_nc<4>(h, p, s);
-            else e = launch_step1_nc<16>(h, p, s);
-        }
-    }
+    if (is_multi(p)) e = ngw_launch_rollout(h, p, s);   // ngw_rollout.cu
+    else if (nc == 0 || nc > 16) e = launch_one_step<0>(h, p, s);
+    else if (nc == 1) e = launch_one_step<1>(h, p, s);
+    else if (nc <= 4) e = launch_one_step<4>(h, p, s);
+    else e = launch_one_step<16>(h, p, s);
     if (e != cudaSuccess) return fail(std::string("step kernel launch: ") + cudaGetErrorString(e));
     h->launches++;
     if (p.actions != nullptr && p.auto_reset && !is_multi(p)) {     // regenerate the episodes the step kernel queued

@@ -89,6 +89,10 @@ struct EnvRow {
     int32_t* inv;                         // staged inventory row
     int ms;
     int r, c, facing, sel;
+    __device__ __forceinline__ void set_pose(uchar4 ps) { r = ps.x; c = ps.y; facing = ps.z; sel = ps.w; }
+    __device__ __forceinline__ uchar4 pose() const {
+        return make_uchar4((unsigned char)r, (unsigned char)c, (unsigned char)facing, (unsigned char)sel);
+    }
 };
 
 struct StepOut {
@@ -98,6 +102,7 @@ struct StepOut {
     float cost;
     int msg;        // enum ngw_msg | argument << 5
     int goal;       // the goal item is in the inventory after the step (done by success, not by fire / truncation)
+    __device__ __forceinline__ void clear() { reward = 0; done = 0; result = 0; cost = 0.0f; msg = 0; goal = 0; }
 };
 
 __device__ __forceinline__ int msg_of(int code, int arg) { return code | (arg << 5); }
@@ -748,46 +753,29 @@ __device__ __forceinline__ bool reset_candidate(int kind, int id, int wall, int 
          : (id == a);                                                  // novelty_wrappers.py:1130
 }
 
-// A TEAM regenerates one environment: TW == 1, the 32 lanes of one warp (ngw_reset: one env per warp, throughput-bound);
-// TW == 4, a whole CTA of 128 threads (the auto-reset queue consumer: few envs per step, latency-bound — one env per warp
-// took 10 k dependent instructions, 50-65 us, whatever the queue length).  All threads of the team call with the same
-// arguments.  `hist`: NGW_RESET_SCRATCH_WORDS uint32 of shared memory owned by the team.
+// The 32 lanes of one warp regenerate one environment (ngw_reset, the queued auto-resets, the in-place regeneration of
+// the rollout kernels).  All lanes call with the same arguments.  `hist`: NGW_RESET_SCRATCH_WORDS uint32 of shared
+// memory owned by the warp.
 #define NGW_RESET_SCRATCH_WORDS (256 + 32)
-template <int TW> __device__ __forceinline__ void team_sync() { if (TW == 1) __syncwarp(); else __syncthreads(); }
-template <int TW> __device__ __forceinline__ int team_sum(int v, uint32_t* word) {
-    v = __reduce_add_sync(0xFFFFFFFFu, v);
-    if (TW == 1) return v;
-    if (threadIdx.x == 0) *word = 0;
-    __syncthreads();
-    if ((threadIdx.x & 31) == 0) atomicAdd(word, (uint32_t)v);
-    __syncthreads();
-    v = (int)*word;
-    __syncthreads();
-    return v;
-}
-
-template <int TW>
-__device__ __noinline__ uint32_t reset_env_team(const ngw_config* cfg, int8_t* m, int32_t* inv, int ms, int inv_stride,
-                                                uint64_t seed, uint64_t gid, uint32_t episode, bool do_base,
-                                                int op_begin, int op_end, uint32_t* hist, int& pr, int& pc, int& pf,
-                                                int& psel, uint32_t key_mask = 0xFFFFFFFFu) {
+static __device__ __noinline__ uint32_t reset_env_warp(const ngw_config* cfg, int8_t* m, int32_t* inv, int ms, int inv_stride,
+                                                       uint64_t seed, uint64_t gid, uint32_t episode, bool do_base,
+                                                       int op_begin, int op_end, uint32_t* hist, int& pr, int& pc, int& pf,
+                                                       int& psel, uint32_t key_mask = 0xFFFFFFFFu) {
     const uint32_t FULL = 0xFFFFFFFFu;
     const int lane = threadIdx.x & 31;
-    const int tid = TW == 1 ? lane : (int)threadIdx.x, NT = 32 * TW;
-    const bool lead = TW == 1 || threadIdx.x < 32;                    // the warp that does the serial parts
-    uint32_t* xw = hist + 256;                                        // [0] reduction word, [1] boundary-list length, [2..4] scan result
+    uint32_t* xw = hist + 256;                                        // [1] boundary-list length, [2..4] scan result
     const int cells = ms * ms;
     const int wall = cfg->id_wall;
     uint32_t err = 0;
     if (do_base) {
-        for (int i = tid; i < inv_stride; i += NT) inv[i] = 0;         // pogostick_v1_env.py:119-120
+        for (int i = lane; i < inv_stride; i += 32) inv[i] = 0;         // pogostick_v1_env.py:119-120
         psel = 0;
-        for (int r = tid / ms, c = tid - (tid / ms) * ms, i = tid; i < cells; i += NT) {   // pogostick_v1_env.py:129-130
+        for (int r = lane / ms, c = lane - (lane / ms) * ms, i = lane; i < cells; i += 32) {   // pogostick_v1_env.py:129-130
             m[i] = (r == 0 || c == 0 || r == ms - 1 || c == ms - 1) ? (int8_t)wall : (int8_t)0;
-            c += NT;
+            c += 32;
             while (c >= ms) { c -= ms; r++; }
         }
-        team_sync<TW>();
+        __syncwarp();
         Philox rng;
         rng.init(seed, gid, episode, 0);
         const int side = ms - 4;                                      // rows/cols 2 .. ms-3 (pogostick_v1_env.py:136-138)
@@ -818,9 +806,9 @@ __device__ __noinline__ uint32_t reset_env_team(const ngw_config* cfg, int8_t* m
                                 pick--;
                             }
                 }
-                team_sync<TW>();                                      // every thread has read the grid it decided on
-                if (tid == 0) m[where] = (int8_t)item;
-                team_sync<TW>();
+                __syncwarp();                                         // every lane has read the grid it decided on
+                if (lane == 0) m[where] = (int8_t)item;
+                __syncwarp();
             }
         }
     }
@@ -829,55 +817,53 @@ __device__ __noinline__ uint32_t reset_env_team(const ngw_config* cfg, int8_t* m
     for (int k = op_begin; k < op_end; k++) {
         const ngw_reset_op op = cfg->reset_ops[k];
         if (op.kind == NGW_RESET_INVSET) {                            // novelty_wrappers.py:33,460,668-671
-            if (tid == 0) inv[op.a] = op.lo;
-            team_sync<TW>();
+            if (lane == 0) inv[op.a] = op.lo;
+            __syncwarp();
             continue;
         }
         const uint32_t stream = 1 + k;
         if (op.kind == NGW_RESET_TREETAP) {                           // pogostick_v0_env.py:155-178
             // uniform over (tree_log, direction) pairs until the target cell is free == the reference's retry loop;
-            // done by the lead warp (a rare op on 10x10 grids), the draws redundantly by its lanes
+            // done by the whole warp (a rare op on 10x10 grids), the draws redundantly by its lanes
             int target = -1, n_logs = 0;
-            if (lead) {
-                for (int i = lane; i < cells; i += 32) n_logs += (m[i] == (int8_t)op.b);
-                n_logs = __reduce_add_sync(FULL, n_logs);
-                if (n_logs > 1) {
-                    Philox rt;
-                    rt.init(seed, gid, episode, stream);
-                    for (int attempt = 0; attempt < 4096 && target < 0; attempt++) {
-                        int direction = (int)rt.below(4);
-                        int which = (int)rt.below((uint32_t)n_logs);
-                        int log = -1;
-                        for (int base = 0; base < cells && log < 0; base += 32) {     // which-th tree_log in row-major order
-                            int i = base + lane;
-                            uint32_t bal = __ballot_sync(FULL, i < cells && m[i] == (int8_t)op.b);
-                            int c = __popc(bal);
-                            if (which < c) {
-                                int bit = __fns(bal, 0, which + 1);
-                                log = base + bit;
-                            } else which -= c;
-                        }
-                        int r = log / ms, c = log - r * ms;
-                        int tr = r + (direction == NGW_SOUTH) - (direction == NGW_NORTH);
-                        int tc = c + (direction == NGW_EAST) - (direction == NGW_WEST);
-                        if (tr >= 0 && tr < ms && tc >= 0 && tc < ms && m[tr * ms + tc] == 0 && tr * ms + tc != agent)
-                            target = tr * ms + tc;
+            for (int i = lane; i < cells; i += 32) n_logs += (m[i] == (int8_t)op.b);
+            n_logs = __reduce_add_sync(FULL, n_logs);
+            if (n_logs > 1) {
+                Philox rt;
+                rt.init(seed, gid, episode, stream);
+                for (int attempt = 0; attempt < 4096 && target < 0; attempt++) {
+                    int direction = (int)rt.below(4);
+                    int which = (int)rt.below((uint32_t)n_logs);
+                    int log = -1;
+                    for (int base = 0; base < cells && log < 0; base += 32) {     // which-th tree_log in row-major order
+                        int i = base + lane;
+                        uint32_t bal = __ballot_sync(FULL, i < cells && m[i] == (int8_t)op.b);
+                        int c = __popc(bal);
+                        if (which < c) {
+                            int bit = __fns(bal, 0, which + 1);
+                            log = base + bit;
+                        } else which -= c;
                     }
+                    int r = log / ms, c = log - r * ms;
+                    int tr = r + (direction == NGW_SOUTH) - (direction == NGW_NORTH);
+                    int tc = c + (direction == NGW_EAST) - (direction == NGW_WEST);
+                    if (tr >= 0 && tr < ms && tc >= 0 && tc < ms && m[tr * ms + tc] == 0 && tr * ms + tc != agent)
+                        target = tr * ms + tc;
                 }
-                if (lane == 0) { xw[2] = (uint32_t)n_logs; xw[3] = (uint32_t)target; }
             }
-            team_sync<TW>();
+            if (lane == 0) { xw[2] = (uint32_t)n_logs; xw[3] = (uint32_t)target; }
+            __syncwarp();
             n_logs = (int)xw[2]; target = (int)xw[3];
-            team_sync<TW>();
+            __syncwarp();
             if (n_logs <= 1 || target < 0) { err |= NGW_ERR_PLACEMENT; continue; }
-            if (tid == 0) m[target] = (int8_t)op.a;
-            team_sync<TW>();
+            if (lane == 0) m[target] = (int8_t)op.a;
+            __syncwarp();
             continue;
         }
         // ---- n candidates, percentage, m
         int n = 0;
-        for (int i = tid; i < cells; i += NT) n += reset_candidate(op.kind, m[i], wall, op.a);
-        n = team_sum<TW>(n, &xw[0]);
+        for (int i = lane; i < cells; i += 32) n += reset_candidate(op.kind, m[i], wall, op.a);
+        n = __reduce_add_sync(FULL, n);
         Philox rng;
         rng.init(seed, gid, episode, stream);
         const int pct = op.lo + (int)rng.below((uint32_t)(op.hi - op.lo));            // randint(low, high), high exclusive
@@ -890,9 +876,9 @@ __device__ __noinline__ uint32_t reset_env_team(const ngw_config* cfg, int8_t* m
         int bits = 0, remaining = take, bin_count = n;
         const int quads = (cells + 3) >> 2;                           // a thread handles 4 consecutive cells per Philox block
         while (remaining < bin_count && bin_count > 32 && bits < 32) {
-            for (int i = tid; i < 256; i += NT) hist[i] = 0;
-            team_sync<TW>();
-            for (int q = tid; q < quads; q += NT) {
+            for (int i = lane; i < 256; i += 32) hist[i] = 0;
+            __syncwarp();
+            for (int q = lane; q < quads; q += 32) {
                 bool cand[4], any = false;
 #pragma unroll
                 for (int j = 0; j < 4; j++) {
@@ -910,31 +896,29 @@ __device__ __noinline__ uint32_t reset_env_team(const ngw_config* cfg, int8_t* m
                     if (cand[j] && (bits == 0 || (key[j] >> (32 - bits)) == prefix))
                         atomicAdd(&hist[(key[j] >> (24 - bits)) & 0xFF], 1u);
             }
-            team_sync<TW>();
-            if (lead) {                                               // the lead warp scans the 256 bins, 8 per lane
-                uint32_t mine[8], sum = 0;
+            __syncwarp();
+            uint32_t mine[8], sum = 0;                                // scan the 256 bins, 8 per lane
 #pragma unroll
-                for (int j = 0; j < 8; j++) { mine[j] = hist[lane * 8 + j]; sum += mine[j]; }
-                uint32_t incl = sum;
+            for (int j = 0; j < 8; j++) { mine[j] = hist[lane * 8 + j]; sum += mine[j]; }
+            uint32_t incl = sum;
 #pragma unroll
-                for (int o = 1; o < 32; o <<= 1) {
-                    uint32_t t = __shfl_up_sync(FULL, incl, o);
-                    if (lane >= o) incl += t;
-                }
-                uint32_t excl = incl - sum;
-                bool owner = (uint32_t)remaining > excl && (uint32_t)remaining <= incl;   // the bin holding the remaining-th key
-                if (owner) {
-                    uint32_t below = excl;
+            for (int o = 1; o < 32; o <<= 1) {
+                uint32_t t = __shfl_up_sync(FULL, incl, o);
+                if (lane >= o) incl += t;
+            }
+            uint32_t excl = incl - sum;
+            bool owner = (uint32_t)remaining > excl && (uint32_t)remaining <= incl;   // the bin holding the remaining-th key
+            if (owner) {
+                uint32_t below = excl;
 #pragma unroll
-                    for (int j = 0; j < 8; j++) {
-                        if ((uint32_t)remaining <= below + mine[j]) { xw[2] = (uint32_t)(lane * 8 + j); xw[3] = below; xw[4] = mine[j]; break; }
-                        below += mine[j];
-                    }
+                for (int j = 0; j < 8; j++) {
+                    if ((uint32_t)remaining <= below + mine[j]) { xw[2] = (uint32_t)(lane * 8 + j); xw[3] = below; xw[4] = mine[j]; break; }
+                    below += mine[j];
                 }
             }
-            team_sync<TW>();
+            __syncwarp();
             const uint32_t bin = xw[2], below = xw[3], cnt = xw[4];
-            team_sync<TW>();
+            __syncwarp();
             prefix = (prefix << 8) | bin;
             bits += 8;
             remaining -= (int)below;
@@ -944,10 +928,10 @@ __device__ __noinline__ uint32_t reset_env_team(const ngw_config* cfg, int8_t* m
         const bool all_in_bin_win = remaining >= bin_count;
         const bool exact_keys = bits >= 32 && bin_count > 32;
         const int value = op.kind == NGW_RESET_ADDITEM ? op.a : op.b;
-        if (tid == 0) xw[1] = 0;
-        team_sync<TW>();
-        for (int qb = 0; qb < quads; qb += NT) {
-            const int q = qb + tid;
+        if (lane == 0) xw[1] = 0;
+        __syncwarp();
+        for (int qb = 0; qb < quads; qb += 32) {
+            const int q = qb + lane;
             uint32_t key[4] = {0, 0, 0, 0};
             int id[4]; bool cand[4], any = false;
 #pragma unroll
@@ -967,8 +951,8 @@ __device__ __noinline__ uint32_t reset_env_team(const ngw_config* cfg, int8_t* m
                 bool boundary = cand[j] && !all_in_bin_win && top == prefix;
                 uint32_t bal = __ballot_sync(FULL, boundary);
                 if (bal != 0) {
-                    // a slot per boundary cell: warp-aggregated counter in shared memory (visiting order across the team's
-                    // warps is arbitrary, which is fine: the list is ranked by (key, cell) afterwards)
+                    // a slot per boundary cell: warp-aggregated counter in shared memory (the list is ranked by
+                    // (key, cell) afterwards)
                     int base = 0;
                     if (lane == __ffs((int)bal) - 1) base = (int)atomicAdd(&xw[1], (uint32_t)__popc(bal));
                     base = __shfl_sync(FULL, base, __ffs((int)bal) - 1);
@@ -986,9 +970,9 @@ __device__ __noinline__ uint32_t reset_env_team(const ngw_config* cfg, int8_t* m
                 }
             }
         }
-        team_sync<TW>();
+        __syncwarp();
         int n_list = (int)xw[1];
-        if (n_list > 0 && !exact_keys && lead) {
+        if (n_list > 0 && !exact_keys) {
             if (n_list > 32) n_list = 32;                             // unreachable: the loop above ends with <= 32 contenders or exact keys
             uint32_t my_key = 0; int my_idx = -1;
             if (lane < n_list) { my_key = hist[lane]; my_idx = (int)hist[32 + lane]; }
@@ -1003,10 +987,10 @@ __device__ __noinline__ uint32_t reset_env_team(const ngw_config* cfg, int8_t* m
                 else if (my_idx != agent) m[my_idx] = (int8_t)value;
             }
         }
-        team_sync<TW>();
+        __syncwarp();
         if (op.kind == NGW_RESET_FENCE) {                             // add_fence_around, pogostick_v1_env.py:524-536
-            // two phases so that the team's warps do not race: read every mark first, then write the fences
-            for (int i = tid; i < cells; i += NT) {
+            // two phases so that the lanes do not race: read every mark first, then write the fences
+            for (int i = lane; i < cells; i += 32) {
                 int v = m[i];
                 if (!(v & 0x80)) continue;
                 int r = i / ms, c = i - r * ms;
@@ -1015,24 +999,15 @@ __device__ __noinline__ uint32_t reset_env_team(const ngw_config* cfg, int8_t* m
                         if (rr >= 0 && rr < ms && cc >= 0 && cc < ms && m[rr * ms + cc] == 0 && rr * ms + cc != agent)
                             m[rr * ms + cc] = (int8_t)op.a;
             }
-            team_sync<TW>();
-            for (int i = tid; i < cells; i += NT) {
+            __syncwarp();
+            for (int i = lane; i < cells; i += 32) {
                 int v = m[i];
                 if (v & 0x80) m[i] = (int8_t)(v & 0x7F);
             }
-            team_sync<TW>();
+            __syncwarp();
         }
     }
     return err;
-}
-
-// the one-env-per-warp form (ngw_reset, the in-place regeneration of the rollout kernel)
-__device__ __forceinline__ uint32_t reset_env_warp(const ngw_config* cfg, int8_t* m, int32_t* inv, int ms, int inv_stride,
-                                                   uint64_t seed, uint64_t gid, uint32_t episode, bool do_base,
-                                                   int op_begin, int op_end, uint32_t* hist, int& pr, int& pc, int& pf,
-                                                   int& psel, uint32_t key_mask = 0xFFFFFFFFu) {
-    return reset_env_team<1>(cfg, m, inv, ms, inv_stride, seed, gid, episode, do_base, op_begin, op_end, hist, pr, pc, pf,
-                             psel, key_mask);
 }
 
 }  // namespace ngw

@@ -86,7 +86,7 @@ __global__ void __launch_bounds__(32 * NGW_RESET_WARPS) reset_kernel(const Reset
 // observation row and writes the rows back.  Like ngw_reset, the observation of the new episode is taken after
 // reset_obs_after_ops ops (quirk Q3: a novelty wrapped outside LidarInFront patches the state after the observation
 // was computed).  The last CTA to finish empties the queue for the next step.
-// (Measured and rejected: a whole CTA of 4 warps per env, reset_env_team<4> — at 96 registers only 5 such CTAs fit an SM, the
+// (Measured and rejected: a whole CTA of 4 warps per env — at 96 registers only 5 such CTAs fit an SM, the
 // ~2000 queued envs of a C5 step then take three rounds instead of one: 356 vs 315 us per step.)
 // Shared memory is sized for the batch's grid (dynamic: NGW_RESET_WARPS x reset_list_scratch_bytes(cells)), so that one
 // CTA of this kernel fits next to a full set of step CTAs when the next handle's step overlaps it (C5: 11 KB).
@@ -174,8 +174,7 @@ __global__ void observe_masked_kernel(const ResetParams p) {
     env.gm = nullptr;
     env.inv = p.inv + e * p.inv_stride;
     env.ms = p.ms;
-    uchar4 ps = p.pose[e];
-    env.r = ps.x; env.c = ps.y; env.facing = ps.z; env.sel = ps.w;
+    env.set_pose(p.pose[e]);
     ObsRow orow;
     orow.p = p.obs + e * p.obs_row_bytes;
     orow.fmt = p.obs_format;

@@ -8,22 +8,24 @@
         if (_e != cudaSuccess) return fail(std::string("cudaFuncSetAttribute(" #K "): ") + cudaGetErrorString(_e));   \
     } while (0)
 
-int ngw_rollout_init() {
+// the rollout kernels' part of create_init's set_kernel_attributes (the kernels are instantiated in this unit)
+int ngw_rollout_set_attributes() {
     // (rollout_kernel is the fallback behind rollout2_kernel: inline configs for one config, the global table otherwise)
     NGW_SMEM_ATTR((rollout_kernel<0>)); NGW_SMEM_ATTR((rollout_kernel<1>));
+    NGW_SMEM_ATTR((rollout2_kernel<0, 0>)); NGW_SMEM_ATTR((rollout2_kernel<0, 1>)); NGW_SMEM_ATTR((rollout2_kernel<0, 2>));
+    NGW_SMEM_ATTR((rollout2_kernel<0, 3>)); NGW_SMEM_ATTR((rollout2_kernel<0, 4>));
+    NGW_SMEM_ATTR((rollout2_kernel<1, 0>)); NGW_SMEM_ATTR((rollout2_kernel<1, 1>)); NGW_SMEM_ATTR((rollout2_kernel<1, 2>));
+    NGW_SMEM_ATTR((rollout2_kernel<1, 3>)); NGW_SMEM_ATTR((rollout2_kernel<1, 4>));
     return 0;
 }
 
 // K-step rollout launches (ngw_rollout / ngw_rollout_policy): one tile per CTA, tile resident across the steps
 template <int NC>
 static cudaError_t launch_rollout_nc(ngw_handle* h, StepParams p, cudaStream_t s) {
-    static thread_local StepArgs<NC> args;          // host staging of the argument block (copied by the launch); per thread,
-                                                    // so distinct handles stay independent across host threads
     // ---- shared-memory plan: header | lidar tables | reset scratch | grid + inventory tile | observation tile
     const int in_bytes = p.map_bytes + p.inv_bytes;
-    const int luts = (NGW_MAX_MAP_SIZE + NGW_MAX_ITEMS * (NC > 0 ? NC : 0) + 127) & ~127;
     p.off_luts = NGW_SMEM_HDR;
-    p.off_scratch = p.off_luts + luts;
+    p.off_scratch = p.off_luts + lut_bytes<NC>();
     p.off_policy = p.off_scratch + ((NGW_RESET_SCRATCH_WORDS * 4 + 127) & ~127);
     p.off_in = p.off_policy + (p.policy_w ? ((16 + p.obs_dim * p.policy_actions) * 4 + 127) & ~127 : 0);
     const long long tiles = (p.env_end - p.env_begin + 31) / 32;
@@ -32,25 +34,15 @@ static cudaError_t launch_rollout_nc(ngw_handle* h, StepParams p, cudaStream_t s
     // the K-step rollout is all step logic (one lidar pass at the end): one warp per tile keeps more tiles resident
     const int warps = (smem * 12 <= 227 * 1024) ? 1 : h->warps;
     claim_stream(h, s, false);
-    args.p = p;
-    for (int i = 0; i < NC && i < h->n_cfgs; i++) args.cfg[i] = h->h_cfgs[i];
-    cudaLaunchConfig_t lc;
-    memset(&lc, 0, sizeof(lc));
-    lc.gridDim = dim3((unsigned)tiles); lc.blockDim = dim3(32 * warps); lc.dynamicSmemBytes = smem;
-    lc.stream = s;
-    cudaLaunchAttribute attr[1];
-    pdl_attr(lc, attr);
-    return cudaLaunchKernelEx(&lc, rollout_kernel<NC>, args);
+    return launch_tiles<NC>(rollout_kernel<NC>, h, p, dim3((unsigned)tiles), dim3(32 * warps), smem, s);
 }
 
 // K-step rollout launches in the lane-pair shape (rollout2_kernel); cudaErrorNotSupported -> rollout_kernel
 template <int NC, int A4>
 static cudaError_t launch_rollout2_na(ngw_handle* h, StepParams p, cudaStream_t s) {
-    static thread_local StepArgs<NC> args;
     const int in_bytes = p.map_bytes + p.inv_bytes;
-    const int luts = (NGW_MAX_MAP_SIZE + NGW_MAX_ITEMS * (NC > 0 ? NC : 0) + 127) & ~127;
     p.off_luts = NGW_R2_HDR;
-    p.off_scratch = p.off_luts + luts;
+    p.off_scratch = p.off_luts + lut_bytes<NC>();
     p.off_policy = p.off_scratch + (p.auto_reset ? ((2 * NGW_RESET_SCRATCH_WORDS * 4 + 127) & ~127) : 0);
     p.off_in = p.off_policy + (A4 > 0 ? ((16 + p.obs_dim * 4 * A4) * 4 + 127) & ~127 : 0);
     const int obs_tile = p.obs ? p.obs_bytes : 0;
@@ -58,17 +50,7 @@ static cudaError_t launch_rollout2_na(ngw_handle* h, StepParams p, cudaStream_t 
     if (smem > 200 * 1024) return cudaErrorNotSupported;
     const long long tiles = (p.env_end - p.env_begin + 31) / 32;
     claim_stream(h, s, false);
-    args.p = p;
-    for (int i = 0; i < NC && i < h->n_cfgs; i++) args.cfg[i] = h->h_cfgs[i];
-    cudaLaunchConfig_t lc;
-    memset(&lc, 0, sizeof(lc));
-    lc.gridDim = dim3((unsigned)tiles); lc.blockDim = dim3(64); lc.dynamicSmemBytes = smem;
-    lc.stream = s;
-    cudaLaunchAttribute attr[1];
-    pdl_attr(lc, attr);
-    static bool attr_set = false;       // per instantiation
-    if (!attr_set) { cudaFuncSetAttribute(rollout2_kernel<NC, A4>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024); attr_set = true; }
-    return cudaLaunchKernelEx(&lc, rollout2_kernel<NC, A4>, args);
+    return launch_tiles<NC>(rollout2_kernel<NC, A4>, h, p, dim3((unsigned)tiles), dim3(64), smem, s);
 }
 
 template <int NC>

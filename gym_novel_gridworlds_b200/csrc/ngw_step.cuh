@@ -138,6 +138,10 @@ template <int NC>
 struct StepArgs {
     StepParams p;
     DevConfig cfg[NC > 0 ? NC : 1];
+    // the config of an env whose config id is cfg_i
+    __device__ __forceinline__ const DevConfig& config(int cfg_i) const {
+        return (NC == 1) ? cfg[0] : (NC > 1 ? cfg[cfg_i] : p.dcfgs[cfg_i]);
+    }
 };
 
 #define NGW_STAT_SLOTS 512
@@ -147,6 +151,125 @@ __device__ __forceinline__ float warp_sum(float v) {
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xFFFFFFFFu, v, o);
     return v;
+}
+
+// ------------------------------------------------------------------ tile plumbing shared by the step and rollout kernels
+// Lidar tables read with per-lane indices, staged in shared memory: config 0's first-sample table, every inline config's
+// item -> slot table (NC == 0: the lanes read both from the global config table instead).
+template <int NC>
+__device__ __forceinline__ void stage_lidar_luts(const StepArgs<NC>& args, uint8_t* sfirstk, int8_t* sslot) {
+    if (NC > 0) {                                                     // config tables are kernel arguments (constant bank)
+        if (threadIdx.x < NGW_MAX_MAP_SIZE / 4)
+            reinterpret_cast<uint32_t*>(sfirstk)[threadIdx.x] =
+                reinterpret_cast<const uint32_t*>(args.cfg[0].lidar.firstk)[threadIdx.x];
+#pragma unroll
+        for (int k = 0; k < NC; k++)
+            if (threadIdx.x < NGW_MAX_ITEMS / 4)
+                reinterpret_cast<uint32_t*>(sslot + k * NGW_MAX_ITEMS)[threadIdx.x] =
+                    reinterpret_cast<const uint32_t*>(args.cfg[k].c.lidar_slot)[threadIdx.x];
+    }
+}
+
+// the lane's lidar tables: the staged ones (stage_lidar_luts), or config cfg_i's in global memory when NC == 0
+template <int NC>
+__device__ __forceinline__ LidarLuts lane_luts(const StepParams& p, const uint8_t* sfirstk, const int8_t* sslot, int cfg_i) {
+    LidarLuts luts;
+    if (NC > 0) { luts.slot = sslot + cfg_i * NGW_MAX_ITEMS; luts.firstk = sfirstk; }
+    else { luts.slot = p.dcfgs[cfg_i].c.lidar_slot; luts.firstk = p.dcfgs[cfg_i].lidar.firstk; }
+    return luts;
+}
+
+// one thread: the tile's grid rows and inventory rows -> shared memory, completing on `bar`, L2 policy `pol`
+__device__ __forceinline__ void issue_tile_loads(const StepParams& p, uint64_t* bar, int8_t* smap, const int8_t* gmap,
+                                                 int32_t* sinv, const int32_t* ginv, uint64_t pol) {
+    mbar_expect_tx(bar, (uint32_t)(p.map_bytes + p.inv_bytes));
+    bulk_g2s_hint(smap, gmap, (uint32_t)p.map_bytes, bar, pol);
+    bulk_g2s_hint(sinv, ginv, (uint32_t)p.inv_bytes, bar, pol);
+}
+
+// the action table entry of `action`; NGW_OP_INVALID for an id outside the config's actions
+__device__ __forceinline__ ngw_action_entry decode_action(const ngw_config& cfg, int action) {
+    ngw_action_entry a;
+    a.op = NGW_OP_INVALID;
+    if (action >= 0 && action < cfg.n_actions) {
+        uint2 raw = *reinterpret_cast<const uint2*>(&cfg.actions[action]);
+        memcpy(&a, &raw, sizeof(a));
+    }
+    return a;
+}
+
+// One-step kernels: episode bookkeeping after a valid step of env e — truncation at max_episode_steps (a harness knob: it
+// sets o.done), the episode length, and whether the env is reset.  ld.cg: another grid may overlap this one.  (The
+// rollouts keep this inline with a plain load: there ep_len is read once per step on the step's dependent chain, and
+// ld.cg measured 1.6 % fewer env-steps/s on the C2 rollout, B200 at 1000 W.)
+__device__ __forceinline__ int end_of_step(const StepParams& p, long long e, StepOut& o) {
+    int finished = o.done;
+    if (p.max_episode_steps > 0) {
+        int len = __ldcg(&p.ep_len[e]) + 1;
+        if (len >= p.max_episode_steps) { finished = 1; o.done = 1; }
+        p.ep_len[e] = finished && p.auto_reset ? 0 : len;
+    }
+    return finished && p.auto_reset;
+}
+
+// whole warp: append the lanes with did_reset to the auto-reset queue that reset_list_kernel consumes
+__device__ __forceinline__ void queue_resets(const StepParams& p, int lane, long long e, int did_reset) {
+    const uint32_t bal = __ballot_sync(0xFFFFFFFFu, did_reset);
+    if (bal != 0) {
+        int base = 0;
+        if (lane == 0) base = atomicAdd(p.reset_count, __popc(bal));
+        base = __shfl_sync(0xFFFFFFFFu, base, 0);
+        if (did_reset) p.reset_list[base + __popc(bal & ((1u << lane) - 1u))] = (int)e;
+    }
+}
+
+// one thread: add one set of episode statistics into statistics slot `slot` (mod NGW_STAT_SLOTS)
+__device__ __forceinline__ void flush_stats(double* stats, unsigned slot, int steps, int reward, float cost, int done,
+                                            int succ, int reset, int invalid) {
+    double* s = stats + (size_t)(slot % NGW_STAT_SLOTS) * NGW_STAT_COUNT;
+    atomicAdd(&s[NGW_STAT_STEPS], (double)steps);
+    atomicAdd(&s[NGW_STAT_REWARD_SUM], (double)reward);
+    atomicAdd(&s[NGW_STAT_COST_SUM], (double)cost);
+    if (done) atomicAdd(&s[NGW_STAT_EPISODES], (double)done);
+    if (succ) atomicAdd(&s[NGW_STAT_SUCCESSES], (double)succ);
+    if (reset) atomicAdd(&s[NGW_STAT_RESETS], (double)reset);
+    if (invalid) atomicAdd(&s[NGW_STAT_INVALID], (double)invalid);
+}
+
+// threads t, t + nt, ...: copy `bytes` (a multiple of 16) in 16-byte words
+__device__ __forceinline__ void copy16(void* dst, const void* src, int bytes, int t, int nt) {
+    const uint4* s4 = reinterpret_cast<const uint4*>(src);
+    uint4* d4 = reinterpret_cast<uint4*>(dst);
+    for (int i = t; i < (bytes >> 4); i += nt) d4[i] = s4[i];
+}
+
+// threads t, t + nt, ...: the valid rows of a partial observation tile -> HBM (srow: the row stride in shared memory)
+__device__ __forceinline__ void copy_obs_rows(const StepParams& p, long long e0, const unsigned char* sobs, int srow, int t,
+                                              int nt) {
+    const int rows = (int)(p.env_end - e0 < 32 ? p.env_end - e0 : 32), words = p.obs_row_bytes >> 2;
+    for (int r = 0; r < rows; r++) {
+        uint32_t* grow = reinterpret_cast<uint32_t*>(p.obs + (e0 + r) * p.obs_row_bytes);
+        const uint32_t* srow_p = reinterpret_cast<const uint32_t*>(sobs + r * srow);
+        for (int i = t; i < words; i += nt) grow[i] = srow_p[i];
+    }
+}
+
+// zero the shared memory [a, end) (shared-memory addresses), 16 bytes per thread and pass, `step` bytes apart
+__device__ __forceinline__ void zero_span(uint32_t a, uint32_t end, uint32_t step) {
+#pragma unroll 4
+    for (; a < end; a += step) asm volatile("st.shared.v4.b32 [%0], {%1, %1, %1, %1};" ::"r"(a), "r"(0) : "memory");
+}
+
+// one warp: a full observation tile -> HBM (L2 policy `pol`), one bulk store when the tile's rows are contiguous in shared
+// memory, else one per row (lane l stores row l)
+__device__ __forceinline__ void store_obs_tile(const StepParams& p, long long e0, const unsigned char* sobs, int lane,
+                                               uint64_t pol) {
+    unsigned char* gobs = p.obs + e0 * p.obs_row_bytes;
+    if (p.obs_srow == p.obs_row_bytes) {
+        if (lane == 0) bulk_s2g_hint(gobs, sobs, (uint32_t)p.obs_bytes, pol);
+    } else {
+        bulk_s2g_hint(gobs + lane * p.obs_row_bytes, sobs + lane * p.obs_srow, (uint32_t)p.obs_row_bytes, pol);
+    }
 }
 
 // Cold: fused auto-reset.  Called by the whole step warp; every lane that finished an episode is regenerated in turn by
@@ -180,7 +303,7 @@ static __device__ __noinline__ void auto_reset_warp(const StepParams& p, const D
 }
 
 // Episode statistics of one tile: warp reductions + one atomic per counter into one of NGW_STAT_SLOTS slots.
-__device__ __forceinline__ void tile_stats(double* stats, int slot, int lane, int valid, int done, int success, int did_reset,
+__device__ __forceinline__ void tile_stats(double* stats, unsigned slot, int lane, int valid, int done, int success, int did_reset,
                                            int invalid, int reward, float cost) {
     // five small counts (each <= 32) share one reduction: 6 bits apiece
     unsigned packed = (unsigned)(valid ? done : 0) | ((unsigned)success << 6) | ((unsigned)did_reset << 12) |
@@ -191,14 +314,7 @@ __device__ __forceinline__ void tile_stats(double* stats, int slot, int lane, in
     if (lane == 0) {
         const int n_done = packed & 63, n_succ = (packed >> 6) & 63, n_reset = (packed >> 12) & 63;
         const int n_inv = (packed >> 18) & 63, n_valid = (packed >> 24) & 63;
-        double* s = stats + (size_t)(slot % NGW_STAT_SLOTS) * NGW_STAT_COUNT;
-        atomicAdd(&s[NGW_STAT_STEPS], (double)(n_valid - n_inv));
-        atomicAdd(&s[NGW_STAT_REWARD_SUM], (double)r_sum);
-        atomicAdd(&s[NGW_STAT_COST_SUM], (double)c_sum);
-        if (n_done) atomicAdd(&s[NGW_STAT_EPISODES], (double)n_done);
-        if (n_succ) atomicAdd(&s[NGW_STAT_SUCCESSES], (double)n_succ);
-        if (n_reset) atomicAdd(&s[NGW_STAT_RESETS], (double)n_reset);
-        if (n_inv) atomicAdd(&s[NGW_STAT_INVALID], (double)n_inv);
+        flush_stats(stats, slot, n_valid - n_inv, r_sum, c_sum, n_done, n_succ, n_reset, n_inv);
     }
 }
 
@@ -243,16 +359,7 @@ __global__ void __launch_bounds__(256) rollout_kernel(const __grid_constant__ St
         mbar_init(bar, 1);
         *reinterpret_cast<uint64_t*>(szero) = 0ull;
     }
-    if (NC > 0) {                                                    // config tables are kernel arguments (constant bank)
-        if (threadIdx.x < NGW_MAX_MAP_SIZE / 4)
-            reinterpret_cast<uint32_t*>(sfirstk)[threadIdx.x] =
-                reinterpret_cast<const uint32_t*>(args.cfg[0].lidar.firstk)[threadIdx.x];
-#pragma unroll
-        for (int k = 0; k < NC; k++)
-            if (threadIdx.x < NGW_MAX_ITEMS / 4)
-                reinterpret_cast<uint32_t*>(sslot + k * NGW_MAX_ITEMS)[threadIdx.x] =
-                    reinterpret_cast<const uint32_t*>(args.cfg[k].c.lidar_slot)[threadIdx.x];
-    }
+    stage_lidar_luts<NC>(args, sfirstk, sslot);
     if (p.obs != nullptr) {
         const uint4 z = make_uint4(0, 0, 0, 0);
         uint4* o4 = reinterpret_cast<uint4*>(sobs);
@@ -262,12 +369,7 @@ __global__ void __launch_bounds__(256) rollout_kernel(const __grid_constant__ St
     asm volatile("griddepcontrol.wait;" ::: "memory");               // previous kernel of the stream done + visible
 
     // ---- stage the tile: grid rows + inventory rows (state arrays are padded, a full tile is always readable)
-    if (threadIdx.x == 0) {
-        mbar_expect_tx(bar, (uint32_t)(p.map_bytes + p.inv_bytes));
-        uint64_t pol = policy_evict_first();
-        bulk_g2s_hint(smap, gmap, (uint32_t)p.map_bytes, bar, pol);
-        bulk_g2s_hint(sinv, ginv, (uint32_t)p.inv_bytes, bar, pol);
-    }
+    if (threadIdx.x == 0) issue_tile_loads(p, bar, smap, gmap, sinv, ginv, policy_evict_first());
     if (closed_loop) {                                               // the policy's weights, once per CTA
         const int n_w = p.obs_dim * p.policy_actions;
         for (int i = threadIdx.x; i < 16; i += blockDim.x) spol[i] = i < p.policy_actions ? p.policy_b[i] : 0;
@@ -276,18 +378,11 @@ __global__ void __launch_bounds__(256) rollout_kernel(const __grid_constant__ St
 
     // ---- while the copies fly: per-lane scalars
     const int cfg_i = (NC == 1) ? 0 : (int)p.cfg_id[e];
-    const DevConfig& dc = (NC == 1) ? args.cfg[0] : (NC > 1 ? args.cfg[cfg_i] : p.dcfgs[cfg_i]);
+    const DevConfig& dc = args.config(cfg_i);
     const ngw_config& cfg = dc.c;
     const LidarDev& beam_tables = (NC > 1 && p.lidar_uniform) ? args.cfg[0].lidar : dc.lidar;
-    LidarLuts luts;
-    if (NC > 0) {
-        luts.slot = sslot + cfg_i * NGW_MAX_ITEMS;
-        luts.firstk = (NC == 1 || p.lidar_uniform) ? sfirstk : nullptr;
-        if (luts.firstk == nullptr) luts.slot = nullptr;              // heterogeneous beam tables: pointer-walking path
-    } else {
-        luts.slot = p.dcfgs[cfg_i].c.lidar_slot;
-        luts.firstk = p.dcfgs[cfg_i].lidar.firstk;
-    }
+    LidarLuts luts = lane_luts<NC>(p, sfirstk, sslot, cfg_i);
+    if (NC > 1 && !p.lidar_uniform) luts.slot = nullptr;              // heterogeneous beam tables: pointer-walking path
     ObsRow orow;
     orow.p = sobs + lane * p.obs_row_bytes;
     orow.fmt = p.obs_format;
@@ -309,9 +404,9 @@ __global__ void __launch_bounds__(256) rollout_kernel(const __grid_constant__ St
     env.ms = p.ms;
 
     if (g == 0) {
-        env.r = ps.x; env.c = ps.y; env.facing = ps.z; env.sel = ps.w;
+        env.set_pose(ps);
         StepOut o;
-        o.reward = 0; o.done = 0; o.result = 0; o.cost = 0.0f; o.msg = 0; o.goal = 0;
+        o.clear();
         float reward_sum = 0.0f, cost_sum = 0.0f;
         int done_count = 0;
         // the sink needs the line-gather lidar (lidar_observe would take the same branch); otherwise the observation row
@@ -349,15 +444,10 @@ __global__ void __launch_bounds__(256) rollout_kernel(const __grid_constant__ St
                 action = rpol.draw(p.policy_seed, (uint64_t)(p.first_gid + e), (uint32_t)t, (uint32_t)(cfg.n_actions > 0 ? cfg.n_actions : 1));
             }
             if (p.actions_out != nullptr && valid) p.actions_out[t * p.act_stride + e] = action;
-            o.reward = 0; o.done = 0; o.result = 0; o.cost = 0.0f; o.msg = 0; o.goal = 0;
+            o.clear();
             int invalid = 0, did_reset = 0, success = 0;
             if (valid) {
-                ngw_action_entry a;
-                a.op = NGW_OP_INVALID;
-                if (action >= 0 && action < cfg.n_actions) {
-                    uint2 raw = *reinterpret_cast<const uint2*>(&cfg.actions[action]);
-                    memcpy(&a, &raw, sizeof(a));
-                }
+                const ngw_action_entry a = decode_action(cfg, action);
                 if (a.op == NGW_OP_INVALID) {                         // wrappers.py:76 / pogostick_v1_env.py:236 would raise
                     invalid = 1;
                     p.err[e] |= NGW_ERR_INVALID_ACTION;
@@ -372,17 +462,17 @@ __global__ void __launch_bounds__(256) rollout_kernel(const __grid_constant__ St
                     }
                     if (finished && p.auto_reset) did_reset = 1;
                 }
-                ps = make_uchar4((unsigned char)env.r, (unsigned char)env.c, (unsigned char)env.facing, (unsigned char)env.sel);
+                ps = env.pose();
                 reward_sum += (float)o.reward; cost_sum += o.cost; done_count += o.done;
             }
             if (p.auto_reset) {
                 // the next step needs the new episode now -> regenerate in place, warp-cooperatively
                 if (__ballot_sync(0xFFFFFFFFu, did_reset) != 0) {
                     auto_reset_warp(p, p.dcfgs, cfg_i, did_reset != 0, smap, sinv, sscratch, e0, ps);
-                    env.r = ps.x; env.c = ps.y; env.facing = ps.z; env.sel = ps.w;
+                    env.set_pose(ps);
                 }
             }
-            tile_stats(p.stats, (int)blockIdx.x, lane, valid, o.done, success, did_reset, invalid, o.reward, o.cost);
+            tile_stats(p.stats, blockIdx.x, lane, valid, o.done, success, did_reset, invalid, o.reward, o.cost);
             action = next_action;
         }
         if (closed_loop && !use_sink) {                               // the last policy observation must not leak into the final one
@@ -403,7 +493,7 @@ __global__ void __launch_bounds__(256) rollout_kernel(const __grid_constant__ St
     if (G > 1) {
         __syncthreads();                                             // step results (grid, inventory, pose) visible to all warps
         ps = spose[lane];
-        env.r = ps.x; env.c = ps.y; env.facing = ps.z; env.sel = ps.w;
+        env.set_pose(ps);
     }
 
     // ---- LidarInFront observation of the final state into the shared-memory tile
@@ -424,15 +514,8 @@ __global__ void __launch_bounds__(256) rollout_kernel(const __grid_constant__ St
             bulk_wait_read<0>();                                     // shared memory must outlive the bulk stores' reads
         }
     } else {
-        const uint4* s4 = reinterpret_cast<const uint4*>(sinv);
-        uint4* d4 = reinterpret_cast<uint4*>(ginv);
-        for (int i = threadIdx.x; i < (p.inv_bytes >> 4); i += blockDim.x) d4[i] = s4[i];
-        if (p.obs != nullptr) {
-            const int n = (int)((p.env_end - e0 < 32 ? p.env_end - e0 : 32)) * (p.obs_row_bytes >> 2);
-            uint32_t* gobs = reinterpret_cast<uint32_t*>(p.obs + e0 * p.obs_row_bytes);
-            const uint32_t* so = reinterpret_cast<const uint32_t*>(sobs);
-            for (int i = threadIdx.x; i < n; i += blockDim.x) gobs[i] = so[i];
-        }
+        copy16(ginv, sinv, p.inv_bytes, threadIdx.x, blockDim.x);
+        if (p.obs != nullptr) copy_obs_rows(p, e0, sobs, p.obs_row_bytes, threadIdx.x, blockDim.x);
     }
 }
 
@@ -511,16 +594,7 @@ __global__ void __launch_bounds__(512) step1_kernel(const __grid_constant__ Step
         mbar_init(bar, 1);
         *reinterpret_cast<uint64_t*>(szero) = 0ull;
     }
-    if (NC > 0) {                                                     // config tables are kernel arguments (constant bank)
-        if (threadIdx.x < NGW_MAX_MAP_SIZE / 4)
-            reinterpret_cast<uint32_t*>(sfirstk)[threadIdx.x] =
-                reinterpret_cast<const uint32_t*>(args.cfg[0].lidar.firstk)[threadIdx.x];
-#pragma unroll
-        for (int k = 0; k < NC; k++)
-            if (threadIdx.x < NGW_MAX_ITEMS / 4)
-                reinterpret_cast<uint32_t*>(sslot + k * NGW_MAX_ITEMS)[threadIdx.x] =
-                    reinterpret_cast<const uint32_t*>(args.cfg[k].c.lidar_slot)[threadIdx.x];
-    }
+    stage_lidar_luts<NC>(args, sfirstk, sslot);
     __syncthreads();                                                  // the only CTA-wide barrier
 
     // ---- stage the tile: grid rows + inventory rows (state arrays are padded, a full tile is always readable).
@@ -530,14 +604,9 @@ __global__ void __launch_bounds__(512) step1_kernel(const __grid_constant__ Step
     // predecessor's tail.  Otherwise they follow the wait.
     const int8_t* gmap = p.map + e0 * p.cells;
     int32_t* ginv = p.inv + e0 * p.inv_stride;
-    uint64_t pol_first = 0;
+    const uint64_t pol_first = policy_evict_first();
     auto issue_loads = [&]() {
-        if (gt == 0) {
-            mbar_expect_tx(bar, (uint32_t)(p.map_bytes + p.inv_bytes));
-            pol_first = policy_evict_first();
-            bulk_g2s_hint(smap, gmap, (uint32_t)p.map_bytes, bar, pol_first);
-            bulk_g2s_hint(sinv, ginv, (uint32_t)p.inv_bytes, bar, pol_first);
-        }
+        if (gt == 0) issue_tile_loads(p, bar, smap, gmap, sinv, ginv, pol_first);
     };
     const int n_cls = G >= 2 ? 2 : 1;                                 // warps that take part in the step
     uchar4 ps = make_uchar4(0, 0, 0, 0);
@@ -546,17 +615,9 @@ __global__ void __launch_bounds__(512) step1_kernel(const __grid_constant__ Step
         issue_loads();
         if (g < n_cls) ps = __ldcg(&p.pose[e]);
     }
-    if (p.obs != nullptr) {                                           // the group zeroes its observation tile while the loads fly
-        uint32_t a = smem_u32(sobs) + (uint32_t)gt * 16u + (kAlias ? in_bytes : 0u);   // (alias: only the part beyond the rows)
-        const uint32_t end = smem_u32(sobs) + 32u * (uint32_t)p.obs_srow, st = 512u * (uint32_t)G;
-        for (; a + 3u * st < end; a += 4u * st) {
-            asm volatile("st.shared.v4.b32 [%0], {%1, %1, %1, %1};" ::"r"(a), "r"(0) : "memory");
-            asm volatile("st.shared.v4.b32 [%0], {%1, %1, %1, %1};" ::"r"(a + st), "r"(0) : "memory");
-            asm volatile("st.shared.v4.b32 [%0], {%1, %1, %1, %1};" ::"r"(a + 2u * st), "r"(0) : "memory");
-            asm volatile("st.shared.v4.b32 [%0], {%1, %1, %1, %1};" ::"r"(a + 3u * st), "r"(0) : "memory");
-        }
-        for (; a < end; a += st) asm volatile("st.shared.v4.b32 [%0], {%1, %1, %1, %1};" ::"r"(a), "r"(0) : "memory");
-    }
+    if (p.obs != nullptr)                                             // the group zeroes its observation tile while the loads fly
+        zero_span(smem_u32(sobs) + (uint32_t)gt * 16u + (kAlias ? in_bytes : 0u),   // (alias: only the part beyond the rows)
+                  smem_u32(sobs) + 32u * (uint32_t)p.obs_srow, 512u * (uint32_t)G);
     if (!p.concurrent) {
         asm volatile("griddepcontrol.wait;" ::: "memory");            // previous kernel of the stream done + visible
         // trigger right after the wait (rather than once the stores are issued): C2 7.70 -> 7.60 us/step
@@ -567,7 +628,7 @@ __global__ void __launch_bounds__(512) step1_kernel(const __grid_constant__ Step
 
     // ---- while the copies fly: per-lane scalars
     const int cfg_i = (NC == 1) ? 0 : (int)__ldcg(&p.cfg_id[e]);
-    const DevConfig& dc = (NC == 1) ? args.cfg[0] : (NC > 1 ? args.cfg[cfg_i] : p.dcfgs[cfg_i]);
+    const DevConfig& dc = args.config(cfg_i);
     const ngw_config& cfg = dc.c;
     int action = 0;
     if (g < n_cls) {
@@ -584,12 +645,14 @@ __global__ void __launch_bounds__(512) step1_kernel(const __grid_constant__ Step
     env.ms = p.ms;
 
     if (g < n_cls) {
-        env.r = ps.x; env.c = ps.y; env.facing = ps.z; env.sel = ps.w;
+        env.set_pose(ps);
         bool mine = !stepping && g == 0;                              // this warp publishes this lane's hand-over record
         uint32_t bits = 0;
         StepOut o;
-        o.reward = 0; o.done = 0; o.result = 0; o.cost = 0.0f; o.msg = 0; o.goal = 0;
+        o.clear();
         if (stepping) {
+            // (decode_action plus the lane's validity: calling it with an id of -1 for past-the-end lanes costs
+            // step1_kernel<1, true, true> a register)
             ngw_action_entry a;
             a.op = NGW_OP_INVALID;
             if (valid && action >= 0 && action < cfg.n_actions) {
@@ -607,29 +670,15 @@ __global__ void __launch_bounds__(512) step1_kernel(const __grid_constant__ Step
                 } else {
                     step_env(env, cfg, a, o);
                     if (o.goal) bits |= 1u << 18;
-                    int finished = o.done;
-                    if (p.max_episode_steps > 0) {
-                        int len = __ldcg(&p.ep_len[e]) + 1;
-                        if (len >= p.max_episode_steps) { finished = 1; o.done = 1; }   // harness truncation knob
-                        p.ep_len[e] = finished && p.auto_reset ? 0 : len;
-                    }
-                    if (finished && p.auto_reset) { did_reset = 1; bits |= 1u << 19; }
+                    did_reset = end_of_step(p, e, o);
+                    if (did_reset) bits |= 1u << 19;
                 }
-                ps = make_uchar4((unsigned char)env.r, (unsigned char)env.c, (unsigned char)env.facing,
-                                 (unsigned char)env.sel);
+                ps = env.pose();
                 bits |= ((uint32_t)o.reward & 0xFFFFu) | ((uint32_t)o.done << 16) | ((uint32_t)o.result << 17);
             }
-            if (p.auto_reset) {
-                // queue the finished envs; reset_list_kernel (next in the stream, one warp per env at full occupancy)
-                // regenerates them and overwrites their observation rows
-                const uint32_t bal = __ballot_sync(0xFFFFFFFFu, did_reset);
-                if (bal != 0) {
-                    int base = 0;
-                    if (lane == 0) base = atomicAdd(p.reset_count, __popc(bal));
-                    base = __shfl_sync(0xFFFFFFFFu, base, 0);
-                    if (did_reset) p.reset_list[base + __popc(bal & ((1u << lane) - 1u))] = (int)e;
-                }
-            }
+            // queue the finished envs; reset_list_kernel (next in the stream, one warp per env at full occupancy)
+            // regenerates them and overwrites their observation rows
+            if (p.auto_reset) queue_resets(p, lane, e, did_reset);
         }
         if (mine) {                                                   // one 16-byte record per lane, written by its stepping warp
             TileOut t;
@@ -639,16 +688,14 @@ __global__ void __launch_bounds__(512) step1_kernel(const __grid_constant__ Step
     }
     group_sync<kOne>(grp, G);                                               // step results (grid, inventory, hand-over) visible to the group
     ps = sout[lane].ps;
-    env.r = ps.x; env.c = ps.y; env.facing = ps.z; env.sel = ps.w;
+    env.set_pose(ps);
     if (kAlias && stepping) {                                         // the inventory tile leaves before its rows are overwritten
         if (full_tile) {
             fence_async_smem();
             group_sync<kOne>(grp, G);
             if (gt == 0) { bulk_s2g(ginv, sinv, (uint32_t)p.inv_bytes); bulk_commit(); }
         } else {
-            const uint4* s4 = reinterpret_cast<const uint4*>(sinv);
-            uint4* d4 = reinterpret_cast<uint4*>(ginv);
-            for (int i = gt; i < (p.inv_bytes >> 4); i += 32 * G) d4[i] = s4[i];
+            copy16(ginv, sinv, p.inv_bytes, gt, 32 * G);
         }
     }
 
@@ -659,20 +706,15 @@ __global__ void __launch_bounds__(512) step1_kernel(const __grid_constant__ Step
             sink.init(p.obs_format);
             const bool look = valid && cfg.n_beams > 0;
             if (look) {
-                LidarLuts luts;
-                if (NC > 0) { luts.slot = sslot + cfg_i * NGW_MAX_ITEMS; luts.firstk = sfirstk; }
-                else { luts.slot = p.dcfgs[cfg_i].c.lidar_slot; luts.firstk = p.dcfgs[cfg_i].lidar.firstk; }
+                LidarLuts luts = lane_luts<NC>(p, sfirstk, sslot, cfg_i);
                 if (NC > 1 && !p.lidar_uniform) luts.slot = nullptr;
                 lidar_observe<false, RegSink<NGW_REGSINK_TAIL> >(env, dc, (NC > 1 && p.lidar_uniform) ? args.cfg[0].lidar : dc.lidar,
                                                                  luts, sink, szero, g, G, g == G - 1);
             }
             if (gt == 0) bulk_wait_read<0>();                         // the inventory store has read its rows
             group_sync<kOne>(grp, G);                                 // ... and every warp is done with the grid rows
-            {
-                const uint32_t z0 = smem_u32(sobs), zend = z0 + min(in_bytes, 32u * (uint32_t)p.obs_srow);
-                for (uint32_t a = z0 + (uint32_t)gt * 16u; a < zend; a += 512u * (uint32_t)G)
-                    asm volatile("st.shared.v4.b32 [%0], {%1, %1, %1, %1};" ::"r"(a), "r"(0) : "memory");
-            }
+            zero_span(smem_u32(sobs) + (uint32_t)gt * 16u, smem_u32(sobs) + min(in_bytes, 32u * (uint32_t)p.obs_srow),
+                      512u * (uint32_t)G);
             group_sync<kOne>(grp, G);
             if (look) {
                 sink.flush(smem_u32(sobs) + (uint32_t)(lane * p.obs_srow), smem_u32(gbase + 16), cfg.n_lidar_items,
@@ -684,9 +726,7 @@ __global__ void __launch_bounds__(512) step1_kernel(const __grid_constant__ Step
         ObsRow orow;
         orow.p = sobs + lane * p.obs_srow;
         orow.fmt = p.obs_format;
-        LidarLuts luts;
-        if (NC > 0) { luts.slot = sslot + cfg_i * NGW_MAX_ITEMS; luts.firstk = sfirstk; }
-        else { luts.slot = p.dcfgs[cfg_i].c.lidar_slot; luts.firstk = p.dcfgs[cfg_i].lidar.firstk; }
+        LidarLuts luts = lane_luts<NC>(p, sfirstk, sslot, cfg_i);
         if (p.lidar_mode == 1) {                                      // every config: line gather, one shared geometry
             const int sel = lidar_line_share(g, G);
             if (sel) lidar_lines<false, ObsRow>(env, cfg, (NC > 0) ? args.cfg[0].lidar : dc.lidar, luts, orow, sel);
@@ -702,33 +742,13 @@ __global__ void __launch_bounds__(512) step1_kernel(const __grid_constant__ Step
     //      writes to the tiles before the async proxy reads them (fence before the barrier), then one thread issues.
     fence_async_smem();
     group_sync<kOne>(grp, G);
-    const bool padded_rows = p.obs_srow != p.obs_row_bytes;
     if (full_tile) {
         if (!kAlias && gt == 0 && stepping) bulk_s2g(ginv, sinv, (uint32_t)p.inv_bytes);
-        if (p.obs != nullptr) {
-            unsigned char* gobs = p.obs + e0 * p.obs_row_bytes;
-            if (!padded_rows) {                                       // the tile is one contiguous span on both sides
-                if (gt == 0) bulk_s2g_hint(gobs, sobs, (uint32_t)p.obs_bytes, pol_first);
-            } else if (g == 0) {                                      // padded rows in shared memory: lane l stores row l
-                bulk_s2g_hint(gobs + lane * p.obs_row_bytes, sobs + lane * p.obs_srow, (uint32_t)p.obs_row_bytes,
-                              lane == 0 ? pol_first : policy_evict_first());
-            }
-        }
+        if (p.obs != nullptr && g == 0) store_obs_tile(p, e0, sobs, lane, pol_first);
         if (g == 0) bulk_commit();
     } else {
-        if (stepping && !kAlias) {
-            const uint4* s4 = reinterpret_cast<const uint4*>(sinv);
-            uint4* d4 = reinterpret_cast<uint4*>(ginv);
-            for (int i = gt; i < (p.inv_bytes >> 4); i += 32 * G) d4[i] = s4[i];
-        }
-        if (p.obs != nullptr) {
-            const int rows = (int)(p.env_end - e0 < 32 ? p.env_end - e0 : 32), words = p.obs_row_bytes >> 2;
-            for (int r = 0; r < rows; r++) {
-                uint32_t* grow = reinterpret_cast<uint32_t*>(p.obs + (e0 + r) * p.obs_row_bytes);
-                const uint32_t* srow = reinterpret_cast<const uint32_t*>(sobs + r * p.obs_srow);
-                for (int i = gt; i < words; i += 32 * G) grow[i] = srow[i];
-            }
-        }
+        if (stepping && !kAlias) copy16(ginv, sinv, p.inv_bytes, gt, 32 * G);
+        if (p.obs != nullptr) copy_obs_rows(p, e0, sobs, p.obs_srow, gt, 32 * G);
     }
 
     // ---- per-env outputs (full lines, one warp) and episode statistics, behind the tile stores
@@ -776,14 +796,7 @@ __global__ void __launch_bounds__(512) step1_kernel(const __grid_constant__ Step
             if (flush) {
                 const int n_step = a_tot & 1023, n_done = (a_tot >> 10) & 1023, n_succ = (a_tot >> 20) & 1023;
                 const int n_reset = b_tot & 1023, n_inv = (b_tot >> 10) & 1023;
-                double* sg = p.stats + (size_t)(blockIdx.x % NGW_STAT_SLOTS) * NGW_STAT_COUNT;
-                atomicAdd(&sg[NGW_STAT_STEPS], (double)(n_step - n_inv));
-                atomicAdd(&sg[NGW_STAT_REWARD_SUM], (double)r_tot);
-                atomicAdd(&sg[NGW_STAT_COST_SUM], (double)c_tot);
-                if (n_done) atomicAdd(&sg[NGW_STAT_EPISODES], (double)n_done);
-                if (n_succ) atomicAdd(&sg[NGW_STAT_SUCCESSES], (double)n_succ);
-                if (n_reset) atomicAdd(&sg[NGW_STAT_RESETS], (double)n_reset);
-                if (n_inv) atomicAdd(&sg[NGW_STAT_INVALID], (double)n_inv);
+                flush_stats(p.stats, blockIdx.x, n_step - n_inv, r_tot, c_tot, n_done, n_succ, n_reset, n_inv);
             }
         }
     }
@@ -811,11 +824,6 @@ __global__ void __launch_bounds__(512) step1_kernel(const __grid_constant__ Step
 //   outputs pose / reward / step_cost / done / result straight from registers (lane = env: full lines), statistics
 #define NGW_WTILE_HDR 128            // mbarrier (8) | dump word at +16
 #define NGW_WCTA_HDR 384            // [0] tiles done | per-warp statistics partials at +64: int4[16]
-
-__device__ __forceinline__ void zero_span(uint32_t a, uint32_t end) {      // 16 bytes per lane, 512 per warp and pass
-#pragma unroll 4
-    for (; a < end; a += 512u) asm volatile("st.shared.v4.b32 [%0], {%1, %1, %1, %1};" ::"r"(a), "r"(0) : "memory");
-}
 
 // NT: compile-time bound of the inventory tail kept in registers (8 when every config has n_inv_obs <= 8, else 16)
 template <int NC, int NT>
@@ -847,16 +855,7 @@ __global__ void __launch_bounds__(512, 2) step1w_kernel(const __grid_constant__ 
     // ---- prologue without global state
     if (threadIdx.x == 0) scta[0] = 0;
     if (lane == 0 && wid < p.tiles_per_cta) mbar_init(bar, 1);   // (the CTA's last warp is the gate warp: it owns no tile)
-    if (NC > 0) {
-        if (threadIdx.x < NGW_MAX_MAP_SIZE / 4)
-            reinterpret_cast<uint32_t*>(sfirstk)[threadIdx.x] =
-                reinterpret_cast<const uint32_t*>(args.cfg[0].lidar.firstk)[threadIdx.x];
-#pragma unroll
-        for (int k = 0; k < NC; k++)
-            if (threadIdx.x < NGW_MAX_ITEMS / 4)
-                reinterpret_cast<uint32_t*>(sslot + k * NGW_MAX_ITEMS)[threadIdx.x] =
-                    reinterpret_cast<const uint32_t*>(args.cfg[k].c.lidar_slot)[threadIdx.x];
-    }
+    stage_lidar_luts<NC>(args, sfirstk, sslot);
     __syncthreads();                                                  // the only CTA-wide barrier
 
     // The GATE warp (the CTA's last) keeps the stream's order: it waits for the preceding grid and only then lets the
@@ -872,11 +871,7 @@ __global__ void __launch_bounds__(512, 2) step1w_kernel(const __grid_constant__ 
     int32_t* ginv = p.inv + e0 * p.inv_stride;
     const uint64_t pol_first = policy_evict_first();
     auto issue_loads = [&]() {
-        if (lane == 0) {
-            mbar_expect_tx(bar, in_bytes);
-            bulk_g2s_hint(smap, gmap, (uint32_t)p.map_bytes, bar, pol_first);
-            bulk_g2s_hint(sinv, ginv, (uint32_t)p.inv_bytes, bar, pol_first);
-        }
+        if (lane == 0) issue_tile_loads(p, bar, smap, gmap, sinv, ginv, pol_first);
     };
     uchar4 ps = make_uchar4(0, 0, 0, 0);
     const bool early = p.early_state && active;
@@ -885,7 +880,7 @@ __global__ void __launch_bounds__(512, 2) step1w_kernel(const __grid_constant__ 
         ps = __ldcg(&p.pose[e]);   // L2 only: launches overlap, an SM's L1 is not a safe place for another grid's data
     }
     // the part of the observation tile that lies beyond the rows it aliases is zeroed while the loads fly
-    zero_span(region_a + in_bytes + (uint32_t)lane * 16u, region_a + obs_tile);
+    zero_span(region_a + in_bytes + (uint32_t)lane * 16u, region_a + obs_tile, 512u);
     if (!p.concurrent) asm volatile("griddepcontrol.wait;" ::: "memory");   // previous kernel of the stream done + visible
     // (the gate warp has let the dependent launch start by now or will: it is co-resident — half an SM per launch)
     if (!active) return;
@@ -895,7 +890,7 @@ __global__ void __launch_bounds__(512, 2) step1w_kernel(const __grid_constant__ 
     }
 
     const int cfg_i = (NC == 1) ? 0 : (int)__ldcg(&p.cfg_id[e]);
-    const DevConfig& dc = (NC == 1) ? args.cfg[0] : (NC > 1 ? args.cfg[cfg_i] : p.dcfgs[cfg_i]);
+    const DevConfig& dc = args.config(cfg_i);
     const ngw_config& cfg = dc.c;
     int action = 0;
     if (stepping && valid) action = __ldcg(&p.actions[e]);
@@ -907,47 +902,28 @@ __global__ void __launch_bounds__(512, 2) step1w_kernel(const __grid_constant__ 
     env.gm = p.map + e * p.cells;
     env.inv = sinv + lane * p.inv_stride;
     env.ms = p.ms;
-    env.r = ps.x; env.c = ps.y; env.facing = ps.z; env.sel = ps.w;
+    env.set_pose(ps);
 
     // ---- step
     uint32_t counts = 0;                                              // steps | episodes << 6 | successes << 12 | resets << 18 | invalid << 24
     StepOut o;
-    o.reward = 0; o.done = 0; o.result = 0; o.cost = 0.0f; o.msg = 0; o.goal = 0;
+    o.clear();
     if (stepping) {
         int did_reset = 0;
         if (valid) {
-            ngw_action_entry a;
-            a.op = NGW_OP_INVALID;
-            if (action >= 0 && action < cfg.n_actions) {
-                uint2 raw = *reinterpret_cast<const uint2*>(&cfg.actions[action]);
-                memcpy(&a, &raw, sizeof(a));
-            }
+            const ngw_action_entry a = decode_action(cfg, action);
             counts = 1u;
             if (a.op == NGW_OP_INVALID) {                             // wrappers.py:76 / pogostick_v1_env.py:236 would raise
                 counts |= 1u << 24;
                 atomicOr(&p.err[e], NGW_ERR_INVALID_ACTION);
             } else {
                 step_env(env, cfg, a, o);
-                int finished = o.done;
-                if (p.max_episode_steps > 0) {
-                    int len = __ldcg(&p.ep_len[e]) + 1;
-                    if (len >= p.max_episode_steps) { finished = 1; o.done = 1; }   // harness truncation knob
-                    p.ep_len[e] = finished && p.auto_reset ? 0 : len;
-                }
-                did_reset = finished && p.auto_reset;
+                did_reset = end_of_step(p, e, o);
                 counts |= ((uint32_t)o.done << 6) | ((uint32_t)o.goal << 12) | ((uint32_t)did_reset << 18);
             }
-            ps = make_uchar4((unsigned char)env.r, (unsigned char)env.c, (unsigned char)env.facing, (unsigned char)env.sel);
+            ps = env.pose();
         }
-        if (p.auto_reset) {                                           // queue the finished envs for reset_list_kernel
-            const uint32_t bal = __ballot_sync(0xFFFFFFFFu, did_reset);
-            if (bal != 0) {
-                int base = 0;
-                if (lane == 0) base = atomicAdd(p.reset_count, __popc(bal));
-                base = __shfl_sync(0xFFFFFFFFu, base, 0);
-                if (did_reset) p.reset_list[base + __popc(bal & ((1u << lane) - 1u))] = (int)e;
-            }
-        }
+        if (p.auto_reset) queue_resets(p, lane, e, did_reset);       // queue the finished envs for reset_list_kernel
         // ---- store 1: the inventory tile leaves as soon as the step is done
         if (full_tile) {
             fence_async_smem();
@@ -955,9 +931,7 @@ __global__ void __launch_bounds__(512, 2) step1w_kernel(const __grid_constant__ 
             if (lane == 0) { bulk_s2g(ginv, sinv, (uint32_t)p.inv_bytes); bulk_commit(); }
         } else {
             __syncwarp();
-            const uint4* s4 = reinterpret_cast<const uint4*>(sinv);
-            uint4* d4 = reinterpret_cast<uint4*>(ginv);
-            for (int i = lane; i < (p.inv_bytes >> 4); i += 32) d4[i] = s4[i];
+            copy16(ginv, sinv, p.inv_bytes, lane, 32);
         }
     }
 
@@ -967,16 +941,14 @@ __global__ void __launch_bounds__(512, 2) step1w_kernel(const __grid_constant__ 
         sink.init(p.obs_format);
         const bool look = valid && cfg.n_beams > 0;
         if (look) {
-            LidarLuts luts;
-            if (NC > 0) { luts.slot = sslot + cfg_i * NGW_MAX_ITEMS; luts.firstk = sfirstk; }
-            else { luts.slot = p.dcfgs[cfg_i].c.lidar_slot; luts.firstk = p.dcfgs[cfg_i].lidar.firstk; }
+            const LidarLuts luts = lane_luts<NC>(p, sfirstk, sslot, cfg_i);
             lidar_lines<false, RegSink<NT> >(env, cfg, (NC > 0) ? args.cfg[0].lidar : dc.lidar, luts, sink, 0xF);
             obs_tail<RegSink<NT>, NT>(env, cfg, sink, dc.lidar.tail_first);
         }
         // ---- store 2: the rows have been consumed (and read by the inventory store) -> the region becomes the observation tile
         if (lane == 0) bulk_wait_read<0>();
         __syncwarp();
-        zero_span(region_a + (uint32_t)lane * 16u, region_a + (in_bytes < obs_tile ? in_bytes : obs_tile));
+        zero_span(region_a + (uint32_t)lane * 16u, region_a + (in_bytes < obs_tile ? in_bytes : obs_tile), 512u);
         __syncwarp();
         if (look) {
             sink.flush(region_a + (uint32_t)(lane * p.obs_srow), smem_u32(gbase + 16), cfg.n_lidar_items,
@@ -985,21 +957,11 @@ __global__ void __launch_bounds__(512, 2) step1w_kernel(const __grid_constant__ 
         if (full_tile) {
             fence_async_smem();
             __syncwarp();
-            unsigned char* gobs = p.obs + e0 * p.obs_row_bytes;
-            if (p.obs_srow == p.obs_row_bytes) {                      // the tile is one contiguous span on both sides
-                if (lane == 0) bulk_s2g_hint(gobs, sobs, (uint32_t)p.obs_bytes, pol_first);
-            } else {                                                  // padded rows in shared memory: lane l stores row l
-                bulk_s2g_hint(gobs + lane * p.obs_row_bytes, sobs + lane * p.obs_srow, (uint32_t)p.obs_row_bytes, pol_first);
-            }
+            store_obs_tile(p, e0, sobs, lane, pol_first);
             bulk_commit();
         } else {
             __syncwarp();
-            const int rows = (int)(p.env_end - e0 < 32 ? p.env_end - e0 : 32), words = p.obs_row_bytes >> 2;
-            for (int r = 0; r < rows; r++) {
-                uint32_t* grow = reinterpret_cast<uint32_t*>(p.obs + (e0 + r) * p.obs_row_bytes);
-                const uint32_t* srow = reinterpret_cast<const uint32_t*>(sobs + r * p.obs_srow);
-                for (int i = lane; i < words; i += 32) grow[i] = srow[i];
-            }
+            copy_obs_rows(p, e0, sobs, p.obs_srow, lane, 32);
         }
     }
 
@@ -1042,14 +1004,7 @@ __global__ void __launch_bounds__(512, 2) step1w_kernel(const __grid_constant__ 
             if (lane == 0) {
                 const int n_step = a_tot & 1023, n_done = (a_tot >> 10) & 1023, n_succ = (a_tot >> 20) & 1023;
                 const int n_reset = b_tot & 1023, n_inv = (b_tot >> 10) & 1023;
-                double* sg = p.stats + (size_t)(blockIdx.x % NGW_STAT_SLOTS) * NGW_STAT_COUNT;
-                atomicAdd(&sg[NGW_STAT_STEPS], (double)(n_step - n_inv));
-                atomicAdd(&sg[NGW_STAT_REWARD_SUM], (double)r_tot);
-                atomicAdd(&sg[NGW_STAT_COST_SUM], (double)c_tot);
-                if (n_done) atomicAdd(&sg[NGW_STAT_EPISODES], (double)n_done);
-                if (n_succ) atomicAdd(&sg[NGW_STAT_SUCCESSES], (double)n_succ);
-                if (n_reset) atomicAdd(&sg[NGW_STAT_RESETS], (double)n_reset);
-                if (n_inv) atomicAdd(&sg[NGW_STAT_INVALID], (double)n_inv);
+                flush_stats(p.stats, blockIdx.x, n_step - n_inv, r_tot, c_tot, n_done, n_succ, n_reset, n_inv);
             }
         }
     }
@@ -1177,16 +1132,7 @@ __global__ void __launch_bounds__(64, 14) rollout2_kernel(const __grid_constant_
     const int8_t* gmap = p.map + e0 * p.cells;
     int32_t* ginv = p.inv + e0 * p.inv_stride;
     if (threadIdx.x == 0) mbar_init(bar, 1);
-    if (NC > 0) {
-        if (threadIdx.x < NGW_MAX_MAP_SIZE / 4)
-            reinterpret_cast<uint32_t*>(sfirstk)[threadIdx.x] =
-                reinterpret_cast<const uint32_t*>(args.cfg[0].lidar.firstk)[threadIdx.x];
-#pragma unroll
-        for (int k = 0; k < NC; k++)
-            if (threadIdx.x < NGW_MAX_ITEMS / 4)
-                reinterpret_cast<uint32_t*>(sslot + k * NGW_MAX_ITEMS)[threadIdx.x] =
-                    reinterpret_cast<const uint32_t*>(args.cfg[k].c.lidar_slot)[threadIdx.x];
-    }
+    stage_lidar_luts<NC>(args, sfirstk, sslot);
     __syncthreads();
     asm volatile("griddepcontrol.wait;" ::: "memory");
     if (threadIdx.x == 0) {
@@ -1203,12 +1149,10 @@ __global__ void __launch_bounds__(64, 14) rollout2_kernel(const __grid_constant_
         }
     }
     const int cfg_i = (NC == 1) ? 0 : (int)p.cfg_id[valid ? e : e0];
-    const DevConfig& dc = (NC == 1) ? args.cfg[0] : (NC > 1 ? args.cfg[cfg_i] : p.dcfgs[cfg_i]);
+    const DevConfig& dc = args.config(cfg_i);
     const ngw_config& cfg = dc.c;
     const LidarDev& geom = (NC > 0) ? args.cfg[0].lidar : dc.lidar;
-    LidarLuts luts;
-    if (NC > 0) { luts.slot = sslot + cfg_i * NGW_MAX_ITEMS; luts.firstk = sfirstk; }
-    else { luts.slot = p.dcfgs[cfg_i].c.lidar_slot; luts.firstk = p.dcfgs[cfg_i].lidar.firstk; }
+    const LidarLuts luts = lane_luts<NC>(p, sfirstk, sslot, cfg_i);
     const bool given_actions = A4 == 0 && !p.random_policy;
     uchar4 ps = p.pose[valid ? e : e0];
     int action = 0;
@@ -1221,10 +1165,10 @@ __global__ void __launch_bounds__(64, 14) rollout2_kernel(const __grid_constant_
     env.gm = p.map + e * p.cells;
     env.inv = sinv + el * p.inv_stride;
     env.ms = p.ms;
-    env.r = ps.x; env.c = ps.y; env.facing = ps.z; env.sel = ps.w;
+    env.set_pose(ps);
 
     StepOut o;
-    o.reward = 0; o.done = 0; o.result = 0; o.cost = 0.0f; o.msg = 0; o.goal = 0;
+    o.clear();
     float cost_sum = 0.0f;
     int reward_sum = 0, n_done = 0, n_succ = 0, n_reset = 0, n_invalid = 0;
     const int n_lidar = cfg.n_lidar_items * cfg.n_beams;
@@ -1265,7 +1209,8 @@ __global__ void __launch_bounds__(64, 14) rollout2_kernel(const __grid_constant_
         __syncwarp();                                                 // the high lanes have read the rows
         if (valid && low) {
             if (p.actions_out != nullptr) p.actions_out[t * p.act_stride + e] = action;
-            o.reward = 0; o.done = 0; o.result = 0; o.cost = 0.0f; o.msg = 0; o.goal = 0;
+            o.clear();
+            // (decode_action, inlined by hand: the call shifts this kernel's spills)
             ngw_action_entry a;
             a.op = NGW_OP_INVALID;
             if (action >= 0 && action < cfg.n_actions) {
@@ -1290,10 +1235,10 @@ __global__ void __launch_bounds__(64, 14) rollout2_kernel(const __grid_constant_
         }
         if (p.auto_reset) {
             if (__ballot_sync(0xFFFFFFFFu, did_reset) != 0) {         // regenerate in place, warp-cooperatively (this warp's 16 envs)
-                uchar4 q = make_uchar4((unsigned char)env.r, (unsigned char)env.c, (unsigned char)env.facing, (unsigned char)env.sel);
+                uchar4 q = env.pose();
                 auto_reset_warp(p, p.dcfgs, cfg_i, did_reset != 0, smap + 16 * g * p.cells, sinv + 16 * g * p.inv_stride,
                                 sscratch, e0 + 16 * g, q);
-                env.r = q.x; env.c = q.y; env.facing = q.z; env.sel = q.w;
+                env.set_pose(q);
             }
         }
         // the pair's high lane follows the low lane's pose; the step's writes to the tile become visible to it
@@ -1308,7 +1253,7 @@ __global__ void __launch_bounds__(64, 14) rollout2_kernel(const __grid_constant_
 
     // ---- outputs and statistics (low lanes own them)
     if (valid && low) {
-        p.pose[e] = make_uchar4((unsigned char)env.r, (unsigned char)env.c, (unsigned char)env.facing, (unsigned char)env.sel);
+        p.pose[e] = env.pose();
         p.reward[e] = (float)reward_sum;
         p.done[e] = (uint8_t)o.done;
         p.cost[e] = cost_sum;
@@ -1321,16 +1266,7 @@ __global__ void __launch_bounds__(64, 14) rollout2_kernel(const __grid_constant_
     const int s_done = __reduce_add_sync(0xFFFFFFFFu, n_done), s_succ = __reduce_add_sync(0xFFFFFFFFu, n_succ);
     const int s_reset = __reduce_add_sync(0xFFFFFFFFu, n_reset), s_inv = __reduce_add_sync(0xFFFFFFFFu, n_invalid);
     const float s_cost = warp_sum(cost_sum);
-    if (lane == 0) {
-        double* sg = p.stats + (size_t)(blockIdx.x % NGW_STAT_SLOTS) * NGW_STAT_COUNT;
-        atomicAdd(&sg[NGW_STAT_STEPS], (double)s_steps);
-        atomicAdd(&sg[NGW_STAT_REWARD_SUM], (double)s_rew);
-        atomicAdd(&sg[NGW_STAT_COST_SUM], (double)s_cost);
-        if (s_done) atomicAdd(&sg[NGW_STAT_EPISODES], (double)s_done);
-        if (s_succ) atomicAdd(&sg[NGW_STAT_SUCCESSES], (double)s_succ);
-        if (s_reset) atomicAdd(&sg[NGW_STAT_RESETS], (double)s_reset);
-        if (s_inv) atomicAdd(&sg[NGW_STAT_INVALID], (double)s_inv);
-    }
+    if (lane == 0) flush_stats(p.stats, blockIdx.x, s_steps, s_rew, s_cost, s_done, s_succ, s_reset, s_inv);
 
     // ---- inventory tile out, final observation into the aliased region, observation tile out
     fence_async_smem();
@@ -1339,9 +1275,7 @@ __global__ void __launch_bounds__(64, 14) rollout2_kernel(const __grid_constant_
     if (full_tile) {
         if (threadIdx.x == 0) { bulk_s2g(ginv, sinv, (uint32_t)p.inv_bytes); bulk_commit(); }
     } else {
-        const uint4* s4 = reinterpret_cast<const uint4*>(sinv);
-        uint4* d4 = reinterpret_cast<uint4*>(ginv);
-        for (int i = threadIdx.x; i < (p.inv_bytes >> 4); i += 64) d4[i] = s4[i];
+        copy16(ginv, sinv, p.inv_bytes, threadIdx.x, 64);
     }
     if (p.obs != nullptr) {
         uint32_t hit[4] = {0u, 0u, 0u, 0u};
@@ -1358,8 +1292,7 @@ __global__ void __launch_bounds__(64, 14) rollout2_kernel(const __grid_constant_
         if (threadIdx.x == 0) bulk_wait_read<0>();
         __syncthreads();                                              // rows consumed by everyone (and by the inventory store)
         const uint32_t region_a = smem_u32(region);
-        for (uint32_t a = region_a + threadIdx.x * 16u; a < region_a + (uint32_t)p.obs_bytes; a += 1024u)
-            asm volatile("st.shared.v4.b32 [%0], {%1, %1, %1, %1};" ::"r"(a), "r"(0) : "memory");
+        zero_span(region_a + threadIdx.x * 16u, region_a + (uint32_t)p.obs_bytes, 1024u);
         __syncthreads();
         if (look) {
             ObsRow orow;
@@ -1383,6 +1316,7 @@ __global__ void __launch_bounds__(64, 14) rollout2_kernel(const __grid_constant_
             }
         } else {
             __syncthreads();
+            // the rows are contiguous on both sides: one flat copy (copy_obs_rows costs this kernel spill stores)
             const int n = (int)((p.env_end - e0 < 32 ? p.env_end - e0 : 32)) * (p.obs_row_bytes >> 2);
             uint32_t* gobs = reinterpret_cast<uint32_t*>(p.obs + e0 * p.obs_row_bytes);
             const uint32_t* so = reinterpret_cast<const uint32_t*>(sobs);
