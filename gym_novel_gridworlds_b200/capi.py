@@ -85,6 +85,7 @@ EXPORTS = {
                            C.c_int32, C.c_int32, C.c_void_p]),
     'ngw_step_many': (C.c_int, [C.c_void_p, C.c_int32, C.c_int32, C.c_int32, C.c_void_p]),
     'ngw_set_message_buffer': (C.c_int, [C.c_void_p, C.c_void_p]),
+    'ngw_set_episode_end_buffers': (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p]),
     'ngw_step_host': (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
                                 C.c_int32, C.c_int32]),
     'ngw_rollout': (C.c_int, [C.c_void_p, C.c_void_p, C.c_int32, C.c_uint64, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,

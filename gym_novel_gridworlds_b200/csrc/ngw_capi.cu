@@ -433,6 +433,7 @@ static ResetParams reset_params(ngw_handle* h, const uint8_t* mask, int phase) {
     p.ep_len = h->ep_len; p.err = h->err; p.mask = mask; p.n_envs = h->n; p.first_gid = h->first_gid; p.seed = h->seed;
     p.ms = h->ms; p.cells = h->cells; p.inv_stride = h->inv_stride; p.phase = phase; p.zero_byte = h->zero_byte;
     p.reset_list = h->reset_list; p.reset_count = h->reset_ctl; p.done_ctas = h->reset_ctl + 1; p.obs = nullptr;
+    p.final_obs = nullptr;
     p.obs_dim = h->obs_dim; p.obs_row_bytes = h->obs_row_bytes; p.obs_format = h->obs_format;
     p.key_mask = h->key_mask;
     return p;
@@ -484,6 +485,10 @@ static StepParams step_params(ngw_handle* h, const int32_t* actions, void* obs, 
     p.auto_reset = auto_reset; p.max_episode_steps = max_episode_steps;
     p.lidar_uniform = h->lidar_uniform ? 1 : 0;
     p.msg = h->msg; p.reset_list = h->reset_list; p.reset_count = h->reset_ctl;
+    // episode-end buffers: stepping launches only (observe-only launches leave them alone; the rollouts clear them), and
+    // a final observation only where there is one
+    p.trunc = actions != nullptr ? h->trunc : nullptr;
+    p.final_obs = actions != nullptr && p.obs != nullptr ? h->final_obs : nullptr;
     p.n_steps = 1;
     return p;
 }
@@ -519,6 +524,8 @@ static StreamTail launch_tail(const StepParams& p) {
     add(me.wr, me.n_wr, p.reward, (size_t)n_env * 4); add(me.wr, me.n_wr, p.cost, (size_t)n_env * 4);
     add(me.wr, me.n_wr, p.done, (size_t)n_env); add(me.wr, me.n_wr, p.result, (size_t)n_env);
     add(me.wr, me.n_wr, p.msg, (size_t)n_env * 2);
+    // (the queued-reset kernel behind the step writes final_obs: the step's record covers it, see launch_step)
+    add(me.wr, me.n_wr, p.trunc, (size_t)n_env); add(me.wr, me.n_wr, p.final_obs, (size_t)n_env * p.obs_row_bytes);
     return me;
 }
 
@@ -651,6 +658,7 @@ static int launch_step(ngw_handle* h, const StepParams& p, cudaStream_t s) {
     if (p.actions != nullptr && p.auto_reset && !is_multi(p)) {     // regenerate the episodes the step kernel queued
         ResetParams rp = reset_params(h, nullptr, 2);
         rp.obs = p.obs;
+        rp.final_obs = p.final_obs;
         // Grid: alone, four CTAs per SM regenerate the queue fastest (C5: ~2000 envs in 52 us).  When this step overlapped
         // its predecessor — rotating handles inside a capture — the NEXT handle's step will overlap this kernel: then ONE
         // CTA per SM (11 KB, 16 K registers) fits next to that step's full set of CTAs and the resets hide behind it.
@@ -723,6 +731,7 @@ int ngw_rollout(ngw_handle* h, const int32_t* actions, int32_t n_steps, uint64_t
                                0, h->n);
     p.n_steps = n_steps; p.random_policy = actions ? 0 : 1; p.act_stride = h->n; p.policy_seed = policy_seed;
     p.done_count = done_count; p.actions_out = actions_out;
+    p.trunc = nullptr; p.final_obs = nullptr;              // per-step episode ends have no place in a rollout's sums
     return launch_step(h, p, (cudaStream_t)stream);
 }
 
@@ -745,6 +754,7 @@ int ngw_rollout_policy(ngw_handle* h, const int32_t* weights, const int32_t* bia
                                last_result, auto_reset, max_episode_steps, 0, h->n);
     p.n_steps = n_steps; p.random_policy = 0; p.act_stride = h->n; p.done_count = done_count; p.actions_out = actions_out;
     p.policy_w = weights; p.policy_b = bias; p.policy_actions = n_policy_actions;
+    p.trunc = nullptr; p.final_obs = nullptr;
     return launch_step(h, p, (cudaStream_t)stream);
 }
 
@@ -788,6 +798,14 @@ static int ensure_host_path(ngw_handle* h) {
 int ngw_set_message_buffer(ngw_handle* h, uint16_t* msg_dev) {
     if (!h) return fail("null handle");
     h->msg = msg_dev;
+    return 0;
+}
+
+int ngw_set_episode_end_buffers(ngw_handle* h, uint8_t* truncated_dev, void* final_obs_dev) {
+    if (!h) return fail("null handle");
+    if ((uintptr_t)final_obs_dev & 15) return fail("ngw_set_episode_end_buffers: final_obs must be 16-byte aligned");
+    h->trunc = truncated_dev;
+    h->final_obs = static_cast<unsigned char*>(final_obs_dev);
     return 0;
 }
 

@@ -30,6 +30,8 @@ struct ngw_handle {
     uint32_t* episode = nullptr; int32_t* ep_len = nullptr; uint32_t* err = nullptr; double* stats = nullptr;
     uint8_t* zero_byte = nullptr;
     uint16_t* msg = nullptr;                       // caller-owned message-code buffer (ngw_set_message_buffer)
+    uint8_t* trunc = nullptr;                      // caller-owned episode-end buffers (ngw_set_episode_end_buffers): truncated
+    unsigned char* final_obs = nullptr;            // flags, last observation rows of auto-reset envs
     int32_t* reset_list = nullptr; int32_t* reset_ctl = nullptr;   // auto-reset queue; ctl[0] = count, ctl[1] = finished CTAs
     int sm_count = 148;
     long long launches = 0, concurrent_launches = 0;
@@ -51,7 +53,8 @@ struct StreamTail {                       // the latest library launch on a stre
     cudaGraphNode_t node = nullptr;       // its graph node (captures only)
     bool pure_step = false;               // 'gated': a one-step launch or the queued-reset kernel behind one — kernels that let
                                           // their dependents start only after everything before THEM has completed
-    MemRange rd[2], wr[6];                // caller buffers it reads (actions) / writes (obs, reward, done, cost, result, msg)
+    MemRange rd[2], wr[8];                // caller buffers it reads (actions) / writes (obs, reward, done, cost, result, msg,
+                                          // truncated, final_obs)
     int n_rd = 0, n_wr = 0;
 };
 

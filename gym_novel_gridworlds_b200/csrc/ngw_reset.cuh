@@ -25,6 +25,7 @@ struct ResetParams {
     int32_t* reset_count;
     int32_t* done_ctas;
     unsigned char* obs;         // observation rows of obs_row_bytes bytes (layout as in the step kernel)
+    unsigned char* final_obs;   // reset_list_kernel, optional: a regenerated env's row of obs is copied here before it is replaced
     int obs_dim, obs_row_bytes, obs_format;
     uint32_t key_mask;          // 0xFFFFFFFF; test knob NGW_DEBUG_KEY_MASK forces ties between the subset-sampling keys
 };
@@ -128,6 +129,10 @@ __global__ void __launch_bounds__(32 * NGW_RESET_WARPS) reset_list_kernel(const 
             orow.p = p.obs + e * p.obs_row_bytes;
             orow.fmt = p.obs_format;
             uint32_t* row = reinterpret_cast<uint32_t*>(orow.p);
+            if (p.final_obs != nullptr) {                             // the finished episode's last observation is kept
+                uint32_t* frow = reinterpret_cast<uint32_t*>(p.final_obs + e * p.obs_row_bytes);
+                for (int k = lane; k < (p.obs_row_bytes >> 2); k += 32) frow[k] = row[k];
+            }
             for (int k = lane; k < (p.obs_row_bytes >> 2); k += 32) row[k] = 0;
             if (lane == 0) sc.hist[0] = 0;                                // a shared-memory byte that reads 0
             __syncwarp();

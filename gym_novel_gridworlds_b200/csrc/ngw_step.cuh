@@ -130,6 +130,8 @@ struct StepParams {
     uint16_t* msg;              // optional: info['message'] codes (enum ngw_msg | arg << 5)
     int32_t* reset_list;        // single-step auto-reset: finished envs are queued here ...
     int32_t* reset_count;       // ... and regenerated by reset_list_kernel right after this launch
+    uint8_t* trunc;             // optional, one-step launches: 1 where the step hit max_episode_steps and the env did not end it
+    unsigned char* final_obs;   // optional, one-step launches: reset_list_kernel copies a regenerated env's row here first
 };
 
 // Kernel argument block: the parameters plus up to NC configs INLINE, so that every config read in the hot path
@@ -202,14 +204,16 @@ __device__ __forceinline__ ngw_action_entry decode_action(const ngw_config& cfg,
 // sets o.done), the episode length, and whether the env is reset.  ld.cg: another grid may overlap this one.  (The
 // rollouts keep this inline with a plain load: there ep_len is read once per step on the step's dependent chain, and
 // ld.cg measured 1.6 % fewer env-steps/s on the C2 rollout, B200 at 1000 W.)
+// Returns did_reset | truncated << 1.  truncated is gym's TimeLimit rule: the limit was reached and the env's own step did
+// not end the episode (when both happen, the env reports terminated).
 __device__ __forceinline__ int end_of_step(const StepParams& p, long long e, StepOut& o) {
-    int finished = o.done;
+    int finished = o.done, trunc = 0;
     if (p.max_episode_steps > 0) {
         int len = __ldcg(&p.ep_len[e]) + 1;
-        if (len >= p.max_episode_steps) { finished = 1; o.done = 1; }
+        if (len >= p.max_episode_steps) { trunc = !finished; finished = 1; o.done = 1; }
         p.ep_len[e] = finished && p.auto_reset ? 0 : len;
     }
-    return finished && p.auto_reset;
+    return (finished && p.auto_reset ? 1 : 0) | (trunc << 1);
 }
 
 // whole warp: append the lanes with did_reset to the auto-reset queue that reset_list_kernel consumes
@@ -535,6 +539,7 @@ __global__ void __launch_bounds__(256) rollout_kernel(const __grid_constant__ St
 struct TileOut {            // per-env hand-over from the warp that stepped the lane: 16 bytes
     uchar4 ps;              // pose after the step
     uint32_t bits;          // reward (int16) | done << 16 | result << 17 | success << 18 | reset << 19 | invalid << 20 | stepped << 21
+                            // | truncated << 22
     float cost;
     uint32_t msg;
 };
@@ -670,8 +675,9 @@ __global__ void __launch_bounds__(512) step1_kernel(const __grid_constant__ Step
                 } else {
                     step_env(env, cfg, a, o);
                     if (o.goal) bits |= 1u << 18;
-                    did_reset = end_of_step(p, e, o);
-                    if (did_reset) bits |= 1u << 19;
+                    const int eos = end_of_step(p, e, o);
+                    did_reset = eos & 1;
+                    bits |= (uint32_t)did_reset << 19 | (uint32_t)(eos >> 1) << 22;   // bit 22: truncated
                 }
                 ps = env.pose();
                 bits |= ((uint32_t)o.reward & 0xFFFFu) | ((uint32_t)o.done << 16) | ((uint32_t)o.result << 17);
@@ -764,6 +770,7 @@ __global__ void __launch_bounds__(512) step1_kernel(const __grid_constant__ Step
             p.cost[e] = cost;
             p.result[e] = (uint8_t)((bits >> 17) & 1u);
             if (p.msg != nullptr) p.msg[e] = (uint16_t)raw.w;
+            if (p.trunc != nullptr) p.trunc[e] = (uint8_t)((bits >> 22) & 1u);
         }
         // warp reductions, then shared-memory accumulators of the CTA; the last group to arrive flushes them with one
         // set of global atomics per CTA
@@ -905,7 +912,9 @@ __global__ void __launch_bounds__(512, 2) step1w_kernel(const __grid_constant__ 
     env.set_pose(ps);
 
     // ---- step
-    uint32_t counts = 0;                                              // steps | episodes << 6 | successes << 12 | resets << 18 | invalid << 24
+    // steps | episodes << 6 | successes << 12 | resets << 18 | invalid << 24, and the lane's own truncated flag at bit 30
+    // (masked off before the counts are summed)
+    uint32_t counts = 0;
     StepOut o;
     o.clear();
     if (stepping) {
@@ -918,8 +927,10 @@ __global__ void __launch_bounds__(512, 2) step1w_kernel(const __grid_constant__ 
                 atomicOr(&p.err[e], NGW_ERR_INVALID_ACTION);
             } else {
                 step_env(env, cfg, a, o);
-                did_reset = end_of_step(p, e, o);
-                counts |= ((uint32_t)o.done << 6) | ((uint32_t)o.goal << 12) | ((uint32_t)did_reset << 18);
+                const int eos = end_of_step(p, e, o);
+                did_reset = eos & 1;
+                counts |= ((uint32_t)o.done << 6) | ((uint32_t)o.goal << 12) | ((uint32_t)did_reset << 18) |
+                          ((uint32_t)(eos >> 1) << 30);
             }
             ps = env.pose();
         }
@@ -974,10 +985,11 @@ __global__ void __launch_bounds__(512, 2) step1w_kernel(const __grid_constant__ 
             p.cost[e] = o.cost;
             p.result[e] = (uint8_t)o.result;
             if (p.msg != nullptr) p.msg[e] = (uint16_t)o.msg;
+            if (p.trunc != nullptr) p.trunc[e] = (uint8_t)(counts >> 30);
         }
         // warp reductions -> this warp's slot in shared memory; the last warp of the CTA to arrive folds the slots and
         // issues one set of global atomics per CTA
-        const uint32_t c_all = __reduce_add_sync(0xFFFFFFFFu, counts);            // five counts <= 32: 6 bits apiece
+        const uint32_t c_all = __reduce_add_sync(0xFFFFFFFFu, counts & 0x3FFFFFFFu);   // five counts <= 32: 6 bits apiece
         const int r_sum = __reduce_add_sync(0xFFFFFFFFu, o.reward);
         const float c_sum = warp_sum(o.cost);
         int4* slots = reinterpret_cast<int4*>(smem + 64);

@@ -31,7 +31,7 @@ class NovelGridworldBatchEnv(Env):
     _PLACES_TREE_TAP = False           # pogostick_v0_env.py:155-178
 
     def __init__(self, env=None, num_envs=1, device=None, seed=0, first_env_gid=0, auto_reset=False,
-                 max_episode_steps=0, messages=False, strict_actions=False, obs_format='i32'):
+                 max_episode_steps=0, messages=False, strict_actions=False, obs_format='i32', episode_end_info=False):
         self.env = env                                  # env to restore in reset (pogostick_v1_env.py:29,89-109)
         self.num_envs = int(num_envs)
         self.device = device
@@ -48,6 +48,10 @@ class NovelGridworldBatchEnv(Env):
         # rows (runtime.obs_to_vector turns the narrow ones back into the reference's vector).
         self.strict_actions = bool(strict_actions)
         self.obs_format = obs_format
+        # episode_end_info: a batched step's info also carries 'TimeLimit.truncated' (the step hit max_episode_steps and
+        # the env did not end the episode itself) and 'terminal_observation' (with auto_reset, the last observation of
+        # each finished episode, valid where done) — what a learner needs to bootstrap at a time limit
+        self.episode_end_info = bool(episode_end_info)
 
         self.map_size = 10
         self.direction_id = {'NORTH': 0, 'SOUTH': 1, 'WEST': 2, 'EAST': 3}

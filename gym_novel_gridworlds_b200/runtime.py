@@ -85,7 +85,11 @@ def obs_to_vector(rows, compiled, obs_format, cfg_ids=None):
         if cfg_ids is not None:
             cfg_ids = torch.from_numpy(np.asarray(cfg_ids, dtype=np.int64))
     width = max([cc.c.n_lidar_items * cc.c.n_beams + cc.c.n_inv_obs for cc in compiled if cc.c.n_beams > 0] or [0])
-    if obs_format == 'i32':
+    if rows.shape[0] == 0:
+        # no rows, e.g. the terminal observations of a step that ended no episode (an empty NumPy selection has strides
+        # (0, 0), which a narrow row's int32 tail view cannot take)
+        out = torch.zeros((0, width), dtype=torch.int32, device=rows.device)
+    elif obs_format == 'i32':
         out = rows[:, :width].to(torch.int32).clone()
     else:
         out = torch.zeros((rows.shape[0], width), dtype=torch.int32, device=rows.device)
@@ -319,6 +323,20 @@ class BatchHandle(object):
             self.msg = None
         return self.msg
 
+    def enable_episode_end(self, on=True):
+        """Make every following one-step call (step, step_host, StepGroup) also write self.truncated (uint8 [n]: 1 where
+        the step hit max_episode_steps and the env did not end the episode itself, gym's info['TimeLimit.truncated']) and,
+        for the envs its auto-reset regenerated, self.final_obs (rows like self.obs: the observation the step produced,
+        before the reset observation replaced it).  on=False switches both off and releases them."""
+        if on and getattr(self, 'truncated', None) is None:
+            self.truncated = torch.zeros(self.n, dtype=torch.uint8, device=self.device)
+            self.final_obs = torch.zeros_like(self.obs)
+        if not on:
+            self.truncated = self.final_obs = None
+        capi.check(self.lib, self.lib.ngw_set_episode_end_buffers(
+            self._h, _ptr(self.truncated), _ptr(self.final_obs) if self.obs_dim else None))
+        return self.truncated, self.final_obs
+
     def observe(self):
         if self.obs_dim:
             capi.check(self.lib, self.lib.ngw_observe(self._h, _ptr(self.obs), self._stream()))
@@ -469,11 +487,19 @@ def decode_message(code, compiled):
 
 
 class LazyInfo(object):
-    """info of a batched step: tensors; the reference's strings are formatted only when 'message' is asked for."""
+    """info of a batched step: tensors; the reference's strings are formatted only when 'message' is asked for.
+    `episode_end` (truncated, terminal observation rows), when given, adds 'TimeLimit.truncated' and
+    'terminal_observation'; a host-path step passes a callable that fetches them on first access."""
 
-    def __init__(self, result, step_cost, msg=None, compiled=None, cfg_ids=None, flags=None):
+    def __init__(self, result, step_cost, msg=None, compiled=None, cfg_ids=None, flags=None, episode_end=None):
         self.result, self.step_cost = result, step_cost
         self._msg, self._compiled, self._cfg_ids, self._flags = msg, compiled, cfg_ids, flags
+        self._episode_end = episode_end
+
+    def _end(self):
+        if callable(self._episode_end):
+            self._episode_end = self._episode_end()
+        return self._episode_end
 
     def __getitem__(self, key):
         if key == 'result':
@@ -489,10 +515,21 @@ class LazyInfo(object):
             if self._cfg_ids is None:
                 return [decode_message(c, self._compiled[0]) for c in codes]
             return [decode_message(c, self._compiled[int(i)]) for c, i in zip(codes, self._cfg_ids)]
+        if self._episode_end is not None and key == 'TimeLimit.truncated':
+            return self._end()[0]
+        if self._episode_end is not None and key == 'terminal_observation':
+            return self._end()[1]
         raise KeyError(key)
 
+    def __contains__(self, key):
+        return key in self.keys()
+
+    def get(self, key, default=None):
+        return self[key] if key in self.keys() else default
+
     def keys(self):
-        return ['result', 'step_cost', 'message', 'invalid']
+        keys = ['result', 'step_cost', 'message', 'invalid']
+        return keys + ['TimeLimit.truncated', 'terminal_observation'] if self._episode_end is not None else keys
 
 
 class ChainRuntime(object):
@@ -506,6 +543,7 @@ class ChainRuntime(object):
         self.auto_reset = base.auto_reset
         self.max_episode_steps = base.max_episode_steps
         self.messages = base.messages
+        self.episode_end_info = getattr(base, 'episode_end_info', False)
 
     # ------------------------------------------------------------------
     def _ensure(self):
@@ -520,6 +558,8 @@ class ChainRuntime(object):
                                       obs_format='i32' if self.base.num_envs == 1 else self.base.obs_format)
             if self.single or self.messages:
                 self.handle.enable_messages()
+            if self.episode_end_info and not self.single:       # (the reference has no auto-reset: N == 1 is unchanged)
+                self.handle.enable_episode_end()
         return self.handle
 
     def close(self):
@@ -671,12 +711,20 @@ class ChainRuntime(object):
             obs, reward, done, cost, result = h.step(action, self.auto_reset, self.max_episode_steps)
             self._check_actions(action)
             o = obs[:, lidar_cols] if cc.obs_dim else self.dict_observation()
+            end = None
+            if self.episode_end_info:
+                end = (h.truncated.view(torch.bool), h.final_obs[:, lidar_cols] if cc.obs_dim else None)
             return o, reward, done.view(torch.bool), LazyInfo(result.view(torch.bool), cost, getattr(h, 'msg', None), [cc],
-                                                              flags=h.error_flags)
+                                                              flags=h.error_flags, episode_end=end)
         obs, reward, done, cost, result = h.step_host(action, self.auto_reset, self.max_episode_steps)
         self._check_actions(action)
         o = obs[:, lidar_cols] if cc.obs_dim else self.dict_observation()
-        return o, reward, done.view(np.bool_), LazyInfo(result.view(np.bool_), cost, flags=h.error_flags)
+        end = None
+        if self.episode_end_info:
+            def end():                          # the step's device buffers, fetched on access
+                trunc = h.truncated.cpu().numpy().view(np.bool_)
+                return trunc, (h.final_obs[:, lidar_cols].cpu().numpy() if cc.obs_dim else None)
+        return o, reward, done.view(np.bool_), LazyInfo(result.view(np.bool_), cost, flags=h.error_flags, episode_end=end)
 
     def _check_actions(self, action):
         """strict_actions: raise what the reference raises as soon as one env of the batch got a rejected id."""

@@ -304,6 +304,21 @@ int ngw_step_many(const ngw_step_item* items, int32_t n_items, int32_t auto_rese
  * (NULL switches it off again; off by default — the hot path then writes nothing). */
 int ngw_set_message_buffer(ngw_handle* h, uint16_t* msg_dev);
 
+/* Optional episode-end outputs of the one-step calls (ngw_step, ngw_step_many, ngw_step_host, _begin/_end), what a learner
+ * needs to bootstrap at a time limit (gym 0.18's info['TimeLimit.truncated'], and the last observation of an episode that
+ * the auto-reset replaced).  Each pointer may be NULL, which switches that output off; both are off by default.
+ *   truncated_dev: DEVICE uint8[n_envs].  Every valid env of a call gets 1 when this step reached max_episode_steps and the
+ *                  env's own step did not end the episode (gym's TimeLimit rule), else 0; invalid-action lanes get 0.
+ *                  done == terminated | truncated, the two disjoint: an env that terminates on the limit's step reports
+ *                  terminated.  Without auto_reset an env past the limit reports done, and so truncated, on every step.
+ *   final_obs_dev: DEVICE rows of obs_row_bytes in the handle's layout, 16-byte aligned.  Row e is written only for the
+ *                  envs this call's auto-reset regenerated: the observation the step produced, byte for byte what obs
+ *                  would hold without auto_reset, before the new episode's reset observation replaced it.  Other rows
+ *                  are left untouched.  Ignored without a LidarInFront observation (obs_dim == 0) or an obs buffer.
+ * The host-buffer path writes the same DEVICE buffers on the handle's stream (valid once ngw_step_host / _end returned).
+ * ngw_observe, ngw_reset, ngw_rollout and ngw_rollout_policy never touch either buffer. */
+int ngw_set_episode_end_buffers(ngw_handle* h, uint8_t* truncated_dev, void* final_obs_dev);
+
 /* Same call with HOST buffers (the reference-facing path): copies actions in (H2D), steps, copies
  * obs/reward/done/step_cost/result out (D2H) on the handle's own stream; returns after the outputs are valid
  * on the host.  The step is ordered after everything earlier calls on this handle enqueued on the caller's streams
