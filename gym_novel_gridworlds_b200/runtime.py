@@ -724,7 +724,9 @@ class ChainRuntime(object):
             def end():                          # the step's device buffers, fetched on access
                 trunc = h.truncated.cpu().numpy().view(np.bool_)
                 return trunc, (h.final_obs[:, lidar_cols].cpu().numpy() if cc.obs_dim else None)
-        return o, reward, done.view(np.bool_), LazyInfo(result.view(np.bool_), cost, flags=h.error_flags, episode_end=end)
+        # the message codes sit in the handle's device buffer, complete once step_host returned; decoded on access
+        return o, reward, done.view(np.bool_), LazyInfo(result.view(np.bool_), cost, getattr(h, 'msg', None), [cc],
+                                                        flags=h.error_flags, episode_end=end)
 
     def _check_actions(self, action):
         """strict_actions: raise what the reference raises as soon as one env of the batch got a rejected id."""

@@ -150,7 +150,10 @@ typedef struct {
     int done;
     int result;
     float cost;
+    int msg;           /* info['message'] as enum ngw_msg | argument << 5 (include/ngw.h) */
 } out_t;
+
+static int msg_code(int kind, int arg) { return kind | (arg << 5); }
 
 /* the "Update after each step" block every step path ends with (pogostick_v1_env.py:349-357,
  * duplicated e.g. at novelty_wrappers.py:86-97): entities, then done / reward_done */
@@ -166,21 +169,28 @@ static void post_step(env_t* e, out_t* o) {
 /* craft (pogostick_v1_env.py:413-474, bow_v1_env.py:386-441, novelty_wrappers.py:371-436) */
 static void craft(env_t* e, const ngw_recipe* rc, out_t* o) {
     o->reward = -1; o->result = 1; o->cost = 0.0f;
-    int have_all = 1;
+    int missing = 0;                             /* "Missing items: ..." lists the short inputs in recipe order */
     for (int i = 0; i < rc->n_inputs; i++) {
         int item = rc->in_item[i];
-        if (item == NGW_NONE || e->inv[item] < rc->in_qty[i]) have_all = 0;
+        if (item == NGW_NONE || e->inv[item] < rc->in_qty[i]) missing |= 1 << i;
     }
-    if (!have_all) { o->result = 0; o->cost = rc->cost_missing; return; }
+    if (missing) {
+        o->result = 0; o->cost = rc->cost_missing;
+        o->msg = msg_code(NGW_MSG_MISSING, (int)(rc - e->cfg->recipes) | (missing << 3));
+        return;
+    }
     if (rc->needs_table) {
         int fr, fc;
         front_of(e, &fr, &fc);
-        if (CELL(e, fr, fc) != e->cfg->id_crafting_table) { o->result = 0; o->cost = rc->cost_no_table; return; }
+        if (CELL(e, fr, fc) != e->cfg->id_crafting_table) {
+            o->result = 0; o->cost = rc->cost_no_table; o->msg = NGW_MSG_NEED_TABLE; return;
+        }
     }
     o->reward = rc->reward_ok;
     for (int i = 0; i < rc->n_inputs; i++) e->inv[rc->in_item[i]] -= rc->in_qty[i];
     e->inv[rc->out_item] += rc->out_qty;
     o->cost = rc->cost_ok;
+    o->msg = msg_code(NGW_MSG_CRAFTED, rc->out_item);
 }
 
 /* The Break family.  Every variant starts with update_block_in_front and the unbreakable test. */
@@ -191,7 +201,7 @@ static void do_break(env_t* e, const ngw_action_entry* a, out_t* o) {
     int front = CELL(e, fr, fc);
     int sel = e->pose[3];
     o->reward = -1; o->result = 1; o->cost = 3600.0f;
-    if (in_mask(cfg->unbreakable_mask, front)) { o->result = 0; return; }
+    if (in_mask(cfg->unbreakable_mask, front)) { o->result = 0; o->msg = msg_code(NGW_MSG_CANNOT_BREAK, front); return; }
     switch (a->variant) {
         case NGW_BRK_BASE:                       /* pogostick_v1_env.py:283-289 */
             CELL(e, fr, fc) = 0;
@@ -219,8 +229,8 @@ static void do_break(env_t* e, const ngw_action_entry* a, out_t* o) {
             } else if (e->inv[a->arg] >= 1 && cfg->id_iron_axe != NGW_NONE && sel == cfg->id_iron_axe) {
                 CELL(e, fr, fc) = 0; e->inv[front] += 1;
                 o->reward = cfg->reward_intermediate; o->cost = 900.0f;
-            } else {
-                o->result = 0;
+            } else {                             /* "Cannot break without <axe> selected" */
+                o->result = 0; o->msg = msg_code(NGW_MSG_NEED_AXE, a->arg);
             }
             break;
         case NGW_BRK_INCREASE:                   /* novelty_wrappers.py:1444-1454 */
@@ -238,12 +248,12 @@ static void terminal_step(env_t* e, const ngw_action_entry* a, out_t* o) {
     int r = e->pose[0], c = e->pose[1], f = e->pose[2];
     int fr, fc;
     front_of(e, &fr, &fc);
-    o->reward = -1; o->result = 1; o->cost = 0.0f; o->done = 0;     /* pogostick_v1_env.py:239-242 */
+    o->reward = -1; o->result = 1; o->cost = 0.0f; o->done = 0; o->msg = NGW_MSG_NONE;   /* pogostick_v1_env.py:239-242 */
     switch (a->op) {
         case NGW_OP_NOOP: break;
         case NGW_OP_FORWARD:                      /* pogostick_v1_env.py:244-257 */
             if (CELL(e, fr, fc) == 0) { e->pose[0] = (uint8_t)fr; e->pose[1] = (uint8_t)fc; }
-            else o->result = 0;
+            else { o->result = 0; o->msg = NGW_MSG_BLOCK_IN_PATH; }
             o->cost = 27.906975f;
             break;
         case NGW_OP_LEFT: {                       /* pogostick_v1_env.py:258-268: N->W, S->E, W->S, E->N */
@@ -261,8 +271,9 @@ static void terminal_step(env_t* e, const ngw_action_entry* a, out_t* o) {
                     CELL(e, fr, fc) = (int8_t)cfg->id_tree_tap;
                     e->inv[cfg->id_tree_tap] -= 1;
                     if (front_next_to(e, cfg->id_tree_log)) o->reward = cfg->reward_intermediate;
-                } else o->result = 0;
-            } else o->result = 0;
+                    o->msg = NGW_MSG_TAP_PLACED;
+                } else { o->result = 0; o->msg = msg_code(NGW_MSG_BLOCK_EXISTS, CELL(e, fr, fc)); }
+            } else { o->result = 0; o->msg = NGW_MSG_NOT_IN_INVENTORY; }
             o->cost = 300.0f;
             break;
         case NGW_OP_EXTRACT_RUBBER:               /* pogostick_v1_env.py:315-331, novelty_wrappers.py:1537-1551 */
@@ -271,8 +282,8 @@ static void terminal_step(env_t* e, const ngw_action_entry* a, out_t* o) {
                 if (front_next_to(e, cfg->id_tree_log)) {
                     e->inv[cfg->id_rubber] += a->arg;
                     o->reward = cfg->reward_intermediate; o->cost = 50000.0f;
-                } else o->result = 0;
-            } else o->result = 0;
+                } else { o->result = 0; o->msg = NGW_MSG_NO_LOG_NEAR_TAP; }
+            } else { o->result = 0; o->msg = NGW_MSG_NO_TAP; }
             break;
         case NGW_OP_EXTRACT_STRING:               /* bow_v1_env.py:293-304, novelty_wrappers.py:1524-1536 */
             o->cost = 120.0f;
@@ -280,27 +291,27 @@ static void terminal_step(env_t* e, const ngw_action_entry* a, out_t* o) {
                 e->inv[cfg->id_string] += a->arg;
                 CELL(e, fr, fc) = 0;
                 o->reward = cfg->reward_intermediate; o->cost = 5000.0f;
-            } else o->result = 0;
+            } else { o->result = 0; o->msg = NGW_MSG_NO_WOOL; }
             break;
         case NGW_OP_CRAFT: craft(e, &cfg->recipes[a->arg], o); break;
         case NGW_OP_SELECT:                       /* pogostick_v1_env.py:338-347 */
             o->cost = 120.0f;
             if (a->arg != NGW_NONE && e->inv[a->arg] >= 1) e->pose[3] = a->arg;
-            else o->result = 0;
+            else { o->result = 0; o->msg = NGW_MSG_NOT_IN_INVENTORY; }
             break;
         case NGW_OP_CHOP: {                       /* novelty_wrappers.py:1291-1307 */
             int front = CELL(e, fr, fc);
             o->cost = 3600.0f * 1.2f;
             if (!in_mask(cfg->unbreakable_mask, front)) {
                 CELL(e, fr, fc) = 0; e->inv[front] += 2; o->reward = cfg->reward_intermediate;
-            } else o->result = 0;
+            } else { o->result = 0; o->msg = msg_code(NGW_MSG_CANNOT_CHOP, front); }
             break;
         }
         case NGW_OP_JUMP: {                       /* novelty_wrappers.py:1363-1382: 2 ahead, middle cell ignored */
             int tr = r + 2 * (fr - r), tc = c + 2 * (fc - c);
             if (tr >= 0 && tr <= e->ms - 1 && tc >= 0 && tc <= e->ms - 1 && CELL(e, tr, tc) == 0) {
                 e->pose[0] = (uint8_t)tr; e->pose[1] = (uint8_t)tc;
-            } else o->result = 0;
+            } else { o->result = 0; o->msg = NGW_MSG_BLOCK_IN_PATH; }
             o->cost = 27.906975f * 2.0f;
             break;
         }
@@ -329,7 +340,7 @@ static void layered_step(env_t* e, const ngw_action_entry* a, int i, out_t* o) {
         else if (r + 1 >= 0 && r + 1 <= hi && CELL(e, r + 1, c) == fw) close_to = 1;
         else if (c - 1 >= 0 && c - 1 <= hi && CELL(e, r, c - 1) == fw) close_to = 1;
         else if (c + 1 >= 0 && c + 1 <= hi && CELL(e, r, c + 1) == fw) close_to = 1;
-        if (close_to) { o->reward = cfg->reward_firewall; o->done = 1; }
+        if (close_to) { o->reward = cfg->reward_firewall; o->done = 1; o->msg = NGW_MSG_FIRE_WALL; }
         return;
     }
     /* FenceRestriction medium / hard (novelty_wrappers.py:918-973) */
@@ -337,7 +348,7 @@ static void layered_step(env_t* e, const ngw_action_entry* a, int i, out_t* o) {
         int fr, fc;
         front_of(e, &fr, &fc);
         int front = CELL(e, fr, fc), fence = cfg->id_fence;
-        int result = 1;
+        int result = 1, msg = NGW_MSG_NONE;
         o->reward = -1;
         if (!in_mask(cfg->unbreakable_mask, front)) {
             if (front == fence) {
@@ -358,30 +369,32 @@ static void layered_step(env_t* e, const ngw_action_entry* a, int i, out_t* o) {
                                 restricted = 1;
                 }
                 if (!restricted) layered_step(e, a, i + 1, o);
-                else result = 0;
+                else { result = 0; msg = NGW_MSG_FENCE_RESTRICTION; }
             }
-        } else result = 0;
+        } else { result = 0; msg = msg_code(NGW_MSG_CANNOT_BREAK, front); }
         /* the outer post block always re-runs and OVERWRITES info (SURVEY Q5, novelty_wrappers.py:960-973) */
         int reward = o->reward;
         grab_entities(e);
         o->done = 0;
         if (e->inv[cfg->id_goal] >= 1) { reward = cfg->reward_done; o->done = 1; }
-        o->reward = reward; o->result = result; o->cost = 3600.0f;
+        o->reward = reward; o->result = result; o->cost = 3600.0f; o->msg = msg;
     }
 }
 
 /* ------------------------------------------------------------------ public: one env step */
-/* returns 0, or NGW_ERR_INVALID_ACTION (state untouched, outputs zeroed) */
+/* returns 0, or NGW_ERR_INVALID_ACTION (state untouched, outputs zeroed, message code 0).  msg may be NULL. */
 int ngo_step(const ngw_config* cfg, int ms, int8_t* map, uint8_t* pose, int32_t* inv, int32_t action,
-             float* reward, uint8_t* done, float* cost, uint8_t* result) {
+             float* reward, uint8_t* done, float* cost, uint8_t* result, uint16_t* msg) {
     env_t e = {cfg, ms, map, pose, inv};
     if (action < 0 || action >= cfg->n_actions || cfg->actions[action].op == NGW_OP_INVALID) {
         *reward = 0.0f; *done = 0; *cost = 0.0f; *result = 0;
+        if (msg) *msg = NGW_MSG_NONE;
         return NGW_ERR_INVALID_ACTION;
     }
-    out_t o = {-1, 0, 1, 0.0f};
+    out_t o = {-1, 0, 1, 0.0f, NGW_MSG_NONE};
     layered_step(&e, &cfg->actions[action], 0, &o);
     *reward = (float)o.reward; *done = (uint8_t)o.done; *cost = o.cost; *result = (uint8_t)o.result;
+    if (msg) *msg = (uint16_t)o.msg;
     return 0;
 }
 
@@ -547,7 +560,7 @@ typedef struct {
     const ngw_config* cfgs; const uint8_t* cfg_id; int ms; int64_t begin, end;
     int8_t* map; uint8_t* pose; int32_t* inv; int inv_stride;
     const int32_t* actions; int32_t* obs; int obs_stride;
-    float* reward; uint8_t* done; float* cost; uint8_t* result; uint32_t* err;
+    float* reward; uint8_t* done; float* cost; uint8_t* result; uint32_t* err; uint16_t* msg;
 } job_t;
 
 static void* batch_worker(void* arg) {
@@ -559,7 +572,7 @@ static void* batch_worker(void* arg) {
         uint8_t* pose = j->pose + i * 4;
         int32_t* inv = j->inv + i * j->inv_stride;
         int rc = ngo_step(cfg, j->ms, map, pose, inv, j->actions[i], &j->reward[i], &j->done[i], &j->cost[i],
-                          &j->result[i]);
+                          &j->result[i], j->msg ? &j->msg[i] : NULL);
         if (j->err) j->err[i] |= (uint32_t)rc;
         if (j->obs) {
             int32_t* o = j->obs + i * j->obs_stride;
@@ -571,10 +584,10 @@ static void* batch_worker(void* arg) {
     return NULL;
 }
 
-/* One lock-step pass over n envs with n_threads host threads (envs are independent). */
+/* One lock-step pass over n envs with n_threads host threads (envs are independent).  msg (uint16 [n]) may be NULL. */
 int ngo_step_batch(const ngw_config* cfgs, const uint8_t* cfg_id, int ms, int64_t n, int8_t* map, uint8_t* pose,
                    int32_t* inv, int inv_stride, const int32_t* actions, int32_t* obs, int obs_stride, float* reward,
-                   uint8_t* done, float* cost, uint8_t* result, uint32_t* err, int n_threads) {
+                   uint8_t* done, float* cost, uint8_t* result, uint32_t* err, int n_threads, uint16_t* msg) {
     if (n_threads < 1) n_threads = 1;
     if (n_threads > 1024) n_threads = 1024;
     job_t* jobs = (job_t*)malloc(sizeof(job_t) * (size_t)n_threads);
@@ -585,7 +598,7 @@ int ngo_step_batch(const ngw_config* cfgs, const uint8_t* cfg_id, int ms, int64_
         if (b > n) b = n;
         if (e > n) e = n;
         job_t j = {cfgs, cfg_id, ms, b, e, map, pose, inv, inv_stride, actions, obs, obs_stride,
-                   reward, done, cost, result, err};
+                   reward, done, cost, result, err, msg};
         jobs[t] = j;
         if (n_threads == 1) batch_worker(&jobs[t]);
         else pthread_create(&th[t], NULL, batch_worker, &jobs[t]);
@@ -624,7 +637,7 @@ int ngo_rollout(const ngw_config* cfgs, const uint8_t* cfg_id, int ms, int64_t n
         if (b > n) b = n;
         if (e > n) e = n;
         job_t j = {cfgs, cfg_id, ms, b, e, map, pose, inv, inv_stride, NULL, obs, obs_stride,
-                   reward, done, cost, result, err};
+                   reward, done, cost, result, err, NULL};
         jobs[t].j = j; jobs[t].action_sets = action_sets; jobs[t].n_action_sets = n_action_sets;
         jobs[t].n_steps = n_steps; jobs[t].n = n;
         if (n_threads == 1) rollout_worker(&jobs[t]);

@@ -41,10 +41,10 @@ def lib():
                                        C.c_int, C.c_int, C.c_int]
         L.ngo_observe.argtypes = [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
         L.ngo_step.argtypes = [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32,
-                               C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
+                               C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
         L.ngo_step_batch.argtypes = [C.c_void_p, C.c_void_p, C.c_int, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p,
                                      C.c_int, C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p,
-                                     C.c_void_p, C.c_void_p, C.c_int]
+                                     C.c_void_p, C.c_void_p, C.c_int, C.c_void_p]
         L.ngo_rollout.argtypes = [C.c_void_p, C.c_void_p, C.c_int, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p,
                                   C.c_int, C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p,
                                   C.c_void_p, C.c_void_p, C.c_void_p, C.c_int]
@@ -95,6 +95,7 @@ class OracleBatch(object):
         self.pose = np.zeros((self.n, 4), np.uint8)
         self.inv = np.zeros((self.n, self.inv_stride), np.int32)
         self.err = np.zeros(self.n, np.uint32)
+        self.msg = np.zeros(self.n, np.uint16)       # info['message'] codes of the last step (enum ngw_msg | arg << 5)
 
     def reset_legacy(self, seed0):
         """env i <- reference reset under np.random.seed(seed0 + i)."""
@@ -135,7 +136,7 @@ class OracleBatch(object):
         result = np.zeros(self.n, np.uint8)
         lib().ngo_step_batch(self.cfgs, _p(self.cfg_id), self.ms, self.n, _p(self.map), _p(self.pose), _p(self.inv),
                              self.inv_stride, _p(actions), _p(obs), self.obs_dim, _p(reward), _p(done), _p(cost),
-                             _p(result), _p(self.err), n_threads)
+                             _p(result), _p(self.err), n_threads, _p(self.msg))
         return obs, reward, done, cost, result
 
     def rollout(self, action_sets, n_steps, n_threads=1):

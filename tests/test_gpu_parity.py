@@ -281,10 +281,8 @@ def test_batched_gym_api_auto_reset_messages_and_mixed_batch():
     assert st[0] == 500 and st[6] == 500
 
 
-@pytest.mark.parametrize('n_cfg', [6, 20])
-def test_many_configs_in_one_batch_inline_and_global_tables(n_cfg):
-    """NC = 16 inline-config kernel (6 configs) and the global-memory fallback (20 configs > 16)."""
-    import gym_novel_gridworlds_b200 as gym
+def many_config_inputs(n_cfg):
+    """(compiled configs, batch size, cfg_id) of a batch of n_cfg novelty variants of C2, env i -> config 7 i mod n_cfg."""
     variants = [('addchop', 'hard', '', '', ['Chop']), ('addjump', 'hard', '', '', ['Jump']),
                 ('additem', 'easy', 'spring', '', []), ('breakincrease', 'hard', '', '', []),
                 ('axe', 'easy', 'wooden', 'true', ['Select_wooden_axe']), ('fence', 'medium', 'oak', '', [])]
@@ -295,7 +293,13 @@ def test_many_configs_in_one_batch_inline_and_global_tables(n_cfg):
                 'chain': [['limit', scenarios.C2_SET + extra], ['lidar', 8], ['novelty', name, diff, a1, a2]]}
         compiled.append(_compiled(desc))
     n = 64 * n_cfg + 5
-    cfg_id = (np.arange(n) * 7 % n_cfg).astype(np.uint8)
+    return compiled, n, (np.arange(n) * 7 % n_cfg).astype(np.uint8)
+
+
+@pytest.mark.parametrize('n_cfg', [6, 20])
+def test_many_configs_in_one_batch_inline_and_global_tables(n_cfg):
+    """NC = 16 inline-config kernel (6 configs) and the global-memory fallback (20 configs > 16)."""
+    compiled, n, cfg_id = many_config_inputs(n_cfg)
     _parity_vs_oracle(compiled, n, 40, seed0=777, cfg_id=cfg_id)
 
 
@@ -787,17 +791,11 @@ def _c4_descs():
         ([], ['novelty', 'additem', 'medium', 'spring', '']), ([], ['novelty', 'remapaction', 'hard', '', '']))]
 
 
-@pytest.mark.parametrize('case', ['pogo_ms23', 'bow_ms13', 'c4_mixed', 'c3_layers', 'pogo_ms40', 'bow12_16beams', 'c2_u8', 'pogo_ms40_u8'])
-@pytest.mark.parametrize('mode', ['given', 'given+autoreset', 'policy', 'random'])
-def test_rollout_kernels_equal_repeated_steps_on_other_shapes(case, mode):
-    """The K-step rollout kernels (lane-pair kernel on grids up to 32x32 incl. its generic-size lidar, mixed configs through
-    the global config table, layered novelties; the one-warp-per-tile kernel on 40x40 grids and 16 beams) against the same
-    steps issued one launch at a time: states, sums, final observation, episode counters; closed loop: every action is the
-    argmax of the integer policy on the twin's observation; auto-reset with truncation regenerates the same episodes."""
+def rollout_case_inputs(case):
+    """(compiled configs, batch size, cfg_id or None) of a case of test_rollout_kernels_equal_repeated_steps_on_other_shapes:
+    grids up to 32x32 take the lane-pair rollout kernel (rollout2_kernel), 40x40 grids and 16 beams the one-warp-per-tile
+    kernel (rollout_kernel)."""
     cfg_id = None
-    fmt = 'u8' if case.endswith('_u8') else 'i32'
-    if fmt == 'u8' and mode == 'policy':
-        pytest.skip("the device policy reads int32 observation rows")
     if case == 'c2_u8':
         compiled, n = [_compiled(C2_DESC)], 32 * 20 + 11
     elif case == 'pogo_ms40_u8':
@@ -815,6 +813,20 @@ def test_rollout_kernels_equal_repeated_steps_on_other_shapes(case, mode):
         compiled, n = [_compiled(golden_util.get('pogo_ms40_additem_hard')['meta'])], 32 * 3 + 5
     else:
         compiled, n = [_compiled({'env': scenarios.BOW, 'map_size': 12, 'chain': [['lidar', 16]]})], 200
+    return compiled, n, cfg_id
+
+
+@pytest.mark.parametrize('case', ['pogo_ms23', 'bow_ms13', 'c4_mixed', 'c3_layers', 'pogo_ms40', 'bow12_16beams', 'c2_u8', 'pogo_ms40_u8'])
+@pytest.mark.parametrize('mode', ['given', 'given+autoreset', 'policy', 'random'])
+def test_rollout_kernels_equal_repeated_steps_on_other_shapes(case, mode):
+    """The K-step rollout kernels (lane-pair kernel on grids up to 32x32 incl. its generic-size lidar, mixed configs through
+    the global config table, layered novelties; the one-warp-per-tile kernel on 40x40 grids and 16 beams) against the same
+    steps issued one launch at a time: states, sums, final observation, episode counters; closed loop: every action is the
+    argmax of the integer policy on the twin's observation; auto-reset with truncation regenerates the same episodes."""
+    fmt = 'u8' if case.endswith('_u8') else 'i32'
+    if fmt == 'u8' and mode == 'policy':
+        pytest.skip("the device policy reads int32 observation rows")
+    compiled, n, cfg_id = rollout_case_inputs(case)
     T = 24
     kw = dict(auto_reset=True, max_episode_steps=7) if mode == 'given+autoreset' else {}
     h1 = BatchHandle(compiled, n, seed=21, cfg_id=cfg_id, obs_format=fmt)   # one launch per step
