@@ -268,7 +268,8 @@ static int create_init(ngw_handle* h, const ngw_config* cfgs, int32_t n_cfgs, in
     h->device = device; h->n = n_envs; h->np = (n_envs + 31) / 32 * 32; h->first_gid = first_env_gid; h->seed = seed;
     h->ms = map_size; h->cells = map_size * map_size; h->n_cfgs = n_cfgs;
     h->concurrent = getenv("NGW_NO_CONCURRENT") == nullptr;
-    if (const char* km = getenv("NGW_DEBUG_KEY_MASK")) h->key_mask = (uint32_t)strtoul(km, nullptr, 0);   // test knob: key ties
+    // test knob: key ties.  It reaches ngw_reset and the one-step auto-resets; the rollouts' in-place resets keep every key bit
+    if (const char* km = getenv("NGW_DEBUG_KEY_MASK")) h->key_mask = (uint32_t)strtoul(km, nullptr, 0);
     for (int i = 0; i < n_cfgs; i++) {
         const ngw_config& c = cfgs[i];
         if (c.n_items < 1 || c.n_items > NGW_MAX_ITEMS || c.n_actions < 0 || c.n_actions > NGW_MAX_ACTIONS ||

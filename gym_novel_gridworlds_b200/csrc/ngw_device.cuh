@@ -731,7 +731,9 @@ __device__ __forceinline__ void lidar_observe(const EnvRow& e, const DevConfig& 
 //  * post-ops ("shuffle the candidate cells, take the first m", m = ceil(n * (pct / 100)) in IEEE doubles as NumPy does):
 //    a uniformly random m-subset.  Every candidate cell gets an independent 32-bit Philox key (counter = cell index) and
 //    the m smallest keys win — found with a warp radix-select (256-bin histogram in shared memory) and, inside the
-//    boundary bin, an exact rank by (key, cell index).  Key ties (probability ~ n^2 / 2^33) fall back to index order.
+//    boundary bin, an exact rank by (key, cell index), so equal keys go by cell index.  Only when more than 32 candidates
+//    share the boundary key exactly (probability ~ n^2 / 2^33) do they win in arrival order instead, which is
+//    (i >> 7, i & 3, i >> 2) for cell i: 128-cell rounds, then the word of the key's Philox block, then the lane.
 __device__ __forceinline__ bool placeable(const int8_t* m, int ms, int r, int c) {
     const int8_t* p = m + r * ms + c;
     return p[0] == 0 && p[-ms] == 0 && p[ms] == 0 && p[-1] == 0 && p[1] == 0;

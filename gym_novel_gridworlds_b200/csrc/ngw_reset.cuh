@@ -66,18 +66,21 @@ __global__ void __launch_bounds__(32 * NGW_RESET_WARPS) reset_kernel(const Reset
     int k = cfg->reset_obs_after_ops;
     int8_t* m = p.map + e * p.cells;
     int32_t* inv = p.inv + e * p.inv_stride;
+    uint32_t err;
     if (p.phase != 1) {
         uint32_t ep = p.episode[e] + 1;
         __syncwarp();
-        uint32_t err = reset_env_warp(cfg, sc.row, sc.inv, p.ms, p.inv_stride, p.seed, gid, ep, true, 0,
-                                      p.phase == 0 ? k : NGW_MAX_RESET_OPS, sc.hist, r, c, f, sel, p.key_mask);
-        if (lane == 0) { p.episode[e] = ep; p.ep_len[e] = 0; p.err[e] = err; }
+        err = reset_env_warp(cfg, sc.row, sc.inv, p.ms, p.inv_stride, p.seed, gid, ep, true, 0,
+                             p.phase == 0 ? k : NGW_MAX_RESET_OPS, sc.hist, r, c, f, sel, p.key_mask);
+        if (lane == 0) { p.episode[e] = ep; p.ep_len[e] = 0; }
     } else {
         uint32_t ep = p.episode[e];
         rows_to_smem(sc, m, inv, p.cells, p.inv_stride, lane);
-        reset_env_warp(cfg, sc.row, sc.inv, p.ms, p.inv_stride, p.seed, gid, ep, false, k, NGW_MAX_RESET_OPS, sc.hist, r, c,
-                       f, sel, p.key_mask);
+        err = reset_env_warp(cfg, sc.row, sc.inv, p.ms, p.inv_stride, p.seed, gid, ep, false, k, NGW_MAX_RESET_OPS, sc.hist,
+                             r, c, f, sel, p.key_mask);
     }
+    // a reset assigns the env's flags; its phase 1 adds those of the ops after the observation to what phase 0 assigned
+    if (lane == 0) p.err[e] = p.phase == 1 ? p.err[e] | err : err;
     rows_from_smem(sc, m, inv, p.cells, p.inv_stride, lane);
     if (lane == 0) p.pose[e] = make_uchar4((unsigned char)r, (unsigned char)c, (unsigned char)f, (unsigned char)sel);
 }

@@ -1,5 +1,7 @@
 /*
- * ngw_oracle.c — CPU restatement of the reference's NovelGridworld step / reset / LidarInFront path.
+ * ngw_oracle.c — CPU restatement of the reference's NovelGridworld step / reset / LidarInFront path, and (last section)
+ * of the DEVICE's Philox map generator and random policy, which by design share the reference's distribution but not
+ * its stream.
  *
  * TEST INFRASTRUCTURE, NOT PRODUCT.  Only tests/, __graft_entry__.smoke() and bench.py's cpu_baseline /
  * --impl reference legs may load this library; the product (gym_novel_gridworlds_b200) never does and
@@ -663,6 +665,373 @@ int ngo_reset_batch(const ngw_config* cfgs, const uint8_t* cfg_id, int ms, int64
         int rc = ngo_reset_legacy(cfg, ms, &mt, map + i * cells, pose + i * 4, v, 1, 0, cfg->n_reset_ops);
         if (err) err[i] = (uint32_t)rc;
     }
+    return 0;
+}
+
+/* ==================================================================================================================
+ * RESTATEMENT OF THE DEVICE'S GENERATOR (gym_novel_gridworlds_b200/csrc/ngw_device.cuh: Philox, RandomPolicy,
+ * reset_env_warp).  Everything above restates the reference; this section does not.  The device's map generator has the
+ * reference's DISTRIBUTION, not its stream, so it cannot be pinned by the golden traces: this is the CPU statement of its
+ * contract, written from that contract (not from the warp code), against which tests/test_gpu_reset_exact.py compares
+ * every GPU reset and random-policy draw bit for bit.
+ *   Philox4x32-10: counter = (gid lo, gid hi, episode word, (stream << 20) | block), key = (seed lo, seed hi); next()
+ *     returns words 0..3 of block 0, then of block 1, ...; below(n) = mask (0xFFFFFFFF >> clz(n - 1)) and reject.
+ *   Base (stream 0): walls on the border, agent = below(side^2), facing = below(4), then each item copy takes up to
+ *     8 side^2 draws for a placeable cell; failing that, below(good) picks among the placeable cells in row-major order.
+ *   Op k (stream 1 + k): INVSET, TREETAP (4096 attempts over (direction, log)), and FENCE / ADDITEM / REPLACE, which pick
+ *     the `take` candidates of smallest (key, cell index), key of cell i = word i % 4 of block 1 + i / 4 — except that a
+ *     tie of more than 32 candidates on the boundary key goes by the device's arrival order (i >> 7, i & 3, i >> 2).
+ *   Random policy: word t & 3 of block 0 at episode word t >> 2, stream 0xFFF; action = high half of x * n, Lemire's
+ *     rejection continuing on stream 0xFFE at episode word t.
+ * ================================================================================================================== */
+void ngo_philox4x32_10(const uint32_t ctr[4], const uint32_t key[2], uint32_t out[4]) {
+    uint32_t x0 = ctr[0], x1 = ctr[1], x2 = ctr[2], x3 = ctr[3], k0 = key[0], k1 = key[1];
+    for (int r = 0; r < 10; r++) {
+        uint64_t p0 = (uint64_t)0xD2511F53u * x0, p1 = (uint64_t)0xCD9E8D57u * x2;
+        uint32_t y0 = (uint32_t)(p1 >> 32) ^ x1 ^ k0, y1 = (uint32_t)p1;
+        uint32_t y2 = (uint32_t)(p0 >> 32) ^ x3 ^ k1, y3 = (uint32_t)p0;
+        x0 = y0; x1 = y1; x2 = y2; x3 = y3;
+        k0 += 0x9E3779B9u; k1 += 0xBB67AE85u;
+    }
+    out[0] = x0; out[1] = x1; out[2] = x2; out[3] = x3;
+}
+
+typedef struct {
+    uint32_t ctr[4], key[2], word[4];
+    uint32_t block;    /* next block to generate */
+    int used;          /* words of `word` already returned (4: generate the next block first) */
+} ngo_pstream;
+
+static void ps_block(uint64_t seed, uint64_t gid, uint32_t episode, uint32_t stream, uint32_t block, uint32_t out[4]) {
+    uint32_t ctr[4] = {(uint32_t)gid, (uint32_t)(gid >> 32), episode, (stream << 20) | block};
+    uint32_t key[2] = {(uint32_t)seed, (uint32_t)(seed >> 32)};
+    ngo_philox4x32_10(ctr, key, out);
+}
+
+static void ps_init(ngo_pstream* s, uint64_t seed, uint64_t gid, uint32_t episode, uint32_t stream) {
+    s->ctr[0] = (uint32_t)gid; s->ctr[1] = (uint32_t)(gid >> 32); s->ctr[2] = episode; s->ctr[3] = stream << 20;
+    s->key[0] = (uint32_t)seed; s->key[1] = (uint32_t)(seed >> 32);
+    s->block = 0; s->used = 4;
+}
+
+static uint32_t ps_next(ngo_pstream* s) {
+    if (s->used == 4) {
+        uint32_t ctr[4] = {s->ctr[0], s->ctr[1], s->ctr[2], s->ctr[3] | s->block};
+        ngo_philox4x32_10(ctr, s->key, s->word);
+        s->block++; s->used = 0;
+    }
+    return s->word[s->used++];
+}
+
+static uint32_t ps_below(ngo_pstream* s, uint32_t n) {
+    uint32_t max = n - 1u, mask = max;
+    if (max == 0) return 0;
+    mask |= mask >> 1; mask |= mask >> 2; mask |= mask >> 4; mask |= mask >> 8; mask |= mask >> 16;
+    uint32_t v;
+    do { v = ps_next(s) & mask; } while (v > max);
+    return v;
+}
+
+/* the first `count` outputs of below(n) on one stream (the test of the word stream and of the rejection rate) */
+void ngo_philox_below(uint64_t seed, uint64_t gid, uint32_t episode, uint32_t stream, uint32_t n, int64_t count,
+                      uint32_t* out, uint32_t* words_used) {
+    ngo_pstream s;
+    ps_init(&s, seed, gid, episode, stream);
+    for (int64_t i = 0; i < count; i++) out[i] = ps_below(&s, n);
+    if (words_used) *words_used = s.block * 4u - (uint32_t)(4 - s.used);
+}
+
+/* The random policy's action for step t of env gid (config with n actions); *branch = 0: plain draw, 1: the low half
+ * was below n and the draw was kept, 2: it was below (2^32 - n) mod n and continued on stream 0xFFE. */
+int32_t ngo_policy_draw(uint64_t seed, uint64_t gid, uint32_t t, uint32_t n, int* branch) {
+    uint32_t w[4];
+    ps_block(seed, gid, t >> 2, 0xFFF, 0, w);
+    uint64_t m = (uint64_t)w[t & 3u] * n;
+    int br = 0;
+    if ((uint32_t)m < n) {
+        uint32_t thr = (0u - n) % n;
+        br = (uint32_t)m < thr ? 2 : 1;
+        ngo_pstream s;
+        ps_init(&s, seed, gid, t, 0xFFE);
+        while ((uint32_t)m < thr) m = (uint64_t)ps_next(&s) * n;
+    }
+    if (branch) *branch = br;
+    return (int32_t)(m >> 32);
+}
+
+/* What a reset did, summed over envs: the events the exact tests must see happen. */
+enum {
+    NGO_RS_FALLBACK = 0,      /* item copies placed by the enumeration after 8 side^2 failed draws */
+    NGO_RS_PLACE_FAIL,        /* base placements that found no placeable cell (PLACEMENT, remaining items skipped) */
+    NGO_RS_TREETAP_FAIL,      /* TREETAP ops that flagged PLACEMENT */
+    NGO_RS_SUBSET,            /* FENCE / ADDITEM / REPLACE ops with 0 < take */
+    NGO_RS_ALL_WIN,           /* ... whose boundary bin won whole (take == n, or a radix bin boundary) */
+    NGO_RS_LIST,              /* ... decided by ranking a boundary list of <= 32 candidates by (key, cell) */
+    NGO_RS_ARRIVAL,           /* ... where > 32 candidates tied on the boundary key and arrival order decided */
+    NGO_RS_COUNT = 8
+};
+
+typedef struct { uint32_t key; int32_t cell; } ngo_cand;
+
+static int cand_by_key_cell(const void* a, const void* b) {
+    const ngo_cand *x = (const ngo_cand*)a, *y = (const ngo_cand*)b;
+    if (x->key != y->key) return x->key < y->key ? -1 : 1;
+    return x->cell < y->cell ? -1 : x->cell > y->cell;
+}
+
+static int64_t arrival_rank(int32_t i) { return ((int64_t)(i >> 7) << 40) | ((int64_t)(i & 3) << 32) | (i >> 2); }
+
+static int cand_by_arrival(const void* a, const void* b) {
+    int64_t x = arrival_rank(((const ngo_cand*)a)->cell), y = arrival_rank(((const ngo_cand*)b)->cell);
+    return x < y ? -1 : x > y;
+}
+
+static int placeable_at(const int8_t* m, int ms, int r, int c) {
+    const int8_t* p = m + r * ms + c;
+    return p[0] == 0 && p[-ms] == 0 && p[ms] == 0 && p[-1] == 0 && p[1] == 0;
+}
+
+/* The outcome of the device's radix-select for `take` of the n candidates sorted by (key, cell): 0 = the boundary bin
+ * wins whole, 1 = a boundary list of <= 32 is ranked, 2 = more than 32 identical boundary keys, arrival order.  Bins are
+ * the top 8, 16, 24, 32 key bits of the take-th smallest key; the select narrows while fewer than all of the bin's
+ * candidates are still needed and the bin holds more than 32. */
+static int radix_outcome(const ngo_cand* c, int n, int take) {
+    const uint32_t kth = c[take - 1].key;
+    int bits = 0, remaining = take, bin_count = n;
+    while (remaining < bin_count && bin_count > 32 && bits < 32) {
+        bits += 8;
+        int less = 0, same = 0;
+        for (int i = 0; i < n; i++) {
+            uint32_t top = c[i].key >> (32 - bits), want = kth >> (32 - bits);
+            less += top < want; same += top == want;
+        }
+        remaining = take - less;
+        bin_count = same;
+    }
+    if (remaining >= bin_count) return 0;
+    return (bits >= 32 && bin_count > 32) ? 2 : 1;
+}
+
+/* Ops [op_begin, op_end) of the reset program, do_base != 0 running the base first, at (seed, gid, episode word).
+ * Returns the PLACEMENT flag of what ran; counters (NGO_RS_COUNT) may be NULL. */
+int ngo_reset_philox(const ngw_config* cfg, int ms, uint64_t seed, uint64_t gid, uint32_t episode, uint32_t key_mask,
+                     int8_t* map, uint8_t* pose, int32_t* inv, int inv_stride, int do_base, int op_begin, int op_end,
+                     int64_t* counters) {
+    const int cells = ms * ms, wall = cfg->id_wall;
+    int64_t dummy[NGO_RS_COUNT];
+    int64_t* ct = counters ? counters : dummy;
+    int err = 0;
+    if (do_base) {
+        for (int i = 0; i < inv_stride; i++) inv[i] = 0;
+        pose[3] = 0;
+        for (int r = 0; r < ms; r++)
+            for (int c = 0; c < ms; c++) map[r * ms + c] = (r == 0 || c == 0 || r == ms - 1 || c == ms - 1) ? (int8_t)wall : 0;
+        ngo_pstream s;
+        ps_init(&s, seed, gid, episode, 0);
+        const int side = ms - 4;
+        const uint32_t n_av = (uint32_t)(side * side);
+        uint32_t a = ps_below(&s, n_av);
+        pose[0] = (uint8_t)(2 + a / side); pose[1] = (uint8_t)(2 + a % side);
+        pose[2] = (uint8_t)ps_below(&s, 4);
+        const int agent = pose[0] * ms + pose[1];
+        int stop = 0;
+        for (int i = 0; i < cfg->n_place && !stop; i++) {
+            for (int count = 0; count < cfg->place_qty[i]; count++) {
+                int where = -1;
+                for (uint32_t attempt = 0; attempt < 8 * n_av && where < 0; attempt++) {
+                    uint32_t d = ps_below(&s, n_av);
+                    int r = 2 + (int)(d / side), c = 2 + (int)(d % side);
+                    if (r * ms + c != agent && placeable_at(map, ms, r, c)) where = r * ms + c;
+                }
+                if (where < 0) {
+                    uint32_t good = 0;
+                    for (int r = 2; r <= ms - 3; r++)
+                        for (int c = 2; c <= ms - 3; c++) good += r * ms + c != agent && placeable_at(map, ms, r, c);
+                    if (good == 0) { err |= NGW_ERR_PLACEMENT; ct[NGO_RS_PLACE_FAIL]++; stop = 1; break; }
+                    uint32_t pick = ps_below(&s, good);
+                    for (int r = 2; r <= ms - 3 && where < 0; r++)
+                        for (int c = 2; c <= ms - 3 && where < 0; c++)
+                            if (r * ms + c != agent && placeable_at(map, ms, r, c) && pick-- == 0) where = r * ms + c;
+                    ct[NGO_RS_FALLBACK]++;
+                }
+                map[where] = (int8_t)cfg->place_item[i];
+            }
+        }
+    }
+    const int agent = pose[0] * ms + pose[1];
+    if (op_end > cfg->n_reset_ops) op_end = cfg->n_reset_ops;
+    ngo_cand* cand = (ngo_cand*)malloc(sizeof(ngo_cand) * (size_t)cells);
+    for (int k = op_begin; k < op_end; k++) {
+        const ngw_reset_op* op = &cfg->reset_ops[k];
+        const uint32_t stream = 1u + (uint32_t)k;
+        if (op->kind == NGW_RESET_INVSET) { inv[op->a] = op->lo; continue; }
+        if (op->kind == NGW_RESET_TREETAP) {
+            int n_logs = 0, target = -1;
+            for (int i = 0; i < cells; i++) n_logs += map[i] == (int8_t)op->b;
+            if (n_logs > 1) {
+                ngo_pstream s;
+                ps_init(&s, seed, gid, episode, stream);
+                for (int attempt = 0; attempt < 4096 && target < 0; attempt++) {
+                    int direction = (int)ps_below(&s, 4);
+                    int which = (int)ps_below(&s, (uint32_t)n_logs), log = -1;
+                    for (int i = 0; i < cells && log < 0; i++)
+                        if (map[i] == (int8_t)op->b && which-- == 0) log = i;
+                    int r = log / ms, c = log % ms;
+                    int tr = r + (direction == NGW_SOUTH) - (direction == NGW_NORTH);
+                    int tc = c + (direction == NGW_EAST) - (direction == NGW_WEST);
+                    if (tr >= 0 && tr < ms && tc >= 0 && tc < ms && map[tr * ms + tc] == 0 && tr * ms + tc != agent)
+                        target = tr * ms + tc;
+                }
+            }
+            if (target < 0) { err |= NGW_ERR_PLACEMENT; ct[NGO_RS_TREETAP_FAIL]++; continue; }
+            map[target] = (int8_t)op->a;
+            continue;
+        }
+        int n = 0;
+        for (int i = 0; i < cells; i++) {
+            int id = map[i];
+            int is = op->kind == NGW_RESET_FENCE ? (id != 0 && id != wall) : op->kind == NGW_RESET_ADDITEM ? id == 0 : id == op->a;
+            if (!is) continue;
+            uint32_t w[4];
+            ps_block(seed, gid, episode, stream, 1u + (uint32_t)(i / 4), w);
+            cand[n].key = w[i % 4] & key_mask;
+            cand[n].cell = i;
+            n++;
+        }
+        ngo_pstream s;
+        ps_init(&s, seed, gid, episode, stream);
+        const int pct = op->lo + (int)ps_below(&s, (uint32_t)(op->hi - op->lo));
+        int take = percent_count(n, pct);
+        if (take > n) take = n;
+        if (take <= 0) continue;
+        ct[NGO_RS_SUBSET]++;
+        qsort(cand, (size_t)n, sizeof(ngo_cand), cand_by_key_cell);
+        const int outcome = radix_outcome(cand, n, take);
+        ct[outcome == 0 ? NGO_RS_ALL_WIN : outcome == 1 ? NGO_RS_LIST : NGO_RS_ARRIVAL]++;
+        if (outcome == 2) {                                /* the tied group [lo, hi) is re-ordered by arrival */
+            int lo = take - 1, hi = take;
+            while (lo > 0 && cand[lo - 1].key == cand[take - 1].key) lo--;
+            while (hi < n && cand[hi].key == cand[take - 1].key) hi++;
+            qsort(cand + lo, (size_t)(hi - lo), sizeof(ngo_cand), cand_by_arrival);
+        }
+        for (int j = 0; j < take; j++) {
+            const int i = cand[j].cell;
+            if (op->kind == NGW_RESET_FENCE) {             /* add_fence_around the winner (fences only go into air) */
+                int r = i / ms, c = i % ms;
+                for (int rr = r - 1; rr <= r + 1; rr++)
+                    for (int cc = c - 1; cc <= c + 1; cc++)
+                        if (rr >= 0 && rr < ms && cc >= 0 && cc < ms && map[rr * ms + cc] == 0 && rr * ms + cc != agent)
+                            map[rr * ms + cc] = (int8_t)op->a;
+            } else if (i != agent) {
+                map[i] = (int8_t)(op->kind == NGW_RESET_ADDITEM ? op->a : op->b);
+            }
+        }
+    }
+    free(cand);
+    return err;
+}
+
+/* Device-generator resets of envs [0, n) with n_threads host threads: env i (skipped where mask[i] == 0) is reset at
+ * gid first_gid + i and episode word episode[i]; its observation (obs may be NULL) is taken after k_obs[i] ops (NULL:
+ * the config's reset_obs_after_ops).  err[i] is assigned the PLACEMENT flag; counters [NGO_RS_COUNT] are summed. */
+typedef struct {
+    const ngw_config* cfgs; const uint8_t* cfg_id; int ms; int64_t begin, end;
+    uint64_t seed, first_gid; const uint32_t* episode; uint32_t key_mask; const uint8_t* mask; const int32_t* k_obs;
+    int8_t* map; uint8_t* pose; int32_t* inv; int inv_stride; int32_t* obs; int obs_stride; uint32_t* err;
+    int64_t counters[NGO_RS_COUNT];
+} preset_t;
+
+static void* preset_worker(void* arg) {
+    preset_t* j = (preset_t*)arg;
+    const int cells = j->ms * j->ms;
+    for (int64_t i = j->begin; i < j->end; i++) {
+        if (j->mask && !j->mask[i]) continue;
+        const ngw_config* cfg = &j->cfgs[j->cfg_id ? j->cfg_id[i] : 0];
+        int8_t* map = j->map + i * cells;
+        uint8_t* pose = j->pose + i * 4;
+        int32_t* inv = j->inv + i * j->inv_stride;
+        const uint64_t gid = j->first_gid + (uint64_t)i;
+        int k = j->k_obs ? j->k_obs[i] : cfg->reset_obs_after_ops;
+        int rc = ngo_reset_philox(cfg, j->ms, j->seed, gid, j->episode[i], j->key_mask, map, pose, inv, j->inv_stride, 1, 0,
+                                  k, j->counters);
+        if (j->obs) {
+            int32_t* o = j->obs + i * j->obs_stride;
+            for (int q = 0; q < j->obs_stride; q++) o[q] = 0;
+            if (cfg->n_beams > 0) ngo_observe(cfg, j->ms, map, pose, inv, o);
+        }
+        rc |= ngo_reset_philox(cfg, j->ms, j->seed, gid, j->episode[i], j->key_mask, map, pose, inv, j->inv_stride, 0, k,
+                               NGW_MAX_RESET_OPS, j->counters);
+        if (j->err) j->err[i] = (uint32_t)rc;
+    }
+    return NULL;
+}
+
+int ngo_reset_philox_batch(const ngw_config* cfgs, const uint8_t* cfg_id, int ms, int64_t n, uint64_t seed,
+                           uint64_t first_gid, const uint32_t* episode, uint32_t key_mask, const uint8_t* mask,
+                           const int32_t* k_obs, int8_t* map, uint8_t* pose, int32_t* inv, int inv_stride, int32_t* obs,
+                           int obs_stride, uint32_t* err, int64_t* counters, int n_threads) {
+    if (n_threads < 1) n_threads = 1;
+    if (n_threads > 1024) n_threads = 1024;
+    preset_t* jobs = (preset_t*)calloc((size_t)n_threads, sizeof(preset_t));
+    pthread_t* th = (pthread_t*)malloc(sizeof(pthread_t) * (size_t)n_threads);
+    int64_t per = (n + n_threads - 1) / n_threads;
+    for (int t = 0; t < n_threads; t++) {
+        int64_t b = t * per, e = b + per;
+        if (b > n) b = n;
+        if (e > n) e = n;
+        preset_t j = {cfgs, cfg_id, ms, b, e, seed, first_gid, episode, key_mask, mask, k_obs, map, pose, inv, inv_stride,
+                      obs, obs_stride, err, {0}};
+        jobs[t] = j;
+        if (n_threads == 1) preset_worker(&jobs[t]);
+        else pthread_create(&th[t], NULL, preset_worker, &jobs[t]);
+    }
+    if (n_threads > 1)
+        for (int t = 0; t < n_threads; t++) pthread_join(th[t], NULL);
+    if (counters)
+        for (int t = 0; t < n_threads; t++)
+            for (int c = 0; c < NGO_RS_COUNT; c++) counters[c] += jobs[t].counters[c];
+    free(jobs); free(th);
+    return 0;
+}
+
+/* out[s][i] = ngo_policy_draw(seed, first_gid + i, t0 + s, n_actions[i]) for s < n_steps, i < n; branch (may be NULL)
+ * receives the branch taken, laid out like out. */
+typedef struct {
+    uint64_t seed, first_gid; int64_t n, begin, end; const int32_t* n_actions; uint32_t t0; int n_steps;
+    int32_t* out; uint8_t* branch;
+} pdraw_t;
+
+static void* pdraw_worker(void* arg) {
+    pdraw_t* j = (pdraw_t*)arg;
+    for (int s = 0; s < j->n_steps; s++)
+        for (int64_t i = j->begin; i < j->end; i++) {
+            int br;
+            j->out[s * j->n + i] = ngo_policy_draw(j->seed, j->first_gid + (uint64_t)i, j->t0 + (uint32_t)s,
+                                                   (uint32_t)j->n_actions[i], &br);
+            if (j->branch) j->branch[s * j->n + i] = (uint8_t)br;
+        }
+    return NULL;
+}
+
+int ngo_policy_draw_batch(uint64_t seed, uint64_t first_gid, int64_t n, const int32_t* n_actions, uint32_t t0, int n_steps,
+                          int32_t* out, uint8_t* branch, int n_threads) {
+    if (n_threads < 1) n_threads = 1;
+    if (n_threads > 1024) n_threads = 1024;
+    pdraw_t* jobs = (pdraw_t*)malloc(sizeof(pdraw_t) * (size_t)n_threads);
+    pthread_t* th = (pthread_t*)malloc(sizeof(pthread_t) * (size_t)n_threads);
+    int64_t per = (n + n_threads - 1) / n_threads;
+    for (int t = 0; t < n_threads; t++) {
+        int64_t b = t * per, e = b + per;
+        if (b > n) b = n;
+        if (e > n) e = n;
+        pdraw_t j = {seed, first_gid, n, b, e, n_actions, t0, n_steps, out, branch};
+        jobs[t] = j;
+        if (n_threads == 1) pdraw_worker(&jobs[t]);
+        else pthread_create(&th[t], NULL, pdraw_worker, &jobs[t]);
+    }
+    if (n_threads > 1)
+        for (int t = 0; t < n_threads; t++) pthread_join(th[t], NULL);
+    free(jobs); free(th);
     return 0;
 }
 

@@ -50,6 +50,18 @@ def lib():
                                   C.c_void_p, C.c_void_p, C.c_void_p, C.c_int]
         L.ngo_reset_batch.argtypes = [C.c_void_p, C.c_void_p, C.c_int, C.c_int64, C.c_uint32, C.c_void_p, C.c_void_p,
                                       C.c_void_p, C.c_int, C.c_void_p]
+        L.ngo_philox4x32_10.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p]
+        L.ngo_philox_below.argtypes = [C.c_uint64, C.c_uint64, C.c_uint32, C.c_uint32, C.c_uint32, C.c_int64, C.c_void_p,
+                                       C.c_void_p]
+        L.ngo_policy_draw.argtypes = [C.c_uint64, C.c_uint64, C.c_uint32, C.c_uint32, C.c_void_p]
+        L.ngo_policy_draw.restype = C.c_int32
+        L.ngo_reset_philox.argtypes = [C.c_void_p, C.c_int, C.c_uint64, C.c_uint64, C.c_uint32, C.c_uint32, C.c_void_p,
+                                       C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p]
+        L.ngo_reset_philox_batch.argtypes = [C.c_void_p, C.c_void_p, C.c_int, C.c_int64, C.c_uint64, C.c_uint64,
+                                             C.c_void_p, C.c_uint32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
+                                             C.c_void_p, C.c_int, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_int]
+        L.ngo_policy_draw_batch.argtypes = [C.c_uint64, C.c_uint64, C.c_int64, C.c_void_p, C.c_uint32, C.c_int,
+                                            C.c_void_p, C.c_void_p, C.c_int]
         _lib = L
     return _lib
 
@@ -75,6 +87,47 @@ class MT(object):
         a = np.ascontiguousarray(arr, dtype=np.int32)
         lib().ngo_shuffle_i32(self.buf, a.ctypes.data, len(a))
         return a
+
+
+_U64 = 2 ** 64 - 1
+# counters of ngo_reset_philox (ngw_oracle.c): what the restated resets did, summed over the envs
+RESET_EVENTS = ('fallback', 'place_fail', 'treetap_fail', 'subset', 'all_win', 'list', 'arrival')
+
+
+def philox4x32_10(ctr, key):
+    """One block of the device's Philox4x32-10 as restated in ngw_oracle.c: 4 uint32 words."""
+    c = np.ascontiguousarray(ctr, np.uint32)
+    k = np.ascontiguousarray(key, np.uint32)
+    out = np.zeros(4, np.uint32)
+    lib().ngo_philox4x32_10(c.ctypes.data, k.ctypes.data, out.ctypes.data)
+    return out
+
+
+def philox_below(seed, gid, episode, stream, n, count):
+    """The first `count` values of the device generator's below(n) on one stream, and the words they consumed."""
+    out = np.zeros(count, np.uint32)
+    used = C.c_uint32()
+    lib().ngo_philox_below(int(seed) & _U64, int(gid) & _U64, int(episode) & 0xFFFFFFFF, stream, n, count, out.ctypes.data,
+                           C.byref(used))
+    return out, used.value
+
+
+def policy_draw(seed, gid, t, n):
+    """(action, branch) of the device's random policy at step t of env gid: branch 0 = plain draw, 1 = inside Lemire's
+    threshold test but kept, 2 = rejected and continued on stream 0xFFE."""
+    br = C.c_int()
+    a = lib().ngo_policy_draw(int(seed) & _U64, int(gid) & _U64, int(t), int(n), C.byref(br))
+    return int(a), br.value
+
+
+def policy_draws(seed, first_gid, n_actions, n_steps, t0=0, n_threads=8):
+    """(actions int32 [n_steps, n], branch uint8 [n_steps, n]) of the device's random policy for envs first_gid + i."""
+    na = np.ascontiguousarray(n_actions, np.int32)
+    out = np.zeros((n_steps, na.size), np.int32)
+    br = np.zeros((n_steps, na.size), np.uint8)
+    lib().ngo_policy_draw_batch(int(seed) & _U64, int(first_gid) & _U64, na.size, na.ctypes.data, int(t0), int(n_steps),
+                                out.ctypes.data, br.ctypes.data, n_threads)
+    return out, br
 
 
 class OracleBatch(object):
@@ -119,6 +172,25 @@ class OracleBatch(object):
             lib().ngo_observe(cfg_ptr, self.ms, _p(m), _p(p), _p(v), _p(obs))
         rc |= lib().ngo_reset_legacy(cfg_ptr, self.ms, mt.buf, _p(m), _p(p), _p(v), 0, k, cc.c.n_reset_ops)
         return rc, obs
+
+    def reset_philox(self, seed, first_gid, episode, key_mask=0xFFFFFFFF, k_obs=None, mask=None, want_obs=True,
+                     n_threads=8):
+        """Resets with the DEVICE's generator (ngw_oracle.c, last section): env i (where mask, default all) is reset at
+        gid first_gid + i and episode word episode (scalar or [n]; the word the reset uses and stores, i.e. the env's
+        previous episode + 1).  Returns (flags uint32 [n]: the reset's PLACEMENT bit, 0 for envs not reset; observation
+        int32 [n, obs_dim] taken after k_obs ops (scalar or [n]; None = each config's reset_obs_after_ops), or None;
+        event counters, a dict over RESET_EVENTS)."""
+        ep = np.ascontiguousarray(np.broadcast_to(np.asarray(episode, np.uint64) & 0xFFFFFFFF, (self.n,)), np.uint32)
+        ko = None if k_obs is None else np.ascontiguousarray(np.broadcast_to(k_obs, (self.n,)), np.int32)
+        mk = None if mask is None else np.ascontiguousarray(mask, np.uint8)
+        flags = np.zeros(self.n, np.uint32)
+        obs = np.zeros((self.n, self.obs_dim), np.int32) if (want_obs and self.obs_dim) else None
+        counters = np.zeros(8, np.int64)
+        lib().ngo_reset_philox_batch(self.cfgs, _p(self.cfg_id), self.ms, self.n, int(seed) & _U64, int(first_gid) & _U64,
+                                     _p(ep), int(key_mask) & 0xFFFFFFFF, _p(mk), _p(ko), _p(self.map), _p(self.pose),
+                                     _p(self.inv), self.inv_stride, _p(obs), self.obs_dim, _p(flags), _p(counters),
+                                     n_threads)
+        return flags, obs, dict(zip(RESET_EVENTS, counters.tolist()))
 
     def observe(self):
         obs = np.zeros((self.n, max(self.obs_dim, 1)), np.int32)
