@@ -37,11 +37,53 @@ int fail(const std::string& m) { g_err = m; return 1; }
 // of this library's kernels, which trigger their dependents only after their own wait — cannot have started its body
 // before that writer had completed.  Launches the library cannot see (the caller's own kernels, copies) only add
 // distance.  The first launch of a stream capture is always conservative: a graph can be replayed after anything.
+//
+// Capture chains.  Inside a stream capture, a run of consecutive stepping one-step launches (nothing else captured
+// between them: the stream's dependency set is exactly the one the library left after the previous launch) is spread
+// over kBranches parallel branches of the graph.  The k-th handle to appear in the chain is pinned to branch
+// k % kBranches; its launch depends only on the tip of that branch (the branch's first launch: on the chain's base, the
+// dependency set the chain started from), and after every launch the stream's dependency set is restored to every
+// branch's tip, so whatever the caller captures next (a kernel, an event record, the end of the capture) waits for all of
+// them.  Branches are unordered against each other, so a launch joins a branch only if its caller buffers (launch_tail)
+// do not conflict with those of any launch already on ANOTHER branch of the chain; otherwise, and for every other
+// library launch, the chain ends there (the launch depends on every tip).  Within a branch the proof above holds with
+// "the stream" read as "the branch": a handle's state is only ever written on its own branch, so the branch predecessor
+// of another handle is gated behind that handle's last writer exactly as the stream predecessor is without branches.
+// With as many branches as handles or more, every launch of a branch belongs to the same handle and waits (mode 0).
+// Only one-wave launches branch (see branchable).
+// W, measured on one B200 (1000 W power limit, 1965 MHz max SM clock) with bench.py's C2 line (18 rotating 65,536-env
+// batches, 1008-launch graphs): 4.88 / 4.89 / 4.82 us per step with W = 2 / 3 / 4, against 5.97 without branches —
+// no W beats another beyond the run-to-run spread; 3 is the shape of bench.py's `overlapped` arm (4.88 there).
+static const int kBranches = 3;
+
+struct Branch {
+    StreamTail tail;                      // its latest launch; tail.node is the branch's tip
+    std::vector<MemRange> rd, wr;         // caller buffers of every launch placed on it in this chain
+};
+struct Chain {
+    bool active = false;
+    std::vector<cudaGraphNode_t> base;    // the dependency set the chain started from,
+    StreamTail base_tail;                 // the stream's latest launch at that point
+    std::vector<ngw_handle*> base_block;  // and the handles whose launches may be nodes of the base
+    std::vector<ngw_handle*> pinned;      // pinned[k] runs on branch k % kBranches
+    Branch br[kBranches];
+    int n_br = 0;                         // branches started
+    int last = -1;                        // branch of the chain's latest launch
+    std::vector<cudaGraphNode_t> left;    // the dependency set the library left after it: every branch's tip
+};
+struct StreamRec {
+    StreamTail tail;                      // the latest library launch on the stream
+    Chain chain;
+};
+
 static std::mutex g_order_mu;
-static std::unordered_map<cudaStream_t, StreamTail> g_last_writer;
+static std::unordered_map<cudaStream_t, StreamRec> g_streams;
 static thread_local bool g_first_in_capture = false; // the latest claim_stream saw the first library launch of a stream capture
 static thread_local bool g_capturing = false;        // capture state of the stream seen by the latest claim_stream of this thread
 static thread_local bool g_adjacent_hint = false;   // ngw_step_many: this launch directly follows the library's previous launch on the stream
+static thread_local int g_branch = -1;               // branch of the chain the latest claim_stream placed its launch on, -1: none
+static thread_local bool g_branch_head = false;      // ... the first launch of a branch other than the chain's first
+static thread_local bool g_cross_branch = false;     // ... a branch other than its stream predecessor's
 
 static bool overlaps(const MemRange* a, int na, const MemRange* b, int nb) {
     for (int i = 0; i < na; i++)
@@ -50,39 +92,123 @@ static bool overlaps(const MemRange* a, int na, const MemRange* b, int nb) {
     return false;
 }
 
-// Returns 0 (conservative), 1 (state loads may precede griddepcontrol.wait) or 2 (the launch is independent of its
-// predecessor: see step1w_kernel's gate warp).  2 needs PROOF that nothing sits between the two launches: inside a stream
-// capture the stream's dependency set must be exactly the graph node of the previous launch; that launch must be a plain
-// one-step launch of ANOTHER handle, and the caller buffers of the two launches must not overlap.  Then everything this
-// launch reads besides its own state (the actions) was complete before the predecessor was let go by ITS gate.
-int claim_stream(ngw_handle* h, cudaStream_t s, bool want_early, const StreamTail* mine) {
+static bool same_set(const std::vector<cudaGraphNode_t>& a, const std::vector<cudaGraphNode_t>& b) {
+    if (a.size() != b.size()) return false;
+    for (cudaGraphNode_t x : a) {
+        bool found = false;
+        for (cudaGraphNode_t y : b) found |= x == y;
+        if (!found) return false;
+    }
+    return true;
+}
+
+static bool contains(const std::vector<ngw_handle*>& v, const ngw_handle* h) {
+    for (const ngw_handle* x : v) if (x == h) return true;
+    return false;
+}
+
+static void add_ranges(std::vector<MemRange>& to, const MemRange* r, int n) {
+    for (int i = 0; i < n; i++) {
+        bool known = false;
+        for (const MemRange& x : to) known |= x.lo <= r[i].lo && r[i].hi <= x.hi;
+        if (!known) to.push_back(r[i]);
+    }
+}
+
+// a read of one branch of what another writes, or two writes of one buffer
+static bool conflicts(const StreamTail& mine, const Branch& other) {
+    const int nr = (int)other.rd.size(), nw = (int)other.wr.size();
+    return overlaps(mine.wr, mine.n_wr, other.wr.data(), nw) || overlaps(mine.wr, mine.n_wr, other.rd.data(), nr) ||
+           overlaps(mine.rd, mine.n_rd, other.wr.data(), nw);
+}
+
+// Mode of a launch against its predecessor t: 0 (conservative), 1 (state loads may precede griddepcontrol.wait) or 2
+// (independent of it: see step1w_kernel's gate warp).  `blocked`: a launch of this handle may be a direct predecessor.
+// 2 needs PROOF that nothing sits between the two launches (`adjacent`: the dependency set is exactly t's graph node, or
+// one call issued both), that t is a plain one-step launch of ANOTHER handle, and that the caller buffers of the two do
+// not overlap.  Then everything this launch reads besides its own state (the actions) was complete before t was let go
+// by ITS gate.
+static int launch_mode(const StreamTail& t, bool blocked, unsigned long long cap_id, bool adjacent, const StreamTail* mine) {
+    if (t.h == nullptr || blocked || t.cap_id != cap_id) return 0;
+    if (mine != nullptr && t.pure_step && adjacent &&
+        !overlaps(mine->wr, mine->n_wr, t.wr, t.n_wr) && !overlaps(mine->wr, mine->n_wr, t.rd, t.n_rd) &&
+        !overlaps(mine->rd, mine->n_rd, t.wr, t.n_wr))
+        return 2;
+    return 1;
+}
+
+// Returns the launch's mode (launch_mode) and, for a stepping one-step launch inside a capture (`can_branch`), places it on
+// a branch of the stream's capture chain: the stream's dependency set is then that branch's predecessor until
+// join_branches.
+int claim_stream(ngw_handle* h, cudaStream_t s, bool want_early, const StreamTail* mine, bool can_branch) {
     unsigned long long cap_id = 0;
     cudaStreamCaptureStatus cap = cudaStreamCaptureStatusNone;
-    const cudaGraphNode_t* deps = nullptr;
-    size_t n_deps = 0;
-    if (cudaStreamGetCaptureInfo(s, &cap, &cap_id, nullptr, &deps, &n_deps) != cudaSuccess) {
-        cudaGetLastError(); cap = cudaStreamCaptureStatusNone; n_deps = 0;
+    const cudaGraphNode_t* d = nullptr;
+    size_t n_d = 0;
+    if (cudaStreamGetCaptureInfo(s, &cap, &cap_id, nullptr, &d, &n_d) != cudaSuccess) {
+        cudaGetLastError(); cap = cudaStreamCaptureStatusNone; n_d = 0;
     }
-    if (cap != cudaStreamCaptureStatusActive) { cap_id = 0; n_deps = 0; }
+    if (cap != cudaStreamCaptureStatusActive) { cap_id = 0; n_d = 0; }
     g_capturing = cap == cudaStreamCaptureStatusActive;
+    const std::vector<cudaGraphNode_t> deps(d, d + n_d);
+    g_branch = -1; g_branch_head = false; g_cross_branch = false;
     std::lock_guard<std::mutex> lk(g_order_mu);
-    auto it = g_last_writer.find(s);
-    g_first_in_capture = cap_id != 0 && (it == g_last_writer.end() || it->second.cap_id != cap_id);
-    int mode = 0;
-    if (want_early && it != g_last_writer.end() && it->second.h != nullptr && it->second.h != h && it->second.cap_id == cap_id) {
-        mode = 1;
-        const StreamTail& t = it->second;
-        const bool adjacent = (cap_id != 0 && n_deps == 1 && t.node != nullptr && deps[0] == t.node) ||   // proven by the capture
-                              (g_adjacent_hint && (cap_id == 0 || n_deps == 1));                        // issued back to back by one call
-        if (mine != nullptr && t.pure_step && adjacent &&
-            !overlaps(mine->wr, mine->n_wr, t.wr, t.n_wr) && !overlaps(mine->wr, mine->n_wr, t.rd, t.n_rd) &&
-            !overlaps(mine->rd, mine->n_rd, t.wr, t.n_wr))
-            mode = 2;
+    StreamRec& r = g_streams[s];
+    const StreamTail t = r.tail;
+    Chain& c = r.chain;
+    g_first_in_capture = cap_id != 0 && t.cap_id != cap_id;
+    // A chain of this capture that no library launch has ended yet: every handle it pinned may own a node of the current
+    // dependency set — its tips — even when something else joined the set (a wait on another stream of the capture).
+    const bool in_chain = c.active && cap_id != 0 && t.cap_id == cap_id;
+    const bool chained = in_chain && same_set(deps, c.left);
+    can_branch = can_branch && cap_id != 0 && mine != nullptr && h->concurrent;
+    int mode = 0, b = -1, pin = -1;
+    if (can_branch && chained) {
+        for (int k = 0; k < (int)c.pinned.size() && pin < 0; k++) if (c.pinned[k] == h) pin = k;
+        b = (pin >= 0 ? pin : (int)c.pinned.size()) % kBranches;
+        for (int o = 0; o < c.n_br && b >= 0; o++)
+            if (o != b && conflicts(*mine, c.br[o])) b = -1;
+    }
+    if (can_branch && b < 0) {            // a new chain starts at this launch, from the current dependency set
+        Chain n;
+        n.active = true; n.base = deps; n.base_tail = t;
+        n.base_block = in_chain ? c.pinned : std::vector<ngw_handle*>{};
+        n.base_block.push_back(t.h);
+        c = n;
+        b = 0; pin = -1;
+    }
+    if (b >= 0) {
+        const bool head = b >= c.n_br;
+        const StreamTail& pred = head ? c.base_tail : c.br[b].tail;
+        std::vector<cudaGraphNode_t> pd = head ? c.base : std::vector<cudaGraphNode_t>{pred.node};
+        if (!same_set(pd, deps) &&
+            cudaStreamUpdateCaptureDependencies(s, pd.data(), pd.size(), cudaStreamSetCaptureDependencies) != cudaSuccess) {
+            cudaGetLastError();
+            c.active = false; b = -1;     // (the dependency set is unchanged: the launch joins every tip)
+        } else {
+            const bool blocked = head ? contains(c.base_block, h) : pred.h == h;
+            const bool adjacent = pd.size() == 1 && pred.node != nullptr && pd[0] == pred.node;
+            mode = want_early ? launch_mode(pred, blocked, cap_id, adjacent, mine) : 0;
+            if (pin < 0) c.pinned.push_back(h);
+            if (head) c.n_br = b + 1;
+            add_ranges(c.br[b].rd, mine->rd, mine->n_rd);
+            add_ranges(c.br[b].wr, mine->wr, mine->n_wr);
+            g_branch = b; g_branch_head = head && b > 0; g_cross_branch = c.last >= 0 && c.last != b;
+            c.last = b;
+        }
+    }
+    if (b < 0) {
+        const bool adjacent = (cap_id != 0 && n_d == 1 && t.node != nullptr && deps[0] == t.node) ||   // proven by the capture
+                              (g_adjacent_hint && (cap_id == 0 || n_d == 1));                        // issued back to back by one call
+        const bool blocked = t.h == h || (in_chain && contains(c.pinned, h));   // (a chain's tips are direct predecessors)
+        mode = want_early ? launch_mode(t, blocked, cap_id, adjacent, mine) : 0;
+        c.active = false;
     }
     StreamTail now;
     if (mine != nullptr) now = *mine;
     now.h = h; now.cap_id = cap_id; now.node = nullptr; now.pure_step = false;
-    g_last_writer[s] = now;
+    r.tail = now;
+    if (g_branch >= 0) c.br[g_branch].tail = now;
     return mode;
 }
 
@@ -95,16 +221,45 @@ static void note_launched(cudaStream_t s, bool pure_step) {
     // (eager launches have no graph node: the driver call is only made while the stream is being captured)
     if (g_capturing && cudaStreamGetCaptureInfo(s, &cap, &cap_id, nullptr, &deps, &n_deps) != cudaSuccess) { cudaGetLastError(); return; }
     std::lock_guard<std::mutex> lk(g_order_mu);
-    auto it = g_last_writer.find(s);
-    if (it == g_last_writer.end()) return;
-    it->second.pure_step = pure_step;
-    it->second.node = (cap == cudaStreamCaptureStatusActive && n_deps == 1) ? deps[0] : nullptr;
+    auto it = g_streams.find(s);
+    if (it == g_streams.end()) return;
+    StreamTail& t = it->second.tail;
+    t.pure_step = pure_step;
+    t.node = (cap == cudaStreamCaptureStatusActive && n_deps == 1) ? deps[0] : nullptr;
+    if (g_branch >= 0 && it->second.chain.active) {
+        StreamTail& bt = it->second.chain.br[g_branch].tail;
+        bt.pure_step = t.pure_step; bt.node = t.node;
+    }
+}
+
+// after the last launch that claim_stream placed on a branch (the step and the queued-reset kernel behind it): the stream
+// depends on every branch's tip again
+static cudaError_t join_branches(cudaStream_t s) {
+    if (g_branch < 0) return cudaSuccess;
+    g_branch = -1;
+    std::lock_guard<std::mutex> lk(g_order_mu);
+    auto it = g_streams.find(s);
+    if (it == g_streams.end() || !it->second.chain.active) return cudaSuccess;
+    Chain& c = it->second.chain;
+    c.left.clear();
+    for (int b = 0; b < c.n_br; b++) {
+        if (c.br[b].tail.node == nullptr) { c.active = false; return cudaErrorStreamCaptureInvalidated; }
+        c.left.push_back(c.br[b].tail.node);
+    }
+    const cudaError_t e = cudaStreamUpdateCaptureDependencies(s, c.left.data(), c.left.size(), cudaStreamSetCaptureDependencies);
+    if (e != cudaSuccess) c.active = false;
+    return e;
 }
 
 static void forget_handle(ngw_handle* h) {
     std::lock_guard<std::mutex> lk(g_order_mu);
-    for (auto& kv : g_last_writer)
-        if (kv.second.h == h) kv.second.h = nullptr;
+    for (auto& kv : g_streams) {
+        const Chain& c = kv.second.chain;
+        if (kv.second.tail.h == h || contains(c.pinned, h) || contains(c.base_block, h)) {
+            kv.second.tail.h = nullptr;
+            kv.second.chain.active = false;
+        }
+    }
 }
 
 static int before_device_call(ngw_handle* h, cudaStream_t s) {
@@ -509,7 +664,8 @@ static int obs_srow(int obs_row_bytes) {
 // after a one-step launch: the stream's record for the next launch's independence proof, and the handle's counters
 static void note_step_launched(ngw_handle* h, cudaStream_t s, const StepParams& p) {
     note_launched(s, p.actions != nullptr);
-    h->concurrent_launches += p.concurrent;
+    // launches that may overlap their stream predecessor: independent of it on one branch, or on another branch
+    h->concurrent_launches += (p.concurrent || g_cross_branch) ? 1 : 0;
     h->last_step_concurrent = p.concurrent != 0;
 }
 
@@ -529,6 +685,11 @@ static StreamTail launch_tail(const StepParams& p) {
     add(me.wr, me.n_wr, p.trunc, (size_t)n_env); add(me.wr, me.n_wr, p.final_obs, (size_t)n_env * p.obs_row_bytes);
     return me;
 }
+
+// Which one-step launches may join a capture chain's branches: stepping launches of ONE wave.  Launches of several waves
+// keep the two-deep chain: on the same B200 as kBranches, branching them too moved C3 23.2 -> 21.4 us per step but C5
+// (auto-reset, map 40) 244 -> 267 us, and C4 not at all (96.9 / 97.2).
+static bool branchable(const StepParams& p, bool one_wave) { return p.actions != nullptr && one_wave; }
 
 // one-step launches (ngw_step / ngw_step_host / ngw_observe): several tile groups per CTA
 template <int NC>
@@ -573,7 +734,7 @@ static cudaError_t launch_step1_nc(ngw_handle* h, StepParams p, cudaStream_t s) 
     // only for one-wave launches: with several waves the loads of later waves never wait anyway, and issuing them ahead
     // of the tile's zero-fill measured 4 % slower (C4 122 vs 127 us)
     const StreamTail me = launch_tail(p);
-    const int mode = claim_stream(h, s, true, &me);
+    const int mode = claim_stream(h, s, true, &me, branchable(p, tiles <= per_sm * h->sm_count));
     // independent of the predecessor (see claim_stream): no thread waits for it except the gate CTA (block 0)
     p.concurrent = (mode == 2 && h->concurrent && p.actions != nullptr) ? 1 : 0;
     p.early_state = (p.concurrent || (mode >= 1 && C > 1)) ? 1 : 0;
@@ -607,7 +768,7 @@ static cudaError_t launch_step1w_nc(ngw_handle* h, StepParams p, cudaStream_t s)
     if (c_cap < 1) return cudaErrorNotSupported;
     const StreamTail me = launch_tail(p);
     const bool one_wave = tiles <= (long long)c_cap * h->sm_count;
-    const int mode = claim_stream(h, s, true, &me);
+    const int mode = claim_stream(h, s, true, &me, branchable(p, one_wave));
     p.early_state = mode >= 1 ? 1 : 0;
     // (one-wave launches overlap whole; with several waves the next launch fills the SMs as the last wave drains)
     p.concurrent = (mode == 2 && h->concurrent && p.actions != nullptr) ? 1 : 0;
@@ -618,8 +779,8 @@ static cudaError_t launch_step1w_nc(ngw_handle* h, StepParams p, cudaStream_t s)
     // leave partial CTAs).
     int C;
     if (!one_wave) C = 8;
-    else if (p.concurrent || (g_first_in_capture && h->concurrent && p.actions != nullptr))
-        C = (int)((tiles + 2 * h->sm_count - 1) / (2 * h->sm_count));   // (a capture's first launch waits, but its successor overlaps it)
+    else if (p.concurrent || g_branch_head || (g_first_in_capture && h->concurrent && p.actions != nullptr))
+        C = (int)((tiles + 2 * h->sm_count - 1) / (2 * h->sm_count));   // (a capture's or a branch's first launch waits, but its successor overlaps it)
     else C = (int)((tiles + h->sm_count - 1) / h->sm_count);
     if (C < 1) C = 1;
     if (C > c_cap) C = c_cap;
@@ -645,7 +806,17 @@ static cudaError_t launch_one_step(ngw_handle* h, const StepParams& p, cudaStrea
 
 static const int kResetCtasPerSmOverlapped = 1;    // queued-reset grid behind an overlapped step, see launch_step
 
+static int launch_step_on_branch(ngw_handle* h, const StepParams& p, cudaStream_t s);
+
 static int launch_step(ngw_handle* h, const StepParams& p, cudaStream_t s) {
+    const int rc = launch_step_on_branch(h, p, s);
+    const cudaError_t e = join_branches(s);             // (no-op unless claim_stream placed the step on a branch)
+    if (rc == 0 && e != cudaSuccess) return fail(std::string("rejoining the capture branches: ") + cudaGetErrorString(e));
+    return rc;
+}
+
+// the step and the queued-reset kernel behind it: on the branch claim_stream chose for the step, if any
+static int launch_step_on_branch(ngw_handle* h, const StepParams& p, cudaStream_t s) {
     if (p.env_end <= p.env_begin) return 0;
     const int nc = h->n_cfgs;
     cudaError_t e;

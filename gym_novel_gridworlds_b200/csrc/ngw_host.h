@@ -60,7 +60,7 @@ struct StreamTail {                       // the latest library launch on a stre
 
 int fail(const std::string& m);
 // see ngw_capi.cu
-int claim_stream(ngw_handle* h, cudaStream_t s, bool want_early, const StreamTail* mine = nullptr);
+int claim_stream(ngw_handle* h, cudaStream_t s, bool want_early, const StreamTail* mine = nullptr, bool can_branch = false);
 // ngw_rollout.cu
 cudaError_t ngw_launch_rollout(ngw_handle* h, const StepParams& p, cudaStream_t s);
 int ngw_rollout_set_attributes();
