@@ -89,6 +89,7 @@ struct EnvRow {
     int32_t* inv;                         // staged inventory row
     int ms;
     int r, c, facing, sel;
+    bool inv_dirty = false;               // the step changed the inventory row (inv_add): step1w_kernel stores only such rows
     __device__ __forceinline__ void set_pose(uchar4 ps) { r = ps.x; c = ps.y; facing = ps.z; sel = ps.w; }
     __device__ __forceinline__ uchar4 pose() const {
         return make_uchar4((unsigned char)r, (unsigned char)c, (unsigned char)facing, (unsigned char)sel);
@@ -104,6 +105,12 @@ struct StepOut {
     int goal;       // the goal item is in the inventory after the step (done by success, not by fire / truncation)
     __device__ __forceinline__ void clear() { reward = 0; done = 0; result = 0; cost = 0.0f; msg = 0; goal = 0; }
 };
+
+// every inventory change a step makes goes through here (resets store whole rows and do not)
+__device__ __forceinline__ void inv_add(EnvRow& e, int item, int delta) {
+    e.inv[item] += delta;
+    e.inv_dirty = true;
+}
 
 __device__ __forceinline__ int msg_of(int code, int arg) { return code | (arg << 5); }
 
@@ -144,7 +151,7 @@ __device__ __forceinline__ void grab_entities(EnvRow& e, const ngw_config& cfg) 
             int id = cell(e, rr, cc);
             if (id != 0 && in_mask(mask, id)) {
                 set_cell(e, rr, cc, 0);
-                e.inv[id] += 1;
+                inv_add(e, id, 1);
             }
         }
 }
@@ -174,8 +181,8 @@ __device__ __forceinline__ void craft(EnvRow& e, const ngw_config& cfg, int slot
     }
     o.reward = rc.reward_ok;
     o.msg = msg_of(NGW_MSG_CRAFTED, rc.out_item);
-    for (int i = 0; i < n_in; i++) e.inv[rc.in_item[i]] -= (int)rc.in_qty[i];
-    e.inv[rc.out_item] += (int)rc.out_qty;
+    for (int i = 0; i < n_in; i++) inv_add(e, rc.in_item[i], -(int)rc.in_qty[i]);
+    inv_add(e, rc.out_item, (int)rc.out_qty);
     o.cost = rc.cost_ok;
 }
 
@@ -203,11 +210,11 @@ __device__ __forceinline__ void terminal_op(EnvRow& e, const ngw_config& cfg, co
             int variant = a.variant;
             if (variant == NGW_BRK_BASE) {                            // pogostick_v1_env.py:283-289
                 set_cell(e, fr, fc, 0);
-                e.inv[front] += 1;
+                inv_add(e, front, 1);
                 if (in_mask(cfg.break_reward_mask, front)) o.reward = cfg.reward_intermediate;
             } else if (variant == NGW_BRK_INCREASE) {                 // novelty_wrappers.py:1444-1454
                 set_cell(e, fr, fc, 0);
-                e.inv[front] += (a.arg == NGW_NONE || a.arg == front) ? 2 : 1;
+                inv_add(e, front, (a.arg == NGW_NONE || a.arg == front) ? 2 : 1);
                 o.reward = cfg.reward_intermediate;
             } else {                                                  // axe / axetobreak, novelty_wrappers.py:55-81, 482-501
                 bool has_axe = e.inv[a.arg] >= 1;
@@ -215,14 +222,14 @@ __device__ __forceinline__ void terminal_op(EnvRow& e, const ngw_config& cfg, co
                 bool iron = has_axe && !wooden && cfg.id_iron_axe != NGW_NONE && e.sel == cfg.id_iron_axe;
                 if (wooden || iron) {
                     set_cell(e, fr, fc, 0);
-                    e.inv[front] += (variant == NGW_BRK_AXE_INC) ? 2 : 1;
+                    inv_add(e, front, (variant == NGW_BRK_AXE_INC) ? 2 : 1);
                     o.reward = cfg.reward_intermediate;
                     o.cost = wooden ? 1800.0f : 900.0f;
                 } else if (variant == NGW_BRK_AXETOBREAK) {
                     o.result = 0; o.msg = msg_of(NGW_MSG_NEED_AXE, a.arg);
                 } else {                                              // breaks, but no reward even for tree_log (Q4)
                     set_cell(e, fr, fc, 0);
-                    e.inv[front] += 1;
+                    inv_add(e, front, 1);
                 }
             }
             break;
@@ -231,7 +238,7 @@ __device__ __forceinline__ void terminal_op(EnvRow& e, const ngw_config& cfg, co
             o.cost = 300.0f;
             if (e.inv[cfg.id_tree_tap] >= 1 && cell(e, fr, fc) == 0) {
                 set_cell(e, fr, fc, cfg.id_tree_tap);
-                e.inv[cfg.id_tree_tap] -= 1;
+                inv_add(e, cfg.id_tree_tap, -1);
                 o.msg = NGW_MSG_TAP_PLACED;
                 if (next_to(e, fr, fc, cfg.id_tree_log)) o.reward = cfg.reward_intermediate;
             } else {
@@ -242,7 +249,7 @@ __device__ __forceinline__ void terminal_op(EnvRow& e, const ngw_config& cfg, co
         case NGW_OP_EXTRACT_RUBBER:                                   // pogostick_v1_env.py:315-331, novelty_wrappers.py:1537-1551
             o.cost = 120.0f;
             if (cell(e, fr, fc) == cfg.id_tree_tap && next_to(e, fr, fc, cfg.id_tree_log)) {
-                e.inv[cfg.id_rubber] += a.arg;
+                inv_add(e, cfg.id_rubber, a.arg);
                 o.reward = cfg.reward_intermediate; o.cost = 50000.0f;
             } else {
                 o.result = 0;
@@ -252,7 +259,7 @@ __device__ __forceinline__ void terminal_op(EnvRow& e, const ngw_config& cfg, co
         case NGW_OP_EXTRACT_STRING:                                   // bow_v1_env.py:293-304, novelty_wrappers.py:1524-1536
             o.cost = 120.0f;
             if (cell(e, fr, fc) == cfg.id_wool) {
-                e.inv[cfg.id_string] += a.arg;
+                inv_add(e, cfg.id_string, a.arg);
                 set_cell(e, fr, fc, 0);
                 o.reward = cfg.reward_intermediate; o.cost = 5000.0f;
             } else { o.result = 0; o.msg = NGW_MSG_NO_WOOL; }
@@ -269,7 +276,7 @@ __device__ __forceinline__ void terminal_op(EnvRow& e, const ngw_config& cfg, co
             o.cost = 3600.0f * 1.2f;
             if (!in_mask(cfg.unbreakable_mask, front)) {
                 set_cell(e, fr, fc, 0);
-                e.inv[front] += 2;
+                inv_add(e, front, 2);
                 o.reward = cfg.reward_intermediate;
             } else { o.result = 0; o.msg = msg_of(NGW_MSG_CANNOT_CHOP, front); }
             break;
@@ -312,7 +319,7 @@ __device__ __forceinline__ void step_env(EnvRow& e, const ngw_config& cfg, const
         if (layer == NGW_LAYER_END) break;
         if (layer == NGW_LAYER_CRATE) {                               // novelty_wrappers.py:1085-1088
             if (front == cfg.id_crate)
-                for (int it = 0; it < cfg.n_items; it++) e.inv[it] += (int)cfg.crate_add[it];
+                for (int it = 0; it < cfg.n_items; it++) inv_add(e, it, (int)cfg.crate_add[it]);
         } else if (layer == NGW_LAYER_FENCE_MEDIUM || layer == NGW_LAYER_FENCE_HARD) {   // novelty_wrappers.py:926-958
             bool pass;
             int fence = cfg.id_fence;
