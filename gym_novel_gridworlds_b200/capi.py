@@ -8,7 +8,7 @@ from . import opcodes as oc
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, 'csrc', 'libngw_b200.so')
-ABI_VERSION = 11
+ABI_VERSION = 12
 OBS_I32, OBS_U8, OBS_HITS = 0, 1, 2
 
 
@@ -67,6 +67,12 @@ class StateViewC(C.Structure):
                 ('obs_format', C.c_int32), ('obs_row_bytes', C.c_int32)]
 
 
+class RolloutRecordC(C.Structure):
+    """struct ngw_rollout_record (include/ngw.h): the per-step buffers a rollout fills, [max_steps][n_envs_padded]."""
+    _fields_ = [('max_steps', C.c_int32), ('obs', C.c_void_p), ('reward', C.c_void_p), ('step_cost', C.c_void_p),
+                ('done', C.c_void_p), ('result', C.c_void_p), ('truncated', C.c_void_p), ('final_obs', C.c_void_p)]
+
+
 # name -> (restype, argtypes); the same list is checked against include/ngw.h by the CPU test-suite
 EXPORTS = {
     'ngw_create': (C.c_int, [C.POINTER(C.c_void_p), C.POINTER(ConfigC), C.c_int32, C.c_int64, C.c_int32,
@@ -86,6 +92,7 @@ EXPORTS = {
     'ngw_step_many': (C.c_int, [C.c_void_p, C.c_int32, C.c_int32, C.c_int32, C.c_void_p]),
     'ngw_set_message_buffer': (C.c_int, [C.c_void_p, C.c_void_p]),
     'ngw_set_episode_end_buffers': (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p]),
+    'ngw_set_rollout_record': (C.c_int, [C.c_void_p, C.POINTER(RolloutRecordC)]),
     'ngw_step_host': (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
                                 C.c_int32, C.c_int32]),
     'ngw_rollout': (C.c_int, [C.c_void_p, C.c_void_p, C.c_int32, C.c_uint64, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,

@@ -652,7 +652,8 @@ static StepParams step_params(ngw_handle* h, const int32_t* actions, void* obs, 
 }  // extern "C" (templates need C++ linkage)
 
 static bool is_multi(const StepParams& p) {
-    return p.n_steps > 1 || p.random_policy || p.done_count != nullptr || p.actions_out != nullptr || p.policy_w != nullptr;
+    return p.n_steps > 1 || p.random_policy || p.done_count != nullptr || p.actions_out != nullptr || p.policy_w != nullptr ||
+           p.record;
 }
 
 // shared-memory row stride of a one-step kernel's observation tile (StepParams::obs_srow): rows of a multiple of 8 words
@@ -888,6 +889,17 @@ int ngw_step_many(const ngw_step_item* items, int32_t n_items, int32_t auto_rese
     return rc;
 }
 
+// a rollout with the handle's record (if one is set; the launcher passes it to the recording kernel); fails when the record
+// holds fewer than n_steps steps
+static int attach_record(const ngw_handle* h, StepParams& p, int32_t n_steps, const char* who) {
+    if (!h->rec_on) return 0;
+    if (n_steps > h->rec.max_steps)
+        return fail(std::string(who) + ": n_steps " + std::to_string(n_steps) + " > the rollout record's max_steps " +
+                    std::to_string(h->rec.max_steps));
+    p.record = 1;
+    return ngw_rollout_record_fits(h, p);
+}
+
 int ngw_rollout(ngw_handle* h, const int32_t* actions, int32_t n_steps, uint64_t policy_seed, void* obs,
                 float* reward_sum, float* cost_sum, int32_t* done_count, uint8_t* last_done, uint8_t* last_result,
                 int32_t* actions_out, int32_t auto_reset, int32_t max_episode_steps, void* stream) {
@@ -895,8 +907,6 @@ int ngw_rollout(ngw_handle* h, const int32_t* actions, int32_t n_steps, uint64_t
     if (n_steps < 1) return fail("ngw_rollout: n_steps must be >= 1");
     if (!reward_sum || !cost_sum || !last_done || !last_result) return fail("ngw_rollout: null output pointer");
     if (h->obs_dim > 0 && obs && ((uintptr_t)obs & 15)) return fail("ngw_rollout: obs must be 16-byte aligned");
-    CK(cudaSetDevice(h->device));
-    before_device_call(h, (cudaStream_t)stream);
     // any non-null pointer marks "stepping"; with the random policy it is never dereferenced
     const int32_t* act = actions ? actions : reinterpret_cast<const int32_t*>(h->zero_byte);
     StepParams p = step_params(h, act, obs, reward_sum, last_done, cost_sum, last_result, auto_reset, max_episode_steps,
@@ -904,6 +914,9 @@ int ngw_rollout(ngw_handle* h, const int32_t* actions, int32_t n_steps, uint64_t
     p.n_steps = n_steps; p.random_policy = actions ? 0 : 1; p.act_stride = h->n; p.policy_seed = policy_seed;
     p.done_count = done_count; p.actions_out = actions_out;
     p.trunc = nullptr; p.final_obs = nullptr;              // per-step episode ends have no place in a rollout's sums
+    if (attach_record(h, p, n_steps, "ngw_rollout")) return 1;   // (the per-step ones go to the record)
+    CK(cudaSetDevice(h->device));
+    before_device_call(h, (cudaStream_t)stream);
     return launch_step(h, p, (cudaStream_t)stream);
 }
 
@@ -920,13 +933,14 @@ int ngw_rollout_policy(ngw_handle* h, const int32_t* weights, const int32_t* bia
     if (n_steps < 1) return fail("ngw_rollout_policy: n_steps must be >= 1");
     if (!reward_sum || !cost_sum || !last_done || !last_result) return fail("ngw_rollout_policy: null output pointer");
     if ((uintptr_t)obs & 15) return fail("ngw_rollout_policy: obs must be 16-byte aligned");
-    CK(cudaSetDevice(h->device));
-    before_device_call(h, (cudaStream_t)stream);
     StepParams p = step_params(h, reinterpret_cast<const int32_t*>(h->zero_byte), obs, reward_sum, last_done, cost_sum,
                                last_result, auto_reset, max_episode_steps, 0, h->n);
     p.n_steps = n_steps; p.random_policy = 0; p.act_stride = h->n; p.done_count = done_count; p.actions_out = actions_out;
     p.policy_w = weights; p.policy_b = bias; p.policy_actions = n_policy_actions;
     p.trunc = nullptr; p.final_obs = nullptr;
+    if (attach_record(h, p, n_steps, "ngw_rollout_policy")) return 1;
+    CK(cudaSetDevice(h->device));
+    before_device_call(h, (cudaStream_t)stream);
     return launch_step(h, p, (cudaStream_t)stream);
 }
 
@@ -978,6 +992,19 @@ int ngw_set_episode_end_buffers(ngw_handle* h, uint8_t* truncated_dev, void* fin
     if ((uintptr_t)final_obs_dev & 15) return fail("ngw_set_episode_end_buffers: final_obs must be 16-byte aligned");
     h->trunc = truncated_dev;
     h->final_obs = static_cast<unsigned char*>(final_obs_dev);
+    return 0;
+}
+
+int ngw_set_rollout_record(ngw_handle* h, const ngw_rollout_record* rec) {
+    if (!h) return fail("null handle");
+    if (!rec) { h->rec_on = false; h->rec = ngw_rollout_record{}; return 0; }
+    if (rec->max_steps < 1) return fail("ngw_set_rollout_record: max_steps must be >= 1");
+    if (h->obs_dim > 0 && (((uintptr_t)rec->obs & 15) || ((uintptr_t)rec->final_obs & 15)))
+        return fail("ngw_set_rollout_record: obs and final_obs must be 16-byte aligned");
+    if (((uintptr_t)rec->reward & 3) || ((uintptr_t)rec->step_cost & 3))
+        return fail("ngw_set_rollout_record: reward and step_cost must be 4-byte aligned");
+    h->rec = *rec;
+    h->rec_on = true;
     return 0;
 }
 

@@ -32,6 +32,8 @@ struct ngw_handle {
     uint16_t* msg = nullptr;                       // caller-owned message-code buffer (ngw_set_message_buffer)
     uint8_t* trunc = nullptr;                      // caller-owned episode-end buffers (ngw_set_episode_end_buffers): truncated
     unsigned char* final_obs = nullptr;            // flags, last observation rows of auto-reset envs
+    ngw_rollout_record rec{};                      // caller-owned per-step record of the rollouts (ngw_set_rollout_record)
+    bool rec_on = false;
     int32_t* reset_list = nullptr; int32_t* reset_ctl = nullptr;   // auto-reset queue; ctl[0] = count, ctl[1] = finished CTAs
     int sm_count = 148;
     long long launches = 0, concurrent_launches = 0;
@@ -64,19 +66,25 @@ int claim_stream(ngw_handle* h, cudaStream_t s, bool want_early, const StreamTai
 // ngw_rollout.cu
 cudaError_t ngw_launch_rollout(ngw_handle* h, const StepParams& p, cudaStream_t s);
 int ngw_rollout_set_attributes();
+int ngw_rollout_record_fits(const ngw_handle* h, const StepParams& p);   // 0, or fail() with a message
 
 // shared memory of the lidar tables a kernel with NC inline configs stages (stage_lidar_luts)
 template <int NC>
 constexpr int lut_bytes() { return (NGW_MAX_MAP_SIZE + NGW_MAX_ITEMS * (NC > 0 ? NC : 0) + 127) & ~127; }
 
-// Launches a tile kernel with its argument block: the parameters plus the handle's first NC configs inline.
-template <int NC>
-cudaError_t launch_tiles(void (*kernel)(StepArgs<NC>), const ngw_handle* h, const StepParams& p, dim3 grid, dim3 block,
-                         size_t smem, cudaStream_t s) {
-    static thread_local StepArgs<NC> args;          // host staging of the argument block (copied by the launch); per thread,
+template <int NC> void set_record(StepArgs<NC>&, const RecordParams*) {}
+template <int NC> void set_record(RecArgs<NC>& a, const RecordParams* rec) { a.rec = *rec; }
+
+// Launches a tile kernel with its argument block: the parameters plus the handle's first NC configs inline (and, for the
+// recording rollout kernels, the record `rec`).
+template <int NC, typename Args = StepArgs<NC> >
+cudaError_t launch_tiles(void (*kernel)(Args), const ngw_handle* h, const StepParams& p, dim3 grid, dim3 block,
+                         size_t smem, cudaStream_t s, const RecordParams* rec = nullptr) {
+    static thread_local Args args;                  // host staging of the argument block (copied by the launch); per thread,
                                                     // so distinct handles stay independent across host threads
     args.p = p;
     for (int i = 0; i < NC && i < h->n_cfgs; i++) args.cfg[i] = h->h_cfgs[i];
+    set_record(args, rec);
     cudaLaunchConfig_t lc;
     memset(&lc, 0, sizeof(lc));
     lc.gridDim = grid; lc.blockDim = block; lc.dynamicSmemBytes = smem;

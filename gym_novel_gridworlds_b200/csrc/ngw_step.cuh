@@ -15,6 +15,8 @@
 #include <stdint.h>
 #include <string.h>
 
+#include <type_traits>
+
 #include "ngw_device.cuh"
 
 namespace ngw {
@@ -127,11 +129,26 @@ struct StepParams {
     const int32_t* policy_w;    // closed-loop linear policy: int32 [obs_dim][policy_actions] (nullptr = off)
     const int32_t* policy_b;    // int32 [policy_actions]
     int policy_actions;
+    int record;                 // K-step rollout with the per-step record (RecordParams) set
     uint16_t* msg;              // optional: info['message'] codes (enum ngw_msg | arg << 5)
     int32_t* reset_list;        // single-step auto-reset: finished envs are queued here ...
     int32_t* reset_count;       // ... and regenerated by reset_list_kernel right after this launch
     uint8_t* trunc;             // optional, one-step launches: 1 where the step hit max_episode_steps and the env did not end it
     unsigned char* final_obs;   // optional, one-step launches: reset_list_kernel copies a regenerated env's row here first
+};
+
+// Per-step record of the K-step rollouts (ngw_set_rollout_record): element [t][e] at t * stride + e.  Only the recording
+// rollout kernels take it (RecArgs), so every other kernel's argument block stays as it was.
+struct RecordParams {
+    unsigned char* obs;         // rows of obs_row_bytes (nullptr = skip, as every field below)
+    float* reward;
+    float* cost;
+    uint8_t* done;
+    uint8_t* result;
+    uint8_t* trunc;
+    unsigned char* final_obs;   // written only for the envs step t's auto-reset regenerated
+    long long stride;           // n_envs_padded: every step's block starts on a 128-byte boundary
+    int off_tile;               // the staging tile of the recorded observations in shared memory (32 rows)
 };
 
 // Kernel argument block: the parameters plus up to NC configs INLINE, so that every config read in the hot path
@@ -145,6 +162,16 @@ struct StepArgs {
         return (NC == 1) ? cfg[0] : (NC > 1 ? cfg[cfg_i] : p.dcfgs[cfg_i]);
     }
 };
+
+template <int NC>
+struct RecArgs : StepArgs<NC> {
+    RecordParams rec;
+};
+// the argument block of a rollout kernel: StepArgs, plus the record when kRec
+template <int NC, bool kRec>
+using RolloutArgs = typename std::conditional<kRec, RecArgs<NC>, StepArgs<NC> >::type;
+template <int NC> __device__ __forceinline__ const RecordParams* record_of(const StepArgs<NC>&) { return nullptr; }
+template <int NC> __device__ __forceinline__ const RecordParams* record_of(const RecArgs<NC>& a) { return &a.rec; }
 
 #define NGW_STAT_SLOTS 512
 #define NGW_SMEM_HDR 256            // mbarriers, zero pad, pose hand-over
@@ -322,6 +349,36 @@ __device__ __forceinline__ void tile_stats(double* stats, unsigned slot, int lan
     }
 }
 
+// K-step rollouts with a record: the scalars of env e's step t, written by the lane that stepped it
+__device__ __forceinline__ void record_scalars(const RecordParams& rec, int t, long long e, const StepOut& o, int trunc) {
+    const long long r = t * rec.stride + e;
+    if (rec.reward != nullptr) rec.reward[r] = (float)o.reward;
+    if (rec.cost != nullptr) rec.cost[r] = o.cost;
+    if (rec.done != nullptr) rec.done[r] = (uint8_t)o.done;
+    if (rec.result != nullptr) rec.result[r] = (uint8_t)o.result;
+    if (rec.trunc != nullptr) rec.trunc[r] = (uint8_t)trunc;
+}
+
+// Cold, rollout_kernel with a record: the observation this step produced, for the envs the auto-reset is about to
+// regenerate (need), into the lane's staging row and on to final_obs element r.  Called by the whole step warp.
+__device__ __forceinline__ void lane_final_obs(const StepParams& p, const RecordParams& rec, const EnvRow& env,
+                                               const DevConfig& dc, const LidarDev& tables, const LidarLuts& luts,
+                                               const int8_t* zero, unsigned char* srow, int lane, bool need, long long r) {
+    if (lane == 0) bulk_wait_read<0>();                               // the previous step's store has read the tile
+    __syncwarp();
+    if (need) {
+        ObsRow row;
+        row.p = srow;
+        row.fmt = p.obs_format;
+        uint32_t* w = reinterpret_cast<uint32_t*>(srow);
+        for (int i = 0; i < (p.obs_row_bytes >> 2); i++) w[i] = 0u;
+        if (dc.c.n_beams > 0) lidar_observe<false>(env, dc, tables, luts, row, zero, 0, 1, true);
+        uint32_t* f = reinterpret_cast<uint32_t*>(rec.final_obs + r * p.obs_row_bytes);
+        for (int i = 0; i < (p.obs_row_bytes >> 2); i++) f[i] = w[i];
+    }
+    __syncwarp();
+}
+
 // ------------------------------------------------------------------ the K-STEP ROLLOUT kernel (ngw_rollout, ngw_rollout_policy)
 // SURVEY §8f N1.  One CTA = one tile of 32 consecutive envs that stays in shared memory for n_steps steps; lane l owns env
 // l.  Warp 0 runs the steps; actions come from a [K][N] tensor (next step's action prefetched behind the current step),
@@ -331,11 +388,15 @@ __device__ __forceinline__ void tile_stats(double* stats, unsigned slot, int lan
 // shared memory.  Finished lanes are regenerated in place by the step warp (auto_reset_warp).  After the last step all G
 // warps cast the final observation, which leaves with the inventory tile through two TMA bulk stores; the other outputs are
 // per-env sums (reward, step_cost, episodes finished) and the last step's done / result.
+// kRec (ngw_set_rollout_record): every step also leaves its transition — the step's scalars straight from registers, and
+// the observation of the state after the step (and its auto-reset) cast into a staging tile of its own (the grid and
+// inventory rows live across the steps) and stored with one bulk store; an env regenerated at step t first has the
+// observation the step produced copied to final_obs.
 #define NGW_CLASS1_OPS ((1u << NGW_OP_FORWARD) | (1u << NGW_OP_BREAK) | (1u << NGW_OP_PLACE_TREE_TAP) | \
                         (1u << NGW_OP_EXTRACT_RUBBER) | (1u << NGW_OP_EXTRACT_STRING) | (1u << NGW_OP_CHOP) | (1u << NGW_OP_JUMP))
 
-template <int NC>
-__global__ void __launch_bounds__(256) rollout_kernel(const __grid_constant__ StepArgs<NC> args) {
+template <int NC, bool kRec>
+__global__ void __launch_bounds__(256) rollout_kernel(const __grid_constant__ RolloutArgs<NC, kRec> args) {
     extern __shared__ __align__(128) unsigned char smem[];
     const StepParams& p = args.p;
     const int lane = threadIdx.x & 31, g = threadIdx.x >> 5, G = blockDim.x >> 5;
@@ -354,6 +415,8 @@ __global__ void __launch_bounds__(256) rollout_kernel(const __grid_constant__ St
     int8_t* smap = reinterpret_cast<int8_t*>(smem + p.off_in);
     int32_t* sinv = reinterpret_cast<int32_t*>(smem + p.off_in + p.map_bytes);
     unsigned char* sobs = smem + p.off_obs;
+    const RecordParams* rec = record_of<NC>(args);                   // kRec: the record, else nullptr
+    unsigned char* srec = kRec ? smem + rec->off_tile : nullptr;     // kRec: staging tile of the recorded observations
     const bool closed_loop = p.policy_w != nullptr;
 
     // ---- prologue without global state: barrier, zero pad, lidar tables, zeroed observation tile
@@ -449,7 +512,7 @@ __global__ void __launch_bounds__(256) rollout_kernel(const __grid_constant__ St
             }
             if (p.actions_out != nullptr && valid) p.actions_out[t * p.act_stride + e] = action;
             o.clear();
-            int invalid = 0, did_reset = 0, success = 0;
+            int invalid = 0, did_reset = 0, success = 0, trunc = 0;
             if (valid) {
                 const ngw_action_entry a = decode_action(cfg, action);
                 if (a.op == NGW_OP_INVALID) {                         // wrappers.py:76 / pogostick_v1_env.py:236 would raise
@@ -461,19 +524,42 @@ __global__ void __launch_bounds__(256) rollout_kernel(const __grid_constant__ St
                     int finished = o.done;
                     if (p.max_episode_steps > 0) {
                         int len = p.ep_len[e] + 1;
-                        if (len >= p.max_episode_steps) { finished = 1; o.done = 1; }   // harness truncation knob
+                        if (len >= p.max_episode_steps) { trunc = !finished; finished = 1; o.done = 1; }   // harness truncation knob
                         p.ep_len[e] = finished && p.auto_reset ? 0 : len;
                     }
                     if (finished && p.auto_reset) did_reset = 1;
                 }
                 ps = env.pose();
                 reward_sum += (float)o.reward; cost_sum += o.cost; done_count += o.done;
+                if (kRec) record_scalars(*rec, t, e, o, trunc);
             }
+            if (kRec && rec->final_obs != nullptr && __ballot_sync(0xFFFFFFFFu, did_reset) != 0)
+                lane_final_obs(p, *rec, env, dc, beam_tables, luts, szero, srec + lane * p.obs_row_bytes, lane, did_reset != 0,
+                               t * rec->stride + e);
             if (p.auto_reset) {
                 // the next step needs the new episode now -> regenerate in place, warp-cooperatively
                 if (__ballot_sync(0xFFFFFFFFu, did_reset) != 0) {
                     auto_reset_warp(p, p.dcfgs, cfg_i, did_reset != 0, smap, sinv, sscratch, e0, ps);
                     env.set_pose(ps);
+                }
+            }
+            if (kRec && rec->obs != nullptr) {                       // the observation after the step, all 32 rows -> record
+                const uint32_t a0 = smem_u32(srec);
+                if (lane == 0) bulk_wait_read<0>();
+                __syncwarp();
+                zero_span(a0 + lane * 16u, a0 + 32u * (uint32_t)p.obs_row_bytes, 512u);
+                __syncwarp();
+                if (valid && cfg.n_beams > 0) {
+                    ObsRow rrow;
+                    rrow.p = srec + lane * p.obs_row_bytes;
+                    rrow.fmt = p.obs_format;
+                    lidar_observe<false>(env, dc, beam_tables, luts, rrow, szero, 0, 1, true);
+                }
+                fence_async_smem();
+                __syncwarp();
+                if (lane == 0) {
+                    bulk_s2g(rec->obs + (t * rec->stride + e0) * p.obs_row_bytes, srec, 32u * (uint32_t)p.obs_row_bytes);
+                    bulk_commit();
                 }
             }
             tile_stats(p.stats, blockIdx.x, lane, valid, o.done, success, did_reset, invalid, o.reward, o.cost);
@@ -521,6 +607,7 @@ __global__ void __launch_bounds__(256) rollout_kernel(const __grid_constant__ St
         copy16(ginv, sinv, p.inv_bytes, threadIdx.x, blockDim.x);
         if (p.obs != nullptr) copy_obs_rows(p, e0, sobs, p.obs_row_bytes, threadIdx.x, blockDim.x);
     }
+    if (kRec && threadIdx.x == 0) bulk_wait_read<0>();              // the record's stores have read the staging tile
 }
 
 // ------------------------------------------------------------------ the ONE-STEP kernel (ngw_step / ngw_observe)
@@ -1122,10 +1209,64 @@ __device__ __forceinline__ void policy_mac(int (&acc)[16], const int32_t* w, int
     }
 }
 
+// kRec: one lane pair's observation row of `env` into the zeroed row `orow` (hits from both lanes, inventory tail from the low one)
+__device__ __forceinline__ void pair_observe(const EnvRow& env, const DevConfig& dc, const LidarDev& geom, const LidarLuts& luts,
+                                             int half, const ObsRow& orow) {
+    const ngw_config& cfg = dc.c;
+    uint32_t hit[4];
+    if (env.ms == 10) pair_lidar<10, true>(env, cfg, geom, luts, half, hit);
+    else pair_lidar<0, true>(env, cfg, geom, luts, half, hit);
+#pragma unroll
+    for (int j = 0; j < 4; j++)
+        if (hit[j]) orow.put((int)(hit[j] >> 16), (int)((hit[j] >> 8) & 0xFFu), cfg.n_lidar_items, (int)(hit[j] & 0xFFu));
+    if (half == 0) {
+        const int tf = dc.lidar.tail_first;
+        int32_t* tl = orow.tail(cfg.n_lidar_items, cfg.n_beams);
+        for (int i = 0; i < cfg.n_inv_obs; i++) tl[i] = env.inv[tf >= 0 ? tf + i : (int)cfg.inv_obs_item[i]];
+    }
+}
+
+// lane pairs (rollout2_kernel): the high lane takes the low lane's pose, and the low lane's writes to the tile become
+// visible to it
+__device__ __forceinline__ void pair_follow_low(EnvRow& env, int lane) {
+    uint32_t pose = (uint32_t)env.r | ((uint32_t)env.c << 8) | ((uint32_t)env.facing << 16) | ((uint32_t)env.sel << 24);
+    __syncwarp();
+    pose = __shfl_sync(0xFFFFFFFFu, pose, lane & 15);
+    env.r = pose & 0xFF; env.c = (pose >> 8) & 0xFF; env.facing = (pose >> 16) & 0xFF; env.sel = pose >> 24;
+}
+
+// Cold, rollout2_kernel with a record: the observation this step produced (env: the state before the auto-reset, pose
+// still the low lane's only), for the envs of this warp in `resets`, into its staging rows `srec` and on to final_obs
+// rows [r0, r0 + 16).  Called by the whole warp.
+__device__ __forceinline__ void pair_final_obs(const StepParams& p, const RecordParams& rec, EnvRow env,
+                                               const DevConfig& dc, const LidarDev& geom, const LidarLuts& luts,
+                                               unsigned char* srec, int lane, bool valid, uint32_t resets, long long r0) {
+    pair_follow_low(env, lane);
+    const uint32_t a0 = smem_u32(srec);
+    if (lane == 0) bulk_wait_read<0>();                               // the previous step's store has read the rows
+    __syncwarp();
+    zero_span(a0 + lane * 16u, a0 + 16u * (uint32_t)p.obs_row_bytes, 512u);
+    __syncwarp();
+    ObsRow orow;
+    orow.p = srec + (lane & 15) * p.obs_row_bytes;
+    orow.fmt = p.obs_format;
+    if (valid && ((resets >> (lane & 15)) & 1u) && dc.c.n_beams > 0) pair_observe(env, dc, geom, luts, lane >> 4, orow);
+    __syncwarp();
+    for (uint32_t m = resets & 0xFFFFu; m != 0; m &= m - 1) {
+        const int r = __ffs(m) - 1;
+        const uint32_t* src = reinterpret_cast<const uint32_t*>(srec + r * p.obs_row_bytes);
+        uint32_t* dst = reinterpret_cast<uint32_t*>(rec.final_obs + (r0 + r) * p.obs_row_bytes);
+        for (int i = lane; i < (p.obs_row_bytes >> 2); i += 32) dst[i] = src[i];
+    }
+    __syncwarp();
+}
+
 #define NGW_R2_HDR 128
-// A4: ceil(policy actions / 4) for the closed loop, 0 = actions given or drawn (no per-step observation)
-template <int NC, int A4>
-__global__ void __launch_bounds__(64, 14) rollout2_kernel(const __grid_constant__ StepArgs<NC> args) {
+// A4: ceil(policy actions / 4) for the closed loop, 0 = actions given or drawn (no per-step observation).
+// kRec: the per-step record, as rollout_kernel's; warp g stages and bulk-stores its own 16 contiguous rows, so the record
+// needs no CTA barrier per step.
+template <int NC, int A4, bool kRec>
+__global__ void __launch_bounds__(64, 14) rollout2_kernel(const __grid_constant__ RolloutArgs<NC, kRec> args) {
     extern __shared__ __align__(128) unsigned char smem[];
     const StepParams& p = args.p;
     const int lane = threadIdx.x & 31, g = threadIdx.x >> 5;
@@ -1145,6 +1286,9 @@ __global__ void __launch_bounds__(64, 14) rollout2_kernel(const __grid_constant_
     int8_t* smap = reinterpret_cast<int8_t*>(region);
     int32_t* sinv = reinterpret_cast<int32_t*>(region + p.map_bytes);
     unsigned char* sobs = region;                                     // aliases the rows above (written after the last step)
+    const RecordParams* rec = record_of<NC>(args);                    // kRec: the record, else nullptr
+    unsigned char* srec = kRec ? smem + rec->off_tile + 16 * g * p.obs_row_bytes : nullptr;   // this warp's 16 record rows
+    const bool rec_rows = kRec && (rec->obs != nullptr || rec->final_obs != nullptr);
     const uint32_t in_bytes = (uint32_t)(p.map_bytes + p.inv_bytes);
 
     const int8_t* gmap = p.map + e0 * p.cells;
@@ -1223,7 +1367,7 @@ __global__ void __launch_bounds__(64, 14) rollout2_kernel(const __grid_constant_
         } else if (p.random_policy && valid && low) {
             action = rpol.draw(p.policy_seed, (uint64_t)(p.first_gid + e), (uint32_t)t, (uint32_t)(cfg.n_actions > 0 ? cfg.n_actions : 1));
         }
-        int did_reset = 0;
+        int did_reset = 0, trunc = 0;
         __syncwarp();                                                 // the high lanes have read the rows
         if (valid && low) {
             if (p.actions_out != nullptr) p.actions_out[t * p.act_stride + e] = action;
@@ -1244,13 +1388,17 @@ __global__ void __launch_bounds__(64, 14) rollout2_kernel(const __grid_constant_
                 int finished = o.done;
                 if (p.max_episode_steps > 0) {
                     int len = p.ep_len[e] + 1;
-                    if (len >= p.max_episode_steps) { finished = 1; o.done = 1; }
+                    if (len >= p.max_episode_steps) { trunc = !finished; finished = 1; o.done = 1; }
                     p.ep_len[e] = finished && p.auto_reset ? 0 : len;
                 }
                 if (finished && p.auto_reset) { did_reset = 1; n_reset++; }
             }
             reward_sum += o.reward; cost_sum += o.cost; n_done += o.done;
+            if (kRec) record_scalars(*rec, t, e, o, trunc);
         }
+        const uint32_t resets = kRec ? __ballot_sync(0xFFFFFFFFu, did_reset) : 0u;   // low lanes: bit l = env l of this warp
+        if (rec_rows && rec->final_obs != nullptr && resets != 0)   // cold: the envs the auto-reset is about to regenerate
+            pair_final_obs(p, *rec, env, dc, geom, luts, srec, lane, valid, resets, t * rec->stride + e0 + 16 * g);
         if (p.auto_reset) {
             if (__ballot_sync(0xFFFFFFFFu, did_reset) != 0) {         // regenerate in place, warp-cooperatively (this warp's 16 envs)
                 uchar4 q = env.pose();
@@ -1259,12 +1407,23 @@ __global__ void __launch_bounds__(64, 14) rollout2_kernel(const __grid_constant_
                 env.set_pose(q);
             }
         }
-        // the pair's high lane follows the low lane's pose; the step's writes to the tile become visible to it
-        {
-            uint32_t pose = (uint32_t)env.r | ((uint32_t)env.c << 8) | ((uint32_t)env.facing << 16) | ((uint32_t)env.sel << 24);
+        pair_follow_low(env, lane);                                   // the pair's high lane follows the low lane's pose
+        if (rec_rows && rec->obs != nullptr) {                       // the observation after the step: 16 rows -> record
+            const uint32_t a0 = smem_u32(srec);
+            if (lane == 0) bulk_wait_read<0>();
             __syncwarp();
-            pose = __shfl_sync(0xFFFFFFFFu, pose, lane & 15);
-            env.r = pose & 0xFF; env.c = (pose >> 8) & 0xFF; env.facing = (pose >> 16) & 0xFF; env.sel = pose >> 24;
+            zero_span(a0 + lane * 16u, a0 + 16u * (uint32_t)p.obs_row_bytes, 512u);
+            __syncwarp();
+            ObsRow orow;
+            orow.p = srec + (lane & 15) * p.obs_row_bytes;
+            orow.fmt = p.obs_format;
+            if (valid && cfg.n_beams > 0) pair_observe(env, dc, geom, luts, half, orow);
+            fence_async_smem();
+            __syncwarp();
+            if (lane == 0) {
+                bulk_s2g(rec->obs + (t * rec->stride + e0 + 16 * g) * p.obs_row_bytes, srec, 16u * (uint32_t)p.obs_row_bytes);
+                bulk_commit();
+            }
         }
         action = next_action;
     }
@@ -1341,7 +1500,7 @@ __global__ void __launch_bounds__(64, 14) rollout2_kernel(const __grid_constant_
             for (int i = threadIdx.x; i < n; i += 64) gobs[i] = so[i];
         }
     }
-    if (threadIdx.x == 0) bulk_wait_read<0>();                        // shared memory must outlive the bulk stores' reads
+    if (kRec ? lane == 0 : threadIdx.x == 0) bulk_wait_read<0>();    // shared memory must outlive the bulk stores' reads
 }
 
 }  // namespace ngw

@@ -104,6 +104,42 @@ def obs_to_vector(rows, compiled, obs_format, cfg_ids=None):
     return out.numpy() if as_numpy else out
 
 
+class RolloutRecord(object):
+    """Reusable per-step buffers of a K-step rollout (BatchHandle.rollout_record, include/ngw.h ngw_set_rollout_record).
+    Padded device tensors [max_steps, n_envs_padded, ...] hold the steps; the attributes below are their [:, :n] views,
+    element [t][e] being what the t-th of as many single steps would report for env e:
+        obs        observation rows (the handle's format) after step t and its auto-reset: what the rollout's policy acts
+                   on at step t + 1, and what observe() returns after the t-th single step
+        reward, step_cost   float32;  done, result, truncated   uint8
+        final_obs  rows like obs, only with final_obs=True: written only where step t's auto-reset regenerated the env
+                   (the observation the step produced); other rows keep what they held.
+    Flatten with obs.reshape(-1, obs.shape[-1]) to decode narrow rows with BatchHandle.obs_vector / obs_to_vector."""
+
+    def __init__(self, handle, max_steps, final_obs=False):
+        if max_steps < 1:
+            raise ValueError("max_steps must be >= 1")
+        self.handle, self.max_steps = handle, int(max_steps)
+        self.obs_format, self.obs_row_bytes = handle.obs_format, handle.obs_row_bytes
+        T, npad, n, dev = self.max_steps, handle.n_padded, handle.n, handle.device
+
+        def rows():
+            if not handle.obs_dim:
+                return None
+            if handle.obs_format == 'i32':
+                return torch.zeros((T, npad, handle.obs_row_bytes // 4), dtype=torch.int32, device=dev)
+            return torch.zeros((T, npad, handle.obs_row_bytes), dtype=torch.uint8, device=dev)
+
+        self.padded = {'obs': rows(), 'final_obs': rows() if final_obs else None}
+        for k, dt in (('reward', torch.float32), ('step_cost', torch.float32), ('done', torch.uint8),
+                      ('result', torch.uint8), ('truncated', torch.uint8)):
+            self.padded[k] = torch.zeros((T, npad), dtype=dt, device=dev)
+        for k, t in self.padded.items():
+            setattr(self, k, None if t is None else t[:, :n])
+        self._c = capi.RolloutRecordC(self.max_steps, *[None if self.padded[k] is None else self.padded[k].data_ptr()
+                                                        for k in ('obs', 'reward', 'step_cost', 'done', 'result',
+                                                                  'truncated', 'final_obs')])
+
+
 class BatchHandle(object):
     def __init__(self, compiled, n_envs, device=None, seed=0, first_env_gid=0, cfg_id=None, obs_format='i32'):
         if not torch.cuda.is_available():
@@ -251,12 +287,31 @@ class BatchHandle(object):
                                                1 if auto_reset else 0, int(max_episode_steps), self._stream()))
         return self.obs, self.reward, self.done, self.step_cost, self.result
 
+    def rollout_record(self, max_steps, final_obs=False):
+        """A reusable per-step record for rollout(..., record=) of up to max_steps steps (see RolloutRecord).  final_obs is
+        opt-in: it is as large as obs.  Preallocated, it keeps a recorded rollout capturable in a CUDA graph."""
+        return RolloutRecord(self, max_steps, final_obs)
+
     def rollout(self, n_steps, actions=None, policy_seed=0, auto_reset=False, max_episode_steps=0,
-                record_actions=False, policy=None):
+                record_actions=False, policy=None, record=None):
         """n_steps consecutive steps in ONE launch (tile resident in shared memory).  actions: int32 CUDA tensor
         [n_steps, n]; None = on-device uniform random policy; policy=(W int32 [obs_dim, A], b int32 [A]) = closed loop,
         action = argmax(b + obs @ W) computed on the device from the current observation.  Returns (obs after the last
-        step, reward sum, step_cost sum, episodes finished, last done, last result[, actions taken])."""
+        step, reward sum, step_cost sum, episodes finished, last done, last result[, actions taken][, record]).
+        record: a RolloutRecord of this handle, filled with every step's transition (set for this call only)."""
+        if record is None:
+            return self._rollout(n_steps, actions, policy_seed, auto_reset, max_episode_steps, record_actions, policy)
+        if record.handle is not self or record.obs_row_bytes != self.obs_row_bytes:
+            raise ValueError("rollout: the record was built for another handle or observation format "
+                             "(rows of %d bytes, this handle's are %d)" % (record.obs_row_bytes, self.obs_row_bytes))
+        capi.check(self.lib, self.lib.ngw_set_rollout_record(self._h, C.byref(record._c)))
+        try:
+            out = self._rollout(n_steps, actions, policy_seed, auto_reset, max_episode_steps, record_actions, policy)
+        finally:
+            capi.check(self.lib, self.lib.ngw_set_rollout_record(self._h, None))
+        return out + (record,)
+
+    def _rollout(self, n_steps, actions, policy_seed, auto_reset, max_episode_steps, record_actions, policy):
         if policy is not None:
             w = torch.as_tensor(policy[0], device=self.device).to(torch.int32).contiguous()
             b = torch.as_tensor(policy[1], device=self.device).to(torch.int32).contiguous()

@@ -38,7 +38,7 @@
 extern "C" {
 #endif
 
-#define NGW_ABI_VERSION 11
+#define NGW_ABI_VERSION 12
 
 #define NGW_MAX_ITEMS 24          /* reference asserts len(items) <= 20 (pogostick_v1_env.py:75,220) */
 #define NGW_MAX_ACTIONS 48
@@ -319,6 +319,38 @@ int ngw_set_message_buffer(ngw_handle* h, uint16_t* msg_dev);
  * ngw_observe, ngw_reset, ngw_rollout and ngw_rollout_policy never touch either buffer. */
 int ngw_set_episode_end_buffers(ngw_handle* h, uint8_t* truncated_dev, void* final_obs_dev);
 
+/* Optional per-step record of the K-step rollouts (ngw_rollout, ngw_rollout_policy): while it is set, a rollout of n_steps
+ * fills, for every step t < n_steps and env e < n_envs, element [t][e] of each non-NULL buffer with what n_steps single
+ * ngw_step calls would report at their t-th step (same seed, state, actions, auto_reset and max_episode_steps, episode-end
+ * buffers on).  Every buffer is DEVICE memory laid out [max_steps][n_envs_padded] (ngw_state_view.n_envs_padded: each
+ * step's block starts on a 128-byte boundary; what padding elements hold is unspecified).
+ *   obs       rows of obs_row_bytes in the observation format in force at launch, 16-byte aligned: the observation of
+ *             env e after step t and its auto-reset, observed after ALL of the reset ops — what ngw_observe returns right
+ *             after the t-th ngw_step, and what the rollout's policy acts on at step t + 1 (so obs[n_steps - 1] equals the
+ *             rollout's obs output).  It differs from ngw_step's obs row only for an env regenerated at step t under a
+ *             config with reset_obs_after_ops < n_reset_ops.
+ *   reward, step_cost, done, result   as ngw_step's outputs (step_cost bit for bit; no summation).
+ *   truncated 1 where step t reached max_episode_steps and the env's own step did not end the episode (gym's TimeLimit
+ *             rule, as ngw_set_episode_end_buffers); 0 on invalid-action lanes.
+ *   final_obs rows like obs, written ONLY where step t's auto-reset regenerated env e: the observation the step produced,
+ *             before the reset.  Every other row is left untouched.
+ * Invalid actions record zeros and the observation of the unchanged state, as ngw_step does.  obs / final_obs are ignored
+ * without a LidarInFront observation (obs_dim == 0).  A rollout with n_steps > max_steps fails and enqueues nothing.
+ * Everything a rollout returns without a record is bit-identical with one.  ngw_step, ngw_step_many, the host-buffer path,
+ * ngw_observe and ngw_reset never touch the record.  The buffers are the caller's; the handle keeps the pointers. */
+typedef struct ngw_rollout_record {
+    int32_t max_steps;      /* steps the buffers hold (>= 1) */
+    void* obs;              /* rows of obs_row_bytes, [max_steps][n_envs_padded], 16-byte aligned; NULL = skip */
+    float* reward;          /* [max_steps][n_envs_padded]; NULL = skip (same for every field below) */
+    float* step_cost;
+    uint8_t* done;
+    uint8_t* result;
+    uint8_t* truncated;
+    void* final_obs;        /* rows like obs, 16-byte aligned; written only for envs regenerated at step t */
+} ngw_rollout_record;
+/* rec is copied; NULL switches the record off (the default).  Fails on misaligned pointers or max_steps < 1. */
+int ngw_set_rollout_record(ngw_handle* h, const ngw_rollout_record* rec);
+
 /* Same call with HOST buffers (the reference-facing path): copies actions in (H2D), steps, copies
  * obs/reward/done/step_cost/result out (D2H) on the handle's own stream; returns after the outputs are valid
  * on the host.  The step is ordered after everything earlier calls on this handle enqueued on the caller's streams
@@ -334,7 +366,8 @@ int ngw_step_host(ngw_handle* h, const int32_t* actions, void* obs, float* rewar
  * (policy_seed, global env id, step index / 4: one block serves four steps; exact uniformity by multiply-shift with
  * rejection) — the tests/random_action.py loop without the host.  reward_sum / cost_sum
  * accumulate over the steps, done_count counts finished episodes, last_done / last_result are the final step's, obs is
- * the observation after the last step; actions_out (DEVICE int32[n_steps][n_envs], NULL = skip) records the actions. */
+ * the observation after the last step; actions_out (DEVICE int32[n_steps][n_envs], NULL = skip) records the actions.
+ * ngw_set_rollout_record adds the per-step transitions (observation, reward, done, truncation, terminal observation). */
 int ngw_rollout(ngw_handle* h, const int32_t* actions, int32_t n_steps, uint64_t policy_seed, void* obs,
                 float* reward_sum, float* cost_sum, int32_t* done_count, uint8_t* last_done, uint8_t* last_result,
                 int32_t* actions_out, int32_t auto_reset, int32_t max_episode_steps, void* stream);
@@ -343,7 +376,8 @@ int ngw_rollout(ngw_handle* h, const int32_t* actions, int32_t n_steps, uint64_t
  * env's valid action ids, computed on the device from the current LidarInFront observation (lowest id wins ties).
  * weights: DEVICE int32[obs_dim][n_policy_actions], bias: DEVICE int32[n_policy_actions], n_policy_actions <= 16.
  * Integer arithmetic => bit-reproducible on the host.  Outputs as ngw_rollout.  Needs NGW_OBS_I32 rows.  With auto_reset,
- * an env regenerated inside a rollout is observed after ALL of its reset ops (the next step needs the final state). */
+ * an env regenerated inside a rollout is observed after ALL of its reset ops (the next step needs the final state); the
+ * per-step record (ngw_set_rollout_record) holds the observations the policy acted on. */
 int ngw_rollout_policy(ngw_handle* h, const int32_t* weights, const int32_t* bias, int32_t n_policy_actions,
                        int32_t n_steps, void* obs, float* reward_sum, float* cost_sum, int32_t* done_count,
                        uint8_t* last_done, uint8_t* last_result, int32_t* actions_out, int32_t auto_reset,
