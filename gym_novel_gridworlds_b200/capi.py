@@ -8,8 +8,9 @@ from . import opcodes as oc
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, 'csrc', 'libngw_b200.so')
-ABI_VERSION = 12
+ABI_VERSION = 13
 OBS_I32, OBS_U8, OBS_HITS = 0, 1, 2
+RNG_PHILOX, RNG_NUMPY = 0, 1
 
 
 class ActionEntryC(C.Structure):
@@ -87,6 +88,9 @@ EXPORTS = {
     'ngw_load_state': (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_int64, C.c_void_p]),
     'ngw_export_state': (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_int64, C.c_void_p]),
     'ngw_reset': (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
+    'ngw_set_reset_rng': (C.c_int, [C.c_void_p, C.c_int32, C.c_void_p]),
+    'ngw_load_rng_state': (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_int64, C.c_void_p]),
+    'ngw_export_rng_state': (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_int64, C.c_void_p]),
     'ngw_step': (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
                            C.c_int32, C.c_int32, C.c_void_p]),
     'ngw_step_many': (C.c_int, [C.c_void_p, C.c_int32, C.c_int32, C.c_int32, C.c_void_p]),

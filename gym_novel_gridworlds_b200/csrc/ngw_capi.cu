@@ -289,6 +289,7 @@ void ngw_destroy(ngw_handle* h) {
     for (auto p : h->d_luts) cudaFree(p);
     cudaFree(h->d_cfgs); cudaFree(h->map); cudaFree(h->pose); cudaFree(h->inv); cudaFree(h->cfg_id);
     cudaFree(h->episode); cudaFree(h->ep_len); cudaFree(h->err); cudaFree(h->stats); cudaFree(h->zero_byte); cudaFree(h->reset_list); cudaFree(h->reset_ctl);
+    cudaFree(h->mt_key); cudaFree(h->mt_pos);
     cudaFree(h->h_actions); cudaFree(h->h_obs);   // reward / step_cost / done / result staging lives in h_obs's block
     if (h->hs) cudaStreamDestroy(h->hs);
     if (h->ev_dev) cudaEventDestroy(h->ev_dev);
@@ -415,6 +416,10 @@ static int set_kernel_attributes() {
     // the queued-reset kernel shares SMs with the next handle's step CTAs: both must want the same (maximal) shared-memory
     // carve-out, or the SM would have to drain before it can be reconfigured
     CK(cudaFuncSetAttribute(reset_list_kernel, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
+    // the numpy reset stream's candidate lists (ms^2 uint16 per warp) take both reset kernels past the 48 KB a launch gets
+    // without opting in on grids above ~58x58; the Philox plans are below it and do not change
+    CK(cudaFuncSetAttribute(reset_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024 - (int)sizeof(ResetScratch) * NGW_RESET_WARPS));
+    CK(cudaFuncSetAttribute(reset_list_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
     return ngw_rollout_set_attributes();              // ngw_rollout.cu
 }
 
@@ -583,6 +588,80 @@ int ngw_export_state(ngw_handle* h, int8_t* map, uint8_t* pose, int32_t* invento
     return 0;
 }
 
+int ngw_set_reset_rng(ngw_handle* h, int32_t kind, void* stream) {
+    if (!h) return fail("null handle");
+    if (kind != NGW_RNG_PHILOX && kind != NGW_RNG_NUMPY) return fail("ngw_set_reset_rng: unknown generator kind");
+    CK(cudaSetDevice(h->device));
+    if (kind == NGW_RNG_PHILOX) {
+        // (cudaFree waits for the device: no launch still reading the state can outlive it)
+        if (h->mt_key) { CK(cudaFree(h->mt_key)); CK(cudaFree(h->mt_pos)); }
+        h->mt_key = nullptr; h->mt_pos = nullptr;
+        return 0;
+    }
+    if (h->first_gid < 0 || h->seed + (unsigned long long)h->first_gid + (unsigned long long)(h->n - 1) >= (1ull << 32))
+        return fail("ngw_set_reset_rng: np.random.seed takes seeds below 2^32, but seed + first_env_gid + n_envs - 1 = " +
+                    std::to_string(h->seed + (unsigned long long)h->first_gid + (unsigned long long)(h->n - 1)));
+    if (!h->mt_key) {
+        uint32_t* key = nullptr; int32_t* pos = nullptr;
+        CK(cudaMalloc(&key, (size_t)h->np * NGW_MT_WORDS * 4));
+        if (cudaMalloc(&pos, (size_t)h->np * 4) != cudaSuccess) {
+            cudaGetLastError();
+            cudaFree(key);
+            return fail("ngw_set_reset_rng: out of device memory for the np.random states");
+        }
+        h->mt_key = key; h->mt_pos = pos;     // mt_seed_kernel writes every env's state; the padding rows are never read
+    }
+    cudaStream_t s = (cudaStream_t)stream;
+    before_device_call(h, s);
+    note_state_writer(h, s);
+    mt_seed_kernel<<<(unsigned)((h->n + 127) / 128), 128, 0, s>>>(h->mt_key, h->mt_pos, h->n,
+                                                                 h->seed + (unsigned long long)h->first_gid);
+    h->launches++;
+    CK(cudaGetLastError());
+    return 0;
+}
+
+// the checks the two state copies share: a numpy-stream handle and a range inside the batch
+static int rng_state_range(const ngw_handle* h, const char* who, int64_t first, int64_t count) {
+    if (!h) return fail("null handle");
+    if (!h->mt_key) return fail(std::string(who) + ": the handle has no np.random states (ngw_set_reset_rng(NGW_RNG_NUMPY))");
+    if (first < 0 || count < 0 || first + count > h->n) return fail(std::string(who) + ": range outside the batch");
+    return 0;
+}
+
+int ngw_load_rng_state(ngw_handle* h, const uint32_t* key, const int32_t* pos, int64_t first, int64_t count, void* stream) {
+    if (rng_state_range(h, "ngw_load_rng_state", first, count)) return 1;
+    if (count == 0) return 0;
+    if (!key || !pos) return fail("ngw_load_rng_state: null key or pos");
+    CK(cudaSetDevice(h->device));
+    cudaStream_t s = (cudaStream_t)stream;
+    // pos is checked on the host before anything is enqueued: once the stream's earlier work has written it
+    std::vector<int32_t> hp((size_t)count);
+    CK(cudaStreamSynchronize(s));
+    CK(cudaMemcpy(hp.data(), pos, (size_t)count * 4, cudaMemcpyDeviceToHost));
+    for (int64_t i = 0; i < count; i++)
+        if (hp[(size_t)i] < 0 || hp[(size_t)i] > NGW_MT_WORDS)
+            return fail("ngw_load_rng_state: pos[" + std::to_string(i) + "] = " + std::to_string(hp[(size_t)i]) +
+                        " outside [0, 624]");
+    before_device_call(h, s);
+    note_state_writer(h, s);
+    CK(cudaMemcpyAsync(h->mt_key + first * NGW_MT_WORDS, key, (size_t)count * NGW_MT_WORDS * 4, cudaMemcpyDeviceToDevice, s));
+    CK(cudaMemcpyAsync(h->mt_pos + first, pos, (size_t)count * 4, cudaMemcpyDeviceToDevice, s));
+    return 0;
+}
+
+int ngw_export_rng_state(ngw_handle* h, uint32_t* key, int32_t* pos, int64_t first, int64_t count, void* stream) {
+    if (rng_state_range(h, "ngw_export_rng_state", first, count)) return 1;
+    CK(cudaSetDevice(h->device));
+    cudaStream_t s = (cudaStream_t)stream;
+    before_device_call(h, s);
+    note_state_writer(h, s);                  // ends a capture chain: the copies wait for every branch
+    // cudaMemcpyDefault: the destinations may be device or (pinned / pageable) host memory
+    if (key) CK(cudaMemcpyAsync(key, h->mt_key + first * NGW_MT_WORDS, (size_t)count * NGW_MT_WORDS * 4, cudaMemcpyDefault, s));
+    if (pos) CK(cudaMemcpyAsync(pos, h->mt_pos + first, (size_t)count * 4, cudaMemcpyDefault, s));
+    return 0;
+}
+
 static ResetParams reset_params(ngw_handle* h, const uint8_t* mask, int phase) {
     ResetParams p;
     p.dcfgs = h->d_cfgs; p.map = h->map; p.pose = h->pose; p.inv = h->inv; p.cfg_id = h->cfg_id; p.episode = h->episode;
@@ -592,6 +671,7 @@ static ResetParams reset_params(ngw_handle* h, const uint8_t* mask, int phase) {
     p.final_obs = nullptr;
     p.obs_dim = h->obs_dim; p.obs_row_bytes = h->obs_row_bytes; p.obs_format = h->obs_format;
     p.key_mask = h->key_mask;
+    p.mt_key = h->mt_key; p.mt_pos = h->mt_pos;
     return p;
 }
 
@@ -608,17 +688,19 @@ int ngw_reset(ngw_handle* h, const uint8_t* mask, void* obs, void* stream) {
     const bool want_obs = obs != nullptr && h->obs_dim > 0;
     ResetParams po = reset_params(h, mask, split ? 0 : 2);
     po.obs = static_cast<unsigned char*>(obs);
+    // numpy stream: every warp's candidate list (the Philox reset needs no dynamic shared memory)
+    const size_t lists = h->mt_key != nullptr ? (size_t)NGW_RESET_WARPS * 2 * h->cells : 0;
     if (!want_obs || !split) {
-        reset_kernel<<<rblocks, 32 * NGW_RESET_WARPS, 0, s>>>(reset_params(h, mask, 2));
+        reset_kernel<<<rblocks, 32 * NGW_RESET_WARPS, lists, s>>>(reset_params(h, mask, 2));
         h->launches++;
         if (want_obs) {
             observe_masked_kernel<<<blocks, 128, 0, s>>>(po);
             h->launches++;
         }
     } else {
-        reset_kernel<<<rblocks, 32 * NGW_RESET_WARPS, 0, s>>>(reset_params(h, mask, 0));
+        reset_kernel<<<rblocks, 32 * NGW_RESET_WARPS, lists, s>>>(reset_params(h, mask, 0));
         observe_masked_kernel<<<blocks, 128, 0, s>>>(po);
-        reset_kernel<<<rblocks, 32 * NGW_RESET_WARPS, 0, s>>>(reset_params(h, mask, 1));
+        reset_kernel<<<rblocks, 32 * NGW_RESET_WARPS, lists, s>>>(reset_params(h, mask, 1));
         h->launches += 3;
     }
     CK(cudaGetLastError());
@@ -646,6 +728,7 @@ static StepParams step_params(ngw_handle* h, const int32_t* actions, void* obs, 
     p.trunc = actions != nullptr ? h->trunc : nullptr;
     p.final_obs = actions != nullptr && p.obs != nullptr ? h->final_obs : nullptr;
     p.n_steps = 1;
+    p.mt_key = h->mt_key; p.mt_pos = h->mt_pos;
     return p;
 }
 
@@ -839,7 +922,7 @@ static int launch_step_on_branch(ngw_handle* h, const StepParams& p, cudaStream_
         cudaLaunchConfig_t lc;
         memset(&lc, 0, sizeof(lc));
         lc.gridDim = dim3((unsigned)rl_ctas); lc.blockDim = dim3(32 * NGW_RESET_WARPS);
-        lc.dynamicSmemBytes = NGW_RESET_WARPS * reset_list_scratch_bytes(h->cells);
+        lc.dynamicSmemBytes = NGW_RESET_WARPS * reset_list_scratch_bytes(h->cells, h->mt_key != nullptr);
         lc.stream = s;
         // a PLAIN launch: it starts once the step has completed.  (Launched programmatically behind an overlapped step it
         // could start under that step's tail, but that measured no faster — 250.2 vs 250.7 us on C5.)

@@ -730,7 +730,7 @@ __device__ __forceinline__ void lidar_observe(const EnvRow& e, const DevConfig& 
 // ------------------------------------------------------------------ reset (pogostick_v1_env.py:86-181 + novelty resets)
 // WARP-COOPERATIVE: the 32 lanes of one warp regenerate ONE environment (rows in shared or global memory).
 //
-// Same DISTRIBUTION as the reference, not the same stream:
+// Same DISTRIBUTION as the reference, not the same stream (reset_env_numpy_warp below draws the reference's own stream):
 //  * placement: the reference draws uniformly from a list it shrinks by popping every drawn cell; a popped cell is the
 //    agent cell, a placed item or a cell that can never become placeable again, so "first placeable cell in a uniformly
 //    random order" == uniform over the currently placeable cells == draw-with-replacement-until-placeable (no list).
@@ -1016,6 +1016,220 @@ static __device__ __noinline__ uint32_t reset_env_warp(const ngw_config* cfg, in
             __syncwarp();
         }
     }
+    return err;
+}
+
+// ------------------------------------------------------------------ reset with the reference's own stream (NGW_RNG_NUMPY)
+// The same program as ngo_reset_legacy (oracle/ngw_oracle.c), draw for draw, on the env's persistent legacy np.random
+// state: MT19937 key[624] + pos in global memory, numpy's get_state() layout.  One warp per env; lane l holds the tempered
+// output of word wbase + l, and every draw is broadcast with a shuffle, so all lanes take the same (sequential) decisions.
+#define NGW_MT_WORDS 624
+// TREETAP attempts before the numpy reset gives up with NGW_ERR_PLACEMENT.  The reference retries forever; when at least
+// one target is free an attempt finds one with probability >= 1 / (4 ms^2), so with the cap's 2^20 attempts a 40x40
+// grid stops early with probability below e^-163.  Only a grid where no log has a free neighbour reaches it.
+#define NGW_NUMPY_TREETAP_CAP (1 << 20)
+
+// MT19937 twist: key[i] for i in [a, b) from key[i + o], key[i], key[i + 1]; every lane reads before any lane writes
+__device__ __forceinline__ void mt_twist_span(uint32_t* key, int a, int b, int o, int lane) {
+    for (int base = a; base < b; base += 32) {
+        const int i = base + lane;
+        uint32_t v = 0;
+        if (i < b) {
+            const uint32_t y = (key[i] & 0x80000000u) | (key[i + 1] & 0x7fffffffu);
+            v = key[i + o] ^ (y >> 1) ^ ((y & 1u) ? 0x9908b0dfu : 0u);
+        }
+        __syncwarp();
+        if (i < b) key[i] = v;
+        __syncwarp();
+    }
+}
+// mt_refill (oracle/ngw_oracle.c) in phases whose reads are complete before they start: [0, 227) reads words >= 397,
+// [227, 454) and [454, 623) read words 227 back, which the previous phase wrote; word 623 last
+static __device__ __noinline__ void mt_twist(uint32_t* key, int lane) {
+    mt_twist_span(key, 0, 227, 397, lane);
+    mt_twist_span(key, 227, 454, -227, lane);
+    mt_twist_span(key, 454, 623, -227, lane);
+    if (lane == 0) {
+        const uint32_t y = (key[623] & 0x80000000u) | (key[0] & 0x7fffffffu);
+        key[623] = key[396] ^ (y >> 1) ^ ((y & 1u) ? 0x9908b0dfu : 0u);
+    }
+    __syncwarp();
+}
+
+struct MtWarp {
+    uint32_t* key;   // the env's 624 words (global memory)
+    int pos;         // next word, 624 = twist first
+    int wbase;       // first word of the lanes' window
+    uint32_t win;    // lane l: tempered key[wbase + l]
+
+    __device__ __forceinline__ uint32_t next(int lane) {
+        if (pos == NGW_MT_WORDS) { mt_twist(key, lane); pos = 0; wbase = -64; }
+        if (pos - wbase >= 32) {
+            wbase = pos;
+            uint32_t y = pos + lane < NGW_MT_WORDS ? key[pos + lane] : 0u;
+            y ^= (y >> 11);
+            y ^= (y << 7) & 0x9d2c5680u;
+            y ^= (y << 15) & 0xefc60000u;
+            y ^= (y >> 18);
+            win = y;
+        }
+        return __shfl_sync(0xFFFFFFFFu, win, pos++ - wbase);
+    }
+    // uniform in [0, max]: masked rejection on 32-bit outputs (legacy random_interval)
+    __device__ __forceinline__ uint32_t interval(uint32_t max, int lane) {
+        if (max == 0) return 0;
+        uint32_t mask = max;
+        mask |= mask >> 1; mask |= mask >> 2; mask |= mask >> 4; mask |= mask >> 8; mask |= mask >> 16;
+        uint32_t v;
+        do { v = next(lane) & mask; } while (v > max);
+        return v;
+    }
+    // np.random.randint(lo, hi) / np.random.choice(hi) with lo = 0
+    __device__ __forceinline__ uint32_t randint(uint32_t lo, uint32_t hi, int lane) { return lo + interval(hi - 1u - lo, lane); }
+};
+
+// list.pop(idx) on the warp's shared-memory list of n entries
+__device__ __forceinline__ void list_pop(uint16_t* list, int idx, int n, int lane) {
+    for (int base = idx; base < n - 1; base += 32) {
+        const int i = base + lane;
+        const uint16_t v = i < n - 1 ? list[i + 1] : (uint16_t)0;
+        __syncwarp();
+        if (i < n - 1) list[i] = v;
+        __syncwarp();
+    }
+}
+
+// The 32 lanes of one warp regenerate one env from its np.random state (key[624] and *pos_io, global memory) exactly as
+// the reference does under that state.  Arguments as reset_env_warp's; `list`: ms * ms uint16 of shared memory owned by
+// the warp (the reference's candidate lists).  A placement that runs out of cells, or a TREETAP with no log to tap (or
+// past NGW_NUMPY_TREETAP_CAP attempts), returns NGW_ERR_PLACEMENT and skips the rest of the program, as the reference's
+// AssertionError does; the caller skips a second part too.  *pos_io is written back in every case.
+static __device__ __noinline__ uint32_t reset_env_numpy_warp(const ngw_config* cfg, int8_t* m, int32_t* inv, int ms,
+                                                             int inv_stride, uint32_t* key, int32_t* pos_io, bool do_base,
+                                                             int op_begin, int op_end, uint16_t* list, int& pr, int& pc,
+                                                             int& pf, int& psel) {
+    const uint32_t FULL = 0xFFFFFFFFu;
+    const int lane = threadIdx.x & 31;
+    const int cells = ms * ms;
+    const int wall = cfg->id_wall;
+    MtWarp mt;
+    mt.key = key; mt.pos = *pos_io; mt.wbase = -64; mt.win = 0;
+    uint32_t err = 0;
+    if (do_base) {                                                    // pogostick_v1_env.py:118-157
+        for (int i = lane; i < inv_stride; i += 32) inv[i] = 0;
+        psel = 0;
+        for (int r = lane / ms, c = lane - (lane / ms) * ms, i = lane; i < cells; i += 32) {
+            m[i] = (r == 0 || c == 0 || r == ms - 1 || c == ms - 1) ? (int8_t)wall : (int8_t)0;
+            c += 32;
+            while (c >= ms) { c -= ms; r++; }
+        }
+        const int side = ms - 4;                                      // interior cells 2 .. ms-3, row-major
+        int n = side * side;
+        for (int i = lane; i < n; i += 32) list[i] = (uint16_t)((2 + i / side) * ms + 2 + i % side);
+        __syncwarp();
+        const int a = (int)mt.randint(0, (uint32_t)n, lane);          // agent cell (stays in the list)
+        pr = 2 + a / side; pc = 2 + a % side;
+        pf = (int)mt.randint(0, 4, lane);                             // choice(['NORTH','SOUTH','WEST','EAST'])
+        const int agent = pr * ms + pc;
+        for (int i = 0; i < cfg->n_place && err == 0; i++) {         // add_item_to_map, pogostick_v1_env.py:159-181
+            const int item = cfg->place_item[i], qty = cfg->place_qty[i];
+            for (int count = 0; count != qty;) {
+                if (n < 1) { err = NGW_ERR_PLACEMENT; break; }
+                const int idx = (int)mt.randint(0, (uint32_t)n, lane);
+                const int cell = list[idx];
+                const int r = cell / ms, c = cell - r * ms;
+                const bool put = cell != agent && placeable(m, ms, r, c);
+                __syncwarp();
+                if (put && lane == 0) m[cell] = (int8_t)item;
+                __syncwarp();
+                count += put;
+                list_pop(list, idx, n, lane);                         // popped whether or not the cell was taken
+                n--;
+            }
+        }
+    }
+    const int agent = pr * ms + pc;
+    if (op_end > cfg->n_reset_ops) op_end = cfg->n_reset_ops;
+    for (int k = op_begin; k < op_end && err == 0; k++) {
+        const ngw_reset_op op = cfg->reset_ops[k];
+        if (op.kind == NGW_RESET_INVSET) {
+            if (lane == 0) inv[op.a] = op.lo;
+            __syncwarp();
+            continue;
+        }
+        if (op.kind == NGW_RESET_TREETAP) {                           // pogostick_v0_env.py:155-178
+            int n_logs = 0, target = -1;
+            for (int i = lane; i < cells; i += 32) n_logs += (m[i] == (int8_t)op.b);
+            n_logs = __reduce_add_sync(FULL, n_logs);
+            if (n_logs <= 1) { err = NGW_ERR_PLACEMENT; break; }      // assert len(result[0]) > 1
+            for (int attempt = 0; attempt < NGW_NUMPY_TREETAP_CAP && target < 0; attempt++) {
+                const int direction = (int)mt.randint(0, 4, lane);
+                int which = (int)mt.randint(0, (uint32_t)n_logs, lane);
+                int log = -1;
+                for (int base = 0; base < cells && log < 0; base += 32) {   // which-th tree_log in row-major order
+                    const int i = base + lane;
+                    const uint32_t bal = __ballot_sync(FULL, i < cells && m[i] == (int8_t)op.b);
+                    const int cnt = __popc(bal);
+                    if (which < cnt) log = base + (int)__fns(bal, 0, which + 1);
+                    else which -= cnt;
+                }
+                const int r = log / ms, c = log - r * ms;
+                const int tr = r + (direction == NGW_SOUTH) - (direction == NGW_NORTH);
+                const int tc = c + (direction == NGW_EAST) - (direction == NGW_WEST);
+                if (tr >= 0 && tr < ms && tc >= 0 && tc < ms && m[tr * ms + tc] == 0 && tr * ms + tc != agent)
+                    target = tr * ms + tc;
+            }
+            if (target < 0) { err = NGW_ERR_PLACEMENT; break; }
+            __syncwarp();
+            if (lane == 0) m[target] = (int8_t)op.a;
+            __syncwarp();
+            continue;
+        }
+        // FENCE / ADDITEM / REPLACE: candidates in row-major order (np.where), shuffled whole, THEN the percentage
+        int n = 0;
+        for (int base = 0; base < cells; base += 32) {
+            const int i = base + lane;
+            const bool cand = i < cells && reset_candidate(op.kind, m[i], wall, op.a);
+            const uint32_t bal = __ballot_sync(FULL, cand);
+            if (cand) list[n + __popc(bal & ((1u << lane) - 1u))] = (uint16_t)i;
+            n += __popc(bal);
+        }
+        __syncwarp();
+        for (int i = n - 1; i >= 1; i--) {                            // Fisher-Yates from the top (legacy shuffle)
+            const int j = (int)mt.interval((uint32_t)i, lane);
+            if (lane == 0) { const uint16_t t = list[i]; list[i] = list[j]; list[j] = t; }
+        }
+        __syncwarp();
+        const int pct = (int)mt.randint(op.lo, op.hi, lane);
+        int take = (int)ceil((double)n * ((double)pct / 100.0));     // novelty_wrappers.py:881,1025,1139
+        if (take > n) take = n;
+        const int value = op.kind == NGW_RESET_ADDITEM ? op.a : op.b;
+        for (int t = lane; t < take; t += 32) {                       // distinct cells: the first `take` in list order
+            const int i = list[t];
+            if (op.kind == NGW_RESET_FENCE) m[i] = (int8_t)(m[i] | 0x80);   // mark; fences go in afterwards
+            else if (i != agent) m[i] = (int8_t)value;
+        }
+        __syncwarp();
+        if (op.kind == NGW_RESET_FENCE) {                             // add_fence_around: the union does not depend on order
+            for (int i = lane; i < cells; i += 32) {
+                const int v = m[i];
+                if (!(v & 0x80)) continue;
+                const int r = i / ms, c = i - r * ms;
+                for (int rr = r - 1; rr <= r + 1; rr++)
+                    for (int cc = c - 1; cc <= c + 1; cc++)
+                        if (rr >= 0 && rr < ms && cc >= 0 && cc < ms && m[rr * ms + cc] == 0 && rr * ms + cc != agent)
+                            m[rr * ms + cc] = (int8_t)op.a;
+            }
+            __syncwarp();
+            for (int i = lane; i < cells; i += 32) {
+                const int v = m[i];
+                if (v & 0x80) m[i] = (int8_t)(v & 0x7F);
+            }
+            __syncwarp();
+        }
+    }
+    __syncwarp();
+    if (lane == 0) *pos_io = mt.pos;
     return err;
 }
 

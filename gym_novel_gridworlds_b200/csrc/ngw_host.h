@@ -35,6 +35,7 @@ struct ngw_handle {
     ngw_rollout_record rec{};                      // caller-owned per-step record of the rollouts (ngw_set_rollout_record)
     bool rec_on = false;
     int32_t* reset_list = nullptr; int32_t* reset_ctl = nullptr;   // auto-reset queue; ctl[0] = count, ctl[1] = finished CTAs
+    uint32_t* mt_key = nullptr; int32_t* mt_pos = nullptr;   // NGW_RNG_NUMPY: per-env np.random state (ngw_set_reset_rng)
     int sm_count = 148;
     long long launches = 0, concurrent_launches = 0;
     bool last_step_concurrent = false;             // the latest one-step launch overlapped its predecessor

@@ -28,6 +28,8 @@ struct ResetParams {
     unsigned char* final_obs;   // reset_list_kernel, optional: a regenerated env's row of obs is copied here before it is replaced
     int obs_dim, obs_row_bytes, obs_format;
     uint32_t key_mask;          // 0xFFFFFFFF; test knob NGW_DEBUG_KEY_MASK forces ties between the subset-sampling keys
+    uint32_t* mt_key;           // NGW_RNG_NUMPY: the envs' np.random states, key [n][624] and pos [n]; nullptr = Philox
+    int32_t* mt_pos;
 };
 
 #define NGW_RESET_WARPS 4
@@ -52,12 +54,16 @@ __device__ __forceinline__ void rows_from_smem(const ResetScratch& sc, int8_t* m
     for (int i = lane; i < inv_stride; i += 32) inv[i] = sc.inv[i];
 }
 
+// With the numpy stream (p.mt_key) each warp also owns `cells` uint16 of dynamic shared memory for its candidate lists.
 __global__ void __launch_bounds__(32 * NGW_RESET_WARPS) reset_kernel(const ResetParams p) {
     __shared__ ResetScratch scratch[NGW_RESET_WARPS];
+    extern __shared__ __align__(16) uint16_t rk_lists[];
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     long long e = (long long)blockIdx.x * NGW_RESET_WARPS + warp;       // one warp regenerates one env
     if (e >= p.n_envs) return;
     if (p.mask != nullptr && p.mask[e] == 0) return;
+    // numpy stream: a phase 0 that failed ended the reset program (the reference raised there)
+    if (p.mt_key != nullptr && p.phase == 1 && (p.err[e] & NGW_ERR_PLACEMENT)) return;
     ResetScratch& sc = scratch[warp];
     const ngw_config* cfg = &p.dcfgs[p.cfg_id[e]].c;
     uchar4 ps = p.pose[e];
@@ -70,19 +76,41 @@ __global__ void __launch_bounds__(32 * NGW_RESET_WARPS) reset_kernel(const Reset
     if (p.phase != 1) {
         uint32_t ep = p.episode[e] + 1;
         __syncwarp();
-        err = reset_env_warp(cfg, sc.row, sc.inv, p.ms, p.inv_stride, p.seed, gid, ep, true, 0,
-                             p.phase == 0 ? k : NGW_MAX_RESET_OPS, sc.hist, r, c, f, sel, p.key_mask);
+        const int end = p.phase == 0 ? k : NGW_MAX_RESET_OPS;
+        if (p.mt_key != nullptr)
+            err = reset_env_numpy_warp(cfg, sc.row, sc.inv, p.ms, p.inv_stride, p.mt_key + e * NGW_MT_WORDS, p.mt_pos + e,
+                                       true, 0, end, rk_lists + warp * p.cells, r, c, f, sel);
+        else
+            err = reset_env_warp(cfg, sc.row, sc.inv, p.ms, p.inv_stride, p.seed, gid, ep, true, 0, end, sc.hist, r, c, f,
+                                 sel, p.key_mask);
         if (lane == 0) { p.episode[e] = ep; p.ep_len[e] = 0; }
     } else {
         uint32_t ep = p.episode[e];
         rows_to_smem(sc, m, inv, p.cells, p.inv_stride, lane);
-        err = reset_env_warp(cfg, sc.row, sc.inv, p.ms, p.inv_stride, p.seed, gid, ep, false, k, NGW_MAX_RESET_OPS, sc.hist,
-                             r, c, f, sel, p.key_mask);
+        if (p.mt_key != nullptr)
+            err = reset_env_numpy_warp(cfg, sc.row, sc.inv, p.ms, p.inv_stride, p.mt_key + e * NGW_MT_WORDS, p.mt_pos + e,
+                                       false, k, NGW_MAX_RESET_OPS, rk_lists + warp * p.cells, r, c, f, sel);
+        else
+            err = reset_env_warp(cfg, sc.row, sc.inv, p.ms, p.inv_stride, p.seed, gid, ep, false, k, NGW_MAX_RESET_OPS,
+                                 sc.hist, r, c, f, sel, p.key_mask);
     }
     // a reset assigns the env's flags; its phase 1 adds those of the ops after the observation to what phase 0 assigned
     if (lane == 0) p.err[e] = p.phase == 1 ? p.err[e] | err : err;
     rows_from_smem(sc, m, inv, p.cells, p.inv_stride, lane);
     if (lane == 0) p.pose[e] = make_uchar4((unsigned char)r, (unsigned char)c, (unsigned char)f, (unsigned char)sel);
+}
+
+// NGW_RNG_NUMPY seeding: env e's state becomes np.random.seed(seed0 + e)'s (init_genrand, pos = 624)
+__global__ void mt_seed_kernel(uint32_t* key, int32_t* pos, long long n, unsigned long long seed0) {
+    const long long e = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (e >= n) return;
+    uint32_t s = (uint32_t)(seed0 + (unsigned long long)e);
+    uint32_t* k = key + e * NGW_MT_WORDS;
+    for (int i = 0; i < NGW_MT_WORDS; i++) {
+        k[i] = s;
+        s = 1812433253u * (s ^ (s >> 30)) + (uint32_t)i + 1u;
+    }
+    pos[e] = NGW_MT_WORDS;
 }
 
 // Second half of the single-step auto-reset: a grid-stride loop of warps over the queue the step kernel filled.  Each
@@ -94,8 +122,9 @@ __global__ void __launch_bounds__(32 * NGW_RESET_WARPS) reset_kernel(const Reset
 // ~2000 queued envs of a C5 step then take three rounds instead of one: 356 vs 315 us per step.)
 // Shared memory is sized for the batch's grid (dynamic: NGW_RESET_WARPS x reset_list_scratch_bytes(cells)), so that one
 // CTA of this kernel fits next to a full set of step CTAs when the next handle's step overlaps it (C5: 11 KB).
-__host__ __device__ inline int reset_list_scratch_bytes(int cells) {
-    return NGW_RESET_SCRATCH_WORDS * 4 + NGW_MAX_ITEMS * 4 + ((cells + 15) & ~15);
+// With the numpy stream a warp's scratch also holds its candidate list: cells uint16 more.
+__host__ __device__ inline int reset_list_scratch_bytes(int cells, bool numpy = false) {
+    return NGW_RESET_SCRATCH_WORDS * 4 + NGW_MAX_ITEMS * 4 + ((cells + 15) & ~15) + (numpy ? (2 * cells + 15) & ~15 : 0);
 }
 struct ResetScratchView { uint32_t* hist; int32_t* inv; int8_t* row; };
 
@@ -104,7 +133,7 @@ __global__ void __launch_bounds__(32 * NGW_RESET_WARPS) reset_list_kernel(const 
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     ResetScratchView sc;
     {
-        unsigned char* base = rl_smem + warp * reset_list_scratch_bytes(p.cells);
+        unsigned char* base = rl_smem + warp * reset_list_scratch_bytes(p.cells, p.mt_key != nullptr);
         sc.hist = reinterpret_cast<uint32_t*>(base);
         sc.inv = reinterpret_cast<int32_t*>(base + NGW_RESET_SCRATCH_WORDS * 4);
         sc.row = reinterpret_cast<int8_t*>(base + NGW_RESET_SCRATCH_WORDS * 4 + NGW_MAX_ITEMS * 4);
@@ -125,8 +154,12 @@ __global__ void __launch_bounds__(32 * NGW_RESET_WARPS) reset_list_kernel(const 
         __syncwarp();
         int k_obs = dc.c.reset_obs_after_ops;
         if (p.obs == nullptr || k_obs >= dc.c.n_reset_ops) k_obs = NGW_MAX_RESET_OPS;
-        uint32_t err = reset_env_warp(&dc.c, sc.row, sc.inv, p.ms, p.inv_stride, p.seed, gid, ep, true, 0, k_obs, sc.hist,
-                                      r, c, f, sel, p.key_mask);
+        uint16_t* list = reinterpret_cast<uint16_t*>(sc.row + ((p.cells + 15) & ~15));   // numpy stream only
+        uint32_t err = p.mt_key != nullptr
+            ? reset_env_numpy_warp(&dc.c, sc.row, sc.inv, p.ms, p.inv_stride, p.mt_key + e * NGW_MT_WORDS, p.mt_pos + e,
+                                   true, 0, k_obs, list, r, c, f, sel)
+            : reset_env_warp(&dc.c, sc.row, sc.inv, p.ms, p.inv_stride, p.seed, gid, ep, true, 0, k_obs, sc.hist, r, c, f,
+                             sel, p.key_mask);
         if (p.obs != nullptr) {                                       // observation of the new episode replaces the row
             ObsRow orow;
             orow.p = p.obs + e * p.obs_row_bytes;
@@ -152,7 +185,10 @@ __global__ void __launch_bounds__(32 * NGW_RESET_WARPS) reset_list_kernel(const 
             }
             __syncwarp();
         }
-        if (k_obs < dc.c.n_reset_ops)
+        if (k_obs < dc.c.n_reset_ops && p.mt_key != nullptr && !(err & NGW_ERR_PLACEMENT))
+            err |= reset_env_numpy_warp(&dc.c, sc.row, sc.inv, p.ms, p.inv_stride, p.mt_key + e * NGW_MT_WORDS,
+                                        p.mt_pos + e, false, k_obs, NGW_MAX_RESET_OPS, list, r, c, f, sel);
+        else if (k_obs < dc.c.n_reset_ops && p.mt_key == nullptr)
             err |= reset_env_warp(&dc.c, sc.row, sc.inv, p.ms, p.inv_stride, p.seed, gid, ep, false, k_obs,
                                   NGW_MAX_RESET_OPS, sc.hist, r, c, f, sel, p.key_mask);
         __syncwarp();

@@ -47,6 +47,13 @@ static int record_tile_bytes(const RecordParams& rec, const StepParams& p) {
     return rec.obs != nullptr || rec.final_obs != nullptr ? 32 * p.obs_row_bytes : 0;
 }
 
+// numpy stream only: candidate lists for the `warps` warps that regenerate envs, appended at the plan's end `end`
+static size_t numpy_lists(StepParams& p, size_t end, int warps) {
+    if (p.mt_key == nullptr || !p.auto_reset) return end;
+    p.off_lists = (int)((end + 127) & ~(size_t)127);
+    return (size_t)p.off_lists + (size_t)warps * 2 * p.cells;
+}
+
 // rollout_kernel's shared-memory plan (offsets into p, the record's staging tile into rec) -> bytes per CTA
 template <int NC>
 static size_t rollout_plan(const ngw_handle* h, StepParams& p, RecordParams& rec) {
@@ -58,7 +65,8 @@ static size_t rollout_plan(const ngw_handle* h, StepParams& p, RecordParams& rec
     p.off_in = p.off_policy + (p.policy_w ? ((16 + p.obs_dim * p.policy_actions) * 4 + 127) & ~127 : 0);
     p.off_obs = p.off_in + in_bytes;
     rec = record_params(h, (p.off_obs + p.obs_bytes + 127) & ~127);
-    return p.record ? (size_t)rec.off_tile + record_tile_bytes(rec, p) : (size_t)p.off_obs + p.obs_bytes;
+    const size_t end = p.record ? (size_t)rec.off_tile + record_tile_bytes(rec, p) : (size_t)p.off_obs + p.obs_bytes;
+    return numpy_lists(p, end, 1);
 }
 
 // A rollout with a record runs rollout2_kernel where its plan fits 200 KB, else rollout_kernel, whose plan (grid,
@@ -97,8 +105,8 @@ static cudaError_t launch_rollout2_na(ngw_handle* h, StepParams p, cudaStream_t 
     p.off_in = p.off_policy + (A4 > 0 ? ((16 + p.obs_dim * 4 * A4) * 4 + 127) & ~127 : 0);
     const int obs_tile = p.obs ? p.obs_bytes : 0;
     const RecordParams rec = record_params(h, (p.off_in + (in_bytes > obs_tile ? in_bytes : obs_tile) + 127) & ~127);
-    const size_t smem = p.record ? (size_t)rec.off_tile + record_tile_bytes(rec, p)
-                                 : (size_t)p.off_in + (in_bytes > obs_tile ? in_bytes : obs_tile);
+    const size_t smem = numpy_lists(p, p.record ? (size_t)rec.off_tile + record_tile_bytes(rec, p)
+                                                : (size_t)p.off_in + (in_bytes > obs_tile ? in_bytes : obs_tile), 2);
     if (smem > 200 * 1024) return cudaErrorNotSupported;
     const long long tiles = (p.env_end - p.env_begin + 31) / 32;
     claim_stream(h, s, false);

@@ -135,6 +135,9 @@ struct StepParams {
     int32_t* reset_count;       // ... and regenerated by reset_list_kernel right after this launch
     uint8_t* trunc;             // optional, one-step launches: 1 where the step hit max_episode_steps and the env did not end it
     unsigned char* final_obs;   // optional, one-step launches: reset_list_kernel copies a regenerated env's row here first
+    uint32_t* mt_key;           // NGW_RNG_NUMPY: the envs' np.random states (key [n][624], pos [n]); nullptr = Philox
+    int32_t* mt_pos;
+    int off_lists;              // rollout kernels, numpy stream: the resetting warps' candidate lists (cells uint16 each)
 };
 
 // Per-step record of the K-step rollouts (ngw_set_rollout_record): element [t][e] at t * stride + e.  Only the recording
@@ -321,8 +324,16 @@ static __device__ __noinline__ void auto_reset_warp(const StepParams& p, const D
         int8_t* m = smap + src * p.cells;
         int32_t* inv = sinv + src * p.inv_stride;
         int r = 0, c = 0, f = 0, sel = 0;
-        uint32_t err = reset_env_warp(&dcfgs[ci].c, m, inv, p.ms, p.inv_stride, p.seed, (uint64_t)(p.first_gid + e), ep,
-                                      true, 0, NGW_MAX_RESET_OPS, hist, r, c, f, sel);
+        uint32_t err;
+        if (p.mt_key != nullptr) {
+            extern __shared__ __align__(128) unsigned char ar_smem[];
+            uint16_t* list = reinterpret_cast<uint16_t*>(ar_smem + p.off_lists) + (threadIdx.x >> 5) * p.cells;
+            err = reset_env_numpy_warp(&dcfgs[ci].c, m, inv, p.ms, p.inv_stride, p.mt_key + e * NGW_MT_WORDS, p.mt_pos + e,
+                                       true, 0, NGW_MAX_RESET_OPS, list, r, c, f, sel);
+        } else {
+            err = reset_env_warp(&dcfgs[ci].c, m, inv, p.ms, p.inv_stride, p.seed, (uint64_t)(p.first_gid + e), ep, true, 0,
+                                 NGW_MAX_RESET_OPS, hist, r, c, f, sel);
+        }
         int8_t* grow = p.map + e * p.cells;
         for (int i = lane; i < p.cells; i += 32) grow[i] = m[i];
         if (lane == src) {

@@ -31,7 +31,8 @@ class NovelGridworldBatchEnv(Env):
     _PLACES_TREE_TAP = False           # pogostick_v0_env.py:155-178
 
     def __init__(self, env=None, num_envs=1, device=None, seed=0, first_env_gid=0, auto_reset=False,
-                 max_episode_steps=0, messages=False, strict_actions=False, obs_format='i32', episode_end_info=False):
+                 max_episode_steps=0, messages=False, strict_actions=False, obs_format='i32', episode_end_info=False,
+                 reset_rng='philox'):
         self.env = env                                  # env to restore in reset (pogostick_v1_env.py:29,89-109)
         self.num_envs = int(num_envs)
         self.device = device
@@ -52,6 +53,13 @@ class NovelGridworldBatchEnv(Env):
         # the env did not end the episode itself) and 'terminal_observation' (with auto_reset, the last observation of
         # each finished episode, valid where done) — what a learner needs to bootstrap at a time limit
         self.episode_end_info = bool(episode_end_info)
+        # reset_rng: 'philox' (default) draws maps from the counter-based generator keyed by (seed, env id, episode) — the
+        # reference's distribution, not its stream.  'numpy' draws them from the reference's own legacy np.random stream:
+        # env i starts from np.random.seed(seed + first_env_gid + i) and continues it episode after episode; with
+        # num_envs == 1, reset() instead draws from (and advances) the process's global np.random, as the reference does.
+        if reset_rng not in ('philox', 'numpy'):
+            raise ValueError("reset_rng must be 'philox' or 'numpy'")
+        self.reset_rng = reset_rng
 
         self.map_size = 10
         self.direction_id = {'NORTH': 0, 'SOUTH': 1, 'WEST': 2, 'EAST': 3}
@@ -116,13 +124,31 @@ class NovelGridworldBatchEnv(Env):
         return ids
 
     def add_new_items(self, new_items_quantity):
-        """pogostick_v1_env.py:495-501.  The reference also calls reset() here; a batched reset at
-        wrapper-construction time would be thrown away by the user's own reset(), so it is skipped."""
+        """pogostick_v1_env.py:495-501.  The reference also calls reset() here.  A batched reset at wrapper-construction
+        time would be thrown away by the user's own reset(), so it is skipped, except for one env on the numpy stream:
+        there the reference's reset consumes draws of the global np.random, which a seeded script's later maps depend on."""
         for item in new_items_quantity:
             self.items.add(item)
             self.items_id.setdefault(item, len(self.items_id))
             self.items_quantity.update({item: new_items_quantity[item]})
         self.inventory_items_quantity = {item: 0 for item in self.items}
+        if self.reset_rng == 'numpy' and self.num_envs == 1:
+            self._construction_reset()
+
+    def _construction_reset(self):
+        """The base env's reset() with its tables as they are now, on a one-env numpy-stream batch: it advances the global
+        np.random exactly as the reference's reset does, and raises where that raises."""
+        import torch
+        from .compiler import compile_chain
+        from .runtime import BatchHandle, global_stream_reset
+        h = BatchHandle([compile_chain(self)], 1, self.device, self.rng_seed, self.first_env_gid, reset_rng='numpy')
+        try:
+            global_stream_reset(h, want_obs=False)
+            torch.cuda.current_stream(h.device).synchronize()
+            if int(h.error_flags[0].item()) & oc.ERR_PLACEMENT:
+                raise AssertionError("Cannot place items, increase map size!")      # pogostick_v1_env.py:167
+        finally:
+            h.close()
 
     def remap_action(self, actions_id, start_action_id):
         """Shuffle names until the mapping changes (pogostick_v1_env.py:476-493); draws from the global
@@ -251,7 +277,9 @@ class NovelGridworldBatchEnv(Env):
         return text
 
     def seed(self, seed=None):
-        """The reference has no seed() (it draws from the global np.random); here it re-keys the Philox generator."""
+        """The reference has no seed() (it draws from the global np.random).  Here it re-keys the Philox generator, or on
+        the numpy stream re-seeds env gid with np.random.seed(seed + gid) (one env: reset() follows the global
+        np.random instead, see reset_rng)."""
         if seed is not None:
             self.rng_seed = int(seed)
             self.close()                       # the next reset() builds a handle with the new key

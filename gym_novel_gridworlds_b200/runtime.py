@@ -31,6 +31,7 @@ def _ptr(t):
 
 
 _OBS_FORMATS = {'i32': capi.OBS_I32, 'u8': capi.OBS_U8, 'hits': capi.OBS_HITS}
+_RESET_RNGS = {'philox': capi.RNG_PHILOX, 'numpy': capi.RNG_NUMPY}
 
 
 def _tail_offset(c, obs_format):
@@ -141,7 +142,8 @@ class RolloutRecord(object):
 
 
 class BatchHandle(object):
-    def __init__(self, compiled, n_envs, device=None, seed=0, first_env_gid=0, cfg_id=None, obs_format='i32'):
+    def __init__(self, compiled, n_envs, device=None, seed=0, first_env_gid=0, cfg_id=None, obs_format='i32',
+                 reset_rng='philox'):
         if not torch.cuda.is_available():
             raise RuntimeError("gym_novel_gridworlds_b200 needs a CUDA device (B200, sm_100a); there is no CPU path")
         self.lib = capi.load_library()
@@ -199,6 +201,9 @@ class BatchHandle(object):
         self._host = None
         if cfg_id is not None:
             self.set_env_configs(cfg_id)
+        self.reset_rng = 'philox'
+        if reset_rng != 'philox':
+            self.set_reset_rng(reset_rng)
 
     # ------------------------------------------------------------------
     def _stream(self):
@@ -252,6 +257,37 @@ class BatchHandle(object):
         if host:
             torch.cuda.current_stream(self.device).synchronize()
         return m.view(count, self.map_size, self.map_size), p, v
+
+    def set_reset_rng(self, kind):
+        """'philox' (default): the counter-based map generator.  'numpy': the reference's own legacy np.random stream, one
+        state per env, env i seeded as np.random.seed(seed + first_env_gid + i) (ngw_set_reset_rng; calling it again
+        re-seeds)."""
+        if kind not in _RESET_RNGS:
+            raise ValueError("reset_rng must be 'philox' or 'numpy'")
+        capi.check(self.lib, self.lib.ngw_set_reset_rng(self._h, _RESET_RNGS[kind], self._stream()))
+        self.reset_rng = kind
+
+    def rng_state(self, first=0, count=None):
+        """(key uint32 [count, 624], pos int32 [count]): the np.random states of envs first .. first + count - 1 in
+        np.random.get_state()'s layout (numpy stream only)."""
+        count = self.n - first if count is None else int(count)
+        key = torch.empty((count, 624), dtype=torch.int32, device=self.device)
+        pos = torch.empty(count, dtype=torch.int32, device=self.device)
+        capi.check(self.lib, self.lib.ngw_export_rng_state(self._h, _ptr(key), _ptr(pos), int(first), count, self._stream()))
+        return key.cpu().numpy().view(np.uint32), pos.cpu().numpy()
+
+    def load_rng_state(self, key, pos, first=0):
+        """Set the np.random states of envs first .. first + len(pos) - 1 (numpy stream only): key uint32 [count, 624],
+        pos int32 [count] in [0, 624], as np.random.RandomState(s).get_state()[1:3] gives them."""
+        k = np.ascontiguousarray(np.asarray(key, dtype=np.uint32).reshape(-1, 624))
+        p = np.ascontiguousarray(np.asarray(pos, dtype=np.int32).reshape(-1))
+        if k.shape[0] != p.shape[0]:
+            raise ValueError("key and pos must describe the same number of envs")
+        kt = torch.from_numpy(k.view(np.int32)).to(self.device)
+        pt = torch.from_numpy(p).to(self.device)
+        capi.check(self.lib, self.lib.ngw_load_rng_state(self._h, _ptr(kt), _ptr(pt), int(first), int(p.shape[0]),
+                                                         self._stream()))
+        torch.cuda.current_stream(self.device).synchronize()      # kt / pt are temporaries
 
     def split_obs(self, obs, cfg=0):
         """(lidar part, inventory tail int32 [n, I_obs]) views of an observation buffer of this handle's format (torch
@@ -587,6 +623,18 @@ class LazyInfo(object):
         return keys + ['TimeLimit.truncated', 'terminal_observation'] if self._episode_end is not None else keys
 
 
+def global_stream_reset(h, want_obs=True):
+    """Reset env 0 of a numpy-stream handle from the process's global np.random and advance that stream by the draws the
+    reset took, as the reference's reset() does: get_state -> load into env 0 -> reset -> export -> set_state (the cached
+    Gaussian is kept)."""
+    name, key, pos, has_gauss, cached = np.random.get_state()
+    h.load_rng_state(np.asarray(key, np.uint32).reshape(1, 624), np.array([pos], np.int32))
+    obs = h.reset(want_obs=want_obs)
+    k, p = h.rng_state(0, 1)
+    np.random.set_state((name, k[0].copy(), int(p[0]), has_gauss, cached))
+    return obs
+
+
 class ChainRuntime(object):
     """Drives one wrapper chain (one config) through a BatchHandle with the reference's return conventions."""
 
@@ -610,7 +658,8 @@ class ChainRuntime(object):
             self.compiled, self._fingerprint = cc, fp
             self.handle = BatchHandle([cc], self.base.num_envs, self.base.device, self.base.rng_seed,
                                       self.base.first_env_gid,
-                                      obs_format='i32' if self.base.num_envs == 1 else self.base.obs_format)
+                                      obs_format='i32' if self.base.num_envs == 1 else self.base.obs_format,
+                                      reset_rng=self.base.reset_rng)
             if self.single or self.messages:
                 self.handle.enable_messages()
             if self.episode_end_info and not self.single:       # (the reference has no auto-reset: N == 1 is unchanged)
@@ -625,6 +674,12 @@ class ChainRuntime(object):
     @property
     def single(self):
         return self.base.num_envs == 1
+
+
+    @property
+    def global_stream(self):
+        """num_envs == 1 on the numpy stream: reset() draws from the process's global np.random, as the reference does."""
+        return self.single and self.base.reset_rng == 'numpy'
 
     def dict_observation(self):
         h = self.handle
@@ -708,7 +763,10 @@ class ChainRuntime(object):
         else:
             h = self._ensure()
             cc = self.compiled
-            obs = h.reset(want_obs=(cc.reset_returns == 'lidar'))
+            if self.global_stream:
+                obs = global_stream_reset(h, want_obs=(cc.reset_returns == 'lidar'))
+            else:
+                obs = h.reset(want_obs=(cc.reset_returns == 'lidar'))
         if self.single:
             torch.cuda.current_stream(h.device).synchronize()
             if int(h.error_flags[0].item()) & oc.ERR_PLACEMENT:
@@ -801,7 +859,8 @@ class ChainRuntime(object):
 class MixedBatch(object):
     """Several wrapper chains (configs) in one batch: env i runs config cfg_id[i] — one launch per step."""
 
-    def __init__(self, tops, num_envs, cfg_id=None, device=None, seed=0, first_env_gid=0, assignment='interleaved'):
+    def __init__(self, tops, num_envs, cfg_id=None, device=None, seed=0, first_env_gid=0, assignment='interleaved',
+                 reset_rng='philox'):
         self.compiled = [compile_chain(t) for t in tops]
         n_cfg = len(self.compiled)
         if cfg_id is None:
@@ -809,7 +868,8 @@ class MixedBatch(object):
             gid = idx + int(first_env_gid)
             cfg_id = (gid % n_cfg) if assignment == 'interleaved' else np.minimum(idx * n_cfg // num_envs, n_cfg - 1)
         self.cfg_id_host = np.asarray(cfg_id, dtype=np.int32)
-        self.handle = BatchHandle(self.compiled, num_envs, device, seed, first_env_gid, cfg_id=self.cfg_id_host)
+        self.handle = BatchHandle(self.compiled, num_envs, device, seed, first_env_gid, cfg_id=self.cfg_id_host,
+                                  reset_rng=reset_rng)
         self.n_actions = np.array([cc.c.n_actions for cc in self.compiled], dtype=np.int32)
 
     def reset(self, mask=None):

@@ -38,7 +38,7 @@
 extern "C" {
 #endif
 
-#define NGW_ABI_VERSION 12
+#define NGW_ABI_VERSION 13
 
 #define NGW_MAX_ITEMS 24          /* reference asserts len(items) <= 20 (pogostick_v1_env.py:75,220) */
 #define NGW_MAX_ACTIONS 48
@@ -270,9 +270,34 @@ int ngw_load_state(ngw_handle* h, const int8_t* map, const uint8_t* pose, const 
 int ngw_export_state(ngw_handle* h, int8_t* map, uint8_t* pose, int32_t* inventory, int64_t first, int64_t count,
                      void* stream);
 
-/* Reset envs whose mask byte is non-zero (mask DEVICE uint8[n_envs], NULL = all) with the Philox
- * map generator; obs (DEVICE rows of obs_row_bytes, NULL = skip) receives the reset observation of
- * the reset envs, taken after cfg.reset_obs_after_ops ops as the reference does. */
+/* The generator every regeneration of this handle draws its maps from: ngw_reset, the auto-resets of ngw_step /
+ * ngw_step_many / the host-buffer path, and the in-kernel resets of ngw_rollout / ngw_rollout_policy.
+ *   NGW_RNG_PHILOX (default): counter-based, keyed by (seed, global env id, episode); the reference's distribution, not
+ *                  its stream.  Setting it frees the np.random states.
+ *   NGW_RNG_NUMPY: the reference's own stream.  Allocates one legacy np.random (MT19937) state per env (2.5 KB) and seeds
+ *                  env e exactly as np.random.seed(seed + first_env_gid + e) does (init_genrand, pos = 624), so sharding
+ *                  does not change the episodes.  Calling it again re-seeds.  Every reset then draws what the reference's
+ *                  reset draws under that state, in its order, and leaves the state where the reference leaves it, so the
+ *                  env's episodes continue the stream as consecutive reference resets do.  The only difference: a TREETAP
+ *                  reset op (v0 envs) whose logs have no free neighbour makes the reference retry forever; here it gives up
+ *                  after 2^20 attempts with NGW_ERR_PLACEMENT.  A reset that fails skips the rest of its program, as the
+ *                  reference's AssertionError does.  Fails, and enqueues nothing, if seed + first_env_gid + n_envs - 1
+ *                  >= 2^32.  The random policy of ngw_rollout keeps drawing from Philox (it picks actions, not maps).
+ * The states are handle state: only this handle's own launches read or write them. */
+enum { NGW_RNG_PHILOX = 0, NGW_RNG_NUMPY = 1 };
+int ngw_set_reset_rng(ngw_handle* h, int32_t kind, void* stream);
+
+/* The np.random states of envs [first, first + count) of a NGW_RNG_NUMPY handle in numpy's get_state() layout:
+ * key uint32 [count][624], pos int32 [count].  Load reads DEVICE memory; it reads pos back to check it (a synchronising
+ * copy, so not inside a stream capture).  Export writes device or host memory (asynchronous on `stream`).  A handle
+ * without np.random states, a range outside the batch, or a pos outside [0, 624] fails with a message and enqueues
+ * nothing. */
+int ngw_load_rng_state(ngw_handle* h, const uint32_t* key, const int32_t* pos, int64_t first, int64_t count, void* stream);
+int ngw_export_rng_state(ngw_handle* h, uint32_t* key, int32_t* pos, int64_t first, int64_t count, void* stream);
+
+/* Reset envs whose mask byte is non-zero (mask DEVICE uint8[n_envs], NULL = all) with the handle's map generator
+ * (ngw_set_reset_rng: Philox by default); obs (DEVICE rows of obs_row_bytes, NULL = skip) receives the reset observation
+ * of the reset envs, taken after cfg.reset_obs_after_ops ops as the reference does. */
 int ngw_reset(ngw_handle* h, const uint8_t* mask, void* obs, void* stream);
 
 /* One fused step of every env: action semantics + novelties + reward/done/step_cost + LidarInFront
